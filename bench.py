@@ -4,6 +4,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload reddit|arxiv|physics|pubmed|cora] [--f F] [--order K] [--scales S]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic graph of the named
 shape: K fused Chebyshev orders (SpMM over the implicit scaled Laplacian +
@@ -58,6 +59,7 @@ UNIT = "nnz*K*F/s"
 DEFAULT_F = {"reddit": 1, "arxiv": 128, "physics": 1, "pubmed": 1, "cora": 1}
 REFERENCE_MAX_TIMED_RUNS = 2     # stock-function runs of the reference arm (the full Reddit graph takes ~1 min each)
 REFERENCE_FULL_GRAPH_LIMIT = 8   # K*F above which the CPU arm falls back to a scaled sample of the workload
+DUMP_MAX_BYTES = 64_000_000      # --dump-outputs: bound on what one run writes
 
 
 def parse_args():
@@ -91,7 +93,16 @@ def parse_args():
                          "edge flips around a random target node applied on top of the resident graph")
     ap.add_argument("--no-check", action="store_true",
                     help="N>1: skip the comparison of every rank's rows with the single-GPU path (outside the timed region)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU only: after the timed steps, write the features the last timed step returned as "
+                         "DIR/features.npy (float32); above 64 MB a fixed, seeded sample of rows, with the sampled row "
+                         "ids in DIR/features_rows.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
+    return args
 
 
 def scale_list(n_scales):
@@ -367,6 +378,21 @@ def make_flips(n, budget, seed, graph_rowptr=None, graph_colidx=None):
     return ([target] * len(others) + others, others + [target] * len(others), [1.0] * (2 * len(others)))
 
 
+def dump_features(out_dir, feats):
+    """Writes the features a step returned ([N, S*F]) as ``out_dir/features.npy`` in float32, so that two builds
+    can be compared output for output on the same seeded inputs.  Above DUMP_MAX_BYTES a fixed, seeded sample of
+    whole rows is written instead, with the sampled row ids (ascending) in ``out_dir/features_rows.npy``."""
+    os.makedirs(out_dir, exist_ok=True)
+    h = feats.detach().float().cpu().numpy()
+    n, width = h.shape
+    if h.nbytes > DUMP_MAX_BYTES:
+        budget = (DUMP_MAX_BYTES - 1024) // (4 * width + 8)        # float32 row + its float64 id, minus the headers
+        rows = np.sort(np.random.default_rng(0).choice(n, budget, replace=False))
+        h = h[rows]
+        np.save(os.path.join(out_dir, "features_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "features.npy"), h)
+
+
 def time_steps(fn, steps, warmup):
     for _ in range(warmup):
         fn()
@@ -499,18 +525,20 @@ def run_ours(args, rank, local_rank, world):
         if i % EV_STRIDE == 0 and replay_events:
             row = ev[i // EV_STRIDE]
             row[0].record()
-            session()
+            out = session()
             row[1].record()
         elif i % EV_STRIDE == 0:
-            step(ev_arrays[i // EV_STRIDE])
+            out = step(ev_arrays[i // EV_STRIDE])
         elif session is not None:
-            session()
+            out = session()
         else:
-            step()
+            out = step()
     stop.record()
     torch.cuda.synchronize()
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs:
+        dump_features(args.dump_outputs, out)     # before anything else replays the session into the same buffer
     ms_per_step = start.elapsed_time(stop) / args.steps
     value = work / (ms_per_step * 1e-3)
 
@@ -733,6 +761,9 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs is implemented for the one-GPU run only; a multi-GPU run compares every "
+                         "rank's rows with the single-GPU path instead (the 'check' record; off with --no-check)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

@@ -40,7 +40,61 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+import numpy as np  # noqa: E402
 import pytest  # noqa: E402
+import torch  # noqa: E402
+
+
+def test_bad_steps_and_dump_outputs_of_the_reference_arm_are_refused(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cora", *extra],
+                             capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", extra
+    assert os.listdir(tmp_path) == []
+
+
+def test_dump_features_bounds_the_size_with_a_fixed_row_sample(tmp_path):
+    import bench
+    feats = torch.randn(300_000, 60, generator=torch.Generator().manual_seed(0))      # 72 MB of float32
+    for d in ("a", "b"):
+        bench.dump_features(str(tmp_path / d), feats)
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_MAX_BYTES
+    rows, got = np.load(tmp_path / "a" / "features_rows.npy"), np.load(tmp_path / "a" / "features.npy")
+    assert rows.dtype == np.float64 and got.dtype == np.float32 and np.all(np.diff(rows) > 0)
+    np.testing.assert_array_equal(got, feats.numpy()[rows.astype(np.int64)])
+    for name in ("features_rows.npy", "features.npy"):                 # the same sample on every run
+        np.testing.assert_array_equal(np.load(tmp_path / "b" / name), np.load(tmp_path / "a" / name))
+    small = torch.randn(10, 3, dtype=torch.float64)
+    bench.dump_features(str(tmp_path / "c"), small)
+    assert os.listdir(tmp_path / "c") == ["features.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "c" / "features.npy"), small.float().numpy())
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("f", [1, 8])
+def test_gpu_arm_dumps_the_features_of_its_last_step(tmp_path, f):
+    """--dump-outputs: what the last timed step returned equals the same call made here on the bench's seeded
+    graph and signal, and --steps is the number of timed steps."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "pubmed", "--f", str(f),
+                          "--steps", "3", "--warmup", "1", "--no-cpu-baseline", "--no-e2e", "--no-ugca",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 3
+    assert os.listdir(tmp_path) == ["features.npy"]
+    got = np.load(tmp_path / "features.npy")
+
+    import efficient_gnn_b200 as egnn
+    from efficient_gnn_b200 import synth
+    rp, ci, n = synth.synth_csr("pubmed", self_loops=True, device="cuda")
+    x0 = None
+    if f > 1:
+        x0 = torch.randn(n, f, device="cuda", generator=torch.Generator(device="cuda").manual_seed(synth.SHAPES["pubmed"].seed))
+    graph = egnn.CsrGraph(rp, ci, None, n)
+    want = egnn.graph_wavelet_features(graph, k=3, s=0.8, X0=x0).cpu().numpy()
+    s = egnn.graph_wavelet_features(graph, k=3, s=0.8, X0=x0, return_parts=True).combined.reshape(n, -1).cpu().numpy()
+    sure = np.abs(s) > 1e-4 * np.abs(s).max()         # away from sign flips of S ~ 0 (F = 1: H = sign(S))
+    assert got.dtype == np.float32 and got.shape == (n, f)
+    np.testing.assert_allclose(got[sure], want[sure], rtol=0, atol=1e-6)
 
 
 @pytest.mark.gpu
