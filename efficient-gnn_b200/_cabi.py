@@ -13,7 +13,7 @@ import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("EGNN_LIB_PATH") or os.path.join(_HERE, "lib", "libegnn_b200.so")   # override: tuning builds
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 # every symbol include/egnn_b200.h declares: name -> (restype, argtypes)
 _P, _I32, _I64, _F32, _SZ = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -42,6 +42,14 @@ SYMBOLS = {
     "egnn_cheb_workspace_bytes": (_SZ, [_I64, _I32]),
     "egnn_cheb_wavelet": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _I64, _I32, _I32, _I32, _P, _F32, _F32,
                                     _P, _P, _I32, _P, _P, _P, _I32, _P, _SZ, _P, _P, _P, _P, _P, _I32, _P, _P, _I32]),
+    "egnn_cheb_adjoint": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I64, _I32, _I32, _I32, _P, _F32, _F32,
+                                    _P, _P, _P, _P, _P, _P, _I32, _P, _SZ, _P, _P, _P]),
+    "egnn_l1_normalize": (C.c_int, [_P, _P, _I64, _I32, _P]),
+    "egnn_l1_normalize_backward": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P]),
+    "egnn_cheb_coeff_grad_ws_bytes": (_SZ, [_I32, _I32]),
+    "egnn_cheb_coeff_grad": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _P, _P, _SZ, _P]),
+    "egnn_csr_transpose_ws_bytes": (_SZ, [_I64, _I64]),
+    "egnn_csr_transpose": (C.c_int, [_P, _P, _P, _I64, _I64, _P, _P, _P, _P, _SZ, _P]),
     "egnn_row_order_ws_bytes": (_SZ, [_I64]),
     "egnn_row_order": (C.c_int, [_P, _I64, _P, _P, _SZ, _P]),
     "egnn_sell_step_sharded": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _I32, _I32, _I32, _P,

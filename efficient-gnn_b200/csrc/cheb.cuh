@@ -45,6 +45,12 @@ struct OrderParams {
     float c_prev[EGNN_MAX_SCALES];
     float c_k[EGNN_MAX_SCALES];
     DeltaList delta;
+    // adjoint instantiation (ADJ): b = c_adj * (M^T b_{k+1})_i - b_{k+2} + v_k with
+    // v_k[i, :] = tbar[i, :] + sum_s c_k[s] * cbar[i, s, :]; tprev_own = b_{k+1}, tprev2_own = b_{k+2}
+    // (NULL: zero), tk_own = b_k, y_own = dinv * b_k.  Appended so the forward layout is unchanged.
+    const float* cbar;       // [n_rows, S, F]
+    const float* tbar;       // [n_rows, F] or NULL
+    float c_adj;             // 2, or 1 on the last application (it yields the signal's gradient)
 };
 
 template <int VEC> struct FeatVec;
@@ -134,7 +140,7 @@ __device__ __forceinline__ void accumulate_row(const OrderParams& p, int q_first
         for (int v = 0; v < VEC; ++v) acc[u][v] = (float)(hi[u][v] + (double)acc[u][v]);
 }
 
-template <int VEC, int U, bool HAS_VALS, bool PRESCALED>
+template <int VEC, int U, bool HAS_VALS, bool PRESCALED, bool ADJ = false>
 __global__ void __launch_bounds__(kOrderBlock)
 cheb_order_kernel(const __grid_constant__ OrderParams p) {
     const int lane = threadIdx.x & 31;
@@ -250,6 +256,39 @@ cheb_order_kernel(const __grid_constant__ OrderParams p) {
 #pragma unroll
                 for (int v = 0; v < VEC; ++v) acc[u][v] += t.v[v];
             }
+    }
+
+    if constexpr (ADJ) {         // adjoint epilogue (Clenshaw step): no scale accumulation
+        if (!writer) return;
+        const float di = __ldg(p.dinv + grow);
+        const float theta = fmaf(p.a, 1.f - (float)__ldg(p.iso + grow), p.b);
+        const float nscale = -p.a * di;
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            if (!fok[u]) continue;
+            const int64_t off = row * F + fidx[u];
+            FeatVec<VEC> own, b2, v, t;
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) { own.v[j] = 0.f; b2.v[j] = 0.f; v.v[j] = 0.f; }
+            if (theta != 0.f) own.load_plain(p.tprev_own + off);
+            if (p.tprev2_own) b2.load_plain(p.tprev2_own + off);
+            if (p.tbar) v.load_plain(p.tbar + off);
+            for (int s = 0; s < p.S; ++s) {
+                t.load_plain(p.cbar + (row * p.S + s) * F + fidx[u]);
+#pragma unroll
+                for (int j = 0; j < VEC; ++j) v.v[j] = fmaf(p.c_k[s], t.v[j], v.v[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < VEC; ++j)
+                t.v[j] = fmaf(p.c_adj, fmaf(theta, own.v[j], nscale * acc[u][j]), v.v[j] - b2.v[j]);
+            if (p.tk_own) t.store(p.tk_own + off);       // may alias tprev2_own: read above
+            if (p.y_own) {
+#pragma unroll
+                for (int j = 0; j < VEC; ++j) t.v[j] *= di;
+                t.store(p.y_own + off);
+            }
+        }
+        return;
     }
 
     // ---- epilogue: Laplacian scaling, recurrence, scale accumulation -------

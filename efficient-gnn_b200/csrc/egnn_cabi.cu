@@ -4,6 +4,7 @@
 #include <stdarg.h>
 #include <stdlib.h>
 
+#include "adjoint.cuh"
 #include "cheb.cuh"
 #include "common.cuh"
 #include "head.cuh"
@@ -75,26 +76,28 @@ static OrderConfig choose_config(int64_t n_rows, int64_t nnz, int32_t F) {
     return c;
 }
 
-template <int VEC, int U>
+template <int VEC, int U, bool ADJ>
 static void launch_order_vu(const OrderParams& p, bool has_vals, bool prescaled, dim3 grid,
                             cudaStream_t st) {
     if (has_vals) {
-        if (prescaled) cheb_order_kernel<VEC, U, true, true><<<grid, kOrderBlock, 0, st>>>(p);
-        else cheb_order_kernel<VEC, U, true, false><<<grid, kOrderBlock, 0, st>>>(p);
+        if (prescaled) cheb_order_kernel<VEC, U, true, true, ADJ><<<grid, kOrderBlock, 0, st>>>(p);
+        else cheb_order_kernel<VEC, U, true, false, ADJ><<<grid, kOrderBlock, 0, st>>>(p);
     } else {
-        if (prescaled) cheb_order_kernel<VEC, U, false, true><<<grid, kOrderBlock, 0, st>>>(p);
-        else cheb_order_kernel<VEC, U, false, false><<<grid, kOrderBlock, 0, st>>>(p);
+        if (prescaled) cheb_order_kernel<VEC, U, false, true, ADJ><<<grid, kOrderBlock, 0, st>>>(p);
+        else cheb_order_kernel<VEC, U, false, false, ADJ><<<grid, kOrderBlock, 0, st>>>(p);
     }
 }
 
+// ADJ: the adjoint instantiation (an application of M^T in the backward pass)
+template <bool ADJ = false>
 static int launch_order(const OrderParams& p, const OrderConfig& c, cudaStream_t st) {
     if (p.n_rows == 0) return EGNN_OK;
     const int rows_per_block = (kOrderBlock / 32) * (32 >> (c.fl_log2 + c.nz_log2));
     dim3 grid((unsigned)ceil_div64(p.n_rows, rows_per_block), (unsigned)c.grid_y, 1);
     const bool has_vals = p.vals != nullptr;
-    if (c.vec == 4) launch_order_vu<4, 1>(p, has_vals, c.prescaled, grid, st);
-    else if (c.u == 1) launch_order_vu<1, 1>(p, has_vals, c.prescaled, grid, st);
-    else launch_order_vu<1, 4>(p, has_vals, c.prescaled, grid, st);
+    if (c.vec == 4) launch_order_vu<4, 1, ADJ>(p, has_vals, c.prescaled, grid, st);
+    else if (c.u == 1) launch_order_vu<1, 1, ADJ>(p, has_vals, c.prescaled, grid, st);
+    else launch_order_vu<1, 4, ADJ>(p, has_vals, c.prescaled, grid, st);
     EGNN_LAUNCH_CHECK("cheb_order_kernel launch");
     return EGNN_OK;
 }
@@ -112,45 +115,49 @@ static RingConfig ring_config(int ldy) {
     return c;
 }
 
-template <int NZ_LOG2, bool PEER, bool DYN>
+template <int NZ_LOG2, bool PEER, bool DYN, bool ADJ>
 static int launch_wide_npd(const WideParams& p, dim3 grid, cudaStream_t st) {
     const bool aligned = (p.F % 4) == 0;
     if (p.vals) {
-        if (aligned) cheb_wide_kernel<NZ_LOG2, true, true, PEER, DYN><<<grid, kWideBlock, 0, st>>>(p);
-        else cheb_wide_kernel<NZ_LOG2, true, false, PEER, DYN><<<grid, kWideBlock, 0, st>>>(p);
+        if (aligned) cheb_wide_kernel<NZ_LOG2, true, true, PEER, DYN, ADJ><<<grid, kWideBlock, 0, st>>>(p);
+        else cheb_wide_kernel<NZ_LOG2, true, false, PEER, DYN, ADJ><<<grid, kWideBlock, 0, st>>>(p);
     } else {
-        if (aligned) cheb_wide_kernel<NZ_LOG2, false, true, PEER, DYN><<<grid, kWideBlock, 0, st>>>(p);
-        else cheb_wide_kernel<NZ_LOG2, false, false, PEER, DYN><<<grid, kWideBlock, 0, st>>>(p);
+        if (aligned) cheb_wide_kernel<NZ_LOG2, false, true, PEER, DYN, ADJ><<<grid, kWideBlock, 0, st>>>(p);
+        else cheb_wide_kernel<NZ_LOG2, false, false, PEER, DYN, ADJ><<<grid, kWideBlock, 0, st>>>(p);
     }
     EGNN_LAUNCH_CHECK("cheb_wide_kernel launch");
     return EGNN_OK;
 }
 
 // DYN instantiation (single GPU only): rows handed out from p.row_counter
-template <int NZ_LOG2, bool PEER>
+template <int NZ_LOG2, bool PEER, bool ADJ>
 static int launch_wide_np(const WideParams& p, dim3 grid, cudaStream_t st) {
-    if (!PEER && p.row_counter) return launch_wide_npd<NZ_LOG2, false, true>(p, grid, st);
-    return launch_wide_npd<NZ_LOG2, PEER, false>(p, grid, st);
+    if (!PEER && p.row_counter) return launch_wide_npd<NZ_LOG2, false, true, ADJ>(p, grid, st);
+    return launch_wide_npd<NZ_LOG2, PEER, false, ADJ>(p, grid, st);
 }
 
-// PEER instantiation: operand in the exchange window, written by the other GPUs (world > 1)
-template <int NZ_LOG2>
+// PEER instantiation: operand in the exchange window, written by the other GPUs (world > 1).
+// The adjoint (ADJ) runs on one GPU only.
+template <int NZ_LOG2, bool ADJ>
 static int launch_wide_n(const WideParams& p, dim3 grid, cudaStream_t st) {
-    return p.peer.world > 1 ? launch_wide_np<NZ_LOG2, true>(p, grid, st) : launch_wide_np<NZ_LOG2, false>(p, grid, st);
+    if constexpr (ADJ) return launch_wide_np<NZ_LOG2, false, true>(p, grid, st);
+    else return p.peer.world > 1 ? launch_wide_np<NZ_LOG2, true, false>(p, grid, st)
+                                 : launch_wide_np<NZ_LOG2, false, false>(p, grid, st);
 }
 
 // (Measured and dropped: pinning the gather operand in L2 with an access-policy window and the
 // persisting set-aside - arxiv F = 128 0.283 -> 0.276 ms per order, Reddit F = 64 2.13 -> 2.28,
 // Physics F = 8415 2.77 -> 3.6: the set-aside shrinks the L2 left for the other four slabs.)
 // Wide kernel: persistent grid of kWideMinBlocks CTAs per SM per feature tile.
+template <bool ADJ = false>
 static int launch_wide(const WideParams& p, const RingConfig& c, int sm_count, cudaStream_t st) {
     dim3 grid((unsigned)(sm_count * kWideMinBlocks), (unsigned)c.grid_y, 1);
     switch (c.nz_log2) {
-        case 0: return launch_wide_n<0>(p, grid, st);
-        case 1: return launch_wide_n<1>(p, grid, st);
-        case 2: return launch_wide_n<2>(p, grid, st);
-        case 3: return launch_wide_n<3>(p, grid, st);
-        default: return launch_wide_n<4>(p, grid, st);
+        case 0: return launch_wide_n<0, ADJ>(p, grid, st);
+        case 1: return launch_wide_n<1, ADJ>(p, grid, st);
+        case 2: return launch_wide_n<2, ADJ>(p, grid, st);
+        case 3: return launch_wide_n<3, ADJ>(p, grid, st);
+        default: return launch_wide_n<4, ADJ>(p, grid, st);
     }
 }
 
@@ -334,7 +341,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 6; }
+int egnn_abi_version(void) { return 7; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -807,6 +814,226 @@ int egnn_cheb_wavelet(const int32_t* rowptr, const int32_t* colidx, const float*
         EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
     }
     return EGNN_OK;
+}
+
+// ---- backward of the wavelet pass (csrc/adjoint.cuh) ------------------------------------------------
+int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                      const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
+                      int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                      const float* cbar, const float* tbar_or_null, float* xbar,
+                      const int32_t* delta_row_host, const int32_t* delta_col_host,
+                      const float* delta_val_host, int32_t n_delta, void* workspace,
+                      size_t workspace_bytes, egnn_stream_t stream, void* const* app_events_host,
+                      const int32_t* row_order_or_null) {
+    EGNN_REQUIRE(rowptr_t && dinv && iso && cbar && xbar && coeffs_host, "null pointer");
+    EGNN_REQUIRE(nnz == 0 || colidx_t, "null colidx");
+    EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
+    EGNN_REQUIRE(f >= 1, "f must be >= 1");
+    EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "k out of range");
+    EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
+    if (n == 0) return EGNN_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    OrderParams p{};
+    int rc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    if (rc) return rc;
+    for (int i = 0; i < n_delta; ++i)
+        EGNN_REQUIRE(p.delta.row[i] >= 0 && p.delta.row[i] < n && p.delta.col[i] >= 0 && p.delta.col[i] < n,
+                     "delta index out of range");
+    const size_t slab_elems = (size_t)n * (size_t)f;
+    auto coef_row = [&](int m) {
+        CoefRow c{};
+        for (int s = 0; s < n_scales; ++s) c.c[s] = coeffs_host[s * (k + 1) + m];
+        return c;
+    };
+    auto tbar_at = [&](int m) { return tbar_or_null ? tbar_or_null + (size_t)m * slab_elems : nullptr; };
+    if (k == 0) {
+        adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
+            cbar, tbar_at(0), dinv, xbar, nullptr, n, f, n_scales, f, coef_row(0));
+        EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+        return EGNN_OK;
+    }
+    const size_t need = egnn_cheb_workspace_bytes(n, f);
+    if (workspace == nullptr || workspace_bytes < need) {
+        set_error("workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+        return EGNN_ERR_WORKSPACE;
+    }
+    char* ws = (char*)align_up((size_t)workspace, 256);
+    // application j = 1..K produces b_m, m = K - j (b_0 = the signal's gradient)
+    if (f >= kWideMinF) {
+        const int ldy = (f + 3) / 4 * 4;
+        const RingConfig rcfg = ring_config(ldy);
+        const size_t yslab = align_up(sizeof(float) * (size_t)n * (size_t)ldy, 256);
+        float* yb[2] = {(float*)ws, (float*)(ws + yslab)};        // dinv (.) b, rows padded to 16 bytes
+        unsigned* counters = (unsigned*)(ws + 2 * yslab);
+        rc = check_cuda(cudaMemsetAsync(counters, 0, sizeof(unsigned) * (size_t)k * (size_t)rcfg.grid_y, st), "memset row counters");
+        if (rc) return rc;
+        adjoint_prologue_kernel<<<grid_for((int64_t)n * ldy, 256), 256, 0, st>>>(
+            cbar, tbar_at(k), dinv, nullptr, yb[0], n, f, n_scales, ldy, coef_row(k));
+        EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+        WideParams wp{};
+        wp.delta = p.delta;
+        wp.rowptr = rowptr_t; wp.colidx = colidx_t; wp.vals = vals_t_or_null;
+        wp.perm = row_order_or_null; wp.n_hub = row_order_or_null ? row_order_or_null + n : nullptr;
+        wp.dinv = dinv; wp.iso = iso; wp.out = nullptr; wp.n_rows = n; wp.row0 = 0; wp.F = f; wp.ldy = ldy;
+        wp.S = n_scales; wp.a = op_scale; wp.b = op_shift; wp.first = 0; wp.normalize = 0;
+        wp.cbar = cbar; wp.x0_own = nullptr;
+        const bool dynamic_rows = rcfg.grid_y == 1 && nnz < (int64_t)kWideDynamicMaxDegree * n;   // as the forward
+        const int sms = device_sm_count();
+        for (int j = 1; j <= k; ++j) {
+            const int m = k - j;
+            wp.row_counter = dynamic_rows ? counters + (size_t)(j - 1) * (size_t)rcfg.grid_y : nullptr;
+            wp.ysrc = yb[(j - 1) & 1];
+            wp.y2_own = j == 1 ? nullptr : yb[j & 1];
+            wp.y_out = m == 0 ? nullptr : yb[j & 1];             // in place over dinv (.) b_{m+2} (own row only)
+            wp.tk_out = m == 0 ? xbar : nullptr;
+            wp.tbar = tbar_at(m);
+            wp.c_adj = m == 0 ? 1.f : 2.f;
+            for (int s = 0; s < n_scales; ++s) wp.c_k[s] = coeffs_host[s * (k + 1) + m];
+            if (app_events_host) {
+                rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1)], st), "event record");
+                if (rc) return rc;
+            }
+            rc = launch_wide<true>(wp, rcfg, sms, st);
+            if (rc) return rc;
+            if (app_events_host) {
+                rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1) + 1], st), "event record");
+                if (rc) return rc;
+            }
+        }
+        return EGNN_OK;
+    }
+    const OrderConfig cfg = choose_config(n, nnz, f);
+    const size_t slab = align_up(sizeof(float) * slab_elems, 256);
+    float* tbuf[2] = {(float*)ws, (float*)(ws + slab)};
+    float* ybuf[2] = {(float*)(ws + 2 * slab), (float*)(ws + 3 * slab)};
+    adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
+        cbar, tbar_at(k), dinv, tbuf[0], cfg.prescaled ? ybuf[0] : nullptr, n, f, n_scales, f, coef_row(k));
+    EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+    p.rowptr = rowptr_t; p.colidx = colidx_t; p.vals = vals_t_or_null; p.dinv = dinv; p.iso = iso;
+    p.out = nullptr; p.acc_ws = nullptr; p.n_rows = n; p.row0 = 0; p.F = f; p.S = n_scales;
+    p.a = op_scale; p.b = op_shift; p.mode = 0; p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
+    p.first = 0; p.normalize = 0; p.cbar = cbar;
+    for (int j = 1; j <= k; ++j) {
+        const int m = k - j;
+        p.tprev_own = tbuf[(j - 1) & 1];
+        p.tprev2_own = j == 1 ? nullptr : tbuf[j & 1];
+        p.tk_own = m == 0 ? xbar : tbuf[j & 1];                  // in place over b_{m+2}
+        p.gsrc = cfg.prescaled ? ybuf[(j - 1) & 1] : tbuf[(j - 1) & 1];
+        p.y_own = (cfg.prescaled && m > 0) ? ybuf[j & 1] : nullptr;
+        p.tbar = tbar_at(m);
+        p.c_adj = m == 0 ? 1.f : 2.f;
+        for (int s = 0; s < n_scales; ++s) p.c_k[s] = coeffs_host[s * (k + 1) + m];
+        if (app_events_host) {
+            rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1)], st), "event record");
+            if (rc) return rc;
+        }
+        rc = launch_order<true>(p, cfg, st);
+        if (rc) return rc;
+        if (app_events_host) {
+            rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1) + 1], st), "event record");
+            if (rc) return rc;
+        }
+    }
+    return EGNN_OK;
+}
+
+int egnn_l1_normalize(const float* c, float* h, int64_t n_vec, int32_t f, egnn_stream_t stream) {
+    EGNN_REQUIRE(c && h, "null pointer");
+    EGNN_REQUIRE(n_vec >= 0 && f >= 1, "bad shape");
+    if (n_vec == 0) return EGNN_OK;
+    l1_normalize_out_kernel<<<grid_for(n_vec * 32, 256), 256, 0, (cudaStream_t)stream>>>(c, h, n_vec, f);
+    EGNN_LAUNCH_CHECK("l1_normalize_out_kernel launch");
+    return EGNN_OK;
+}
+
+int egnn_l1_normalize_backward(const float* c, const float* hbar, const float* cbar_in_or_null, float* cbar_out,
+                               int64_t n_vec, int32_t f, egnn_stream_t stream) {
+    EGNN_REQUIRE(c && hbar && cbar_out, "null pointer");
+    EGNN_REQUIRE(n_vec >= 0 && f >= 1, "bad shape");
+    if (n_vec == 0) return EGNN_OK;
+    l1_normalize_backward_kernel<<<grid_for(n_vec * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+        c, hbar, cbar_in_or_null, cbar_out, n_vec, f);
+    EGNN_LAUNCH_CHECK("l1_normalize_backward_kernel launch");
+    return EGNN_OK;
+}
+
+size_t egnn_cheb_coeff_grad_ws_bytes(int32_t k, int32_t n_scales) {
+    const int64_t q = (int64_t)(k > 0 ? k + 1 : 1) * (n_scales > 0 ? n_scales : 1);
+    return align_up(sizeof(double) * (size_t)kCoefGradBlocks * (size_t)q, 256) + 256;
+}
+
+int egnn_cheb_coeff_grad(const float* cbar, const float* t_all, int64_t n, int32_t f, int32_t k, int32_t n_scales,
+                         double* grad_out, void* workspace, size_t workspace_bytes, egnn_stream_t stream) {
+    EGNN_REQUIRE(cbar && t_all && grad_out, "null pointer");
+    EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && f >= 1, "bad shape");
+    EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "k out of range");
+    EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
+    const size_t need = egnn_cheb_coeff_grad_ws_bytes(k, n_scales);
+    if (workspace == nullptr || workspace_bytes < need) {
+        set_error("coefficient-gradient workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+        return EGNN_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    double* partial = (double*)align_up((size_t)workspace, 256);
+    coeff_grad_partial_kernel<<<kCoefGradBlocks, kCoefGradThreads, 0, st>>>(cbar, t_all, n, f, k, n_scales, partial);
+    EGNN_LAUNCH_CHECK("coeff_grad_partial_kernel launch");
+    const int n_out = n_scales * (k + 1);
+    coeff_grad_finish_kernel<<<(unsigned)ceil_div64(n_out, 128), 128, 0, st>>>(partial, kCoefGradBlocks, n_out, grad_out);
+    EGNN_LAUNCH_CHECK("coeff_grad_finish_kernel launch");
+    return EGNN_OK;
+}
+
+static size_t transpose_cub_bytes(int64_t n, int64_t nnz) {
+    size_t a = 0, b = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, a, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const int32_t*)nullptr,
+                                    (int32_t*)nullptr, (int)nnz);
+    cub::DeviceScan::ExclusiveSum(nullptr, b, (int32_t*)nullptr, (int32_t*)nullptr, (int)(n + 1));
+    return (a > b ? a : b) + 256;
+}
+
+size_t egnn_csr_transpose_ws_bytes(int64_t n, int64_t nnz) {
+    if (n < 0 || nnz < 0) return 256;
+    return 3 * align_up(4 * (size_t)(nnz > 0 ? nnz : 1), 256) + align_up(4 * (size_t)(n + 1), 256) +
+           transpose_cub_bytes(n, nnz) + 256;
+}
+
+int egnn_csr_transpose(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null, int64_t n,
+                       int64_t nnz, int32_t* rowptr_t, int32_t* colidx_t, float* vals_t_or_null, void* workspace,
+                       size_t workspace_bytes, egnn_stream_t stream) {
+    EGNN_REQUIRE(rowptr && rowptr_t, "null pointer");
+    EGNN_REQUIRE(nnz == 0 || (colidx && colidx_t), "null colidx");
+    EGNN_REQUIRE((vals_or_null == nullptr) == (vals_t_or_null == nullptr), "vals and vals_t come together");
+    EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
+    const size_t need = egnn_csr_transpose_ws_bytes(n, nnz);
+    if (workspace == nullptr || workspace_bytes < need) {
+        set_error("transpose workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+        return EGNN_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t arr = align_up(4 * (size_t)(nnz > 0 ? nnz : 1), 256);
+    char* ws = (char*)align_up((size_t)workspace, 256);
+    uint32_t* keys_sorted = (uint32_t*)ws;
+    int32_t* ids = (int32_t*)(ws + arr);
+    int32_t* ids_sorted = (int32_t*)(ws + 2 * arr);
+    int32_t* counts = (int32_t*)(ws + 3 * arr);
+    void* cub_temp = ws + 3 * arr + align_up(4 * (size_t)(n + 1), 256);
+    size_t cub_bytes = transpose_cub_bytes(n, nnz);
+    int rc = check_cuda(cudaMemsetAsync(counts, 0, sizeof(int32_t) * (size_t)(n + 1), st), "memset column counts");
+    if (rc) return rc;
+    if (nnz > 0) {
+        transpose_count_kernel<<<grid_for(nnz, 256), 256, 0, st>>>(colidx, nnz, ids, counts);
+        EGNN_LAUNCH_CHECK("transpose_count_kernel launch");
+        // stable: entries of one column keep their CSR (row-major) order, so the rows come out sorted
+        const int end_bit = pow2_ceil_log2(n > 1 ? n : 2);
+        rc = check_cuda(cub::DeviceRadixSort::SortPairs(cub_temp, cub_bytes, (const uint32_t*)colidx, keys_sorted, ids,
+                                                        ids_sorted, (int)nnz, 0, end_bit, st), "sort entries by column");
+        if (rc) return rc;
+        transpose_fill_kernel<<<grid_for(nnz, 256), 256, 0, st>>>(rowptr, n, vals_or_null, ids_sorted, nnz, colidx_t,
+                                                                 vals_t_or_null);
+        EGNN_LAUNCH_CHECK("transpose_fill_kernel launch");
+    }
+    return check_cuda(cub::DeviceScan::ExclusiveSum(cub_temp, cub_bytes, counts, rowptr_t, (int)(n + 1), st),
+                      "scan column counts");
 }
 
 int egnn_cheb_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,

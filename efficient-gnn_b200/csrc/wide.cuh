@@ -72,6 +72,12 @@ struct WideParams {
     float c_k[EGNN_MAX_SCALES];
     DeltaList delta;
     PeerPush peer;              // world > 1: y_out rows also go to every rank's exchange window
+    // adjoint instantiation (ADJ, single GPU): b_k = c_adj * (M^T b_{k+1}) - b_{k+2} + v_k with
+    // v_k = tbar + sum_s c_k[s] * cbar[:, s, :]; ysrc = dinv (.) b_{k+1}, y2_own = dinv (.) b_{k+2}
+    // (NULL: zero), y_out = dinv (.) b_k, tk_out = b_k (the last application: the signal's gradient)
+    const float* cbar;          // [n_rows, S, F]
+    const float* tbar;          // [n_rows, F] or NULL
+    float c_adj;
 };
 
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
@@ -141,7 +147,7 @@ __device__ __forceinline__ void store_user4(float* base, int64_t off, int ncol, 
 
 // Fused epilogue of one row tile; `writer` lanes (entry slot 0, column inside
 // the padded row) hold the row's sum in acc.  ncol = valid user columns of the lane.
-template <bool ALIGNED, bool PEER>
+template <bool ALIGNED, bool PEER, bool ADJ>
 __device__ __forceinline__ void wide_epilogue(const WideParams& p, int row, int grow, int FL, int fcol, int ncol,
                                               bool writer, float (&acc)[4], uint64_t pol_stream, bool have_own,
                                               const float (&own)[4]) {
@@ -163,6 +169,39 @@ __device__ __forceinline__ void wide_epilogue(const WideParams& p, int row, int 
     }
     const float nscale = -p.a * di;
     const float inv_di = 1.f / di;
+    if constexpr (ADJ) {                    // adjoint epilogue (Clenshaw step): no scale accumulation
+        if (!writer) return;
+        const int64_t uoff = (int64_t)row * F + fcol;
+        const int64_t yoff = (int64_t)row * ldy + fcol;
+        float bown[4] = {0.f, 0.f, 0.f, 0.f}, b2[4] = {0.f, 0.f, 0.f, 0.f}, v[4] = {0.f, 0.f, 0.f, 0.f};
+        if (theta != 0.f) {                                     // b_{k+1} of the own row = y / dinv
+            const float4 t = ld_operand_f4<PEER>(p.ysrc + (int64_t)grow * ldy + fcol);
+            bown[0] = t.x * inv_di; bown[1] = t.y * inv_di; bown[2] = t.z * inv_di; bown[3] = t.w * inv_di;
+        }
+        if (have_own) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) b2[j] = own[j] * inv_di;
+        } else if (p.y2_own) {
+            const float4 t = ld_stream_f4(p.y2_own + yoff, pol_stream);
+            b2[0] = t.x * inv_di; b2[1] = t.y * inv_di; b2[2] = t.z * inv_di; b2[3] = t.w * inv_di;
+        }
+        if (p.tbar) load_user4<ALIGNED>(p.tbar, uoff, ncol, pol_stream, v);
+        for (int s = 0; s < p.S; ++s) {
+            float t[4];
+            load_user4<ALIGNED>(p.cbar, ((int64_t)row * p.S + s) * F + fcol, ncol, pol_stream, t);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) v[j] = fmaf(p.c_k[s], t[j], v[j]);
+        }
+        float b[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            b[j] = fmaf(p.c_adj, fmaf(theta, bown[j], nscale * acc[j]), v[j] - b2[j]);
+            if (j >= ncol) b[j] = 0.f;                          // padding columns stay zero
+        }
+        if (p.tk_out) store_user4<ALIGNED>(p.tk_out, uoff, ncol, pol_stream, b);
+        if (p.y_out) *reinterpret_cast<float4*>(p.y_out + yoff) = make_float4(di * b[0], di * b[1], di * b[2], di * b[3]);
+        return;
+    }
     float tk[4] = {0.f, 0.f, 0.f, 0.f}, xprev[4] = {0.f, 0.f, 0.f, 0.f};
     if (writer) {
         const int64_t uoff = (int64_t)row * F + fcol;          // user arrays
@@ -301,7 +340,7 @@ __device__ __forceinline__ void wide_accumulate(const WideParams& p, int qs, int
     for (int v = 0; v < 4; ++v) sum[v] = hi[v] + acc[v];
 }
 
-template <int NZ_LOG2, bool HAS_VALS, bool ALIGNED, bool PEER, bool DYN>
+template <int NZ_LOG2, bool HAS_VALS, bool ALIGNED, bool PEER, bool DYN, bool ADJ = false>
 __global__ void __launch_bounds__(kWideBlock, kWideMinBlocks)
 cheb_wide_kernel(const __grid_constant__ WideParams p) {
     __shared__ float hub_part[kWideWarps][128];
@@ -358,7 +397,7 @@ cheb_wide_kernel(const __grid_constant__ WideParams p) {
                 for (int w = 0; w < kWideWarps; ++w) t += hub_part[w][fl * 4 + v];     // fixed order
                 acc[v] = t;
             }
-            wide_epilogue<ALIGNED, PEER>(p, row, grow, FL, fcol, ncol, writer, acc, pol_stream, false, none);
+            wide_epilogue<ALIGNED, PEER, ADJ>(p, row, grow, FL, fcol, ncol, writer, acc, pol_stream, false, none);
         }
     }
 
@@ -379,17 +418,19 @@ cheb_wide_kernel(const __grid_constant__ WideParams p) {
     int row = 0, start = 0, end = 0, pre_c = 0;
     float pre_w = 0.f;
     float own[4] = {0.f, 0.f, 0.f, 0.f};
-    // the own-row operand of the epilogue (T_0 row at order 1, dinv (.) T_{k-2} later) is requested a row ahead
+    // the own-row operand of the epilogue (T_0 row at order 1, dinv (.) T_{k-2} later; adjoint:
+    // dinv (.) b_{k+2} when there is one) is requested a row ahead
     auto load_own = [&](int rw, float (&dst)[4]) {
         if (!writer) return;
-        if (p.first) {
+        if (ADJ && !p.y2_own) return;
+        if (!ADJ && p.first) {
             if (ALIGNED) load_user4<true>(p.x0_own, (int64_t)rw * p.F + fcol, ncol, pol_stream, dst);
         } else {
             const float4 t = ld_stream_f4(p.y2_own + (int64_t)rw * p.ldy + fcol, pol_stream);
             dst[0] = t.x; dst[1] = t.y; dst[2] = t.z; dst[3] = t.w;
         }
     };
-    const bool have_own = !p.first || ALIGNED;
+    const bool have_own = ADJ ? p.y2_own != nullptr : (!p.first || ALIGNED);
     if (r < n_rows) {
         row = p.perm ? __ldg(p.perm + r) : r;
         start = __ldg(p.rowptr + row);
@@ -432,7 +473,7 @@ cheb_wide_kernel(const __grid_constant__ WideParams p) {
 #pragma unroll
             for (int v = 0; v < 4; ++v) acc[v] += __shfl_xor_sync(0xffffffffu, acc[v], o);
         }
-        wide_epilogue<ALIGNED, PEER>(p, row, grow, FL, fcol, ncol, writer, acc, pol_stream, have_own, own);
+        wide_epilogue<ALIGNED, PEER, ADJ>(p, row, grow, FL, fcol, ncol, writer, acc, pol_stream, have_own, own);
         r = r_next; r_next = r_nn; row = row_n; start = start_n; end = end_n; pre_c = pre_c_n; pre_w = pre_w_n;
 #pragma unroll
         for (int v = 0; v < 4; ++v) own[v] = own_n[v];

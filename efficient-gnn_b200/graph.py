@@ -198,6 +198,7 @@ class CsrGraph:
         self._sorted = None        # lazily read result of the degree pass's sortedness check
         self._scratch = None       # lazily built scratch copies of dinv / iso / x0 / y0 for the in-place UGCA patches
         self._y0 = None            # lazily built dinv * x0 (first operand of the narrow path, default signal)
+        self._adjoint = None       # lazily built transposed graph of the backward pass (False: symmetric)
 
     def _release_scratch(self):
         self._diag = self._colsum = None
@@ -230,6 +231,36 @@ class CsrGraph:
                                                            _stream()), "egnn_prescale")
             self._y0 = y
         return self._y0
+
+    def adjoint(self) -> "CsrGraph":
+        """The graph the backward pass gathers over: ``self`` when the sorted CSR
+        equals its transpose (every undirected graph), else the transposed
+        adjacency carrying THIS graph's degree vectors (scipy normalises by the
+        column sums on both sides of ``L``, so they are not re-derived from the
+        transpose).  Built once on the device (one 1-byte host read)."""
+        if self._adjoint is None:
+            lib = _cabi.load()
+            n, nnz = self.n, self.nnz
+            with torch.cuda.device(self.device):
+                rp = torch.empty(n + 1, dtype=torch.int32, device=self.device)
+                ci = torch.empty(nnz, dtype=torch.int32, device=self.device)
+                vv = None if self.vals is None else torch.empty(nnz, dtype=torch.float32, device=self.device)
+                ws_bytes = int(lib.egnn_csr_transpose_ws_bytes(n, nnz))
+                ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
+                _cabi.check(lib.egnn_csr_transpose(_cabi.ptr(self.rowptr), _cabi.ptr(self.colidx), _cabi.ptr(self.vals),
+                                                   n, nnz, _cabi.ptr(rp), _cabi.ptr(ci), _cabi.ptr(vv), _cabi.ptr(ws),
+                                                   ws_bytes, _stream()), "egnn_csr_transpose")
+                same = torch.equal(rp, self.rowptr) and torch.equal(ci, self.colidx) and \
+                    (vv is None or torch.equal(vv, self.vals))
+            if same:
+                self._adjoint = False
+            else:
+                g = CsrGraph(rp, ci, vv, n, _prepare=False)
+                g.dinv, g.iso, g.x0, g.w, g.rowsum = self.dinv, self.iso, self.x0, self.w, self.rowsum
+                g._release_scratch()
+                g._sorted = True                     # the transpose comes out with sorted rows
+                self._adjoint = g
+        return self._adjoint or self
 
     # -- processing order for the wide (F >= 8) kernel ----------------------------
     def row_order(self):

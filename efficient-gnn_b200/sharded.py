@@ -398,6 +398,8 @@ class ShardedWavelet:
     ``rowptr_local`` / ``colidx_local``: the rank's rows (global column ids),
     rows assigned by :class:`RowPartition`.  ``engine`` defaults to the CUDA
     engine; tests inject a CPU engine to drive this logic over gloo.
+    Forward-only: the sharded pass has no backward (single-GPU
+    ``graph_wavelet_features`` does).
     """
 
     def __init__(self, rowptr_local, colidx_local, n_global: int, *, group=None, engine=None, device=None,

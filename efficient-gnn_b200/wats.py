@@ -11,6 +11,13 @@ New behaviour is keyword-only.  All arithmetic of the path runs in
 libegnn_b200 (hand-written sm_100a CUDA behind a C ABI); this module is tensor
 plumbing.  There is no CPU fallback: without the shared library or a CUDA
 device every entry point raises ``EgnnError``.
+
+``graph_wavelet_features``, ``chebyshev_polynomials`` and both operators'
+``@`` are differentiable w.r.t. the signal (and the features w.r.t. a tensor
+``s``): when grad mode is on and an input requires grad, the pass runs inside
+an autograd function whose backward is the adjoint (Clenshaw) pass of
+``egnn_cheb_adjoint``.  Otherwise nothing changes: same kernels, nothing saved.
+``WATS``, ``WaveletSession`` and the sharded path stay forward-only.
 """
 from __future__ import annotations
 
@@ -21,6 +28,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
+from torch.autograd.function import once_differentiable
 
 from . import _cabi
 from .graph import CsrGraph, as_graph, deltas_from_dense
@@ -114,6 +122,144 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
     return out, t_all
 
 
+def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, op_scale: float, op_shift: float,
+                 cbar: torch.Tensor, tbar=None, deltas=None, app_events=None) -> torch.Tensor:
+    """One call of egnn_cheb_adjoint: the signal's gradient ``[N, F]`` from ``cbar`` ``[N, S, F]`` (and
+    ``tbar`` ``[K+1, N, F]``).  ``graph_t``: the transposed graph (:meth:`CsrGraph.adjoint`),
+    ``degree_vectors``: the forward's ``(dinv, iso)``, ``deltas``: the forward's flips, not yet
+    transposed."""
+    lib = _cabi.load()
+    n, f, dev = graph_t.n, int(cbar.shape[2]), graph_t.device
+    dinv, iso = degree_vectors
+    d_rows, d_cols, d_vals = ([], [], []) if deltas is None else deltas
+    row_order = graph_t.row_order() if (f >= WIDE_MIN_F and k >= 1) else None
+    with torch.cuda.device(dev):
+        xbar = torch.empty((n, f), dtype=torch.float32, device=dev)
+        ws_bytes = int(lib.egnn_cheb_workspace_bytes(n, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        coeffs32 = np.ascontiguousarray(coeffs, dtype=np.float32)
+        _cabi.check(lib.egnn_cheb_adjoint(
+            _cabi.ptr(graph_t.rowptr), _cabi.ptr(graph_t.colidx), _cabi.ptr(graph_t.vals), _cabi.ptr(dinv),
+            _cabi.ptr(iso), n, graph_t.nnz, f, k, int(coeffs.shape[0]), coeffs32.ctypes.data_as(C.c_void_p),
+            float(op_scale), float(op_shift), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar),
+            _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),       # transposed flips: rows <-> cols
+            _cabi.host_array(C.c_int32, [int(v) for v in d_rows]),
+            _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows),
+            _cabi.ptr(ws), ws_bytes, _stream(), app_events, _cabi.ptr(row_order)), "egnn_cheb_adjoint")
+    return xbar
+
+
+def _coeff_grad(cbar: torch.Tensor, t_all: torch.Tensor) -> torch.Tensor:
+    """``G[s, k] = <cbar[:, s, :], T_k>`` in float64 on the device (egnn_cheb_coeff_grad)."""
+    lib = _cabi.load()
+    n, n_scales, f = cbar.shape
+    k = int(t_all.shape[0]) - 1
+    with torch.cuda.device(cbar.device):
+        g = torch.empty((n_scales, k + 1), dtype=torch.float64, device=cbar.device)
+        ws_bytes = int(lib.egnn_cheb_coeff_grad_ws_bytes(k, n_scales))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=cbar.device)
+        _cabi.check(lib.egnn_cheb_coeff_grad(_cabi.ptr(cbar), _cabi.ptr(t_all), n, f, k, n_scales, _cabi.ptr(g),
+                                             _cabi.ptr(ws), ws_bytes, _stream()), "egnn_cheb_coeff_grad")
+    return g
+
+
+class _PassSpec:
+    """Everything of one pass but its differentiable inputs (the signal and the scales)."""
+
+    def __init__(self, graph, adjoint, k, coeffs, op_scale, op_shift, want_orders, deltas=None, degree_vectors=None,
+                 use_sell=None, default_signal=False, y0=None):
+        self.graph, self.adjoint, self.k, self.coeffs = graph, adjoint, k, coeffs
+        self.op_scale, self.op_shift, self.want_orders = op_scale, op_shift, want_orders
+        self.deltas, self.degree_vectors, self.use_sell = deltas, degree_vectors, use_sell
+        self.default_signal, self.y0 = default_signal, y0
+
+
+class _WaveletPass(torch.autograd.Function):
+    """``(C [N,S,F], T [K+1,N,F])`` of one un-normalised pass as a function of the signal ``x0`` and
+    the scales ``s`` (a tensor, or None when they need no gradient).  ``T`` is empty unless the
+    orders are wanted or ``s`` needs a gradient (its backward reads them).  Backward: the adjoint
+    pass on the transposed graph, and ``ds_j = -sum_k k alpha[j,k] <Cbar_j, T_k>``."""
+
+    @staticmethod
+    def forward(ctx, x0, s, spec):
+        ctx.set_materialize_grads(False)        # an output nobody differentiates arrives as None
+        s_grad = s is not None and ctx.needs_input_grad[1]
+        comb, t_all = _run_cheb(spec.graph, x0, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, False,
+                                spec.want_orders or s_grad, spec.deltas, spec.degree_vectors, use_sell=spec.use_sell,
+                                default_signal=spec.default_signal, y0=spec.y0)
+        if t_all is None:
+            t_all = comb.new_empty((0,))
+            ctx.mark_non_differentiable(t_all)
+        ctx.spec, ctx.x_shape = spec, x0.shape
+        ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
+        ctx.save_for_backward(t_all if s_grad else None)
+        return comb, t_all
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_comb, g_orders):
+        spec = ctx.spec
+        (t_all,) = ctx.saved_tensors
+        g = spec.graph
+        n_scales = int(spec.coeffs.shape[0])
+        f = 1 if len(ctx.x_shape) == 1 else int(ctx.x_shape[1])
+        cbar = (g_comb.to(torch.float32).contiguous() if g_comb is not None else
+                torch.zeros((g.n, n_scales, f), dtype=torch.float32, device=g.device))
+        tbar = g_orders.to(torch.float32).contiguous() if (g_orders is not None and g_orders.numel()) else None
+        x_grad = s_grad = None
+        if ctx.needs_input_grad[0]:
+            dv = spec.degree_vectors if spec.degree_vectors is not None else (g.dinv, g.iso)
+            x_grad = _run_adjoint(spec.adjoint(), dv, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, cbar, tbar,
+                                  spec.deltas).reshape(ctx.x_shape)
+        if ctx.needs_input_grad[1]:
+            G = _coeff_grad(cbar, t_all)
+            alpha = torch.from_numpy(np.ascontiguousarray(spec.coeffs, dtype=np.float64)).to(G.device)
+            kk = torch.arange(spec.k + 1, dtype=torch.float64, device=G.device)
+            shape, dev, dtype = ctx.s_meta
+            s_grad = (-(kk * alpha * G).sum(dim=1)).to(device=dev, dtype=dtype).reshape(shape)
+        return x_grad, s_grad, None
+
+
+class _L1Normalize(torch.autograd.Function):
+    """``H = C / (sum_f |C| + 1e-8)`` per (row, scale) out of place, backward by egnn_l1_normalize_backward
+    (``r`` recomputed from ``C``)."""
+
+    @staticmethod
+    def forward(ctx, comb):
+        h = torch.empty_like(comb)
+        n_vec = comb.shape[0] * comb.shape[1]
+        with torch.cuda.device(comb.device):
+            _cabi.check(_cabi.load().egnn_l1_normalize(_cabi.ptr(comb), _cabi.ptr(h), n_vec, comb.shape[2], _stream()),
+                        "egnn_l1_normalize")
+        ctx.save_for_backward(comb)
+        return h
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_h):
+        (comb,) = ctx.saved_tensors
+        g_h = g_h.to(torch.float32).contiguous()
+        cbar = torch.empty_like(comb)
+        n_vec = comb.shape[0] * comb.shape[1]
+        with torch.cuda.device(comb.device):
+            _cabi.check(_cabi.load().egnn_l1_normalize_backward(_cabi.ptr(comb), _cabi.ptr(g_h), None, _cabi.ptr(cbar),
+                                                                n_vec, comb.shape[2], _stream()),
+                        "egnn_l1_normalize_backward")
+        return cbar
+
+
+def _needs_grad(x0, s=None) -> bool:
+    """The autograd path engages only in grad mode with an input that requires grad."""
+    return torch.is_grad_enabled() and (x0.requires_grad or (isinstance(s, torch.Tensor) and s.requires_grad))
+
+
+def _differentiable_pass(spec: _PassSpec, x0: torch.Tensor, s=None):
+    """``(C, T)`` through :class:`_WaveletPass`; the device / dtype conversion of ``x0`` stays outside
+    the function, so autograd routes the gradient back to a CPU or float64 leaf."""
+    x0 = x0.to(device=spec.graph.device, dtype=torch.float32)
+    return _WaveletPass.apply(x0, s if (isinstance(s, torch.Tensor) and s.requires_grad) else None, spec)
+
+
 def _patches_in_kernel(graph: CsrGraph, f: int, k: int, use_sell) -> bool:
     """Will a perturbed pass of this shape run on the SELL plan (whose kernel applies the degree
     patches of the flips itself)?  Mirrors the plan choice of :func:`_run_cheb`."""
@@ -169,10 +315,16 @@ class LaplacianOperator:
         return LaplacianOperator(self.graph, self.scale, self.shift + self._identity_multiple(other, self.graph.n))
 
     def __matmul__(self, x):
-        """One operator application through the fused kernel (order-1 pass)."""
+        """One operator application through the fused kernel (order-1 pass); differentiable
+        w.r.t. ``x`` (backward: one application of the transposed operator)."""
         xt = torch.as_tensor(x)
         vec = xt.dim() == 1
-        out, _ = _run_cheb(self.graph, xt, 1, np.array([[0.0, 1.0]]), self.scale, self.shift, False, False)
+        coeffs = np.array([[0.0, 1.0]])
+        if _needs_grad(xt):
+            out, _ = _differentiable_pass(_PassSpec(self.graph, self.graph.adjoint, 1, coeffs, self.scale, self.shift,
+                                                    False), xt)
+        else:
+            out, _ = _run_cheb(self.graph, xt, 1, coeffs, self.scale, self.shift, False, False)
         y = out[:, 0, :]
         return y[:, 0] if vec else y
 
@@ -193,7 +345,10 @@ class ExplicitOperator:
     """An explicit sparse matrix (what the reference hands to ``chebyshev_polynomials``: the scipy
     ``L_rescaled`` of calibration/WATS.py:55) as a device operator.  The off-diagonal entries go
     through the same fused kernels as a weighted CSR (unit normaliser, no implicit diagonal), the
-    stored diagonal is applied as a per-row scale; entries are rounded to float32."""
+    stored diagonal is applied as a per-row scale; entries are rounded to float32.  ``@`` is
+    differentiable w.r.t. its operand; the backward gathers over the transposed off-diagonal part,
+    built on first use (the matrix is not assumed symmetric: scipy's two float32 divisions make the
+    rescaled Laplacian asymmetric in the last bit)."""
 
     def __init__(self, mat):
         import scipy.sparse as sp
@@ -215,14 +370,31 @@ class ExplicitOperator:
         self.diag = torch.from_numpy(diag).to(dev)
         self.unit = (torch.ones(n, dtype=torch.float32, device=dev), torch.ones(n, dtype=torch.uint8, device=dev))
         self.shape = (n, n)
+        self._off = off
+        self._transposed = None
+
+    def _transpose(self) -> CsrGraph:
+        if self._transposed is None:
+            t = self._off.T.tocsr()
+            t.sort_indices()
+            dev = self.diag.device
+            self._transposed = CsrGraph(torch.from_numpy(t.indptr.astype(np.int32)).to(dev),
+                                        torch.from_numpy(t.indices.astype(np.int32)).to(dev),
+                                        torch.from_numpy(t.data.astype(np.float32)).to(dev), self.shape[0])
+        return self._transposed
 
     def __matmul__(self, x):
         xt = torch.as_tensor(x)
         vec = xt.dim() == 1
         xt = (xt.unsqueeze(1) if vec else xt).to(device=self.diag.device, dtype=torch.float32)
         # kernel: theta * x - a * dinv_i * sum_{j != i} v_ij dinv_j x_j with a = -1, dinv = 1, theta = 0
-        out, _ = _run_cheb(self.graph, xt, 1, np.array([[0.0, 1.0]]), -1.0, 0.0, False, False,
-                           degree_vectors=self.unit, use_sell=False)
+        coeffs = np.array([[0.0, 1.0]])
+        if _needs_grad(xt):
+            out, _ = _differentiable_pass(_PassSpec(self.graph, self._transpose, 1, coeffs, -1.0, 0.0, False,
+                                                    degree_vectors=self.unit, use_sell=False), xt)
+        else:
+            out, _ = _run_cheb(self.graph, xt, 1, coeffs, -1.0, 0.0, False, False,
+                               degree_vectors=self.unit, use_sell=False)
         y = out[:, 0, :] + self.diag.unsqueeze(1) * xt
         return y[:, 0] if vec else y
 
@@ -232,7 +404,8 @@ def chebyshev_polynomials(L, k, X0):
     (calibration/WATS.py:29-37).  ``L`` is a :class:`LaplacianOperator` (what
     ``compute_normalized_laplacian`` returns, normally rescaled: all orders in the
     fused kernels) or an explicit scipy sparse matrix as in the reference (one
-    kernel application per order); returns k+1 float32 device tensors ``[N,F]``."""
+    kernel application per order); returns k+1 float32 device tensors ``[N,F]``,
+    differentiable w.r.t. ``X0`` when it requires grad."""
     k = int(k)
     if not isinstance(L, LaplacianOperator):
         try:
@@ -252,7 +425,11 @@ def chebyshev_polynomials(L, k, X0):
             t_k.append(2 * (op @ t_k[-1]) - t_k[-2])
         return t_k
     coeffs = np.zeros((1, k + 1))
-    _, t_all = _run_cheb(L.graph, torch.as_tensor(X0), k, coeffs, L.scale, L.shift, False, True)
+    x0 = torch.as_tensor(X0)
+    if _needs_grad(x0):
+        _, t_all = _differentiable_pass(_PassSpec(L.graph, L.graph.adjoint, k, coeffs, L.scale, L.shift, True), x0)
+    else:
+        _, t_all = _run_cheb(L.graph, x0, k, coeffs, L.scale, L.shift, False, True)
     return [t_all[i] for i in range(k + 1)]
 
 
@@ -270,16 +447,25 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
     and the un-normalised combination; ``deltas=(rows, cols, vals)`` applies
     edge flips on top of the graph without rebuilding it (UGCA recompute).
     Returns a float32 tensor on the graph's device.
+
+    Differentiable w.r.t. ``X0`` and a 0-d / 1-d tensor ``s`` (coefficients are
+    computed from its values as for a float) when grad mode is on and one of
+    them requires grad: every output (``features``, ``combined``, ``orders``)
+    then carries a ``grad_fn``; ``deltas=`` is supported.  The forward then keeps
+    the un-normalised combination and normalises out of place.
     """
     graph = as_graph(adj_matrix)
     k = int(k)
-    coeffs = heat_coefficients(k, s)
+    s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
+    coeffs = heat_coefficients(k, s_vals)
     degree_vectors = None
     x0 = graph.x0 if X0 is None else torch.as_tensor(X0)
+    grad = _needs_grad(x0, s)
     y0 = None
     in_kernel = False
     if deltas is not None and len(deltas[0]) > 0:
-        in_kernel = _patches_in_kernel(graph, 1 if x0.dim() == 1 else int(x0.shape[1]), k, _use_sell)
+        # the backward needs the patched degree vectors, so a differentiable pass patches them itself
+        in_kernel = not grad and _patches_in_kernel(graph, 1 if x0.dim() == 1 else int(x0.shape[1]), k, _use_sell)
         if not in_kernel:
             # degree vectors of the flipped graph: only the touched entries of persistent scratch copies are
             # written, and put back once the pass is queued (no copies of the N-vectors per perturbation)
@@ -293,6 +479,15 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
     op_scale = 2.0 / float(lambda_max)
     default_signal = X0 is None and (deltas is None or in_kernel)
     try:
+        if grad:
+            if degree_vectors is not None:       # the scratch vectors are restored below, the backward runs later
+                degree_vectors = tuple(v.clone() for v in degree_vectors)
+            spec = _PassSpec(graph, graph.adjoint, k, coeffs, op_scale, -1.0, return_parts, deltas, degree_vectors,
+                             _use_sell, default_signal, y0)
+            comb, t_all = _differentiable_pass(spec, x0, s)
+            feats = _L1Normalize.apply(comb) if normalize else comb
+            feats = feats.reshape(graph.n, -1)
+            return WaveletResult(feats, [t_all[i] for i in range(k + 1)], comb) if return_parts else feats
         return _wavelet_pass(graph, x0, k, coeffs, op_scale, normalize, return_parts, deltas, degree_vectors,
                              _order_events, _use_sell, default_signal, y0, in_kernel)
     finally:
@@ -341,6 +536,8 @@ class WATS(nn.Module):
     keep the reference's torch ops).
     ``_features_override`` exists for parity tests only: it injects a feature
     matrix computed elsewhere so two instances differ in nothing else.
+    The wavelet features are an input here, computed without gradients
+    (forward-only, as in the reference).
     """
 
     def __init__(self, base_model, features, labels, adj, val_mask, *, k: int = 3, s=0.8,
@@ -475,7 +672,7 @@ class WaveletSession:
     the per-launch host cost in both cases.  ``target`` is a :class:`CsrGraph`
     or a ``sharded.ShardedWavelet``; ``X0`` (optional) is copied into a static
     buffer before each replay.  The returned tensor is a static buffer that the
-    next call overwrites.
+    next call overwrites.  Forward-only: a replay records no autograd graph.
     """
 
     def __init__(self, target, k=3, s=0.8, *, f: int = 1, lambda_max: float = 2.0, normalize: bool = True,

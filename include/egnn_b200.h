@@ -243,6 +243,59 @@ size_t egnn_row_order_ws_bytes(int64_t n);
 int egnn_row_order(const int32_t* rowptr, int64_t n, int32_t* order_out,
                    void* workspace, size_t workspace_bytes, egnn_stream_t stream);
 
+/* ---- backward of the wavelet pass ------------------------------------------
+ * With M = op_scale * L_sym + op_shift * I and C_s = sum_k alpha[s,k] T_k(M) X
+ * (egnn_cheb_wavelet), the gradient of a loss w.r.t. X given upstream
+ * gradients cbar = dLoss/dC [n, n_scales, f] and tbar_or_null = dLoss/dT_k
+ * [K+1, n, f] is the Clenshaw sum
+ *   v_k = sum_s alpha[s,k] cbar[:, s, :] + tbar_k,
+ *   b_K = v_K,  b_k = v_k + 2 M^T b_{k+1} - b_{k+2} (k = K-1..1),
+ *   xbar = v_0 + M^T b_1 - b_2,
+ * K applications of M^T, each one launch of the adjoint instantiation of the
+ * forward's order kernel (f >= 8: the wide kernel; every f < 8 the generic CSR
+ * kernel, there is no SELL path).  coeffs_host is the forward's [S, K+1].
+ * rowptr_t/colidx_t/vals_t: the TRANSPOSED adjacency (egnn_csr_transpose; the
+ * graph's own CSR when it is symmetric) with the FORWARD's dinv / iso (scipy
+ * normalises by column sums on both sides).  delta_*: the forward's flips with
+ * rows and columns swapped (dinv / iso already patched, as for the forward).
+ * workspace: egnn_cheb_workspace_bytes(n, f).  app_events_host: NULL or 2*K
+ * events recorded around application j = 1..K (events 2(j-1), 2(j-1)+1).
+ * row_order_or_null: egnn_row_order of the transposed CSR (f >= 8).          */
+int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t,
+                      const float* vals_t_or_null, const float* dinv, const uint8_t* iso,
+                      int64_t n, int64_t nnz, int32_t f, int32_t k, int32_t n_scales,
+                      const float* coeffs_host, float op_scale, float op_shift,
+                      const float* cbar, const float* tbar_or_null, float* xbar,
+                      const int32_t* delta_row_host, const int32_t* delta_col_host,
+                      const float* delta_val_host, int32_t n_delta,
+                      void* workspace, size_t workspace_bytes, egnn_stream_t stream,
+                      void* const* app_events_host, const int32_t* row_order_or_null);
+
+/* Row L1 normalisation out of place, h = c / (sum_f |c| + 1e-8) per row of f
+ * values (n_vec rows), and its backward: cbar_out = cbar_in + (hbar -
+ * sign(c) <hbar, h>) / r with r recomputed from c and sign(0) = 0.
+ * cbar_in_or_null may alias cbar_out; NULL adds to zero.                     */
+int egnn_l1_normalize(const float* c, float* h, int64_t n_vec, int32_t f, egnn_stream_t stream);
+int egnn_l1_normalize_backward(const float* c, const float* hbar, const float* cbar_in_or_null,
+                               float* cbar_out, int64_t n_vec, int32_t f, egnn_stream_t stream);
+
+/* Gradient w.r.t. the heat coefficients: grad_out[s*(K+1)+k] = <cbar[:, s, :],
+ * T_k> (device float64 [S, K+1]) from cbar [n, S, f] and the forward's orders
+ * t_all [K+1, n, f].  Summed in float64 in a fixed order: deterministic.      */
+size_t egnn_cheb_coeff_grad_ws_bytes(int32_t k, int32_t n_scales);
+int egnn_cheb_coeff_grad(const float* cbar, const float* t_all, int64_t n, int32_t f, int32_t k,
+                         int32_t n_scales, double* grad_out, void* workspace,
+                         size_t workspace_bytes, egnn_stream_t stream);
+
+/* CSR transpose: rowptr_t [n+1], colidx_t / vals_t [nnz] (vals_t NULL iff
+ * vals NULL).  A stable radix sort by column: every row of the transpose comes
+ * out sorted, and the result does not depend on the launch (deterministic).  */
+size_t egnn_csr_transpose_ws_bytes(int64_t n, int64_t nnz);
+int egnn_csr_transpose(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                       int64_t n, int64_t nnz, int32_t* rowptr_t, int32_t* colidx_t,
+                       float* vals_t_or_null, void* workspace, size_t workspace_bytes,
+                       egnn_stream_t stream);
+
 /* ---- fused temperature head (SURVEY 8f.2) ----------------------------------
  * Inference form of WATS.forward, calibration/WATS.py:122-130:
  *   t_i = w2 . relu(W1 feats_i + b1) + b2;  T_i = log(exp(t_i) + 1.1);
