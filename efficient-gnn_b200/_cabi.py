@@ -136,6 +136,16 @@ def ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def vec_ready(t):
+    """``t`` as a contiguous float32 tensor whose data starts on a 16-byte boundary, copied only when
+    needed.  The kernels read and write rows of ``F % 4 == 0`` values with 16-byte vector accesses;
+    ``.contiguous()`` alone keeps a view at an odd element offset (``buf[1:1 + n * f].view(n, f)``,
+    a slice of a ``torch.cat``), which the library refuses."""
+    import torch
+    t = t.to(torch.float32).contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 def host_array(ctype, values):
     arr = (ctype * max(1, len(values)))(*values)
     return arr

@@ -41,6 +41,12 @@ static int pow2_ceil_log2(int64_t x) {
 
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Caller arrays of row stride f are read and written with 16-byte vector accesses when
+// f % 4 == 0 (FeatVec<4>, load_user4<true>), so their base addresses must be 16-byte aligned then.
+static inline bool vec_aligned(const void* p, int32_t f) {
+    return f % 4 != 0 || p == nullptr || ((uintptr_t)p & 15) == 0;
+}
+
 static int fill_delta(DeltaList& d, const int32_t* r, const int32_t* c, const float* v, int32_t n) {
     EGNN_REQUIRE(n >= 0 && n <= EGNN_MAX_DELTA, "n_delta out of range");
     EGNN_REQUIRE(n == 0 || (r && c && v), "delta arrays missing");
@@ -575,6 +581,8 @@ int egnn_cheb_wavelet(const int32_t* rowptr, const int32_t* colidx, const float*
     EGNN_REQUIRE(f >= 1, "f must be >= 1");
     EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "k out of range");
     EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
+    EGNN_REQUIRE(vec_aligned(x0, f) && vec_aligned(out, f) && vec_aligned(t_all_or_null, f),
+                 "x0, out and t_all must be 16-byte aligned when f % 4 == 0");
     if (n == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
 
@@ -831,6 +839,8 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
     EGNN_REQUIRE(f >= 1, "f must be >= 1");
     EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "k out of range");
     EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
+    EGNN_REQUIRE(vec_aligned(cbar, f) && vec_aligned(tbar_or_null, f) && vec_aligned(xbar, f),
+                 "cbar, tbar and xbar must be 16-byte aligned when f % 4 == 0");
     if (n == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
     OrderParams p{};

@@ -560,7 +560,7 @@ class ShardedWavelet:
             x0 = x0.reshape(-1, 1)
         if x0.shape[0] != self.rows:
             raise ValueError(f"X0_local has {x0.shape[0]} rows, this rank owns {self.rows}")
-        x0 = x0.to(device=dev, dtype=torch.float32).contiguous()
+        x0 = _cabi.vec_ready(x0.to(device=dev))
         f = int(x0.shape[1])
         rp = self.part.rows_per
         op_scale, op_shift = 2.0 / float(lambda_max), -1.0

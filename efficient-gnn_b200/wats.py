@@ -78,7 +78,7 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
         x0 = x0.unsqueeze(1)
     if x0.shape[0] != n:
         raise ValueError(f"X0 has {x0.shape[0]} rows, graph has {n} nodes")
-    x0 = x0.detach().to(device=dev, dtype=torch.float32).contiguous()
+    x0 = _cabi.vec_ready(x0.detach().to(device=dev))
     f = int(x0.shape[1])
     n_scales = int(coeffs.shape[0])
     if coeffs.shape[1] != k + 1:
@@ -203,9 +203,9 @@ class _WaveletPass(torch.autograd.Function):
         g = spec.graph
         n_scales = int(spec.coeffs.shape[0])
         f = 1 if len(ctx.x_shape) == 1 else int(ctx.x_shape[1])
-        cbar = (g_comb.to(torch.float32).contiguous() if g_comb is not None else
+        cbar = (_cabi.vec_ready(g_comb) if g_comb is not None else
                 torch.zeros((g.n, n_scales, f), dtype=torch.float32, device=g.device))
-        tbar = g_orders.to(torch.float32).contiguous() if (g_orders is not None and g_orders.numel()) else None
+        tbar = _cabi.vec_ready(g_orders) if (g_orders is not None and g_orders.numel()) else None
         x_grad = s_grad = None
         if ctx.needs_input_grad[0]:
             dv = spec.degree_vectors if spec.degree_vectors is not None else (g.dinv, g.iso)
@@ -238,7 +238,7 @@ class _L1Normalize(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, g_h):
         (comb,) = ctx.saved_tensors
-        g_h = g_h.to(torch.float32).contiguous()
+        g_h = _cabi.vec_ready(g_h)
         cbar = torch.empty_like(comb)
         n_vec = comb.shape[0] * comb.shape[1]
         with torch.cuda.device(comb.device):

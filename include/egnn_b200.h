@@ -197,6 +197,9 @@ int egnn_sell_fill(const int32_t* rowptr, const int32_t* colidx, int64_t n, int6
  *                 already describe the perturbed graph (egnn_patch_degrees).
  *                 Host pointers, n_delta <= EGNN_MAX_DELTA.
  * workspace: egnn_cheb_workspace_bytes(n, f) bytes, 256-byte aligned.
+ * When f % 4 == 0 the kernels access x0, out and t_all_or_null with 16-byte
+ * vector loads and stores: those must then be 16-byte aligned, else
+ * EGNN_ERR_INVALID_ARG (nothing is launched).
  * order_events_host: NULL, or 2*K cudaEvent_t handles; events 2(k-1) and
  * 2(k-1)+1 are recorded on `stream` around order k's kernel (per-kernel
  * timing for the roofline report; no effect on results).  With a SELL plan the
@@ -258,6 +261,8 @@ int egnn_row_order(const int32_t* rowptr, int64_t n, int32_t* order_out,
  * graph's own CSR when it is symmetric) with the FORWARD's dinv / iso (scipy
  * normalises by column sums on both sides).  delta_*: the forward's flips with
  * rows and columns swapped (dinv / iso already patched, as for the forward).
+ * cbar, tbar_or_null and xbar must be 16-byte aligned when f % 4 == 0 (as
+ * x0 / out / t_all of egnn_cheb_wavelet), else EGNN_ERR_INVALID_ARG.
  * workspace: egnn_cheb_workspace_bytes(n, f).  app_events_host: NULL or 2*K
  * events recorded around application j = 1..K (events 2(j-1), 2(j-1)+1).
  * row_order_or_null: egnn_row_order of the transposed CSR (f >= 8).          */

@@ -43,6 +43,38 @@ def test_invalid_arguments_return_status_not_crash():
     assert lib.egnn_cheb_workspace_bytes(1000, 64) >= 2 * 4 * 64000
 
 
+def test_misaligned_vector_buffers_are_refused_before_any_launch():
+    """At F % 4 == 0 the kernels access the caller's signal, outputs and upstream gradients with
+    16-byte vector loads: a contiguous view at an odd element offset would fault the GPU.  The
+    entry points refuse such pointers before the workspace check, so a NULL workspace still
+    yields the alignment error and nothing runs (the pointers here are never dereferenced)."""
+    lib = _cabi.load()
+    base = 1 << 20
+    ok = lambda i: base + 4096 * i                        # noqa: E731  16-byte aligned fakes
+    bad = lambda i: base + 4096 * i + 4                   # noqa: E731  one float past a boundary
+    coeffs = np.ones(8, dtype=np.float32)
+    cptr = coeffs.ctypes.data
+    for x0, out, t_all in ((bad(5), ok(6), None), (ok(5), bad(6), None), (ok(5), ok(6), bad(7))):
+        rc = lib.egnn_cheb_wavelet(ok(1), ok(2), None, ok(3), ok(4), x0, 4, 4, 4, 3, 1, cptr, 1.0, -1.0,
+                                   out, t_all, 0, None, None, None, 0, None, 0, None, None, None, None, None, 0,
+                                   None, None, 0)
+        assert rc == -1, rc
+        assert b"aligned" in lib.egnn_last_error()
+    for cbar, tbar, xbar in ((bad(5), None, ok(6)), (ok(5), bad(7), ok(6)), (ok(5), ok(7), bad(6))):
+        rc = lib.egnn_cheb_adjoint(ok(1), ok(2), None, ok(3), ok(4), 4, 4, 8, 3, 1, cptr, 1.0, -1.0,
+                                   cbar, tbar, xbar, None, None, None, 0, None, 0, None, None, None)
+        assert rc == -1, rc
+        assert b"aligned" in lib.egnn_last_error()
+    # F % 4 != 0 reads per element: the same offsets pass the check and reach the workspace check
+    rc = lib.egnn_cheb_adjoint(ok(1), ok(2), None, ok(3), ok(4), 4, 4, 3, 3, 1, cptr, 1.0, -1.0,
+                               bad(5), bad(7), bad(6), None, None, None, 0, None, 0, None, None, None)
+    assert rc == -4 and b"workspace" in lib.egnn_last_error()
+    rc = lib.egnn_cheb_wavelet(ok(1), ok(2), None, ok(3), ok(4), bad(5), 4, 4, 5, 3, 1, cptr, 1.0, -1.0,
+                               bad(6), None, 0, None, None, None, 0, None, 0, None, None, None, None, None, 0,
+                               None, None, 0)
+    assert rc == -4 and b"workspace" in lib.egnn_last_error()
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-device failure mode")
 def test_no_cpu_fallback():
     with pytest.raises(egnn.EgnnError):

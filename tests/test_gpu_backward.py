@@ -3,13 +3,14 @@
 * Parity of the signal's gradient with ``tests/vjp_reference.wavelet_vjp`` (float64,
   explicit transposed operator) on the golden graphs, with random upstream
   gradients on the features, the combination and the orders: norm-wise
-  ``||Xbar_gpu - Xbar_ref||_inf / ||Xbar_ref||_inf <= 1e-5`` (the forward's bar),
-  the element-wise ratio printed beside it.  The scales' gradient against the
+  ``||Xbar_gpu - Xbar_ref||_inf / ||Xbar_ref||_inf <= 1e-5`` and element-wise ratio
+  <= 1 at the 5e-2 floor (the forward's bars), the ratio at the 1e-3 floor printed beside them.  The scales' gradient against the
   oracle at the same bar; ``chebyshev_polynomials``, ``L @ x`` and the explicit
   scipy operator.
 * Flips: the gradient on ``deltas=`` equals the gradient on the rebuilt graph.
-* Full size (where the oracle would take minutes): the adjoint identity
-  ``<G, f(X)> = <f*(G), X>`` on the un-normalised output, dots in float64.
+* Full size: the signal's gradient element-wise on chosen columns against the float64
+  transposed operator, and the scales' gradient against float64 sums of the pass's own orders.
+  Every adjoint instantiation at small size: test_gpu_adjoint_matrix.py.
 * Determinism and no change of the forward when nothing needs a gradient.
 """
 import numpy as np
@@ -30,7 +31,8 @@ TOL = 1e-5
 # F = 1 golden signals are checked without the normalisation: there H = sign(C) and its derivative,
 # 1e-8 / r^2, is below the float32 rounding of 1 - |C| / r (it vanishes almost everywhere).
 PARITY = [(name, n_scales, normalize)
-          for name in ["cora_noloop", "cora_loops", "directed_weighted", "cora_k6_s04", "cora_wide8", "small_wide130"]
+          for name in ["cora_noloop", "cora_loops", "directed_weighted", "cora_k0", "cora_k1", "cora_k6_s04", "cora_wide8",
+                       "small_wide130"]
           for n_scales in (1, 3) for normalize in (False, True)
           if normalize is False or name in ("cora_wide8", "small_wide130")]
 
@@ -42,8 +44,10 @@ def scales_for(case, n_scales):
 def report(tag, got, ref):
     err = rel_max_err(got, ref)
     ratio = elementwise_ratio(got, ref, TOL)
-    print(f"\n[{tag}] rel {err:.2e}, elementwise_ratio x{ratio:.2f}")
+    ratio3 = elementwise_ratio(got, ref, TOL, floor=1e-3)
+    print(f"\n[{tag}] rel {err:.2e}, elementwise_ratio x{ratio:.2f} (floor 5e-2), x{ratio3:.2f} (floor 1e-3)")
     assert err <= TOL, f"{tag}: rel max err {err:.3e}"
+    assert ratio <= 1.0, f"{tag}: elementwise ratio {ratio:.2f} at the 5e-2 floor"
     return err
 
 
@@ -174,30 +178,86 @@ def directed_half(rp, ci, n, seed):
     return rp2.to(torch.int32), ci[keep].contiguous()
 
 
+def full_graph(shape, directed):
+    """Device graph of a full-size shape: binary symmetric with self loops; directed=True keeps a
+    seeded half of the entries, "weighted" also gives them seeded weights in [0.5, 2)."""
+    rp, ci, n = synth.synth_csr(shape, self_loops=True, device="cuda")
+    vals = None
+    if directed:
+        rp, ci = directed_half(rp, ci, n, seed=2)
+    if directed == "weighted":
+        gen = torch.Generator(device="cuda").manual_seed(4)
+        vals = 0.5 + 1.5 * torch.rand(ci.numel(), generator=gen, device="cuda")
+    return egnn.CsrGraph(rp, ci, vals, n)
+
+
+_MT = {}
+
+
+@pytest.fixture(scope="module")
+def transposed_operator():
+    """``rescaled_laplacian(adj).T`` (float64 CSR) of a full-size graph, built once per graph."""
+    def get(shape, directed, g):
+        key = (shape, directed)
+        if key not in _MT:
+            data = np.ones(g.nnz, np.float32) if g.vals is None else g.vals.cpu().numpy()
+            adj = sp.csr_matrix((data, g.colidx.cpu().numpy(), g.rowptr.cpu().numpy()), shape=(g.n, g.n))
+            _MT[key] = orc.rescaled_laplacian(adj).T.tocsr()
+        return _MT[key]
+    yield get
+    _MT.clear()
+
+
+def check_columns(f):
+    """Columns on both sides of the 4-column groups and of the 128-column feature tiles."""
+    return sorted(c for c in {0, 1, 3, 4, 31, 32, 63, 64, 127, f - 5, f - 4, f - 1} if 0 <= c < f)
+
+
 FULL = [("arxiv", 128, [0.3, 0.8, 1.6, 2.4], False), ("reddit", 64, [0.8], False),
-        ("reddit", 1, [0.8, 1.6], False), ("arxiv", 16, [0.8, 1.6], True)]
+        ("reddit", 1, [0.8, 1.6], False), ("arxiv", 16, [0.8, 1.6], True), ("arxiv", 37, [0.8, 1.3], "weighted")]
 
 
 @pytest.mark.parametrize("shape,f,scales,directed", FULL)
-def test_adjoint_identity_full_size(shape, f, scales, directed):
-    rp, ci, n = synth.synth_csr(shape, self_loops=True, device="cuda")
-    if directed:
-        rp, ci = directed_half(rp, ci, n, seed=2)
-    g = egnn.CsrGraph(rp, ci, None, n)
+def test_adjoint_identity_full_size(shape, f, scales, directed, transposed_operator):
+    """Full size, element-wise on chosen columns: with normalize=False the columns are independent,
+    so ``Xbar[:, cols]`` is compared with ``sum_i T_i(M^T) v_i`` on those columns (scipy, float64);
+    F = 1 on the Reddit shape checks every row, hub rows included.  The scales' gradient is compared
+    with ``-sum_k k alpha_jk <Cbar_j, T_k>`` summed in float64 from the pass's own orders (checked
+    against the oracle by test_gpu_full_size.py): that isolates the coefficient-gradient reduction."""
+    g = full_graph(shape, directed)
+    n = g.n
     if directed:
         assert g.adjoint() is not g
     gen = torch.Generator(device="cuda").manual_seed(7)
     x = torch.randn(n, f, device="cuda", generator=gen).requires_grad_()
+    s = torch.tensor(scales, dtype=torch.float64, requires_grad=True)
     G = torch.randn(n, len(scales) * f, device="cuda", generator=gen)
-    out = egnn.graph_wavelet_features(g, k=3, s=scales, X0=x, normalize=False)
-    (G * out).sum().backward()
-    lhs = (G.double() * out.detach().double()).sum().item()
-    rhs = (x.grad.double() * x.detach().double()).sum().item()
-    scale = (G.double().abs() * out.detach().double().abs()).sum().item() + \
-        (x.grad.double().abs() * x.detach().double().abs()).sum().item()
-    print(f"\n[{shape} F={f} S={len(scales)} directed={directed}] <G, f(X)> = {lhs:.6e}, <f*(G), X> = {rhs:.6e}, "
-          f"rel {abs(lhs - rhs) / scale:.2e}")
-    assert abs(lhs - rhs) <= 1e-5 * scale
+    res = egnn.graph_wavelet_features(g, k=3, s=s, X0=x, normalize=False, return_parts=True)
+    (G * res.features).sum().backward()
+    k, n_scales = 3, len(scales)
+    alpha = egnn.heat_coefficients(k, scales)
+    cbar = G.reshape(n, n_scales, f)
+    # scale gradient: float64 sums of the pass's own float32 orders
+    terms = torch.stack([torch.stack([(cbar[:, j].double() * res.orders[i].detach().double()).sum()
+                                      for i in range(k + 1)]) for j in range(n_scales)]).cpu().numpy()
+    size = torch.stack([torch.stack([(cbar[:, j].double().abs() * res.orders[i].detach().double().abs()).sum()
+                                     for i in range(k + 1)]) for j in range(n_scales)]).cpu().numpy()
+    kk = np.arange(k + 1)
+    s_ref = -(kk * alpha * terms).sum(axis=1)
+    s_size = (kk * alpha * size).sum(axis=1)
+    s_rel = float((np.abs(s.grad.numpy() - s_ref) / s_size).max())
+    tag = f"{shape} F={f} S={n_scales} directed={directed}"
+    print(f"\n[{tag} sbar] rel to sum|terms| {s_rel:.2e}")
+    assert s_rel <= 1e-10
+    # signal gradient on chosen columns
+    mt = transposed_operator(shape, directed, g)
+    cols = check_columns(f)
+    cb = cbar[:, :, cols].double().cpu().numpy()
+    want = np.zeros((n, len(cols)))
+    for i in range(k + 1):
+        v = np.einsum("s,nsc->nc", alpha[:, i], cb)
+        want += orc.chebyshev_orders(mt, i, v)[i]
+    report(f"{tag} Xbar[:, {cols}]", x.grad[:, cols].cpu().numpy(), want)
 
 
 # ---- determinism and the forward ----------------------------------------------------------------

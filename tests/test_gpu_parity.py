@@ -144,7 +144,7 @@ def test_multi_scale_single_pass():
     assert torch.equal(feats[:, 1:2], one)
 
 
-@pytest.mark.parametrize("f", [1, 2, 3, 4, 8, 20, 33, 64, 128, 130, 260])
+@pytest.mark.parametrize("f", [1, 2, 3, 4, 5, 6, 7, 8, 20, 33, 64, 128, 130, 260])
 def test_feature_widths(f):
     c = load_case("cora_noloop")
     rng = np.random.default_rng(f)
@@ -156,9 +156,10 @@ def test_feature_widths(f):
     np.testing.assert_allclose(fused.cpu().numpy(), np.concatenate(p["H"], axis=1), rtol=0, atol=3e-5)
 
 
-@pytest.mark.parametrize("f", [8, 18, 64, 131])
+@pytest.mark.parametrize("f", [5, 7, 8, 18, 64, 131])
 def test_weighted_directed_graph_wide_signals(f):
-    """Non-symmetric weighted adjacency (in-degree normalisation, stored values) through the wide kernel."""
+    """Non-symmetric weighted adjacency (in-degree normalisation, stored values) through the wide kernel
+    (F >= 8) and the generic kernel without pre-scaled operands (F = 5, 7)."""
     c = load_case("directed_weighted")
     x0 = np.random.default_rng(100 + f).standard_normal((c["n"], f)).astype(np.float32)
     res = egnn.graph_wavelet_features(c["adj"], k=3, s=[0.8, 0.4], X0=torch.from_numpy(x0), return_parts=True)
