@@ -13,7 +13,7 @@ import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("EGNN_LIB_PATH") or os.path.join(_HERE, "lib", "libegnn_b200.so")   # override: tuning builds
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 # every symbol include/egnn_b200.h declares: name -> (restype, argtypes)
 _P, _I32, _I64, _F32, _SZ = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -44,6 +44,13 @@ SYMBOLS = {
                                     _P, _P, _I32, _P, _P, _P, _I32, _P, _SZ, _P, _P, _P, _P, _P, _I32, _P, _P, _I32]),
     "egnn_cheb_adjoint": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I64, _I32, _I32, _I32, _P, _F32, _F32,
                                     _P, _P, _P, _P, _P, _P, _I32, _P, _SZ, _P, _P, _P]),
+    "egnn_cheb_adjoint_all": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I64, _I32, _I32, _I32, _P, _F32, _F32,
+                                        _P, _P, _P, _P, _P, _P, _I32, _P, _SZ, _P, _P, _P, _P]),
+    "egnn_adj_grad_degree_ws_bytes": (_SZ, [_I64]),
+    "egnn_adj_grad_degree": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I32, _I32, _F32, _P, _P, _P, _P,
+                                       _P, _P, _P, _SZ, _P]),
+    "egnn_adj_grad_pairs": (C.c_int, [_P, _P, _I64, _P, _P, _P, _P, _P, _I64, _I32, _I32, _F32, _P, _P]),
+    "egnn_adj_grad_dense": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I32, _I32, _F32, _P, _I64, _P]),
     "egnn_l1_normalize": (C.c_int, [_P, _P, _I64, _I32, _P]),
     "egnn_l1_normalize_backward": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P]),
     "egnn_cheb_coeff_grad_ws_bytes": (_SZ, [_I32, _I32]),

@@ -13,6 +13,7 @@
 #include "prep.cuh"
 #include "sell.cuh"
 #include "sell_step.cuh"
+#include "structure_grad.cuh"
 #include "surrogate.cuh"
 #include "blocked.cuh"
 #include "wide.cuh"
@@ -347,7 +348,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 7; }
+int egnn_abi_version(void) { return 8; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -824,23 +825,27 @@ int egnn_cheb_wavelet(const int32_t* rowptr, const int32_t* colidx, const float*
     return EGNN_OK;
 }
 
+}  // extern "C"
+
 // ---- backward of the wavelet pass (csrc/adjoint.cuh) ------------------------------------------------
-int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
-                      const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
-                      int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
-                      const float* cbar, const float* tbar_or_null, float* xbar,
-                      const int32_t* delta_row_host, const int32_t* delta_col_host,
-                      const float* delta_val_host, int32_t n_delta, void* workspace,
-                      size_t workspace_bytes, egnn_stream_t stream, void* const* app_events_host,
-                      const int32_t* row_order_or_null) {
+// b_all_or_null: [K+1, n, f] receives Xbar (slab 0) and every Clenshaw vector b_m (slab m); the
+// generic path then keeps its b vectors there instead of the workspace ping-pong slabs.
+static int cheb_adjoint_impl(const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                             const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
+                             int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                             const float* cbar, const float* tbar_or_null, float* xbar,
+                             const int32_t* delta_row_host, const int32_t* delta_col_host,
+                             const float* delta_val_host, int32_t n_delta, void* workspace,
+                             size_t workspace_bytes, egnn_stream_t stream, void* const* app_events_host,
+                             const int32_t* row_order_or_null, float* b_all_or_null) {
     EGNN_REQUIRE(rowptr_t && dinv && iso && cbar && xbar && coeffs_host, "null pointer");
     EGNN_REQUIRE(nnz == 0 || colidx_t, "null colidx");
     EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
     EGNN_REQUIRE(f >= 1, "f must be >= 1");
     EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "k out of range");
     EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
-    EGNN_REQUIRE(vec_aligned(cbar, f) && vec_aligned(tbar_or_null, f) && vec_aligned(xbar, f),
-                 "cbar, tbar and xbar must be 16-byte aligned when f % 4 == 0");
+    EGNN_REQUIRE(vec_aligned(cbar, f) && vec_aligned(tbar_or_null, f) && vec_aligned(xbar, f) &&
+                 vec_aligned(b_all_or_null, f), "cbar, tbar, xbar and b_all must be 16-byte aligned when f % 4 == 0");
     if (n == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
     OrderParams p{};
@@ -856,11 +861,17 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
         return c;
     };
     auto tbar_at = [&](int m) { return tbar_or_null ? tbar_or_null + (size_t)m * slab_elems : nullptr; };
+    auto b_at = [&](int m) { return b_all_or_null ? b_all_or_null + (size_t)m * slab_elems : nullptr; };
+    auto copy_xbar = [&]() {
+        return b_all_or_null ? check_cuda(cudaMemcpyAsync(b_all_or_null, xbar, sizeof(float) * slab_elems,
+                                                          cudaMemcpyDeviceToDevice, st), "copy Xbar")
+                             : EGNN_OK;
+    };
     if (k == 0) {
         adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
             cbar, tbar_at(0), dinv, xbar, nullptr, n, f, n_scales, f, coef_row(0));
         EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
-        return EGNN_OK;
+        return copy_xbar();
     }
     const size_t need = egnn_cheb_workspace_bytes(n, f);
     if (workspace == nullptr || workspace_bytes < need) {
@@ -878,7 +889,7 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
         rc = check_cuda(cudaMemsetAsync(counters, 0, sizeof(unsigned) * (size_t)k * (size_t)rcfg.grid_y, st), "memset row counters");
         if (rc) return rc;
         adjoint_prologue_kernel<<<grid_for((int64_t)n * ldy, 256), 256, 0, st>>>(
-            cbar, tbar_at(k), dinv, nullptr, yb[0], n, f, n_scales, ldy, coef_row(k));
+            cbar, tbar_at(k), dinv, b_at(k), yb[0], n, f, n_scales, ldy, coef_row(k));
         EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
         WideParams wp{};
         wp.delta = p.delta;
@@ -895,7 +906,7 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
             wp.ysrc = yb[(j - 1) & 1];
             wp.y2_own = j == 1 ? nullptr : yb[j & 1];
             wp.y_out = m == 0 ? nullptr : yb[j & 1];             // in place over dinv (.) b_{m+2} (own row only)
-            wp.tk_out = m == 0 ? xbar : nullptr;
+            wp.tk_out = m == 0 ? xbar : b_at(m);
             wp.tbar = tbar_at(m);
             wp.c_adj = m == 0 ? 1.f : 2.f;
             for (int s = 0; s < n_scales; ++s) wp.c_k[s] = coeffs_host[s * (k + 1) + m];
@@ -910,14 +921,16 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
                 if (rc) return rc;
             }
         }
-        return EGNN_OK;
+        return copy_xbar();
     }
     const OrderConfig cfg = choose_config(n, nnz, f);
     const size_t slab = align_up(sizeof(float) * slab_elems, 256);
     float* tbuf[2] = {(float*)ws, (float*)(ws + slab)};
     float* ybuf[2] = {(float*)(ws + 2 * slab), (float*)(ws + 3 * slab)};
+    // b_m of application j: tbuf[j & 1] (in place over b_{m+2}), or slab m of b_all
+    auto b_vec = [&](int j) { return b_all_or_null ? b_at(k - j) : tbuf[j & 1]; };
     adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
-        cbar, tbar_at(k), dinv, tbuf[0], cfg.prescaled ? ybuf[0] : nullptr, n, f, n_scales, f, coef_row(k));
+        cbar, tbar_at(k), dinv, b_vec(0), cfg.prescaled ? ybuf[0] : nullptr, n, f, n_scales, f, coef_row(k));
     EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
     p.rowptr = rowptr_t; p.colidx = colidx_t; p.vals = vals_t_or_null; p.dinv = dinv; p.iso = iso;
     p.out = nullptr; p.acc_ws = nullptr; p.n_rows = n; p.row0 = 0; p.F = f; p.S = n_scales;
@@ -925,10 +938,10 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
     p.first = 0; p.normalize = 0; p.cbar = cbar;
     for (int j = 1; j <= k; ++j) {
         const int m = k - j;
-        p.tprev_own = tbuf[(j - 1) & 1];
-        p.tprev2_own = j == 1 ? nullptr : tbuf[j & 1];
-        p.tk_own = m == 0 ? xbar : tbuf[j & 1];                  // in place over b_{m+2}
-        p.gsrc = cfg.prescaled ? ybuf[(j - 1) & 1] : tbuf[(j - 1) & 1];
+        p.tprev_own = b_vec(j - 1);
+        p.tprev2_own = j == 1 ? nullptr : b_vec(j - 2);
+        p.tk_own = m == 0 ? xbar : b_vec(j);
+        p.gsrc = cfg.prescaled ? ybuf[(j - 1) & 1] : b_vec(j - 1);
         p.y_own = (cfg.prescaled && m > 0) ? ybuf[j & 1] : nullptr;
         p.tbar = tbar_at(m);
         p.c_adj = m == 0 ? 1.f : 2.f;
@@ -944,7 +957,38 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const fl
             if (rc) return rc;
         }
     }
-    return EGNN_OK;
+    return copy_xbar();
+}
+
+extern "C" {
+
+int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                      const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
+                      int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                      const float* cbar, const float* tbar_or_null, float* xbar,
+                      const int32_t* delta_row_host, const int32_t* delta_col_host,
+                      const float* delta_val_host, int32_t n_delta, void* workspace,
+                      size_t workspace_bytes, egnn_stream_t stream, void* const* app_events_host,
+                      const int32_t* row_order_or_null) {
+    return cheb_adjoint_impl(rowptr_t, colidx_t, vals_t_or_null, dinv, iso, n, nnz, f, k, n_scales, coeffs_host,
+                             op_scale, op_shift, cbar, tbar_or_null, xbar, delta_row_host, delta_col_host,
+                             delta_val_host, n_delta, workspace, workspace_bytes, stream, app_events_host,
+                             row_order_or_null, nullptr);
+}
+
+int egnn_cheb_adjoint_all(const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                          const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
+                          int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                          const float* cbar, const float* tbar_or_null, float* xbar,
+                          const int32_t* delta_row_host, const int32_t* delta_col_host,
+                          const float* delta_val_host, int32_t n_delta, void* workspace,
+                          size_t workspace_bytes, egnn_stream_t stream, void* const* app_events_host,
+                          const int32_t* row_order_or_null, float* b_all) {
+    EGNN_REQUIRE(b_all, "null b_all");
+    return cheb_adjoint_impl(rowptr_t, colidx_t, vals_t_or_null, dinv, iso, n, nnz, f, k, n_scales, coeffs_host,
+                             op_scale, op_shift, cbar, tbar_or_null, xbar, delta_row_host, delta_col_host,
+                             delta_val_host, n_delta, workspace, workspace_bytes, stream, app_events_host,
+                             row_order_or_null, b_all);
 }
 
 int egnn_l1_normalize(const float* c, float* h, int64_t n_vec, int32_t f, egnn_stream_t stream) {
@@ -1044,6 +1088,84 @@ int egnn_csr_transpose(const int32_t* rowptr, const int32_t* colidx, const float
     }
     return check_cuda(cub::DeviceScan::ExclusiveSum(cub_temp, cub_bytes, counts, rowptr_t, (int)(n + 1), st),
                       "scan column counts");
+}
+
+// ---- gradient w.r.t. the adjacency (csrc/structure_grad.cuh) ---------------------------------------
+// lanes across the K*F products of one entry: the next power of two, at most a warp
+static int stack_fl_log2(int32_t f, int32_t k) {
+    const int64_t kf = (int64_t)f * k;
+    const int l = pow2_ceil_log2(kf > 1 ? kf : 1);
+    return l > 5 ? 5 : l;
+}
+
+size_t egnn_adj_grad_degree_ws_bytes(int64_t n) {
+    return 2 * align_up(sizeof(double) * (size_t)(n > 0 ? n : 1), 256) + 256;
+}
+
+int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                         const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                         const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
+                         float op_scale, const float* lam, const float* t, const float* xbar_or_null,
+                         const float* rowsum_or_null, float* gw, float* grho, void* workspace,
+                         size_t workspace_bytes, egnn_stream_t stream) {
+    EGNN_REQUIRE(rowptr && rowptr_t && dinv && iso && gw && grho, "null pointer");
+    EGNN_REQUIRE(nnz == 0 || (colidx && colidx_t), "null colidx");
+    EGNN_REQUIRE((vals_or_null == nullptr) == (vals_t_or_null == nullptr), "vals and vals_t come together");
+    EGNN_REQUIRE(k == 0 || (lam && t), "null lambda / T stacks");
+    EGNN_REQUIRE((xbar_or_null == nullptr) || rowsum_or_null, "xbar needs rowsum");
+    EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
+    EGNN_REQUIRE(f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER, "bad f / k");
+    const size_t need = egnn_adj_grad_degree_ws_bytes(n);
+    if (workspace == nullptr || workspace_bytes < need) {
+        set_error("adjacency-gradient workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+        return EGNN_ERR_WORKSPACE;
+    }
+    if (n == 0) return EGNN_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    double* r = (double*)align_up((size_t)workspace, 256);
+    double* q = (double*)((char*)r + align_up(sizeof(double) * (size_t)n, 256));
+    const int fl = stack_fl_log2(f, k);
+    const int blocks = grid_for(n * 32, 256);
+    adj_grad_degree_kernel<<<blocks, 256, 0, st>>>(rowptr, colidx, vals_or_null, dinv, lam, t, n, f, k, fl, r);
+    EGNN_LAUNCH_CHECK("adj_grad_degree_kernel launch");
+    adj_grad_degree_kernel<<<blocks, 256, 0, st>>>(rowptr_t, colidx_t, vals_t_or_null, dinv, t, lam, n, f, k, fl, q);
+    EGNN_LAUNCH_CHECK("adj_grad_degree_kernel launch");
+    adj_grad_finish_kernel<<<grid_for(n, 256), 256, 0, st>>>(r, q, dinv, iso, xbar_or_null, rowsum_or_null, n,
+                                                             op_scale, gw, grho);
+    EGNN_LAUNCH_CHECK("adj_grad_finish_kernel launch");
+    return EGNN_OK;
+}
+
+int egnn_adj_grad_pairs(const int32_t* rows, const int32_t* cols, int64_t n_pairs, const float* dinv,
+                        const float* lam, const float* t, const float* gw, const float* grho, int64_t n, int32_t f,
+                        int32_t k, float op_scale, float* out, egnn_stream_t stream) {
+    EGNN_REQUIRE(n_pairs >= 0 && n >= 0 && n < (int64_t(1) << 31) && f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER,
+                 "bad shape");
+    if (n_pairs == 0) return EGNN_OK;
+    EGNN_REQUIRE(rows && cols && dinv && gw && grho && out, "null pointer");
+    EGNN_REQUIRE(k == 0 || (lam && t), "null lambda / T stacks");
+    const int fl = stack_fl_log2(f, k);
+    adj_grad_pairs_kernel<<<grid_for(ceil_div64(n_pairs, 32 >> fl) * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+        rows, cols, n_pairs, dinv, lam, t, gw, grho, n, f, k, fl, op_scale, out);
+    EGNN_LAUNCH_CHECK("adj_grad_pairs_kernel launch");
+    return EGNN_OK;
+}
+
+int egnn_adj_grad_dense(const float* dinv, const float* lam, const float* t, const float* gw, const float* grho,
+                        int64_t n, int32_t f, int32_t k, float op_scale, float* out, int64_t ld,
+                        egnn_stream_t stream) {
+    EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER, "bad shape");
+    EGNN_REQUIRE(ld >= n, "ld must be >= n");
+    if (n == 0) return EGNN_OK;
+    EGNN_REQUIRE(dinv && gw && grho && out, "null pointer");
+    EGNN_REQUIRE(k == 0 || (lam && t), "null lambda / T stacks");
+    const int64_t tiles = ceil_div64(n, kDenseTile);
+    EGNN_REQUIRE(tiles <= 65535, "n too large for the dense gradient");
+    const int vec_ok = (ld % 4 == 0) && ((uintptr_t)out & 15) == 0;
+    adj_grad_dense_kernel<<<dim3((unsigned)tiles, (unsigned)tiles, 1), kDenseThreads, 0, (cudaStream_t)stream>>>(
+        lam, t, dinv, gw, grho, n, f, k, op_scale, out, ld, vec_ok);
+    EGNN_LAUNCH_CHECK("adj_grad_dense_kernel launch");
+    return EGNN_OK;
 }
 
 int egnn_cheb_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,

@@ -16,7 +16,9 @@ device every entry point raises ``EgnnError``.
 ``@`` are differentiable w.r.t. the signal (and the features w.r.t. a tensor
 ``s``): when grad mode is on and an input requires grad, the pass runs inside
 an autograd function whose backward is the adjoint (Clenshaw) pass of
-``egnn_cheb_adjoint``.  Otherwise nothing changes: same kernels, nothing saved.
+``egnn_cheb_adjoint``.  ``graph_wavelet_features`` is also differentiable w.r.t. a
+dense or sparse COO adjacency tensor and a 0-d tensor ``lambda_max`` (DESIGN.md
+section 11).  Otherwise nothing changes: same kernels, nothing saved.
 ``WATS``, ``WaveletSession`` and the sharded path stay forward-only.
 """
 from __future__ import annotations
@@ -123,11 +125,12 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
 
 
 def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, op_scale: float, op_shift: float,
-                 cbar: torch.Tensor, tbar=None, deltas=None, app_events=None) -> torch.Tensor:
+                 cbar: torch.Tensor, tbar=None, deltas=None, app_events=None, keep_all: bool = False):
     """One call of egnn_cheb_adjoint: the signal's gradient ``[N, F]`` from ``cbar`` ``[N, S, F]`` (and
     ``tbar`` ``[K+1, N, F]``).  ``graph_t``: the transposed graph (:meth:`CsrGraph.adjoint`),
     ``degree_vectors``: the forward's ``(dinv, iso)``, ``deltas``: the forward's flips, not yet
-    transposed."""
+    transposed.  ``keep_all``: egnn_cheb_adjoint_all instead, returns ``(xbar, b_all)`` with every
+    Clenshaw vector ``b_all`` ``[K+1, N, F]`` (slab 0: ``xbar``)."""
     lib = _cabi.load()
     n, f, dev = graph_t.n, int(cbar.shape[2]), graph_t.device
     dinv, iso = degree_vectors
@@ -138,15 +141,19 @@ def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, 
         ws_bytes = int(lib.egnn_cheb_workspace_bytes(n, f))
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         coeffs32 = np.ascontiguousarray(coeffs, dtype=np.float32)
-        _cabi.check(lib.egnn_cheb_adjoint(
-            _cabi.ptr(graph_t.rowptr), _cabi.ptr(graph_t.colidx), _cabi.ptr(graph_t.vals), _cabi.ptr(dinv),
-            _cabi.ptr(iso), n, graph_t.nnz, f, k, int(coeffs.shape[0]), coeffs32.ctypes.data_as(C.c_void_p),
-            float(op_scale), float(op_shift), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar),
-            _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),       # transposed flips: rows <-> cols
-            _cabi.host_array(C.c_int32, [int(v) for v in d_rows]),
-            _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows),
-            _cabi.ptr(ws), ws_bytes, _stream(), app_events, _cabi.ptr(row_order)), "egnn_cheb_adjoint")
-    return xbar
+        args = (_cabi.ptr(graph_t.rowptr), _cabi.ptr(graph_t.colidx), _cabi.ptr(graph_t.vals), _cabi.ptr(dinv),
+                _cabi.ptr(iso), n, graph_t.nnz, f, k, int(coeffs.shape[0]), coeffs32.ctypes.data_as(C.c_void_p),
+                float(op_scale), float(op_shift), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar),
+                _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),       # transposed flips: rows <-> cols
+                _cabi.host_array(C.c_int32, [int(v) for v in d_rows]),
+                _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows),
+                _cabi.ptr(ws), ws_bytes, _stream(), app_events, _cabi.ptr(row_order))
+        if not keep_all:
+            _cabi.check(lib.egnn_cheb_adjoint(*args), "egnn_cheb_adjoint")
+            return xbar
+        b_all = torch.empty((k + 1, n, f), dtype=torch.float32, device=dev)
+        _cabi.check(lib.egnn_cheb_adjoint_all(*args, _cabi.ptr(b_all)), "egnn_cheb_adjoint_all")
+    return xbar, b_all
 
 
 def _coeff_grad(cbar: torch.Tensor, t_all: torch.Tensor) -> torch.Tensor:
@@ -164,35 +171,43 @@ def _coeff_grad(cbar: torch.Tensor, t_all: torch.Tensor) -> torch.Tensor:
 
 
 class _PassSpec:
-    """Everything of one pass but its differentiable inputs (the signal and the scales)."""
+    """Everything of one pass but its differentiable inputs (the signal, the scales, the adjacency and
+    ``lambda_max``).  ``pattern``: ``(rows, cols)`` int32 device tensors when the adjacency input is
+    the value vector of a sparse COO pattern (None: a dense ``[N, N]`` adjacency)."""
 
     def __init__(self, graph, adjoint, k, coeffs, op_scale, op_shift, want_orders, deltas=None, degree_vectors=None,
-                 use_sell=None, default_signal=False, y0=None):
+                 use_sell=None, default_signal=False, y0=None, lambda_max=None, pattern=None):
         self.graph, self.adjoint, self.k, self.coeffs = graph, adjoint, k, coeffs
         self.op_scale, self.op_shift, self.want_orders = op_scale, op_shift, want_orders
         self.deltas, self.degree_vectors, self.use_sell = deltas, degree_vectors, use_sell
         self.default_signal, self.y0 = default_signal, y0
+        self.lambda_max, self.pattern = lambda_max, pattern
 
 
 class _WaveletPass(torch.autograd.Function):
-    """``(C [N,S,F], T [K+1,N,F])`` of one un-normalised pass as a function of the signal ``x0`` and
-    the scales ``s`` (a tensor, or None when they need no gradient).  ``T`` is empty unless the
-    orders are wanted or ``s`` needs a gradient (its backward reads them).  Backward: the adjoint
-    pass on the transposed graph, and ``ds_j = -sum_k k alpha[j,k] <Cbar_j, T_k>``."""
+    """``(C [N,S,F], T [K+1,N,F])`` of one un-normalised pass as a function of the signal ``x0``, the
+    scales ``s``, the adjacency ``adj`` (dense float32 ``[N, N]`` on the graph's device, or the float32
+    values of ``spec.pattern``) and a 0-d ``lam`` = ``lambda_max`` (each None when it needs no
+    gradient).  ``T`` is empty unless the orders are wanted or ``s``, ``adj`` or ``lam`` needs a
+    gradient (their backward reads them).  Backward: the adjoint pass on the transposed graph,
+    ``ds_j = -sum_k k alpha[j,k] <Cbar_j, T_k>``, and for ``adj`` / ``lam`` the adjacency terms of
+    DESIGN.md section 11 from every Clenshaw vector (egnn_cheb_adjoint_all)."""
 
     @staticmethod
-    def forward(ctx, x0, s, spec):
+    def forward(ctx, x0, s, adj, lam, spec):
         ctx.set_materialize_grads(False)        # an output nobody differentiates arrives as None
         s_grad = s is not None and ctx.needs_input_grad[1]
+        structure = (adj is not None and ctx.needs_input_grad[2]) or (lam is not None and ctx.needs_input_grad[3])
         comb, t_all = _run_cheb(spec.graph, x0, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, False,
-                                spec.want_orders or s_grad, spec.deltas, spec.degree_vectors, use_sell=spec.use_sell,
-                                default_signal=spec.default_signal, y0=spec.y0)
+                                spec.want_orders or s_grad or structure, spec.deltas, spec.degree_vectors,
+                                use_sell=spec.use_sell, default_signal=spec.default_signal, y0=spec.y0)
         if t_all is None:
             t_all = comb.new_empty((0,))
             ctx.mark_non_differentiable(t_all)
         ctx.spec, ctx.x_shape = spec, x0.shape
         ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
-        ctx.save_for_backward(t_all if s_grad else None)
+        ctx.lam_meta = None if lam is None else (lam.shape, lam.device, lam.dtype)
+        ctx.save_for_backward(t_all if (s_grad or structure) else None)
         return comb, t_all
 
     @staticmethod
@@ -206,18 +221,74 @@ class _WaveletPass(torch.autograd.Function):
         cbar = (_cabi.vec_ready(g_comb) if g_comb is not None else
                 torch.zeros((g.n, n_scales, f), dtype=torch.float32, device=g.device))
         tbar = _cabi.vec_ready(g_orders) if (g_orders is not None and g_orders.numel()) else None
-        x_grad = s_grad = None
-        if ctx.needs_input_grad[0]:
+        x_grad = s_grad = adj_grad = lam_grad = None
+        structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
+        if ctx.needs_input_grad[0] or structure:
             dv = spec.degree_vectors if spec.degree_vectors is not None else (g.dinv, g.iso)
-            x_grad = _run_adjoint(spec.adjoint(), dv, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, cbar, tbar,
-                                  spec.deltas).reshape(ctx.x_shape)
+            xbar = _run_adjoint(spec.adjoint(), dv, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, cbar, tbar,
+                                spec.deltas, keep_all=structure)
+            if structure:
+                xbar, b_all = xbar
+            if ctx.needs_input_grad[0]:
+                x_grad = xbar.reshape(ctx.x_shape)
         if ctx.needs_input_grad[1]:
             G = _coeff_grad(cbar, t_all)
             alpha = torch.from_numpy(np.ascontiguousarray(spec.coeffs, dtype=np.float64)).to(G.device)
             kk = torch.arange(spec.k + 1, dtype=torch.float64, device=G.device)
             shape, dev, dtype = ctx.s_meta
             s_grad = (-(kk * alpha * G).sum(dim=1)).to(device=dev, dtype=dtype).reshape(shape)
-        return x_grad, s_grad, None
+        if ctx.needs_input_grad[2]:
+            adj_grad = _adjacency_grad(spec, b_all, t_all)
+        if ctx.needs_input_grad[3]:
+            shape, dev, dtype = ctx.lam_meta
+            lam_grad = _lambda_max_grad(b_all, t_all, spec.lambda_max).to(device=dev, dtype=dtype).reshape(shape)
+        return x_grad, s_grad, adj_grad, lam_grad, None
+
+
+def _adjacency_grad(spec: _PassSpec, b_all: torch.Tensor, t_all: torch.Tensor) -> torch.Tensor:
+    """``dLoss/dA`` from the Clenshaw vectors ``b_all`` and the orders ``t_all``: the degree terms
+    (egnn_adj_grad_degree over the CSR and its transpose), then either the dense ``[N, N]`` gradient
+    (egnn_adj_grad_dense) or its values at ``spec.pattern`` (egnn_adj_grad_pairs)."""
+    lib = _cabi.load()
+    g, k = spec.graph, spec.k
+    gt = spec.adjoint()
+    n, f = g.n, int(b_all.shape[2])
+    lam, t = b_all[1:], t_all[:k]                    # b_1..b_K and T_0..T_{K-1}: [K, N, F] stacks
+    signal = spec.default_signal and f == 1
+    with torch.cuda.device(g.device):
+        gw = torch.empty(n, dtype=torch.float32, device=g.device)
+        grho = torch.empty(n, dtype=torch.float32, device=g.device)
+        ws_bytes = int(lib.egnn_adj_grad_degree_ws_bytes(n))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=g.device)
+        _cabi.check(lib.egnn_adj_grad_degree(
+            _cabi.ptr(g.rowptr), _cabi.ptr(g.colidx), _cabi.ptr(g.vals), _cabi.ptr(gt.rowptr), _cabi.ptr(gt.colidx),
+            _cabi.ptr(gt.vals), _cabi.ptr(g.dinv), _cabi.ptr(g.iso), n, g.nnz, f, k, float(spec.op_scale),
+            _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(b_all[0]) if signal else None,
+            _cabi.ptr(g.rowsum) if signal else None, _cabi.ptr(gw), _cabi.ptr(grho), _cabi.ptr(ws), ws_bytes,
+            _stream()), "egnn_adj_grad_degree")
+        if spec.pattern is None:
+            out = torch.empty((n, n), dtype=torch.float32, device=g.device)
+            _cabi.check(lib.egnn_adj_grad_dense(_cabi.ptr(g.dinv), _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(gw),
+                                                _cabi.ptr(grho), n, f, k, float(spec.op_scale), _cabi.ptr(out), n,
+                                                _stream()), "egnn_adj_grad_dense")
+            return out
+        rows, cols = spec.pattern
+        out = torch.empty(rows.numel(), dtype=torch.float32, device=g.device)
+        _cabi.check(lib.egnn_adj_grad_pairs(_cabi.ptr(rows), _cabi.ptr(cols), rows.numel(), _cabi.ptr(g.dinv),
+                                            _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(gw), _cabi.ptr(grho), n, f, k,
+                                            float(spec.op_scale), _cabi.ptr(out), _stream()), "egnn_adj_grad_pairs")
+    return out
+
+
+def _lambda_max_grad(b_all: torch.Tensor, t_all: torch.Tensor, lambda_max: float) -> torch.Tensor:
+    """``-(1/lambda_max) sum_k <b_k, T_k + T_{k-2} + m_k T_{k-1}>`` (float64, 0-d): one
+    egnn_cheb_coeff_grad per order k with ``S = 1`` and ``cbar = b_k`` gives every ``<b_k, T_j>``."""
+    k = int(t_all.shape[0]) - 1
+    total = torch.zeros((), dtype=torch.float64, device=t_all.device)
+    for i in range(1, k + 1):
+        G = _coeff_grad(b_all[i].unsqueeze(1), t_all)[0]
+        total = total + G[i] + (1.0 if i == 1 else 2.0) * G[i - 1] + (G[i - 2] if i >= 2 else 0.0)
+    return -total / float(lambda_max)
 
 
 class _L1Normalize(torch.autograd.Function):
@@ -253,11 +324,28 @@ def _needs_grad(x0, s=None) -> bool:
     return torch.is_grad_enabled() and (x0.requires_grad or (isinstance(s, torch.Tensor) and s.requires_grad))
 
 
-def _differentiable_pass(spec: _PassSpec, x0: torch.Tensor, s=None):
-    """``(C, T)`` through :class:`_WaveletPass`; the device / dtype conversion of ``x0`` stays outside
-    the function, so autograd routes the gradient back to a CPU or float64 leaf."""
+def _differentiable_pass(spec: _PassSpec, x0: torch.Tensor, s=None, adj=None, lam=None):
+    """``(C, T)`` through :class:`_WaveletPass`; the device / dtype conversion of ``x0`` (and of ``adj``)
+    stays outside the function, so autograd routes the gradient back to a CPU or float64 leaf."""
     x0 = x0.to(device=spec.graph.device, dtype=torch.float32)
-    return _WaveletPass.apply(x0, s if (isinstance(s, torch.Tensor) and s.requires_grad) else None, spec)
+    if adj is not None:
+        adj = adj.to(device=spec.graph.device, dtype=torch.float32)
+    return _WaveletPass.apply(x0, s if (isinstance(s, torch.Tensor) and s.requires_grad) else None, adj, lam, spec)
+
+
+def _structure_input(adj_matrix, lambda_max, deltas):
+    """The adjacency and ``lambda_max`` inputs that need a gradient: ``(adj, lam)``, each None when not.
+    Only a dense strided ``[N, N]`` tensor and a sparse COO tensor take part, only a 0-d tensor
+    ``lambda_max``, and never with ``deltas``."""
+    if not torch.is_grad_enabled() or deltas is not None:
+        return None, None
+    adj = None
+    if isinstance(adj_matrix, torch.Tensor) and adj_matrix.requires_grad and adj_matrix.dim() == 2 and \
+            adj_matrix.layout in (torch.strided, torch.sparse_coo):
+        adj = adj_matrix
+    lam = lambda_max if isinstance(lambda_max, torch.Tensor) and lambda_max.requires_grad and lambda_max.dim() == 0 \
+        else None
+    return adj, lam
 
 
 def _patches_in_kernel(graph: CsrGraph, f: int, k: int, use_sell) -> bool:
@@ -453,14 +541,45 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
     them requires grad: every output (``features``, ``combined``, ``orders``)
     then carries a ``grad_fn``; ``deltas=`` is supported.  The forward then keeps
     the un-normalised combination and normalises out of place.
+
+    Also differentiable w.r.t. the adjacency and ``lambda_max`` (DESIGN.md
+    section 11) in grad mode, without ``deltas``, when one of these requires grad:
+
+    * ``adj_matrix`` a dense strided ``[N, N]`` tensor (CPU or GPU, any float
+      dtype): its gradient is the full dense ``dLoss/dA``, diagonal and
+      unstored entries included;
+    * ``adj_matrix`` a sparse COO tensor (e.g. ``torch.sparse_coo_tensor(
+      edge_index, w, (N, N))`` with a leaf ``w``): the gradient at the stored
+      pattern, which reaches ``w`` through torch's constructor and
+      ``coalesce()`` (duplicates share their entry's gradient; explicit zeros,
+      dropped from the graph, still get the gradient at their position);
+    * ``lambda_max`` a 0-d tensor.
+
+    An isolated node (zero column sum off the diagonal) has its normaliser held
+    at 1: ``w^-1/2`` has no derivative at ``w = 0``.  That holds for every entry
+    of its column: the unstored entries of a dense gradient, and explicit zeros
+    of a COO pattern (a column of explicit zeros only is isolated).  Every other adjacency
+    format (sparse CSR tensors, scipy matrices, ``CsrGraph``, ``(edge_index,
+    N)``) and every call with ``deltas`` stays forward-only in the adjacency.
     """
-    graph = as_graph(adj_matrix)
+    adj_in, lam_in = _structure_input(adj_matrix, lambda_max, deltas)
+    graph = as_graph(adj_matrix if adj_in is None else adj_matrix.detach())
+    pattern = None
+    if adj_in is not None and adj_in.layout == torch.sparse_coo:
+        # the pattern's values are the function's input: torch routes their gradient back through
+        # coalesce() and the constructor, summing it over duplicates
+        adj_in = adj_in.coalesce()
+        idx = adj_in.indices().to(device=graph.device, dtype=torch.int32)
+        pattern = (idx[0].contiguous(), idx[1].contiguous())
+        adj_in = adj_in.values()
+    elif adj_in is not None and tuple(adj_in.shape) != (graph.n, graph.n):
+        raise ValueError(f"adjacency must be [N, N], got {tuple(adj_in.shape)}")
     k = int(k)
     s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
     coeffs = heat_coefficients(k, s_vals)
     degree_vectors = None
     x0 = graph.x0 if X0 is None else torch.as_tensor(X0)
-    grad = _needs_grad(x0, s)
+    grad = _needs_grad(x0, s) or adj_in is not None or lam_in is not None
     y0 = None
     in_kernel = False
     if deltas is not None and len(deltas[0]) > 0:
@@ -483,8 +602,8 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
             if degree_vectors is not None:       # the scratch vectors are restored below, the backward runs later
                 degree_vectors = tuple(v.clone() for v in degree_vectors)
             spec = _PassSpec(graph, graph.adjoint, k, coeffs, op_scale, -1.0, return_parts, deltas, degree_vectors,
-                             _use_sell, default_signal, y0)
-            comb, t_all = _differentiable_pass(spec, x0, s)
+                             _use_sell, default_signal, y0, float(lambda_max), pattern)
+            comb, t_all = _differentiable_pass(spec, x0, s, adj_in, lam_in)
             feats = _L1Normalize.apply(comb) if normalize else comb
             feats = feats.reshape(graph.n, -1)
             return WaveletResult(feats, [t_all[i] for i in range(k + 1)], comb) if return_parts else feats
@@ -593,6 +712,10 @@ class WATS(nn.Module):
                     return self.wavelet_feats
                 return graph_wavelet_features(self.graph, k=self.k, s=self.s, lambda_max=self.lambda_max,
                                               deltas=flips)
+        # the calibrator's features are an input, not a function of the adjacency: a leaf that requires
+        # grad (the attack's modified_adj) gets no wavelet gradient here, whatever the number of flips
+        if isinstance(adj, torch.Tensor):
+            adj = adj.detach()
         return graph_wavelet_features(adj, k=self.k, s=self.s, lambda_max=self.lambda_max)
 
     def temperatures(self, wavelet_features):

@@ -276,6 +276,55 @@ int egnn_cheb_adjoint(const int32_t* rowptr_t, const int32_t* colidx_t,
                       void* workspace, size_t workspace_bytes, egnn_stream_t stream,
                       void* const* app_events_host, const int32_t* row_order_or_null);
 
+/* egnn_cheb_adjoint that also keeps every Clenshaw vector (new in ABI 8):
+ * b_all [K+1, n, f] receives xbar in slab 0 and b_m in slab m = 1..K (the
+ * lambda_k of the adjacency gradient below).  Same kernels as
+ * egnn_cheb_adjoint; b_all must be 16-byte aligned when f % 4 == 0.          */
+int egnn_cheb_adjoint_all(const int32_t* rowptr_t, const int32_t* colidx_t,
+                          const float* vals_t_or_null, const float* dinv, const uint8_t* iso,
+                          int64_t n, int64_t nnz, int32_t f, int32_t k, int32_t n_scales,
+                          const float* coeffs_host, float op_scale, float op_shift,
+                          const float* cbar, const float* tbar_or_null, float* xbar,
+                          const int32_t* delta_row_host, const int32_t* delta_col_host,
+                          const float* delta_val_host, int32_t n_delta,
+                          void* workspace, size_t workspace_bytes, egnn_stream_t stream,
+                          void* const* app_events_host, const int32_t* row_order_or_null,
+                          float* b_all);
+
+/* ---- gradient w.r.t. the adjacency (ABI 8) ---------------------------------
+ * a = op_scale, d = dinv, lam = [K, n, f] stack b_1..b_K (slabs 1..K of
+ * egnn_cheb_adjoint_all's b_all), t = [K, n, f] stack T_0..T_{K-1} (the
+ * forward's t_all); m_1 = 1, m_k = 2 for k >= 2:
+ *   g_ij   = sum_k m_k <d_i lam_k[i,:], d_j T_{k-1}[j,:]>
+ *   R_i    = sum_{j != i} A_ij g_ij,   Q_i = sum_{j != i} A_ji g_ji
+ *   gw_i   = (a/2) d_i^2 (R_i + Q_i), 0 for an isolated node
+ *   grho_i = xbar_i / (1 + rowsum_i) (default signal x0 = log1p(rowsum)), else 0
+ *   dLoss/dA_ij = [i != j] (-a g_ij + gw_j) + grho_i.
+ * An isolated node's d is held at 1 (w^-1/2 has no derivative at w = 0).
+ * All sums run in a fixed order (float32 chunks, float64 carry, no atomics):
+ * bitwise deterministic.
+ *
+ * egnn_adj_grad_degree: gw and grho [n] from the CSR and its transpose
+ * (egnn_csr_transpose, or the CSR itself when symmetric); xbar_or_null /
+ * rowsum_or_null: the signal's gradient [n] and the row sums, f = 1 default
+ * signal only (NULL: grho = 0).  workspace: egnn_adj_grad_degree_ws_bytes(n).
+ * egnn_adj_grad_pairs: out[p] = dLoss/dA at (rows[p], cols[p]), any pattern
+ * (entries need not be stored in the CSR; indices in [0, n)).
+ * egnn_adj_grad_dense: the whole [n, n] gradient into out with row stride ld. */
+size_t egnn_adj_grad_degree_ws_bytes(int64_t n);
+int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                         const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                         const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f,
+                         int32_t k, float op_scale, const float* lam, const float* t,
+                         const float* xbar_or_null, const float* rowsum_or_null, float* gw, float* grho,
+                         void* workspace, size_t workspace_bytes, egnn_stream_t stream);
+int egnn_adj_grad_pairs(const int32_t* rows, const int32_t* cols, int64_t n_pairs, const float* dinv,
+                        const float* lam, const float* t, const float* gw, const float* grho,
+                        int64_t n, int32_t f, int32_t k, float op_scale, float* out, egnn_stream_t stream);
+int egnn_adj_grad_dense(const float* dinv, const float* lam, const float* t, const float* gw,
+                        const float* grho, int64_t n, int32_t f, int32_t k, float op_scale,
+                        float* out, int64_t ld, egnn_stream_t stream);
+
 /* Row L1 normalisation out of place, h = c / (sum_f |c| + 1e-8) per row of f
  * values (n_vec rows), and its backward: cbar_out = cbar_in + (hbar -
  * sign(c) <hbar, h>) / r with r recomputed from c and sign(0) = 0.
