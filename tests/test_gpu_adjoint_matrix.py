@@ -37,6 +37,12 @@ ISOLATED = range(0, 5)          # nodes without any entry
 LOOPS = range(10, 40)           # nodes with a stored self loop
 OUT_HUB, IN_HUB, LAST_IN = 50, 60, 70
 HUB_DEGREE = 2100               # >= 2048 (kHubDegree): summed by a whole CTA on the wide path
+# the forward matrix's extra graphs ("dense_hubs_*", "sparse_long_*"): nodes whose only entry is a
+# stored self loop, out-hub rows on a graph dense enough for the static wide schedule, and
+# consecutive long rows that share one warp of the generic kernel
+LOOP_ONLY = range(5, 8)
+HUB_ROWS = (50, 51, 52)
+LONG_ROWS = range(208, 216)
 
 
 # ---- graphs ------------------------------------------------------------------------------------
@@ -55,13 +61,17 @@ def _pattern(rng, n, deg, directed):
 def build_graph(name):
     """Seeded scipy CSR (float32): binary symmetric or weighted (0.5-2) directed, with isolated
     nodes and stored self loops; the star variants add a row (out-star) or a column (in-star)
-    of HUB_DEGREE entries to the weighted sparse graph."""
+    of HUB_DEGREE entries to the weighted sparse graph.  "dense_hubs_*" (3000 nodes, ~72
+    entries per row: >= 64 per row, the static wide schedule) adds the out-hub rows HUB_ROWS;
+    "sparse_long_*" gives the rows LONG_ROWS 150-400 entries each.  Both have LOOP_ONLY nodes
+    and a node LAST_IN with exactly one in-edge (from node 80), as "stars_w" has."""
     if name == "empty":
         return sp.csr_matrix((700, 700), dtype=np.float32)
     rng = np.random.default_rng(zlib.crc32(name.encode()))
     dense = name.startswith("dense")
     weighted = not name.endswith("bin")
-    n, deg = (2000, 96) if dense else (3000, 8)
+    extras = name.startswith(("dense_hubs", "sparse_long"))
+    n, deg = (3000, 72) if name.startswith("dense_hubs") else (2000, 96) if dense else (3000, 8)
     a = _pattern(rng, n, deg, directed=weighted)
     r, c = a.row, a.col
     extra_r, extra_c = [np.asarray(LOOPS)], [np.asarray(LOOPS)]
@@ -71,12 +81,22 @@ def build_graph(name):
     if name in ("in_star_w", "stars_w"):
         rows = rng.choice(np.arange(100, n), HUB_DEGREE, replace=False)
         extra_r.append(rows); extra_c.append(np.full(HUB_DEGREE, IN_HUB))
+    if name.startswith("dense_hubs"):
+        for h in HUB_ROWS:
+            extra_r.append(np.full(HUB_DEGREE, h)); extra_c.append(rng.choice(np.arange(100, n), HUB_DEGREE, replace=False))
+    if name.startswith("sparse_long"):
+        for i in LONG_ROWS:
+            d = int(rng.integers(150, 400))
+            extra_r.append(np.full(d, i)); extra_c.append(rng.choice(np.arange(100, n), d, replace=False))
     r, c = np.concatenate([r] + extra_r), np.concatenate([c] + extra_c)
-    if name == "stars_w":                  # LAST_IN keeps exactly one in-edge (from node 80)
+    if name == "stars_w" or extras:        # LAST_IN keeps exactly one in-edge (from node 80)
         keep = c != LAST_IN
         r, c = np.concatenate([r[keep], [80]]), np.concatenate([c[keep], [LAST_IN]])
-    iso = np.isin(r, ISOLATED) | np.isin(c, ISOLATED)
+    cut = list(ISOLATED) + (list(LOOP_ONLY) if extras else [])
+    iso = np.isin(r, cut) | np.isin(c, cut)
     r, c = r[~iso], c[~iso]
+    if extras:
+        r, c = np.concatenate([r, LOOP_ONLY]), np.concatenate([c, LOOP_ONLY])
     a = sp.csr_matrix((np.ones(r.size, np.float32), (r, c)), shape=(n, n))
     a.sum_duplicates()
     a.data[:] = 1.0
@@ -243,12 +263,15 @@ def test_adjoint_matrix_vs_float64(case):
 
 
 # ---- which kernels run -------------------------------------------------------------------------
-_KERNEL = re.compile(r"cheb_(wide|order)_kernel<([^>]*)>")
+_KERNEL = re.compile(r"(cheb_wide|cheb_order|sell_step|blocked_spmv)_kernel<([^>]*)>")
+_SHORT = {"cheb_wide": "wide", "cheb_order": "order"}
 
 
-def adjoint_kernels(names):
-    """Normalised ``wide<...>`` / ``order<...>`` keys of the adjoint (last template argument true)
-    instantiations among kernel names, whichever way the demangler spells the arguments."""
+def kernel_keys(names, adj):
+    """Normalised ``wide<...>`` / ``order<...>`` keys of the order-kernel instantiations among
+    kernel names whose last template argument (ADJ) equals ``adj``, whichever way the demangler
+    spells the arguments.  With ``adj`` false the narrow forward kernels, which have no adjoint
+    instantiation, are kept too: ``sell_step<PEER,PATCH>`` and ``blocked_spmv<HAS_VALS>``."""
     out = set()
     for name in names:
         m = _KERNEL.search(name)
@@ -258,9 +281,18 @@ def adjoint_kernels(names):
         for a in m.group(2).split(","):
             a = re.sub(r"^\((?:bool|int)\)", "", a.strip())
             args.append({"true": 1, "false": 0}[a] if a in ("true", "false") else int(a))
-        if args[-1] == 1:
-            out.add(f"{m.group(1)}<{','.join(map(str, args))}>")
+        family = m.group(1)
+        if family in _SHORT and args[-1] != int(adj):
+            continue
+        if family not in _SHORT and adj:
+            continue
+        out.add(f"{_SHORT.get(family, family)}<{','.join(map(str, args))}>")
     return out
+
+
+def adjoint_kernels(names):
+    """Normalised keys of the adjoint (last template argument true) instantiations."""
+    return kernel_keys(names, adj=True)
 
 
 def _profiled_kernels(fn):

@@ -19,27 +19,35 @@ TOL = 1e-5
 
 
 SURVEY_FLOOR_WORST = {}      # tag -> worst element-wise ratio at SURVEY 8c's original 1e-3 floor (printed, not enforced)
+ENFORCED_FLOOR_WORST = {}    # tag -> worst element-wise ratio at the enforced 5e-2 floor
 
 
-def check_parts(res, ref_T, ref_S, ref_H, tag=""):
+def check_parts(res, ref_T, ref_S, ref_H, tag="", tol=TOL):
+    """Every order and every scale's S against the reference: norm-wise <= tol and element-wise
+    ratio <= 1 at the 5e-2 floor (ratio at the 1e-3 floor recorded); H after the float32 cast."""
     worst = []
     for i, (got, ref) in enumerate(zip(res.orders, ref_T)):
         g = got.cpu().numpy()
         err = rel_max_err(g, ref)
         worst.append(err)
-        assert err <= TOL, f"{tag} order {i}: rel max err {err:.3e}"
-        ratio = elementwise_ratio(g, ref, TOL)
+        assert err <= tol, f"{tag} order {i}: rel max err {err:.3e}"
+        ratio = elementwise_ratio(g, ref, tol)
         assert ratio <= 1.0, f"{tag} order {i}: element-wise bound exceeded x{ratio:.2f}"
-        at_survey_floor = elementwise_ratio(g, ref, TOL, floor=1e-3)
+        at_survey_floor = elementwise_ratio(g, ref, tol, floor=1e-3)
         SURVEY_FLOOR_WORST[tag] = max(SURVEY_FLOOR_WORST.get(tag, 0.0), at_survey_floor)
-    if tag:
-        print(f"\n[{tag}] worst element-wise ratio at the enforced 5e-2 floor <= 1; at SURVEY's 1e-3 floor: "
-              f"x{SURVEY_FLOOR_WORST[tag]:.2f}; norm-wise worst {max(worst):.2e}")
+        ENFORCED_FLOOR_WORST[tag] = max(ENFORCED_FLOOR_WORST.get(tag, 0.0), ratio)
     for j, rs in enumerate(ref_S):
         g = res.combined[:, j, :].cpu().numpy()
-        assert rel_max_err(g, rs) <= TOL, f"{tag} S[{j}]"
-        ratio = elementwise_ratio(g, rs, TOL)
+        err = rel_max_err(g, rs)
+        assert err <= tol, f"{tag} S[{j}]: rel max err {err:.3e}"
+        ratio = elementwise_ratio(g, rs, tol)
         assert ratio <= 1.0, f"{tag} S[{j}]: element-wise bound exceeded x{ratio:.2f}"
+        SURVEY_FLOOR_WORST[tag] = max(SURVEY_FLOOR_WORST.get(tag, 0.0), elementwise_ratio(g, rs, tol, floor=1e-3))
+        ENFORCED_FLOOR_WORST[tag] = max(ENFORCED_FLOOR_WORST.get(tag, 0.0), ratio)
+    if tag:
+        print(f"\n[{tag}] worst element-wise ratio x{ENFORCED_FLOOR_WORST.get(tag, 0.0):.2f} at the enforced 5e-2 "
+              f"floor; at SURVEY's 1e-3 floor: x{SURVEY_FLOOR_WORST.get(tag, 0.0):.2f}; "
+              f"norm-wise worst {max(worst, default=0.0):.2e}")
     f = ref_H[0].shape[1]
     for j, rh in enumerate(ref_H):
         g = res.features[:, j * f:(j + 1) * f].cpu().numpy()
