@@ -1669,6 +1669,8 @@ int egnn_gcn_propagate(const int32_t* rowptr, const int32_t* colidx, const float
     int rc = gcn_check(rowptr, n, h);
     if (rc) return rc;
     EGNN_REQUIRE(m && y, "null pointer");
+    EGNN_REQUIRE(vec_aligned(m, h) && vec_aligned(bias_or_null, h) && vec_aligned(y, h),
+                 "m, bias and y must be 16-byte aligned");
     DeltaList d;
     rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
     if (rc) return rc;
@@ -1692,6 +1694,7 @@ int egnn_gcn_target_logits(const int32_t* rowptr, const int32_t* colidx, const f
     int rc = gcn_check(rowptr, n, h);
     if (rc) return rc;
     EGNN_REQUIRE(z1 && w2 && b2 && logits_out && ctx, "null pointer");
+    EGNN_REQUIRE(vec_aligned(z1, h), "z1 must be 16-byte aligned");
     EGNN_REQUIRE(target >= 0 && target < n && n_classes >= 1, "bad target / classes");
     DeltaList d;
     rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
@@ -1717,6 +1720,7 @@ int egnn_gcn_structure_grad(const int32_t* rowptr, const int32_t* colidx, const 
     int rc = gcn_check(rowptr, n, h);
     if (rc) return rc;
     EGNN_REQUIRE(upstream && w2 && z1 && xw && b1 && deg && ctx && grad_row && grad_col, "null pointer");
+    EGNN_REQUIRE(vec_aligned(z1, h) && vec_aligned(xw, h), "z1 and xw must be 16-byte aligned");
     EGNN_REQUIRE(target >= 0 && target < n && n_classes >= 1, "bad target / classes");
     DeltaList d;
     rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);

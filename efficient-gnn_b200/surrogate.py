@@ -89,7 +89,7 @@ class SparseGCNSurrogate:
         dev = self.graph.device
         self.lib = _cabi.load()
         w1 = gcn.gc1.weight.detach().to(dev, torch.float32)
-        self.b1 = gcn.gc1.bias.detach().to(dev, torch.float32).contiguous()
+        self.b1 = _cabi.vec_ready(gcn.gc1.bias.detach().to(dev))     # read with 16-byte vector loads
         self.w2 = gcn.gc2.weight.detach().to(dev, torch.float32).contiguous()
         self.b2 = gcn.gc2.bias.detach().to(dev, torch.float32).contiguous()
         self.h = int(w1.shape[0])

@@ -375,8 +375,11 @@ int egnn_temperature_head(const float* feats, const float* w1, const float* b1,
  *                           floats) carries (A_n relu(Z1))[target,:], deg and the diagonal entry
  *   egnn_gcn_structure_grad grad_row[m] = dLoss/dA[target,m], grad_col[i] = dLoss/dA[i,target]
  *                           for upstream = dLoss/dlogits[target,:] [n_classes] (device)
- * h: hidden width, a multiple of 4 up to 128.  delta_*: flips as in egnn_cheb_wavelet
- * (the same list must be passed to all three calls of one evaluation).        */
+ * h: hidden width, a multiple of 4 up to 128.  Rows of m, bias, y, z1 and xw are
+ * accessed with 16-byte vector loads and stores, so those pointers must be 16-byte
+ * aligned; a misaligned one is refused with EGNN_ERR_INVALID_ARG before any launch.
+ * delta_*: flips as in egnn_cheb_wavelet (the same list must be passed to all
+ * three calls of one evaluation).                                               */
 #define EGNN_GCN_CTX_FLOATS 136
 int egnn_gcn_propagate(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
                        const float* m, const float* bias_or_null, float* y, float* deg_out_or_null,

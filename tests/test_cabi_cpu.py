@@ -75,6 +75,27 @@ def test_misaligned_vector_buffers_are_refused_before_any_launch():
     assert rc == -4 and b"workspace" in lib.egnn_last_error()
 
 
+@pytest.mark.skipif(torch.cuda.is_available(), reason="fake device pointers: must not reach a launch on a GPU")
+def test_misaligned_surrogate_buffers_are_refused_before_any_launch():
+    """The structure-gradient kernels read rows of m / z1 / xw and the bias, and write y, with 16-byte
+    vector accesses.  Each of the three gcn entry points refuses a misaligned one with the
+    alignment error (without the check the call would reach a launch and fail differently)."""
+    lib = _cabi.load()
+    base = 1 << 20
+    ok = lambda i: base + 4096 * i                        # noqa: E731
+    bad = lambda i: base + 4096 * i + 4                   # noqa: E731
+    for m, bias, y in ((bad(3), ok(4), ok(5)), (ok(3), bad(4), ok(5)), (ok(3), ok(4), bad(5))):
+        rc = lib.egnn_gcn_propagate(ok(1), ok(2), None, m, bias, y, None, 4, 4, None, None, None, 0, None)
+        assert rc == -1 and b"aligned" in lib.egnn_last_error(), (rc, lib.egnn_last_error())
+    rc = lib.egnn_gcn_target_logits(ok(1), ok(2), None, bad(3), ok(4), ok(5), 0, 4, 4, 2, ok(6), ok(7),
+                                    None, None, None, 0, None)
+    assert rc == -1 and b"aligned" in lib.egnn_last_error(), (rc, lib.egnn_last_error())
+    for z1, xw in ((bad(5), ok(6)), (ok(5), bad(6))):
+        rc = lib.egnn_gcn_structure_grad(ok(1), ok(2), None, ok(3), ok(4), z1, xw, ok(7), ok(8), ok(9), 0, 4, 4, 2,
+                                         ok(10), ok(11), None, None, None, 0, None)
+        assert rc == -1 and b"aligned" in lib.egnn_last_error(), (rc, lib.egnn_last_error())
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-device failure mode")
 def test_no_cpu_fallback():
     with pytest.raises(egnn.EgnnError):
