@@ -13,7 +13,7 @@ import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("EGNN_LIB_PATH") or os.path.join(_HERE, "lib", "libegnn_b200.so")   # override: tuning builds
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 # every symbol include/egnn_b200.h declares: name -> (restype, argtypes)
 _P, _I32, _I64, _F32, _SZ = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -77,6 +77,11 @@ SYMBOLS = {
     "egnn_cheb_order_sharded": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
                                           _I64, _I64, _I64, _I64, _I32, _I32, _I32, _I32, _P, _F32, _F32,
                                           _I32, _I32, _P, _P, _P, _I32, _P]),
+    "egnn_cheb_adjoint_sharded": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                            _I64, _I64, _I64, _I64, _I32, _I32, _I32, _I32, _P, _F32, _F32, _I32,
+                                            _P, _P, _P, _I32, _P]),
+    "egnn_wide_adjoint_sharded": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _I32, _I32, _I32, _I32,
+                                            _P, _F32, _F32, _P, _P, _P, _I32, _P, _P]),
 }
 
 

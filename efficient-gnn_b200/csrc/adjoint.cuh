@@ -10,6 +10,7 @@
 #pragma once
 
 #include "common.cuh"
+#include "peer.cuh"
 
 namespace egnn {
 
@@ -37,6 +38,30 @@ adjoint_prologue_kernel(const float* __restrict__ cbar, const float* __restrict_
         }
         if (y_out) y_out[i] = dinv[r] * v;
     }
+}
+
+// Row-sharded twin of adjoint_prologue_kernel + peer_prescale_push_kernel: v_K of the local rows
+// (same sum order), dinv (.) v_K stored into operand buffer 0 of every rank's window (rows ldy wide,
+// padding zeroed) once every peer has finished the kernels before it, then signalled.
+__global__ void __launch_bounds__(1024)
+adjoint_prologue_push_kernel(const float* __restrict__ cbar, const float* __restrict__ tbar,
+                             const float* __restrict__ dinv_full, int64_t n_rows, int64_t row0, int32_t F, int32_t S,
+                             int32_t ldy, const __grid_constant__ CoefRow c, const __grid_constant__ PeerPush pp) {
+    peer_producer_wait_first(pp);
+    const int64_t total = n_rows * ldy;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
+         i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = i / ldy;
+        const int col = (int)(i - r * ldy);
+        float v = 0.f;
+        if (col < F) {
+            if (tbar) v = tbar[r * F + col];
+            for (int s = 0; s < S; ++s) v = fmaf(c.c[s], cbar[(r * S + s) * F + col], v);
+        }
+        const float y = dinv_full[row0 + r] * v;
+        for (int p = 0; p < pp.world; ++p) pp.dst[p][(row0 + r) * ldy + col] = y;
+    }
+    peer_producer_signal(pp);
 }
 
 // h[r, :] = c[r, :] / (sum_f |c[r, f]| + 1e-8), one warp per row vector (as l1_normalize_kernel)

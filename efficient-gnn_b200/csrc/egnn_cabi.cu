@@ -143,13 +143,12 @@ static int launch_wide_np(const WideParams& p, dim3 grid, cudaStream_t st) {
     return launch_wide_npd<NZ_LOG2, PEER, false, ADJ>(p, grid, st);
 }
 
-// PEER instantiation: operand in the exchange window, written by the other GPUs (world > 1).
-// The adjoint (ADJ) runs on one GPU only.
+// PEER instantiation: operand in the exchange window, written by the other GPUs (world > 1),
+// for the forward orders and the adjoint applications alike.
 template <int NZ_LOG2, bool ADJ>
 static int launch_wide_n(const WideParams& p, dim3 grid, cudaStream_t st) {
-    if constexpr (ADJ) return launch_wide_np<NZ_LOG2, false, true>(p, grid, st);
-    else return p.peer.world > 1 ? launch_wide_np<NZ_LOG2, true, false>(p, grid, st)
-                                 : launch_wide_np<NZ_LOG2, false, false>(p, grid, st);
+    return p.peer.world > 1 ? launch_wide_np<NZ_LOG2, true, ADJ>(p, grid, st)
+                            : launch_wide_np<NZ_LOG2, false, ADJ>(p, grid, st);
 }
 
 // (Measured and dropped: pinning the gather operand in L2 with an access-policy window and the
@@ -348,7 +347,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 8; }
+int egnn_abi_version(void) { return 9; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -1612,6 +1611,149 @@ int egnn_wide_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_l
         EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
     }
     return EGNN_OK;
+}
+
+// ---- backward of the row-sharded pass ------------------------------------------------------------
+// Application app = 1..K of the adjoint produces b_m, m = K - app, on the rank's rows (b_0: the
+// signal's gradient); app 0 is the prologue b_K = v_K.  tbar_or_null is the whole [K+1, rows, f] stack.
+static int adjoint_sharded_check(int64_t n, int64_t row_begin, int64_t row_end, int32_t f, int32_t app, int32_t k_max,
+                                 int32_t n_scales) {
+    EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && row_begin >= 0 && row_end >= row_begin && row_end <= n,
+                 "bad row range");
+    EGNN_REQUIRE(f >= 1, "f must be >= 1");
+    EGNN_REQUIRE(k_max >= 0 && k_max <= EGNN_MAX_ORDER && app >= 0 && app <= k_max, "bad application");
+    EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
+    return EGNN_OK;
+}
+
+int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                              const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                              const float* dinv_full, const uint8_t* iso_full, const float* b_prev_full,
+                              const float* b_prev_local, const float* b_prev2_local_or_null, float* b_out_local,
+                              const float* cbar_local, const float* tbar_local_or_null, float* acc_ws,
+                              int64_t n, int64_t nnz_hint, int64_t row_begin, int64_t row_end, int32_t f,
+                              int32_t app, int32_t k_max, int32_t n_scales, const float* coeffs_host,
+                              float op_scale, float op_shift, int32_t phase,
+                              const int32_t* delta_row_host, const int32_t* delta_col_host,
+                              const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+    EGNN_REQUIRE(dinv_full && iso_full && b_out_local && cbar_local && coeffs_host, "null pointer");
+    int rc = adjoint_sharded_check(n, row_begin, row_end, f, app, k_max, n_scales);
+    if (rc) return rc;
+    EGNN_REQUIRE(phase >= 0 && phase <= 2, "bad phase");
+    EGNN_REQUIRE(app == 0 || b_prev_local, "b_{m+1} rows missing");
+    EGNN_REQUIRE(vec_aligned(b_prev_full, f) && vec_aligned(b_prev_local, f) && vec_aligned(b_prev2_local_or_null, f) &&
+                 vec_aligned(b_out_local, f) && vec_aligned(cbar_local, f) && vec_aligned(tbar_local_or_null, f) &&
+                 vec_aligned(acc_ws, f), "b, cbar, tbar and acc_ws must be 16-byte aligned when f % 4 == 0");
+    const int64_t rows = row_end - row_begin;
+    if (rows == 0) return EGNN_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t slab_elems = (size_t)rows * (size_t)f;
+    const int m = k_max - app;
+    const float* tbar_m = tbar_local_or_null ? tbar_local_or_null + (size_t)m * slab_elems : nullptr;
+    if (app == 0) {
+        CoefRow c{};
+        for (int s = 0; s < n_scales; ++s) c.c[s] = coeffs_host[s * (k_max + 1) + k_max];
+        adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
+            cbar_local, tbar_m, dinv_full + row_begin, b_out_local, nullptr, rows, f, n_scales, f, c);
+        EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+        return EGNN_OK;
+    }
+    OrderParams p{};
+    p.delta.n = 0;
+    if (phase != 0) {                 // the flips (already transposed) ride with the launch that sees the exchange
+        rc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+        if (rc) return rc;
+        for (int i = 0; i < n_delta; ++i)
+            EGNN_REQUIRE(p.delta.row[i] >= 0 && p.delta.row[i] < n && p.delta.col[i] >= 0 && p.delta.col[i] < n,
+                         "delta index out of range");
+    }
+    p.vals = nullptr; p.dinv = dinv_full; p.iso = iso_full;
+    p.tprev_own = b_prev_local; p.tprev2_own = b_prev2_local_or_null; p.tk_own = b_out_local; p.y_own = nullptr;
+    p.out = nullptr; p.acc_ws = acc_ws; p.n_rows = rows; p.row0 = row_begin; p.F = f; p.S = n_scales;
+    p.a = op_scale; p.b = op_shift; p.first = 0; p.normalize = 0;
+    p.cbar = cbar_local; p.tbar = tbar_m; p.c_adj = m == 0 ? 1.f : 2.f;
+    for (int s = 0; s < n_scales; ++s) p.c_k[s] = coeffs_host[s * (k_max + 1) + m];
+    OrderConfig cfg = choose_config(rows, nnz_hint, f);
+    cfg.prescaled = false;            // sharded slabs carry plain b (what the exchange moves)
+    p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
+    if (phase == 0) {                 // local columns: gathers hit the rank's own slab
+        EGNN_REQUIRE(rowptr_local && acc_ws, "local half missing");
+        p.rowptr = rowptr_local; p.colidx = colidx_local;
+        p.gsrc = b_prev_local - row_begin * (int64_t)f;      // indexed by global column, only own rows touched
+        p.mode = 1;
+        return launch_order<true>(p, cfg, st);
+    }
+    EGNN_REQUIRE(b_prev_full != nullptr, "gathered b_{m+1} missing");
+    p.gsrc = b_prev_full;
+    if (phase == 1) {                 // remote columns + epilogue
+        EGNN_REQUIRE(rowptr_remote && acc_ws, "remote half missing");
+        p.rowptr = rowptr_remote; p.colidx = colidx_remote; p.mode = 2;
+    } else {                          // one launch over the unsplit rows
+        EGNN_REQUIRE(rowptr_local != nullptr, "csr missing");
+        p.rowptr = rowptr_local; p.colidx = colidx_local; p.mode = 0;
+    }
+    return launch_order<true>(p, cfg, st);
+}
+
+int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                              const int32_t* row_order_or_null, const float* dinv_full, const uint8_t* iso_full,
+                              const float* cbar_local, const float* tbar_local_or_null, float* xbar_local,
+                              int64_t n_global, int64_t row_begin, int64_t row_end, int32_t f, int32_t app,
+                              int32_t k_max, int32_t n_scales, const float* coeffs_host, float op_scale,
+                              float op_shift, const int32_t* delta_row_host, const int32_t* delta_col_host,
+                              const float* delta_val_host, int32_t n_delta, const egnn_peer_window* win,
+                              egnn_stream_t stream) {
+    EGNN_REQUIRE(rowptr_local && dinv_full && iso_full && cbar_local && coeffs_host && win, "null pointer");
+    int rc = adjoint_sharded_check(n_global, row_begin, row_end, f, app, k_max, n_scales);
+    if (rc) return rc;
+    EGNN_REQUIRE(f >= kWideMinF, "the wide sharded adjoint serves f >= 8");
+    EGNN_REQUIRE(k_max >= 1, "k_max = 0 has no application to exchange");
+    EGNN_REQUIRE(app < k_max || xbar_local || row_end == row_begin, "xbar rows missing");
+    EGNN_REQUIRE(vec_aligned(cbar_local, f) && vec_aligned(tbar_local_or_null, f) && vec_aligned(xbar_local, f),
+                 "cbar, tbar and xbar must be 16-byte aligned when f % 4 == 0");
+    rc = peer_check(win);
+    if (rc) return rc;
+    const int ldy = (f + 3) / 4 * 4;
+    EGNN_REQUIRE(win->f == ldy && (int64_t)win->world * win->rows_per >= n_global, "window does not fit the signal");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t rows = row_end - row_begin;
+    const size_t slab_elems = (size_t)rows * (size_t)f;
+    const int m = k_max - app;
+    const float* tbar_m = tbar_local_or_null ? tbar_local_or_null + (size_t)m * slab_elems : nullptr;
+    if (app == 0) {                   // b_K = v_K, its operand into buffer 0 of every window
+        CoefRow c{};
+        for (int s = 0; s < n_scales; ++s) c.c[s] = coeffs_host[s * (k_max + 1) + k_max];
+        PeerPush pp{};
+        fill_peer_push(pp, win, 0, true, true);
+        int64_t blocks = ceil_div64(rows > 0 ? rows * ldy : 1, 1024);        // at most one CTA per SM, as the forward's push
+        const int sms = device_sm_count();
+        if (blocks > sms) blocks = sms;
+        adjoint_prologue_push_kernel<<<(unsigned)blocks, 1024, 0, st>>>(cbar_local, tbar_m, dinv_full, rows, row_begin,
+                                                                       f, n_scales, ldy, c, pp);
+        EGNN_LAUNCH_CHECK("adjoint_prologue_push_kernel launch");
+        return EGNN_OK;
+    }
+    const RingConfig rcfg = ring_config(ldy);
+    WideParams wp{};
+    rc = fill_delta(wp.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    if (rc) return rc;
+    for (int i = 0; i < n_delta; ++i)
+        EGNN_REQUIRE(wp.delta.row[i] >= 0 && wp.delta.row[i] < n_global && wp.delta.col[i] >= 0 && wp.delta.col[i] < n_global,
+                     "delta index out of range");
+    wp.rowptr = rowptr_local; wp.colidx = colidx_local; wp.vals = nullptr;
+    wp.perm = row_order_or_null; wp.n_hub = row_order_or_null ? row_order_or_null + rows : nullptr;
+    wp.dinv = dinv_full; wp.iso = iso_full; wp.out = nullptr; wp.n_rows = rows; wp.row0 = row_begin;
+    wp.F = f; wp.ldy = ldy; wp.S = n_scales; wp.a = op_scale; wp.b = op_shift; wp.first = 0; wp.normalize = 0;
+    wp.ysrc = peer_operand(win, win->rank, (app - 1) & 1);                  // dinv (.) b_{m+1}, global rows
+    wp.x0_own = nullptr;
+    float* own_next = peer_operand(win, win->rank, app & 1) + row_begin * (int64_t)ldy;
+    wp.y2_own = app == 1 ? nullptr : own_next;                              // dinv (.) b_{m+2} of the own rows
+    wp.y_out = (m > 0 && win->world == 1) ? own_next : nullptr;             // single rank: plain store
+    wp.tk_out = m == 0 ? xbar_local : nullptr;
+    wp.cbar = cbar_local; wp.tbar = tbar_m; wp.c_adj = m == 0 ? 1.f : 2.f;
+    for (int s = 0; s < n_scales; ++s) wp.c_k[s] = coeffs_host[s * (k_max + 1) + m];
+    fill_peer_push(wp.peer, win, app & 1, m > 0, false);
+    return launch_wide<true>(wp, rcfg, device_sm_count(), st);
 }
 
 int egnn_graph_prep_sharded(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_or_null,

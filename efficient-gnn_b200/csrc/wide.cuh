@@ -72,9 +72,10 @@ struct WideParams {
     float c_k[EGNN_MAX_SCALES];
     DeltaList delta;
     PeerPush peer;              // world > 1: y_out rows also go to every rank's exchange window
-    // adjoint instantiation (ADJ, single GPU): b_k = c_adj * (M^T b_{k+1}) - b_{k+2} + v_k with
+    // adjoint instantiation (ADJ): b_k = c_adj * (M^T b_{k+1}) - b_{k+2} + v_k with
     // v_k = tbar + sum_s c_k[s] * cbar[:, s, :]; ysrc = dinv (.) b_{k+1}, y2_own = dinv (.) b_{k+2}
-    // (NULL: zero), y_out = dinv (.) b_k, tk_out = b_k (the last application: the signal's gradient)
+    // (NULL: zero), y_out = dinv (.) b_k, tk_out = b_k (the last application: the signal's gradient).
+    // ADJ with PEER (row-sharded): dinv (.) b_k goes to every rank's window as the forward's T_k does.
     const float* cbar;          // [n_rows, S, F]
     const float* tbar;          // [n_rows, F] or NULL
     float c_adj;
@@ -200,6 +201,13 @@ __device__ __forceinline__ void wide_epilogue(const WideParams& p, int row, int 
         }
         if (p.tk_out) store_user4<ALIGNED>(p.tk_out, uoff, ncol, pol_stream, b);
         if (p.y_out) *reinterpret_cast<float4*>(p.y_out + yoff) = make_float4(di * b[0], di * b[1], di * b[2], di * b[3]);
+        if constexpr (PEER) {                                   // row-sharded: dinv (.) b_k into every rank's window
+            if (p.peer.has_data) {
+                const float4 yv = make_float4(di * b[0], di * b[1], di * b[2], di * b[3]);
+                const int64_t goff = (int64_t)grow * ldy + fcol;
+                for (int r = 0; r < p.peer.world; ++r) *reinterpret_cast<float4*>(p.peer.dst[r] + goff) = yv;
+            }
+        }
         return;
     }
     float tk[4] = {0.f, 0.f, 0.f, 0.f}, xprev[4] = {0.f, 0.f, 0.f, 0.f};

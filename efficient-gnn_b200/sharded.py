@@ -13,6 +13,9 @@ Rank r owns rows ``[r * rows_per, (r + 1) * rows_per)`` of the CSR, of
   operand ``dinv * T_{k-1}`` (0.93 MB at Reddit size) is gathered, then the
   shared-memory SpMV + epilogue run on the local rows.
 
+The backward (autograd w.r.t. the local signal and ``s``) runs the adjoint applications the same
+way over the rank's rows of the transposed adjacency (DESIGN.md section 12).
+
 The compute engine is injectable so the host logic (partition, column split,
 exchange order, buffer rotation) is testable on CPU with the gloo backend;
 the product engine is :class:`CudaEngine` (C ABI, no fallback).
@@ -29,9 +32,10 @@ from typing import Optional
 import numpy as np
 import torch
 import torch.distributed as dist
+from torch.autograd.function import once_differentiable
 
 from . import _cabi
-from .wats import WIDE_MIN_F, heat_coefficients
+from .wats import WIDE_MIN_F, _needs_grad, heat_coefficients
 
 __all__ = ["RowPartition", "BalancedOrder", "split_columns", "CudaEngine", "DistComm", "PeerExchange", "ShardedWavelet"]
 
@@ -288,6 +292,39 @@ class CudaEngine:
             n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), 1 if normalize else 0,
             *_delta_args(deltas), C.byref(window), _stream()), "egnn_wide_order_sharded")
 
+    # -- backward ------------------------------------------------------------------
+    def adjoint(self, phase, local, remote, dinv, iso, b_prev_full, b_prev_local, b_prev2_local, b_out_local, cbar,
+                tbar, acc_ws, n_global, nnz_hint, row_begin, row_end, f, app, k_max, n_scales, coeffs, op_scale,
+                op_shift, deltas_t=None):
+        """Application ``app`` of the adjoint on the rank's rows (include/egnn_b200.h
+        ``egnn_cheb_adjoint_sharded``); ``deltas_t``: the forward's flips, rows and columns swapped."""
+        lp, lc = (None, None) if local is None else local
+        rp, rc = (None, None) if remote is None else remote
+        _cabi.check(self.lib.egnn_cheb_adjoint_sharded(
+            _cabi.ptr(lp), _cabi.ptr(lc), _cabi.ptr(rp), _cabi.ptr(rc), _cabi.ptr(dinv), _cabi.ptr(iso),
+            _cabi.ptr(b_prev_full), _cabi.ptr(b_prev_local), _cabi.ptr(b_prev2_local), _cabi.ptr(b_out_local),
+            _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(acc_ws), n_global, nnz_hint, row_begin, row_end, f, app,
+            k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), phase,
+            *_delta_args(deltas_t), _stream()), "egnn_cheb_adjoint_sharded")
+
+    def wide_adjoint(self, rowptr, colidx, row_order, dinv, iso, cbar, tbar, xbar, n_global, row_begin, row_end, f,
+                     app, k_max, n_scales, coeffs, op_scale, op_shift, window, deltas_t=None):
+        _cabi.check(self.lib.egnn_wide_adjoint_sharded(
+            _cabi.ptr(rowptr), _cabi.ptr(colidx), _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
+            _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar), n_global, row_begin, row_end, f, app, k_max, n_scales,
+            coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), *_delta_args(deltas_t),
+            C.byref(window), _stream()), "egnn_wide_adjoint_sharded")
+
+    def coeff_grad(self, cbar, t_all):
+        """``G[s, k] = <cbar[:, s, :], T_k>`` of the local rows, float64 (egnn_cheb_coeff_grad)."""
+        from .wats import _coeff_grad
+        return _coeff_grad(cbar, t_all)
+
+    def l1_normalize(self, comb):
+        """Out-of-place row L1 normalisation with its backward (egnn_l1_normalize)."""
+        from .wats import _L1Normalize
+        return _L1Normalize.apply(comb)
+
     # -- stream plumbing ---------------------------------------------------------
     def side_stream(self):
         return torch.cuda.stream(self.comm_stream)
@@ -319,6 +356,14 @@ class DistComm:
             dist.all_gather_into_tensor(full, slab, group=self.group)
         else:
             full.copy_(slab)
+
+    def alltoall(self, out, inp, out_splits, in_splits):
+        """Rows ``inp[sum(in_splits[:r]) ...]`` go to rank r; ``out`` receives rank r's rows for this
+        rank at ``sum(out_splits[:r])`` (``all_to_all_single``: NCCL and gloo)."""
+        if self.world > 1:
+            dist.all_to_all_single(out, inp, out_splits, in_splits, group=self.group)
+        else:
+            out.copy_(inp)
 
 
 class PeerExchange:
@@ -392,14 +437,71 @@ class PeerExchange:
         self._opened, self._own = [], None
 
 
+class _ShardedSpec:
+    """Everything of one sharded pass but its differentiable inputs: ``s`` holds the scales' values."""
+
+    def __init__(self, k, s, lambda_max, want_orders, deltas):
+        self.k, self.s, self.lambda_max, self.want_orders, self.deltas = k, s, lambda_max, want_orders, deltas
+
+
+class _ShardedPass(torch.autograd.Function):
+    """``(C [rows, S, F], T [K+1, rows, F])`` of the rank's rows of one un-normalised pass as a function
+    of the local signal ``x0`` (None: the default signal) and the scales ``s`` (None when they need no
+    gradient).  ``T`` is empty unless the orders are wanted or ``s`` needs a gradient.  Backward: the
+    adjoint pass over the transposed shard (:meth:`ShardedWavelet._adjoint`) and the scale gradient from
+    every rank's float64 partials (:meth:`ShardedWavelet._scale_grad`); both are collective."""
+
+    @staticmethod
+    def forward(ctx, x0, s, sw, spec):
+        ctx.set_materialize_grads(False)
+        s_grad = s is not None and ctx.needs_input_grad[1]
+        want = spec.want_orders or s_grad
+        res = sw._pass(spec.k, spec.s, None if x0 is None else x0.detach(), spec.lambda_max, False, want, spec.deltas)
+        f = 1 if (x0 is None or x0.dim() == 1) else int(x0.shape[1])
+        if want:
+            _, orders, comb = res
+            t_all = torch.stack([o.reshape(sw.rows, f) for o in orders])
+        else:
+            comb = res
+            t_all = comb.new_empty((0,))
+            ctx.mark_non_differentiable(t_all)
+        comb = comb.reshape(sw.rows, -1, f)
+        ctx.sw, ctx.spec, ctx.f = sw, spec, f
+        ctx.x_shape = None if x0 is None else x0.shape
+        ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
+        ctx.save_for_backward(t_all if s_grad else None)
+        return comb, t_all
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_comb, g_orders):
+        sw, spec, f = ctx.sw, ctx.spec, ctx.f
+        (t_all,) = ctx.saved_tensors
+        n_scales = int(np.atleast_1d(spec.s).shape[0])
+        cbar = (_cabi.vec_ready(g_comb) if g_comb is not None else
+                torch.zeros((sw.rows, n_scales, f), dtype=torch.float32, device=sw.device))
+        tbar = _cabi.vec_ready(g_orders) if (g_orders is not None and g_orders.numel()) else None
+        x_grad = s_grad = None
+        if ctx.needs_input_grad[0]:
+            x_grad = sw._adjoint(spec, cbar, tbar, f).reshape(ctx.x_shape)
+        if ctx.needs_input_grad[1]:
+            shape, dev, dtype = ctx.s_meta
+            s_grad = sw._scale_grad(spec, cbar, t_all).to(device=dev, dtype=dtype).reshape(shape)
+        return x_grad, s_grad, None, None
+
+
 class ShardedWavelet:
     """Wavelet features of a row-sharded graph.
 
     ``rowptr_local`` / ``colidx_local``: the rank's rows (global column ids),
     rows assigned by :class:`RowPartition`.  ``engine`` defaults to the CUDA
     engine; tests inject a CPU engine to drive this logic over gloo.
-    Forward-only: the sharded pass has no backward (single-GPU
-    ``graph_wavelet_features`` does).
+
+    :meth:`features` is differentiable w.r.t. ``X0_local`` and a tensor ``s``
+    (DESIGN.md section 12).  The backward is collective, like DDP's: every rank
+    calls ``backward`` on a loss of its own rows, and the gradients are those of
+    the sum of the ranks' losses.  The adjacency and ``lambda_max`` get no
+    gradient here (single-GPU ``graph_wavelet_features`` gives those).
     """
 
     def __init__(self, rowptr_local, colidx_local, n_global: int, *, group=None, engine=None, device=None,
@@ -480,6 +582,8 @@ class ShardedWavelet:
                 pad[:self.rows] = rowsum_local
                 self._allgather(full, pad)
                 self._rowsum_full = full[:self.n].clone()
+        self._adjoint_shard = None     # what the backward gathers over (built on first use, see _adjoint_csr)
+        self._adjoint_order = None
         self.launches = 0
 
     def _wide_window(self, ldy: int):
@@ -535,7 +639,39 @@ class ShardedWavelet:
         per-perturbation recompute (calib_attack/calib_fga.py:868,908,952) on a
         graph that spans several GPUs.  Every rank passes the same list; each
         patches its replicated dinv/iso and the x0 of its own rows, and the
-        order kernels add the flipped entries of the rows they own."""
+        order kernels add the flipped entries of the rows they own.
+
+        Differentiable w.r.t. ``X0_local`` and a 0-d / 1-d tensor ``s`` when
+        grad mode is on and one of them requires grad: every output then
+        carries a ``grad_fn`` (``deltas=`` is supported).  ``X0_local.grad``
+        receives this rank's rows of the gradient and ``s.grad`` the full scale
+        gradient, identical bits on every rank.  The backward is collective:
+        every rank must call ``backward`` (once per call of ``features``, in
+        the same order on every rank), with the same inputs requiring grad."""
+        x_in = None if X0_local is None else torch.as_tensor(X0_local)
+        if _needs_grad(self.x0 if x_in is None else x_in, s):
+            return self._features_grad(int(k), s, x_in, lambda_max, normalize, return_parts, deltas)
+        return self._pass(k, s, X0_local, lambda_max, normalize, return_parts, deltas)
+
+    def _features_grad(self, k, s, x_in, lambda_max, normalize, return_parts, deltas):
+        """The differentiable pass: un-normalised combination (and the orders when wanted) through
+        :class:`_ShardedPass`, then the out-of-place normalisation (as ``graph_wavelet_features``)."""
+        s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
+        if deltas is None or len(deltas[0]) == 0:
+            deltas = None
+        x0 = x_in
+        if x0 is not None:
+            x0 = x0.to(device=self.device, dtype=torch.float32)
+        spec = _ShardedSpec(k, s_vals, float(lambda_max), return_parts, deltas)
+        s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
+        comb, t_all = _ShardedPass.apply(x0, s_in, self, spec)
+        feats = self.engine.l1_normalize(comb) if normalize else comb
+        feats = feats.reshape(self.rows, -1)
+        if return_parts:
+            return feats, [t_all[i] for i in range(k + 1)], comb
+        return feats
+
+    def _pass(self, k, s, X0_local, lambda_max, normalize, return_parts, deltas):
         eng, dev = self.engine, self.device
         k = int(k)
         coeffs = np.ascontiguousarray(heat_coefficients(k, s), dtype=np.float32)
@@ -695,6 +831,138 @@ class ShardedWavelet:
         full = torch.empty((self.world * rp, local_feats.shape[1]), dtype=local_feats.dtype, device=local_feats.device)
         self._allgather(full, pad)
         return full[:self.n]
+
+    # -- backward ------------------------------------------------------------------
+    def _adjoint_csr(self):
+        """``(rowptr, colidx, local half, remote half)`` the adjoint gathers over: this rank's rows of
+        ``A^T`` (the columns ``[row_begin, row_end)`` of A, whose entries every rank holds some of),
+        global column ids, rows sorted.  Built once, collectively (one ``all_to_all`` of the entries);
+        when every rank's transpose equals its own shard (every symmetric graph with sorted rows) the
+        copy is dropped and the forward's CSR, halves and row order are used."""
+        if self._adjoint_shard is None:
+            dev, n, world = self.device, self.n, self.world
+            counts = (self.rowptr[1:] - self.rowptr[:-1]).long()
+            rows_g = torch.repeat_interleave(torch.arange(self.rows, dtype=torch.int64, device=dev) + self.row_begin,
+                                             counts)
+            cols = self.colidx.long()
+            owner = torch.div(cols, self.part.rows_per, rounding_mode="floor")
+            by_owner = torch.argsort(owner, stable=True)
+            send = torch.stack([cols[by_owner], rows_g[by_owner]], dim=1).contiguous()    # (row, column) in A^T
+            send_counts = torch.bincount(owner, minlength=world)
+            recv_counts = torch.empty_like(send_counts)
+            self.comm.alltoall(recv_counts, send_counts, [1] * world, [1] * world)
+            recv = torch.empty((int(recv_counts.sum()), 2), dtype=torch.int64, device=dev)
+            self.comm.alltoall(recv, send, recv_counts.tolist(), send_counts.tolist())
+            key = ((recv[:, 0] - self.row_begin) * n + recv[:, 1]).sort().values
+            rowptr_t = torch.zeros(self.rows + 1, dtype=torch.int64, device=dev)
+            rowptr_t[1:] = torch.cumsum(torch.bincount(torch.div(key, n, rounding_mode="floor"), minlength=self.rows), 0)
+            rowptr_t, colidx_t = rowptr_t.to(torch.int32), (key % n).to(torch.int32)
+            same = torch.equal(rowptr_t, self.rowptr) and torch.equal(colidx_t, self.colidx)
+            differs = torch.tensor([0.0 if same else 1.0], dtype=torch.float64, device=dev)
+            self._allreduce(differs)
+            if float(differs.item()) == 0.0:
+                self._adjoint_shard = False
+            else:
+                self._adjoint_shard = (rowptr_t, colidx_t) + split_columns(rowptr_t, colidx_t, self.row_begin,
+                                                                           self.row_end)
+        if self._adjoint_shard is False:
+            return self.rowptr, self.colidx, self.local_half, self.remote_half
+        return self._adjoint_shard
+
+    def _adjoint_row_order(self):
+        """egnn_row_order of :meth:`_adjoint_csr` (the fused wide adjoint's processing order)."""
+        rowptr = self._adjoint_csr()[0]
+        if self._adjoint_shard is False:
+            if self._row_order is None:
+                self._row_order = self.engine.row_order(self.rowptr, self.rows)
+            return self._row_order
+        if self._adjoint_order is None:
+            self._adjoint_order = self.engine.row_order(rowptr, self.rows)
+        return self._adjoint_order
+
+    def _adjoint(self, spec, cbar, tbar, f):
+        """This rank's rows of the signal's gradient ``[rows, F]`` from its rows of ``cbar`` ``[rows, S, F]``
+        and ``tbar`` ``[K+1, rows, F]`` (collective: the operand of every application is exchanged).  The
+        forward's flips are applied transposed, with the forward's patched ``dinv`` / ``iso``."""
+        eng, dev, k = self.engine, self.device, spec.k
+        coeffs = np.ascontiguousarray(heat_coefficients(k, spec.s), dtype=np.float32)
+        n_scales = coeffs.shape[0]
+        op_scale, op_shift = 2.0 / spec.lambda_max, -1.0
+        dinv, iso, deltas_t = self.dinv, self.iso, None
+        if spec.deltas is not None:
+            dinv, iso, _ = eng.patch_degrees(self.dinv, self.iso, self.x0, self.n, self.row_begin, self.rows,
+                                             spec.deltas)
+            d_rows, d_cols, d_vals = spec.deltas
+            deltas_t = (d_cols, d_rows, d_vals)
+        if self.rows == 0:            # the fused kernels still take part in the exchange: valid pointers
+            cbar = torch.zeros((1, n_scales, f), dtype=torch.float32, device=dev)
+        xbar = torch.empty((max(1, self.rows), f), dtype=torch.float32, device=dev)
+        coef = (k, n_scales, coeffs, op_scale, op_shift)
+        if k == 0:                    # xbar = v_0: no operator application, nothing exchanged
+            if self.rows:
+                eng.adjoint(2, None, None, dinv, iso, None, None, None, xbar, cbar, tbar, None, self.n, 1,
+                            self.row_begin, self.row_end, f, 0, *coef)
+                self.launches += 1
+            return xbar[:self.rows]
+        rowptr_t, colidx_t, local, remote = self._adjoint_csr()
+        if self.fused_wide and f >= WIDE_MIN_F:
+            # exchange fused: the operand dinv (.) b travels through the forward's window and flags
+            win = self._wide_window((f + 3) // 4 * 4).window
+            order = self._adjoint_row_order()
+            for app in range(k + 1):
+                eng.wide_adjoint(rowptr_t, colidx_t, order, dinv, iso, cbar, tbar, xbar, self.n, self.row_begin,
+                                 self.row_end, f, app, *coef, win, deltas_t)
+                self.launches += 1
+            return xbar[:self.rows]
+        # generic CSR kernel, local / remote column halves around the exchange of b_{m+1} (as the forward)
+        rp = self.part.rows_per
+
+        def slab():
+            return torch.empty((rp, f), dtype=torch.float32, device=dev)
+
+        tail = (self.n, max(1, int(colidx_t.numel())), self.row_begin, self.row_end, f)
+        b_prev = slab()
+        if self.rows:
+            eng.adjoint(2, None, None, dinv, iso, None, None, None, b_prev, cbar, tbar, None, *tail, 0, *coef)
+            self.launches += 1
+        b_prev2 = None
+        full = torch.empty((self.world * rp, f), dtype=torch.float32, device=dev)
+        acc_ws = slab()
+        for app in range(1, k + 1):
+            m = k - app
+            b_out = xbar if m == 0 else (slab() if app <= 2 else b_prev2)    # in place over b_{m+2}
+            eng.fork()
+            with eng.side_stream():
+                self._allgather(full, b_prev)
+            if self.rows:
+                eng.adjoint(0, local, None, dinv, iso, None, b_prev, b_prev2, b_out, cbar, tbar, acc_ws, *tail, app,
+                            *coef)
+            eng.join()
+            if self.rows:
+                eng.adjoint(1, None, remote, dinv, iso, full, b_prev, b_prev2, b_out, cbar, tbar, acc_ws, *tail, app,
+                            *coef, deltas_t=deltas_t)
+                self.launches += 2
+            b_prev2, b_prev = b_prev, b_out
+        return xbar[:self.rows]
+
+    def _scale_grad(self, spec, cbar, t_all):
+        """``ds_j = -sum_k k alpha[j,k] G[j,k]`` with ``G = sum_r <cbar_r, T_r>`` over the ranks' rows: every
+        rank's float64 partial is all-gathered and added in rank order, so each rank holds the same bits."""
+        coeffs = heat_coefficients(spec.k, spec.s)
+        n_scales, k1 = coeffs.shape
+        if self.rows:
+            g = self.engine.coeff_grad(cbar, t_all)
+        else:
+            g = torch.zeros((n_scales, k1), dtype=torch.float64, device=self.device)
+        full = torch.empty((self.world * n_scales, k1), dtype=torch.float64, device=self.device)
+        self._allgather(full, g.contiguous())
+        parts = full.reshape(self.world, n_scales, k1)
+        total = parts[0]
+        for r in range(1, self.world):
+            total = total + parts[r]
+        alpha = torch.from_numpy(coeffs).to(self.device)
+        kk = torch.arange(k1, dtype=torch.float64, device=self.device)
+        return -(kk * alpha * total).sum(dim=1)
 
 
 # --------------------------------------------------------------------------- #

@@ -19,7 +19,8 @@ an autograd function whose backward is the adjoint (Clenshaw) pass of
 ``egnn_cheb_adjoint``.  ``graph_wavelet_features`` is also differentiable w.r.t. a
 dense or sparse COO adjacency tensor and a 0-d tensor ``lambda_max`` (DESIGN.md
 section 11).  Otherwise nothing changes: same kernels, nothing saved.
-``WATS``, ``WaveletSession`` and the sharded path stay forward-only.
+``WATS`` and ``WaveletSession`` stay forward-only; the sharded path's gradients w.r.t. the
+signal and ``s`` are ``ShardedWavelet``'s (DESIGN.md section 12).
 """
 from __future__ import annotations
 

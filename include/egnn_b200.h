@@ -547,6 +547,58 @@ int egnn_wide_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_l
                             const float* delta_val_host, int32_t n_delta,
                             const egnn_peer_window* win, egnn_stream_t stream);
 
+/* ---- backward of the row-sharded pass (new in ABI 9) ------------------------
+ * The Clenshaw sum of egnn_cheb_adjoint on the rows [row_begin, row_end) a
+ * rank owns, one call per application: app = 0 is the prologue b_K = v_K, app
+ * = 1..K produces b_m with m = K - app (m = 0: the signal's gradient xbar).
+ * The CSR is the rank's rows of the TRANSPOSED adjacency (global column ids,
+ * rows sorted), or the rank's own shard when every shard equals its
+ * transpose; dinv_full / iso_full are the forward's (patched when it had
+ * flips).  cbar_local [rows, n_scales, f] and tbar_local_or_null [K+1, rows, f]
+ * are the rank's rows of the upstream gradients.  delta_*: the forward's flips
+ * with rows and columns swapped, GLOBAL ids.
+ *
+ * egnn_cheb_adjoint_sharded: the generic CSR kernel's adjoint instantiation
+ * with the phases of egnn_cheb_order_sharded (0: local columns -> acc_ws while
+ * the exchange of b_{m+1} is in flight, 1: remote columns + epilogue, 2: the
+ * unsplit rows).  app 0 writes b_K to b_out_local and ignores the CSR and the
+ * phase.  b_prev_full: the exchanged [n, f] b_{m+1}; b_prev_local /
+ * b_prev2_local_or_null: the rank's b_{m+1} / b_{m+2} rows (NULL at app 1);
+ * b_out_local receives b_m (may alias b_prev2_local).  Every array is
+ * accessed with 16-byte vectors when f % 4 == 0 and must then be 16-byte
+ * aligned, else EGNN_ERR_INVALID_ARG and nothing is launched.                */
+int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                              const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                              const float* dinv_full, const uint8_t* iso_full, const float* b_prev_full,
+                              const float* b_prev_local, const float* b_prev2_local_or_null,
+                              float* b_out_local, const float* cbar_local,
+                              const float* tbar_local_or_null, float* acc_ws,
+                              int64_t n, int64_t nnz_hint, int64_t row_begin, int64_t row_end,
+                              int32_t f, int32_t app, int32_t k_max, int32_t n_scales,
+                              const float* coeffs_host, float op_scale, float op_shift, int32_t phase,
+                              const int32_t* delta_row_host, const int32_t* delta_col_host,
+                              const float* delta_val_host, int32_t n_delta, egnn_stream_t stream);
+
+/* egnn_wide_adjoint_sharded: f >= 8, k_max >= 1, the exchange fused through
+ * the forward's window (win->f = f rounded up to a multiple of 4) and its
+ * flag protocol.  app 0 forms b_K and stores dinv (.) b_K into buffer 0 of
+ * every rank's window after every peer has finished the kernels before it;
+ * app j runs the wide kernel's adjoint instantiation against buffer (j-1)&1
+ * after the peers' flags and stores dinv (.) b_m of the own rows into buffer
+ * j&1 of every window; app K writes xbar_local [rows, f] instead.
+ * row_order_or_null: egnn_row_order of the CSR passed.  cbar, tbar and xbar
+ * must be 16-byte aligned when f % 4 == 0, else EGNN_ERR_INVALID_ARG.        */
+int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                              const int32_t* row_order_or_null, const float* dinv_full,
+                              const uint8_t* iso_full, const float* cbar_local,
+                              const float* tbar_local_or_null, float* xbar_local,
+                              int64_t n_global, int64_t row_begin, int64_t row_end,
+                              int32_t f, int32_t app, int32_t k_max, int32_t n_scales,
+                              const float* coeffs_host, float op_scale, float op_shift,
+                              const int32_t* delta_row_host, const int32_t* delta_col_host,
+                              const float* delta_val_host, int32_t n_delta,
+                              const egnn_peer_window* win, egnn_stream_t stream);
+
 /* Degree pass of a row shard (scipy semantics as egnn_graph_prep).  phase 0:
  * row sums of the local rows, their diagonal entries into diag_full[row_begin..]
  * and the shard's contribution to the in-degree in colsum_full (both zeroed
