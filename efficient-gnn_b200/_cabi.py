@@ -13,7 +13,7 @@ import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("EGNN_LIB_PATH") or os.path.join(_HERE, "lib", "libegnn_b200.so")   # override: tuning builds
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 # every symbol include/egnn_b200.h declares: name -> (restype, argtypes)
 _P, _I32, _I64, _F32, _SZ = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -92,7 +92,7 @@ class SellPlanStruct(C.Structure):
                 ("n_slices", C.c_int64), ("n_vrows", C.c_int64), ("n_entries", C.c_int64), ("n_rowv", C.c_int64),
                 ("slice_off", C.c_void_p), ("blk_slice_ptr", C.c_void_p), ("idx", C.c_void_p),
                 ("rv_ptr", C.c_void_p), ("vslot", C.c_void_p), ("cta_info", C.c_void_p), ("vpart", C.c_void_p),
-                ("sched", C.c_void_p), ("stamps", C.c_void_p)]
+                ("sched", C.c_void_p), ("stamps", C.c_void_p), ("n_hub", C.c_int64), ("hub", C.c_void_p)]
 
 
 MAX_RANKS = 16

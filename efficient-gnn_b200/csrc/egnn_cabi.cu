@@ -277,7 +277,7 @@ static void fill_peer_push(PeerPush& pp, const egnn_peer_window* w, int which, b
 // ---- the narrow-path step kernel (sell_step.cuh) ------------------------------
 static void step_fill_plan(SellStepParams& sp, const egnn_sell_plan* pl) {
     sp.idx = pl->idx; sp.slice_off = pl->slice_off; sp.blk_slice_ptr = pl->blk_slice_ptr; sp.vslot = pl->vslot;
-    sp.cta_info = pl->cta_info; sp.rv_ptr = pl->rv_ptr; sp.vpart = pl->vpart; sp.sched = pl->sched;
+    sp.cta_info = pl->cta_info; sp.hub = pl->hub; sp.rv_ptr = pl->rv_ptr; sp.vpart = pl->vpart; sp.sched = pl->sched;
     sp.stamps = (unsigned long long*)pl->stamps;
     sp.trace = pl->reserved;          // diagnostic: per-CTA trace behind the stamps (scripts/time_step.py)
     sp.n_cta = pl->n_cta; sp.C = pl->n_blocks; sp.CB = pl->col_block; sp.n_cols = pl->n_cols;
@@ -347,7 +347,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 9; }
+int egnn_abi_version(void) { return 10; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -632,7 +632,7 @@ int egnn_cheb_wavelet(const int32_t* rowptr, const int32_t* colidx, const float*
     if (sell_plan) {
         EGNN_REQUIRE(f == 1 && vals_or_null == nullptr, "the SELL plan serves F = 1 on a binary adjacency");
         EGNN_REQUIRE(sell_plan->n == n && sell_plan->n_cols == n && sell_plan->row0 == 0 && sell_plan->vpart && sell_plan->slice_off && sell_plan->blk_slice_ptr &&
-                     sell_plan->rv_ptr && sell_plan->vslot && sell_plan->cta_info && sell_plan->sched, "SELL plan does not match the graph or is not filled");
+                     sell_plan->rv_ptr && sell_plan->vslot && sell_plan->cta_info && sell_plan->hub && sell_plan->sched, "SELL plan does not match the graph or is not filled");
         // all K orders in one persistent launch (sell_step.cuh); the first operand dinv (.) T_0 is
         // computed inside it
         SellStepParams sp{};
@@ -1292,6 +1292,8 @@ int egnn_sell_prepare(const int32_t* rowptr, const int32_t* colidx, int64_t n, i
     rc = check_cuda(cub::DeviceScan::ExclusiveSum(w.cub_temp, tb, w.slice_sz, w.slice_off, (int)(w.smax + 1), st), "scan slices"); if (rc) return rc;
     sell_totals_kernel<<<1, 32, 0, st>>>(w.slice_off, w.rv_ptr, (int)n, w.totals);
     EGNN_LAUNCH_CHECK("sell_totals_kernel launch");
+    sell_hub_count_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, st>>>(w.rv_ptr, (int)n, w.totals);
+    EGNN_LAUNCH_CHECK("sell_hub_count_kernel launch");
     int64_t tot[8];
     rc = check_cuda(cudaMemcpyAsync(tot, w.totals, 64, cudaMemcpyDeviceToHost, st), "copy totals"); if (rc) return rc;
     rc = check_cuda(cudaStreamSynchronize(st), "sync"); if (rc) return rc;
@@ -1301,6 +1303,7 @@ int egnn_sell_prepare(const int32_t* rowptr, const int32_t* colidx, int64_t n, i
     plan->n_slices = tot[kTotSlices];
     plan->n_entries = tot[kTotEntries];
     plan->n_rowv = tot[kTotRowV];
+    plan->n_hub = tot[kTotHub];
     return EGNN_OK;
 }
 
@@ -1309,7 +1312,9 @@ int egnn_sell_fill(const int32_t* rowptr, const int32_t* colidx, int64_t n, int6
     int rc = sell_check_geometry(n, nnz, plan);
     if (rc) return rc;
     (void)rowptr;
-    EGNN_REQUIRE(plan->slice_off && plan->blk_slice_ptr && plan->rv_ptr && plan->cta_info && plan->sched, "plan buffers not allocated");
+    EGNN_REQUIRE(plan->slice_off && plan->blk_slice_ptr && plan->rv_ptr && plan->cta_info && plan->sched && plan->hub,
+                 "plan buffers not allocated");
+    EGNN_REQUIRE(plan->n_hub >= 0 && plan->n_hub <= n, "n_hub out of range");
     EGNN_REQUIRE(plan->n_cta >= 1 && plan->n_cta <= 4096, "n_cta out of range");
     EGNN_REQUIRE(plan->n_entries == 0 || plan->idx, "plan idx not allocated");
     EGNN_REQUIRE(plan->n_vrows == 0 || plan->vslot, "plan vslot not allocated");
@@ -1325,14 +1330,22 @@ int egnn_sell_fill(const int32_t* rowptr, const int32_t* colidx, int64_t n, int6
     rc = check_cuda(cudaMemcpyAsync(plan->rv_ptr, w.rv_ptr, 4 * (n + 1), cudaMemcpyDeviceToDevice, st), "copy rv_ptr"); if (rc) return rc;
     sell_cta_blocks_kernel<<<1, 32, 0, st>>>(w.slice_off, w.bsp, C, plan->n_cta, plan->cta_info, plan->sched);
     EGNN_LAUNCH_CHECK("sell_cta_blocks_kernel launch");
-    // epilogue row ranges balanced by cost (nvrow / nv of the workspace are free again: reused for the costs and their prefix)
-    sell_row_cost_kernel<<<(unsigned)ceil_div64(n + 1, 256), 256, 0, st>>>(w.rv_ptr, (int)n, w.nvrow);
+    // epilogue row ranges balanced by cost, and the hub rows of every range (nvrow / nv / u_off / key
+    // of the workspace are free again: reused for the costs, the hub flags and their prefixes)
+    int32_t* hub_flag = w.u_off;
+    int32_t* hub_prefix = reinterpret_cast<int32_t*>(w.key);
+    int32_t* cta_rows = plan->cta_info + 2 * plan->n_cta + kSellMaxBlocks;
+    sell_row_cost_kernel<<<(unsigned)ceil_div64(n + 1, 256), 256, 0, st>>>(w.rv_ptr, (int)n, w.nvrow, hub_flag);
     EGNN_LAUNCH_CHECK("sell_row_cost_kernel launch");
     size_t tb = w.cub_bytes;
     rc = check_cuda(cub::DeviceScan::ExclusiveSum(w.cub_temp, tb, w.nvrow, w.nv, (int)(n + 1), st), "scan row costs"); if (rc) return rc;
-    sell_cta_rows_kernel<<<(unsigned)ceil_div64(plan->n_cta + 1, 128), 128, 0, st>>>(w.nv, (int)n, plan->n_cta,
-                                                                                 plan->cta_info + 2 * plan->n_cta + kSellMaxBlocks);
+    sell_cta_rows_kernel<<<(unsigned)ceil_div64(plan->n_cta + 1, 128), 128, 0, st>>>(w.nv, (int)n, plan->n_cta, cta_rows);
     EGNN_LAUNCH_CHECK("sell_cta_rows_kernel launch");
+    tb = w.cub_bytes;
+    rc = check_cuda(cub::DeviceScan::ExclusiveSum(w.cub_temp, tb, hub_flag, hub_prefix, (int)(n + 1), st), "scan hub flags"); if (rc) return rc;
+    sell_cta_hubs_kernel<<<(unsigned)ceil_div64(n > plan->n_cta ? n : plan->n_cta + 1, 256), 256, 0, st>>>(
+        hub_flag, hub_prefix, cta_rows, (int)n, plan->n_cta, plan->hub);
+    EGNN_LAUNCH_CHECK("sell_cta_hubs_kernel launch");
     if (plan->n_slices > 0) {
         rc = check_cuda(cudaFuncSetAttribute(sell_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSellFillSmem),
                         "cudaFuncSetAttribute(sell_fill_kernel)");
@@ -1356,7 +1369,7 @@ int egnn_sell_step_sharded(const egnn_sell_plan* plan, const float* dinv_full, c
                            const egnn_peer_window* win, egnn_stream_t stream) {
     EGNN_REQUIRE(plan && dinv_full && iso_full && out_local && coeffs_host, "null pointer");
     EGNN_REQUIRE((w_base_or_null == nullptr) == (rowsum_base_or_null == nullptr), "w_base and rowsum_base come together");
-    EGNN_REQUIRE(plan->vpart && plan->slice_off && plan->blk_slice_ptr && plan->rv_ptr && plan->vslot && plan->cta_info && plan->sched,
+    EGNN_REQUIRE(plan->vpart && plan->slice_off && plan->blk_slice_ptr && plan->rv_ptr && plan->vslot && plan->cta_info && plan->hub && plan->sched,
                  "SELL plan is not filled");
     EGNN_REQUIRE(order_begin >= 1 && order_begin <= order_end && order_end <= k_max && k_max <= EGNN_MAX_ORDER, "bad order range");
     EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");

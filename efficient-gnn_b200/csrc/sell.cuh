@@ -49,7 +49,7 @@ constexpr int kSellGroup = 8;           // indices per 16-byte load
 constexpr int kSellMaxBlocks = 64;
 
 // totals the host needs after the prepare pass (device int64[8])
-enum SellTotals { kTotU = 0, kTotV = 1, kTotSlices = 2, kTotEntries = 3, kTotRowV = 4 };
+enum SellTotals { kTotU = 0, kTotV = 1, kTotSlices = 2, kTotEntries = 3, kTotRowV = 4, kTotHub = 5 };
 
 // ---- build pass 1: per (column block, row) segment of the sorted CSR row ----
 __global__ void __launch_bounds__(256)
@@ -223,12 +223,27 @@ __global__ void sell_cta_blocks_kernel(const int32_t* __restrict__ slice_off, co
 // degree (or hubs clustered any other way) equal row counts left one CTA with every long row
 // and the grid barrier waiting for it (measured: +17 us per order on a degree-sorted Reddit shape).
 constexpr int kSellEpiWarpRow = 24;
-__global__ void sell_row_cost_kernel(const int32_t* __restrict__ rv_ptr, int n, int32_t* __restrict__ cost) {
+__device__ __forceinline__ bool sell_is_hub_row(const int32_t* rv_ptr, int i) {
+    return rv_ptr[i + 1] - rv_ptr[i] > kSellEpiWarpRow;
+}
+
+// cost[i] of the epilogue ranges and hub[i] = 1 for the rows a warp sums ([n + 1] each, last 0)
+__global__ void sell_row_cost_kernel(const int32_t* __restrict__ rv_ptr, int n, int32_t* __restrict__ cost,
+                                     int32_t* __restrict__ hub) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i > n) return;
-    if (i == n) { cost[i] = 0; return; }
+    if (i == n) { cost[i] = 0; hub[i] = 0; return; }
     const int parts = rv_ptr[i + 1] - rv_ptr[i];
     cost[i] = parts > kSellEpiWarpRow ? 28 + parts / 8 : 4;
+    hub[i] = parts > kSellEpiWarpRow ? 1 : 0;
+}
+
+// number of hub rows (prepare: the caller sizes the plan's hub list with it)
+__global__ void sell_hub_count_kernel(const int32_t* __restrict__ rv_ptr, int n, int64_t* __restrict__ totals) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool hub = i < n && sell_is_hub_row(rv_ptr, i);
+    const unsigned m = __ballot_sync(0xffffffffu, hub);
+    if ((threadIdx.x & 31) == 0 && m) atomicAdd(reinterpret_cast<unsigned long long*>(totals + kTotHub), (unsigned long long)__popc(m));
 }
 
 // cta_rows[g] = first row of CTA g (g = 0 .. n_cta): the first row whose cost prefix reaches
@@ -245,6 +260,16 @@ __global__ void sell_cta_rows_kernel(const int32_t* __restrict__ cost_prefix, in
         if (cost_prefix[mid] < target) lo = mid + 1; else hi = mid;
     }
     cta_rows[g] = lo;
+}
+
+// The hub rows of every CTA's epilogue range, listed once per plan so that the step kernel hands
+// them to its warps statically: CTA g's are hub[n_cta + 1 + hub[g] .. n_cta + 1 + hub[g + 1]),
+// ascending (hub_prefix = exclusive sums of the hub flags, [n + 1]).  Grid: max(n, n_cta + 1) threads.
+__global__ void sell_cta_hubs_kernel(const int32_t* __restrict__ hub_flag, const int32_t* __restrict__ hub_prefix,
+                                     const int32_t* __restrict__ cta_rows, int n, int n_cta, int32_t* __restrict__ hub) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i <= n_cta) hub[i] = hub_prefix[cta_rows[i]];
+    if (i < n && hub_flag[i]) hub[n_cta + 1 + hub_prefix[i]] = i;
 }
 
 __global__ void sell_totals_kernel(const int32_t* __restrict__ slice_off, const int32_t* __restrict__ rv_ptr,

@@ -42,6 +42,10 @@ constexpr int kStepMaxOrders = 16;        // orders per launch (the coefficient 
 constexpr int kSchedBarrier = kSellMaxBlocks * kSellCtrStride;   // sched[c * 32]: next slice of column block c; then the 64-bit barrier counter
 constexpr int kEpiWarpRow = kSellEpiWarpRow;           // rows with more partial sums than this are added up by a whole warp
 constexpr int kStageChunkFloats = 8192;   // one bulk copy = 32 KB
+// partial sums of each of a thread's two epilogue rows requested in the first round trip: a row
+// has about one per column block it touches (five blocks on the Reddit shape); 6 or 8 spill at
+// 64 registers
+constexpr int kEpiFirstParts = 5;
 
 struct SellStepParams {
     // plan
@@ -50,6 +54,7 @@ struct SellStepParams {
     const int32_t* blk_slice_ptr;
     const int32_t* vslot;
     const int32_t* cta_info;      // [n_cta] column block (-1: none), [n_cta] rank inside the block, [64] counter start, [n_cta + 1] epilogue rows
+    const int32_t* hub;           // [n_cta + 1] + rows: the hub rows of every CTA's epilogue range (sell_cta_hubs_kernel)
     const int32_t* rv_ptr;
     float* vpart;
     unsigned* sched;
@@ -193,6 +198,19 @@ struct StepRowPre {
 };
 
 template <bool PATCH>
+__device__ __forceinline__ void step_row_patch(const SellStepParams& p, const StepOrderView& v, int gi, StepRowPre& r) {
+    if (PATCH && v.touched_here) {        // a node an edge flip touches: its degree changed (uniform per CTA; most skip this)
+        const int j = step_patch_find(v.pt_node, v.n_touch, gi);
+        if (j >= 0) {
+            r.di = v.pt_dinv[j];
+            r.theta = fmaf(p.a, 1.f - (float)v.pt_iso[j], p.b);
+            if (v.k == 1) r.xprev = v.pt_x0[j];           // T_0 = x0 = log1p(row sum)
+            if (v.k == 2) r.t2 = v.pt_x0[j];
+        }
+    }
+}
+
+template <bool PATCH>
 __device__ __forceinline__ StepRowPre step_row_prefetch(const SellStepParams& p, const StepOrderView& v, int i) {
     StepRowPre r;
     const int gi = p.row0 + i;
@@ -203,15 +221,36 @@ __device__ __forceinline__ StepRowPre step_row_prefetch(const SellStepParams& p,
     r.xprev = v.tprev[i];
     r.t2 = v.first ? 0.f : v.tprev2[i];
     r.out0 = v.first ? 0.f : p.out[(size_t)i * p.S];
-    if (PATCH && v.touched_here) {        // a node an edge flip touches: its degree changed (uniform per CTA; most skip this)
-        const int j = step_patch_find(v.pt_node, v.n_touch, gi);
-        if (j >= 0) {
-            r.di = v.pt_dinv[j];
-            r.theta = fmaf(p.a, 1.f - (float)v.pt_iso[j], p.b);
-            if (v.k == 1) r.xprev = v.pt_x0[j];           // T_0 = x0 = log1p(row sum)
-            if (v.k == 2) r.t2 = v.pt_x0[j];
-        }
-    }
+    step_row_patch<PATCH>(p, v, gi, r);
+    return r;
+}
+
+// The same words for a row a whole warp sums, spread over the lanes (lane j requests word j:
+// t, e, dinv, iso, T_{k-1}, T_{k-2}, S_0) so that the request costs one register, not seven;
+// step_hub_gather assembles them (every lane, after the grid barrier's wait)
+__device__ __forceinline__ uint32_t step_hub_prefetch(const SellStepParams& p, const StepOrderView& v, int i, int lane) {
+    const int gi = p.row0 + i;
+    uint32_t w = 0u;
+    if (lane == 0) w = (uint32_t)__ldg(p.rv_ptr + i);
+    else if (lane == 1) w = (uint32_t)__ldg(p.rv_ptr + i + 1);
+    else if (lane == 2) w = __float_as_uint(__ldg(p.dinv + gi));
+    else if (lane == 3) w = __ldg(p.iso + gi);
+    else if (lane == 4) w = __float_as_uint(v.tprev[i]);
+    else if (lane == 5 && !v.first) w = __float_as_uint(v.tprev2[i]);
+    else if (lane == 6 && !v.first) w = __float_as_uint(p.out[(size_t)i * p.S]);
+    return w;
+}
+template <bool PATCH>
+__device__ __forceinline__ StepRowPre step_hub_gather(const SellStepParams& p, const StepOrderView& v, int i, uint32_t w) {
+    StepRowPre r;
+    r.t = (int)__shfl_sync(0xffffffffu, w, 0);
+    r.e = (int)__shfl_sync(0xffffffffu, w, 1);
+    r.di = __uint_as_float(__shfl_sync(0xffffffffu, w, 2));
+    r.theta = fmaf(p.a, 1.f - (float)__shfl_sync(0xffffffffu, w, 3), p.b);
+    r.xprev = __uint_as_float(__shfl_sync(0xffffffffu, w, 4));
+    r.t2 = __uint_as_float(__shfl_sync(0xffffffffu, w, 5));
+    r.out0 = __uint_as_float(__shfl_sync(0xffffffffu, w, 6));
+    step_row_patch<PATCH>(p, v, p.row0 + i, r);
     return r;
 }
 
@@ -238,18 +277,46 @@ __device__ __forceinline__ void step_epilogue_finish(const SellStepParams& p, co
     }
 }
 
-// Partial sums of a row with at most kEpiWarpRow virtual rows: loads issued eight at a time,
-// added in float64 in storage order (always the same order: deterministic).
-__device__ __forceinline__ double step_row_sum(const float* vpart, int t, int e) {
-    double a = 0.0;
-    for (; t < e; t += 8) {
-        float x[8];
+// Partial sums of a row with at most kEpiWarpRow virtual rows, added in float64 in storage
+// order (always the same order: deterministic).  The first N are requested by the caller (so
+// that the loads of several rows are in flight together), the rest eight at a time.
+template <int N>
+__device__ __forceinline__ void step_row_load(const float* vpart, int t, int e, float (&x)[N]) {
 #pragma unroll
-        for (int u = 0; u < 8; ++u) x[u] = t + u < e ? __ldcg(vpart + t + u) : 0.f;
+    for (int u = 0; u < N; ++u) x[u] = t + u < e ? __ldcg(vpart + t + u) : 0.f;
+}
+template <int N>
+__device__ __forceinline__ double step_row_sum_rest(const float* vpart, int t, int e, const float (&x0)[N]) {
+    double a = 0.0;
+#pragma unroll
+    for (int u = 0; u < N; ++u) a += (double)x0[u];
+    for (t += N; t < e; t += 8) {
+        float x[8];
+        step_row_load(vpart, t, e, x);
 #pragma unroll
         for (int u = 0; u < 8; ++u) a += (double)x[u];
     }
     return a;
+}
+__device__ __forceinline__ double step_row_sum(const float* vpart, int t, int e) {
+    float x[8];
+    step_row_load(vpart, t, e, x);
+    return step_row_sum_rest(vpart, t, e, x);
+}
+
+// A row with more than kEpiWarpRow partial sums, by a whole warp: lane-strided float64 sums in a
+// fixed shuffle tree; x0 = the lane's first partial (vpart[r.t + lane], 0 past the end).
+__device__ __forceinline__ void step_hub_finish(const SellStepParams& p, const StepOrderView& v, int i,
+                                                const StepRowPre& r, float x0, int lane) {
+    double a = 0.0;
+    a += (double)x0;
+    for (int t = r.t + lane + 32; t < r.e; t += 32) a += (double)__ldcg(p.vpart + t);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    if (lane == 0) step_epilogue_finish(p, v, i, r, a);
+}
+__device__ __forceinline__ float step_hub_first(const float* vpart, int t, int e, int lane) {
+    return t + lane < e ? __ldcg(vpart + t + lane) : 0.f;
 }
 
 template <bool PEER, bool PATCH>
@@ -257,7 +324,7 @@ __global__ void __launch_bounds__(kSellThreads, 1)
 sell_step_kernel(const __grid_constant__ SellStepParams p) {
     extern __shared__ __align__(128) float ysm[];
     __shared__ __align__(8) unsigned long long stage_bar;
-    __shared__ int hub_cnt;
+    __shared__ int hub_first[kSellThreads / 32], hub_span[2];     // the first hub row of every warp (-1: none); CTA's span of the list
     __shared__ float flip_term[EGNN_MAX_DELTA];
     __shared__ int pt_node[PATCH ? 2 * EGNN_MAX_DELTA : 1];
     __shared__ float pt_dinv[PATCH ? 2 * EGNN_MAX_DELTA : 1], pt_x0[PATCH ? 2 * EGNN_MAX_DELTA : 1], pt_y0[PATCH ? 2 * EGNN_MAX_DELTA : 1];
@@ -281,20 +348,26 @@ sell_step_kernel(const __grid_constant__ SellStepParams p) {
     const int col0 = c >= 0 ? c * p.CB : 0;
     const int cnt = c >= 0 ? min(p.CB, p.n_cols - col0) : 0;
     // rows this CTA owns in the epilogue phases (one or two per thread on the named shapes)
-#ifdef EGNN_EQUAL_EPILOGUE_ROWS                                                // A/B builds only
-    const int r0 = (int)((int64_t)p.n_rows * g / p.n_cta);
-    const int r1 = (int)((int64_t)p.n_rows * (g + 1) / p.n_cta);
-#else
     const int r0 = __ldg(p.cta_info + 2 * p.n_cta + kSellMaxBlocks + g);       // ranges of equal cost (sell_cta_rows_kernel)
     const int r1 = __ldg(p.cta_info + 2 * p.n_cta + kSellMaxBlocks + g + 1);
-#endif
+    // the hub rows of that range (summed by whole warps) are dealt to the warps in turn: warp w
+    // takes the w-th, (w + 32)-th, ... of the plan's list
+    if (tid < kWarps) {
+        const int hb = __ldg(p.hub + g), he = __ldg(p.hub + g + 1);
+        hub_first[tid] = hb + tid < he ? __ldg(p.hub + p.n_cta + 1 + hb + tid) : -1;
+        if (tid == 0) { hub_span[0] = hb; hub_span[1] = he; }
+    }
 
     unsigned long long* bar_ctr = reinterpret_cast<unsigned long long*>(p.sched + kSchedBarrier);
-    unsigned long long bar_base = 0;
+    // what only thread 0 uses lives in shared memory, not in every thread's registers
+    __shared__ unsigned long long bar_base;
+    __shared__ int stamp_i, trace_i;
     unsigned epoch_base = 0;
     if (tid == 0) {
         const unsigned long long seen = ld_relaxed_gpu_u64(bar_ctr);
         bar_base = seen - seen % n_cta;
+        stamp_i = 1;
+        trace_i = 0;
         mbar_init(&stage_bar, 1);
         if (p.stamps && g == 0) p.stamps[0] = global_timer_ns();
     }
@@ -302,7 +375,6 @@ sell_step_kernel(const __grid_constant__ SellStepParams p) {
     unsigned bar_done = 0;                                     // grid barriers completed in this launch (same on every thread)
     unsigned signals = 0;                                      // flags this rank has raised in this launch
     unsigned stage_parity = 0;
-    int stamp_i = 1;
     bool pending = false, pending_signal = false;              // a barrier this CTA has arrived at but not yet waited for
     const bool late_done = PEER && p.delta.n > 0;              // the last epilogue reads the window (edge-flip corrections)
     // PATCH: every CTA re-derives dinv / iso / x0 / dinv * x0 of the nodes the flips touch (the
@@ -355,14 +427,17 @@ sell_step_kernel(const __grid_constant__ SellStepParams p) {
         }
     };
     auto stamp = [&]() {
-        if (p.stamps && g == 0 && tid == 0) p.stamps[stamp_i] = global_timer_ns();
-        ++stamp_i;
+        if (tid == 0) {
+            if (p.stamps && g == 0) p.stamps[stamp_i] = global_timer_ns();
+            ++stamp_i;
+        }
     };
     // per-CTA trace (diagnostic; the stamps buffer then holds 64 + 64 * n_cta words)
-    int trace_i = 0;
     auto trace = [&]() {
-        if (p.stamps && p.trace && tid == 0 && trace_i < 64) p.stamps[64 + (size_t)g * 64 + trace_i] = global_timer_ns();
-        ++trace_i;
+        if (tid == 0) {
+            if (p.stamps && p.trace && trace_i < 64) p.stamps[64 + (size_t)g * 64 + trace_i] = global_timer_ns();
+            ++trace_i;
+        }
     };
     // the two halves of a grid barrier (every thread calls both; thread 0 does the work)
     auto bar_arrive = [&](bool sys_scope) {
@@ -508,16 +583,14 @@ sell_step_kernel(const __grid_constant__ SellStepParams p) {
         // while HBM idles here made the step slower for every amount tried, DESIGN.md section 4.2)
 
         // ================= epilogue phase: the CTA's own rows ================================
-        // the row's own operands are requested before the wait for everybody's partial sums
-        // (measured: also starting the long rows' chain before the thread rows finish, with the
-        // partial sums held in registers across it, spills and is 1 us slower per order)
-        int* hub_list = reinterpret_cast<int*>(ysm);
-        const int hub_cap = p.CB;
-        if (tid == 0) hub_cnt = 0;
+        // what a row needs besides its partial sums is requested before the wait for everybody's
+        // partial sums: for the thread's rows A and B and for the warp's first hub row
         const int i_a = r0 + tid, i_b = r0 + tid + kSellThreads;
+        const int i_h = hub_first[wid];                        // uniform per warp
         StepRowPre pre_a{}, pre_b{};
         if (i_a < r1) pre_a = step_row_prefetch<PATCH>(p, v, i_a);
         if (i_b < r1) pre_b = step_row_prefetch<PATCH>(p, v, i_b);
+        const uint32_t wh = i_h >= 0 ? step_hub_prefetch(p, v, i_h, lane) : 0u;
         // (exchange) before this phase stores into the windows, and before a flip's term is read
         // from a column whose owner none of this CTA's waits covered: every rank's latest signal.
         // Polled by warp 0 while the grid barrier completes.
@@ -536,24 +609,29 @@ sell_step_kernel(const __grid_constant__ SellStepParams p) {
         // whose corrections the last epilogue still reads from the operand (signalled after it)
         if (PEER && v.last && !late_done) signal_peers();
         if (g == 0 && tid < p.C) p.sched[tid * kSellCtrStride] = (unsigned)__ldg(p.cta_info + 2 * p.n_cta + tid);   // counters for the next SpMV phase
-        for (int i = i_a; i < r1; i += kSellThreads) {
-            const StepRowPre r = i == i_a ? pre_a : (i == i_b ? pre_b : step_row_prefetch<PATCH>(p, v, i));
-            if (r.e - r.t > kEpiWarpRow) {
-                const int h = atomicAdd(&hub_cnt, 1);
-                if (h < hub_cap) { hub_list[h] = i; continue; }
-            }
-            step_epilogue_finish(p, v, i, r, step_row_sum(p.vpart, r.t, r.e));
-        }
-        __syncthreads();
-        const int n_hub = min(hub_cnt, hub_cap);
-        for (int h = wid; h < n_hub; h += kWarps) {            // long rows: lane-strided float64 sums, fixed shuffle tree
-            const int i = hub_list[h];
+        // the partial sums of rows A and B (the first kEpiFirstParts of each) and of the warp's hub
+        // row (the lanes' first ones) are all requested before any is added: one round trip to L2;
+        // a hub row is left to its warp by the thread whose row it is
+        const bool own_a = i_a < r1 && pre_a.e - pre_a.t <= kEpiWarpRow;
+        const bool own_b = i_b < r1 && pre_b.e - pre_b.t <= kEpiWarpRow;
+        float xa[kEpiFirstParts], xb[kEpiFirstParts];
+        step_row_load(p.vpart, pre_a.t, own_a ? pre_a.e : pre_a.t, xa);
+        step_row_load(p.vpart, pre_b.t, own_b ? pre_b.e : pre_b.t, xb);
+        const float xh = i_h >= 0 ? step_hub_first(p.vpart, (int)__shfl_sync(0xffffffffu, wh, 0),
+                                                   (int)__shfl_sync(0xffffffffu, wh, 1), lane) : 0.f;
+        if (own_a) step_epilogue_finish(p, v, i_a, pre_a, step_row_sum_rest(p.vpart, pre_a.t, pre_a.e, xa));
+        if (own_b) step_epilogue_finish(p, v, i_b, pre_b, step_row_sum_rest(p.vpart, pre_b.t, pre_b.e, xb));
+        for (int i = i_b + kSellThreads; i < r1; i += kSellThreads) {      // ranges of more than 2048 rows
             const StepRowPre r = step_row_prefetch<PATCH>(p, v, i);
-            double a = 0.0;
-            for (int t = r.t + lane; t < r.e; t += 32) a += (double)__ldcg(p.vpart + t);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-            if (lane == 0) step_epilogue_finish(p, v, i, r, a);
+            if (r.e - r.t <= kEpiWarpRow) step_epilogue_finish(p, v, i, r, step_row_sum(p.vpart, r.t, r.e));
+        }
+        if (i_h >= 0) {
+            step_hub_finish(p, v, i_h, step_hub_gather<PATCH>(p, v, i_h, wh), xh, lane);
+            for (int h = hub_span[0] + wid + kWarps; h < hub_span[1]; h += kWarps) {   // more hub rows than warps
+                const int i = __ldg(p.hub + p.n_cta + 1 + h);
+                const StepRowPre r = step_row_prefetch<PATCH>(p, v, i);
+                step_hub_finish(p, v, i, r, step_hub_first(p.vpart, r.t, r.e, lane), lane);
+            }
         }
         // the next order (or a peer) reads what this phase wrote
         if (k < p.order_end || (PEER && (v.push || (v.last && late_done)))) {

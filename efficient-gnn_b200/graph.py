@@ -381,6 +381,7 @@ def build_sell_plan(rowptr: torch.Tensor, colidx: torch.Tensor, n_rows: int, n_c
             "rv_ptr": torch.empty(n_rows + 1, dtype=torch.int32, device=dev),
             "vslot": torch.empty(max(1, plan.n_vrows), dtype=torch.int32, device=dev),
             "cta_info": torch.empty(3 * plan.n_cta + 65, dtype=torch.int32, device=dev),
+            "hub": torch.empty(plan.n_cta + 1 + plan.n_hub, dtype=torch.int32, device=dev),
             "vpart": torch.empty(max(1, plan.n_rowv), dtype=torch.float32, device=dev),
             "sched": torch.zeros(64 * 32 + 64, dtype=torch.int32, device=dev),
         }

@@ -141,7 +141,7 @@ int egnn_patch_nodes(const float* w_base, const float* rowsum_base, const float*
  *                        SYNCHRONISES the stream and fills the size fields;
  *   (caller allocates slice_off[n_slices+1], blk_slice_ptr[n_blocks+1],
  *    idx[n_entries] (uint16, 256-byte aligned), rv_ptr[n+1], vslot[n_vrows], cta_info[3*n_cta+65],
- *    sched[2112] uint32, vpart[n_rowv] float32 scratch: row i's partial sums are
+ *    hub[n_cta+1+n_hub], sched[2112] uint32, vpart[n_rowv] float32 scratch: row i's partial sums are
  *    vpart[rv_ptr[i] .. rv_ptr[i+1]), virtual row v writes vpart[vslot[v]])
  *   egnn_sell_fill       writes the index stream; `workspace` must be the
  *                        one prepare used, untouched in between.
@@ -166,6 +166,9 @@ typedef struct egnn_sell_plan {
                                              initialises them; the kernel leaves them ready for the next launch)      */
     uint64_t* stamps;                     /* optional [4 + 2 * orders per launch]: globaltimer of CTA 0 at kernel start,
                                              after every grid barrier and at the end (phase breakdown for bench.py)   */
+    int64_t n_hub;                        /* rows with more than 24 partial sums, summed by a whole warp (prepare)   */
+    int32_t* hub;                         /* [n_cta + 1 + n_hub]: CTA g's hub rows are hub[n_cta + 1 + hub[g] ..
+                                             n_cta + 1 + hub[g + 1]), ascending (egnn_sell_fill)                      */
 } egnn_sell_plan;
 
 int egnn_sell_geometry(int64_t n_cols, int64_t nnz, int32_t* n_blocks, int32_t* col_block, int32_t* lmax);
