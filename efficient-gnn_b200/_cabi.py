@@ -163,6 +163,16 @@ def host_array(ctype, values):
     return arr
 
 
+def delta_args(deltas, transpose: bool = False):
+    """Edge flips ``(rows, cols, vals)`` (or None) as the four flip arguments of the C ABI: three host
+    arrays and the count.  ``transpose=True`` swaps rows and columns, for the adjoint of a pass."""
+    d_rows, d_cols, d_vals = ([], [], []) if deltas is None else deltas
+    if transpose:
+        d_rows, d_cols = d_cols, d_rows
+    return (host_array(C.c_int32, [int(v) for v in d_rows]), host_array(C.c_int32, [int(v) for v in d_cols]),
+            host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows))
+
+
 _device_ok = {}
 
 

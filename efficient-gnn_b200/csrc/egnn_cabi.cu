@@ -48,12 +48,48 @@ static inline bool vec_aligned(const void* p, int32_t f) {
     return f % 4 != 0 || p == nullptr || ((uintptr_t)p & 15) == 0;
 }
 
-static int fill_delta(DeltaList& d, const int32_t* r, const int32_t* c, const float* v, int32_t n) {
+// The caller's edge flips into `d`.  Every index must address a node below `bound`: n, or the
+// global node count of a row shard.
+static int fill_delta(DeltaList& d, const int32_t* r, const int32_t* c, const float* v, int32_t n, int64_t bound) {
     EGNN_REQUIRE(n >= 0 && n <= EGNN_MAX_DELTA, "n_delta out of range");
     EGNN_REQUIRE(n == 0 || (r && c && v), "delta arrays missing");
     d.n = n;
-    for (int i = 0; i < n; ++i) { d.row[i] = r[i]; d.col[i] = c[i]; d.val[i] = v[i]; }
+    for (int i = 0; i < n; ++i) {
+        EGNN_REQUIRE(r[i] >= 0 && r[i] < bound && c[i] >= 0 && c[i] < bound, "delta index out of range");
+        d.row[i] = r[i]; d.col[i] = c[i]; d.val[i] = v[i];
+    }
     return EGNN_OK;
+}
+
+// `what` names the workspace in the message ("sell workspace", "transpose workspace", ...)
+static int require_workspace(const void* ws, size_t bytes, size_t need, const char* what) {
+    if (ws && bytes >= need) return EGNN_OK;
+    set_error("%s too small: need %zu bytes, got %zu", what, need, bytes);
+    return EGNN_ERR_WORKSPACE;
+}
+
+// Event i of the caller's per-order timing list (two per order: before and after), if it gave one.
+static int record_event(void* const* events, int i, cudaStream_t st) {
+    return events ? check_cuda(cudaEventRecord((cudaEvent_t)events[i], st), "event record") : EGNN_OK;
+}
+
+// Coefficient of order m of every scale, from the caller's [S, k + 1] host table.
+static void order_coefs(float* dst, const float* coeffs_host, int k, int S, int m) {
+    for (int s = 0; s < S; ++s) dst[s] = coeffs_host[s * (k + 1) + m];
+}
+static CoefRow coef_row(const float* coeffs_host, int k, int S, int m) {
+    CoefRow c{};
+    order_coefs(c.c, coeffs_host, k, S, m);
+    return c;
+}
+
+// Row width of the wide kernel's operand slabs and exchange windows: F padded to 16 bytes.
+static inline int wide_ldy(int32_t f) { return (f + 3) / 4 * 4; }
+
+// Slab m of a [*, rows, F] stack, or NULL without one.
+template <typename T>
+static inline T* slab_of(T* stack, size_t slab_elems, int m) {
+    return stack ? stack + (size_t)m * slab_elems : nullptr;
 }
 
 // Lane layout and instantiation for one order launch.
@@ -173,6 +209,124 @@ static int grid_for(int64_t work_items, int threads) {
     if (b > cap) b = cap;
     if (b < 1) b = 1;
     return (int)b;
+}
+
+// Row L1 normalisation of `rows` x S feature vectors of width f, after the last order.
+static int launch_l1_normalize(float* out, int64_t rows, int32_t S, int32_t f, cudaStream_t st) {
+    l1_normalize_kernel<<<grid_for(rows * S * 32, 256), 256, 0, st>>>(out, rows * S, f);
+    EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
+    return EGNN_OK;
+}
+
+// Grid of a kernel that pushes `items` floats into the peer windows with 1024 threads per CTA:
+// at most one CTA per SM, since each CTA issues one system-scope fence.
+static unsigned push_grid(int64_t items) {
+    const int64_t blocks = ceil_div64(items > 0 ? items : 1, 1024);
+    const int sms = device_sm_count();
+    return (unsigned)(blocks > sms ? sms : blocks);
+}
+
+static int launch_degree(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null, int64_t rows,
+                         float* rowsum, float* diag, double* colsum, int32_t* unsorted_flag_or_null, int64_t row0,
+                         cudaStream_t st) {
+    const auto kernel = vals_or_null ? degree_kernel<true> : degree_kernel<false>;
+    kernel<<<grid_for(rows * 32, 256), 256, 0, st>>>(rowptr, colidx, vals_or_null, rows, rowsum, diag, colsum,
+                                                      unsorted_flag_or_null, row0);
+    EGNN_LAUNCH_CHECK("degree_kernel launch");
+    return EGNN_OK;
+}
+
+// Column blocks of the shared-memory staged narrow paths (SELL plan and plan-free blocked kernel)
+static void narrow_geometry(int64_t n, int* n_blocks, int* col_block) {
+    const int64_t cb_max = 49152;                     // 192 KB of float32 operand per CTA
+    const int64_t c = ceil_div64(n, cb_max);
+    int64_t cb = ceil_div64(ceil_div64(n, c), 32) * 32;
+    if (cb > 65504) cb = 65504;
+    *n_blocks = (int)ceil_div64(n, cb);
+    *col_block = (int)cb;
+}
+
+// ---- Chebyshev workspace layout (egnn_cheb_workspace_bytes; forward and adjoint) ---------------
+// f < 8: two T slabs, ping-pong for T_{k-1} / T_{k-2} (the adjoint's b vectors), and for f <= 4
+// two pre-scaled operand slabs dinv (.) T.  f >= 8: two operand slabs with rows padded to 16 bytes
+// and one row counter per (order, feature tile) for the wide kernel's dynamic row schedule.
+// f == 1 adds the segment table, partial sums and counters of the plan-free blocked kernel.
+struct ChebWs {
+    float* t[2];
+    float* y[2];
+    unsigned* row_counters;
+    int C, CB;                   // blocked kernel: column blocks the next three are sized for
+    int32_t* seg;
+    float* part;
+    unsigned* blk_counters;
+    size_t total_bytes;
+};
+
+static ChebWs cheb_ws_layout(void* base, int64_t n, int32_t f) {
+    ChebWs w{};
+    size_t off = 0;
+    char* b = (char*)align_up((size_t)base, 256);
+    auto take = [&](size_t bytes) { void* ptr = b + off; off += align_up(bytes, 256); return ptr; };
+    if (f >= kWideMinF) {
+        const size_t ldy = (size_t)wide_ldy(f);
+        w.y[0] = (float*)take(sizeof(float) * (size_t)n * ldy);
+        w.y[1] = (float*)take(sizeof(float) * (size_t)n * ldy);
+        w.row_counters = (unsigned*)take(sizeof(unsigned) * (size_t)EGNN_MAX_ORDER * ((ldy + 127) / 128));
+    } else {
+        const size_t slab = sizeof(float) * (size_t)n * (size_t)f;
+        w.t[0] = (float*)take(slab);
+        w.t[1] = (float*)take(slab);
+        if (f <= 4) {
+            w.y[0] = (float*)take(slab);
+            w.y[1] = (float*)take(slab);
+        }
+        if (f == 1) {
+            narrow_geometry(n > 0 ? n : 1, &w.C, &w.CB);
+            w.seg = (int32_t*)take(4 * (size_t)(w.C + 1) * (size_t)n);
+            w.part = (float*)take(4 * (size_t)w.C * (size_t)n);
+            w.blk_counters = (unsigned*)take(4 * (size_t)EGNN_MAX_ORDER * (size_t)w.C);
+        }
+    }
+    w.total_bytes = off + 256;
+    return w;
+}
+
+// ---- one pass of the Chebyshev recurrence, forward or adjoint ------------------------------------
+// The rows a pass runs over (all n, or one row shard: local row r is node row0 + r), their CSR (of the
+// transposed graph for the adjoint), the operator a * L_sym + b * I and the [S, k + 1] coefficients.
+struct ChebArgs {
+    const int32_t* rowptr;
+    const int32_t* colidx;
+    const float* vals;           // NULL: binary adjacency
+    const int32_t* row_order;    // wide kernel: degree-descending row order and hub count, or NULL
+    const float* dinv;
+    const uint8_t* iso;
+    int64_t rows, row0, nnz;
+    int32_t f, k, S;
+    const float* coeffs;         // host
+    float a, b;
+    DeltaList delta;
+    void* const* events;         // two per order (application), or NULL
+    cudaStream_t st;
+};
+
+static WideParams wide_params(const ChebArgs& c) {
+    WideParams wp{};
+    wp.delta = c.delta;
+    wp.rowptr = c.rowptr; wp.colidx = c.colidx; wp.vals = c.vals;
+    wp.perm = c.row_order; wp.n_hub = c.row_order ? c.row_order + c.rows : nullptr;
+    wp.dinv = c.dinv; wp.iso = c.iso; wp.n_rows = c.rows; wp.row0 = c.row0;
+    wp.F = c.f; wp.ldy = wide_ldy(c.f); wp.S = c.S; wp.a = c.a; wp.b = c.b;
+    return wp;
+}
+
+static OrderParams order_params(const ChebArgs& c, const OrderConfig& cfg) {
+    OrderParams p{};
+    p.delta = c.delta;
+    p.rowptr = c.rowptr; p.colidx = c.colidx; p.vals = c.vals; p.dinv = c.dinv; p.iso = c.iso;
+    p.n_rows = c.rows; p.row0 = c.row0; p.F = c.f; p.S = c.S; p.a = c.a; p.b = c.b;
+    p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
+    return p;
 }
 
 
@@ -403,17 +557,9 @@ int egnn_degree_rows(const int32_t* rowptr, const int32_t* colidx, const float* 
     EGNN_REQUIRE(n >= 0 && row_begin >= 0 && row_begin <= row_end && row_end <= n, "bad row range");
     const int64_t rows = row_end - row_begin;
     if (rows == 0) return EGNN_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int g = grid_for(rows * 32, 256);
     // rowptr values are absolute positions in colidx, so a row range is the same kernel on shifted row arrays
-    if (vals_or_null)
-        degree_kernel<true><<<g, 256, 0, st>>>(rowptr + row_begin, colidx, vals_or_null, rows, rowsum + row_begin,
-                                               diag + row_begin, colsum, unsorted_flag_or_null, row_begin);
-    else
-        degree_kernel<false><<<g, 256, 0, st>>>(rowptr + row_begin, colidx, nullptr, rows, rowsum + row_begin,
-                                                diag + row_begin, colsum, unsorted_flag_or_null, row_begin);
-    EGNN_LAUNCH_CHECK("degree_kernel launch");
-    return EGNN_OK;
+    return launch_degree(rowptr + row_begin, colidx, vals_or_null, rows, rowsum + row_begin, diag + row_begin, colsum,
+                         unsorted_flag_or_null, row_begin, (cudaStream_t)stream);
 }
 
 int egnn_graph_prep_finish(const double* colsum, const float* diag, const float* rowsum, int64_t n, float* dinv,
@@ -456,10 +602,8 @@ int egnn_patch_degrees(const float* w_base, const float* rowsum_base, const floa
     EGNN_REQUIRE(row_begin >= 0 && n_rows >= 0 && row_begin + n_rows <= n, "bad row range");
     EGNN_REQUIRE(n_rows == 0 || (rowsum_base && x0_base && x0_out), "null pointer");
     DeltaList d;
-    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(d.row[i] >= 0 && d.row[i] < n && d.col[i] >= 0 && d.col[i] < n, "delta index out of range");
     cudaStream_t st = (cudaStream_t)stream;
     rc = check_cuda(cudaMemcpyAsync(dinv_out, dinv_base, sizeof(float) * n, cudaMemcpyDeviceToDevice, st), "copy dinv");
     if (rc) return rc;
@@ -483,10 +627,8 @@ int egnn_patch_nodes(const float* w_base, const float* rowsum_base, const float*
     EGNN_REQUIRE(w_base && rowsum_base && dinv_base && iso_base && x0_base && y0_base && dinv_io && iso_io && x0_io && y0_io,
                  "null pointer");
     DeltaList d;
-    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(d.row[i] >= 0 && d.row[i] < n && d.col[i] >= 0 && d.col[i] < n, "delta index out of range");
     if (n_delta == 0) return EGNN_OK;
     patch_nodes_kernel<<<1, 2 * EGNN_MAX_DELTA, 0, (cudaStream_t)stream>>>(w_base, rowsum_base, dinv_base, iso_base, x0_base,
                                                                           y0_base, d, dinv_io, iso_io, x0_io, y0_io,
@@ -513,11 +655,8 @@ int egnn_row_order(const int32_t* rowptr, int64_t n, int32_t* order_out, void* w
     EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31), "bad shape");
     cudaStream_t st = (cudaStream_t)stream;
     if (n == 0) return check_cuda(cudaMemsetAsync(order_out, 0, sizeof(int32_t), st), "memset n_hub");
-    const size_t need = egnn_row_order_ws_bytes(n);
-    if (!workspace || workspace_bytes < need) {
-        set_error("row-order workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    int rc = require_workspace(workspace, workspace_bytes, egnn_row_order_ws_bytes(n), "row-order workspace");
+    if (rc) return rc;
     const size_t arr = align_up(4 * (size_t)n, 256);
     char* ws = (char*)align_up((size_t)workspace, 256);
     uint32_t* keys = (uint32_t*)ws;
@@ -527,40 +666,196 @@ int egnn_row_order(const int32_t* rowptr, int64_t n, int32_t* order_out, void* w
     size_t cub_bytes = row_order_cub_bytes(n);
     row_order_keys_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, st>>>(rowptr, (int)n, keys, ids);
     EGNN_LAUNCH_CHECK("row_order_keys_kernel launch");
-    int rc = check_cuda(cub::DeviceRadixSort::SortPairs(cub_temp, cub_bytes, keys, keys_sorted, ids, order_out, (int)n, 0,
-                                                        32, st), "sort rows by degree");
+    rc = check_cuda(cub::DeviceRadixSort::SortPairs(cub_temp, cub_bytes, keys, keys_sorted, ids, order_out, (int)n, 0, 32,
+                                                    st), "sort rows by degree");
     if (rc) return rc;
     row_order_hubs_kernel<<<1, 32, 0, st>>>(keys_sorted, (int)n, order_out + n);
     EGNN_LAUNCH_CHECK("row_order_hubs_kernel launch");
     return EGNN_OK;
 }
 
-// Column blocks of the shared-memory staged narrow paths (SELL plan and plan-free blocked kernel)
-static void narrow_geometry(int64_t n, int* n_blocks, int* col_block) {
-    const int64_t cb_max = 49152;                     // 192 KB of float32 operand per CTA
-    const int64_t c = ceil_div64(n, cb_max);
-    int64_t cb = ceil_div64(ceil_div64(n, c), 32) * 32;
-    if (cb > 65504) cb = 65504;
-    *n_blocks = (int)ceil_div64(n, cb);
-    *col_block = (int)cb;
+}  // extern "C"
+
+// ---- the wavelet pass: one static function per path of egnn_cheb_wavelet -------------------------
+// Where order `order` of the forward writes T_k: its slab of t_all; nowhere on the last order (T_K
+// is never read again); else the two T slabs for orders 1 and 2, and in place over T_{k-2} after.
+static float* t_slot(const ChebArgs& c, const ChebWs& ws, float* t_all, int order, const float* t_prev2) {
+    if (t_all) return slab_of(t_all, (size_t)c.rows * (size_t)c.f, order);
+    if (order == c.k) return nullptr;
+    if (order <= 2) return ws.t[order - 1];
+    return const_cast<float*>(t_prev2);
 }
 
-static size_t blocked_ws_bytes(int64_t n) {
-    int C = 1, CB = 32;
-    narrow_geometry(n > 0 ? n : 1, &C, &CB);
-    return align_up(4 * (size_t)(C + 1) * (size_t)n, 256) + align_up(4 * (size_t)C * (size_t)n, 256) +
-           align_up(4 * (size_t)EGNN_MAX_ORDER * (size_t)C, 256);
+static int wavelet_order0(const ChebArgs& c, const float* x0, float* out, float* t_all, int32_t normalize_l1) {
+    const size_t slab_elems = (size_t)c.rows * (size_t)c.f;
+    OrderParams p{};
+    p.delta = c.delta;
+    order_coefs(p.c_prev, c.coeffs, 0, c.S, 0);
+    order0_kernel<<<grid_for((int64_t)slab_elems * c.S, 256), 256, 0, c.st>>>(x0, out, c.rows, c.f, c.S, p);
+    EGNN_LAUNCH_CHECK("order0_kernel launch");
+    if (t_all) {
+        int rc = check_cuda(cudaMemcpyAsync(t_all, x0, sizeof(float) * slab_elems, cudaMemcpyDeviceToDevice, c.st), "copy T0");
+        if (rc) return rc;
+    }
+    return normalize_l1 ? launch_l1_normalize(out, c.rows, c.S, c.f, c.st) : EGNN_OK;
 }
+
+// All K orders in one persistent launch (sell_step.cuh); the first operand dinv (.) T_0 is computed
+// inside it unless the caller keeps it (y0: fixed per graph for the default signal).
+static int wavelet_sell(const ChebArgs& c, const ChebWs& ws, const egnn_sell_plan* plan, const float* x0,
+                        const float* y0, float* out, float* t_all, int32_t normalize_l1, const float* w_base,
+                        const float* rowsum_base, int32_t default_signal) {
+    EGNN_REQUIRE(c.f == 1 && c.vals == nullptr, "the SELL plan serves F = 1 on a binary adjacency");
+    EGNN_REQUIRE(plan->n == c.rows && plan->n_cols == c.rows && plan->row0 == 0 && plan->vpart && plan->slice_off && plan->blk_slice_ptr &&
+                 plan->rv_ptr && plan->vslot && plan->cta_info && plan->hub && plan->sched, "SELL plan does not match the graph or is not filled");
+    SellStepParams sp{};
+    step_fill_plan(sp, plan);
+    sp.delta = c.delta;
+    sp.w_base = w_base; sp.rowsum_base = rowsum_base; sp.patch_x0 = default_signal ? 1 : 0;
+    sp.dinv = c.dinv; sp.iso = c.iso; sp.x0 = x0;
+    sp.operand_first = y0;
+    sp.operand[0] = ws.y[0]; sp.operand[1] = ws.y[1];
+    sp.ydst[0][0] = ws.y[0]; sp.ydst[1][0] = ws.y[1]; sp.n_dst = 1;
+    sp.tbuf[0] = ws.t[0]; sp.tbuf[1] = ws.t[1]; sp.t_all = t_all; sp.out = out;
+    sp.normalize = normalize_l1; sp.a = c.a; sp.b = c.b;
+    sp.world = 1; sp.rank = 0; sp.rows_per = c.rows;
+    int rc = record_event(c.events, 0, c.st);
+    if (rc) return rc;
+    rc = run_sell_step(sp, c.k, c.S, c.coeffs, false, c.st);
+    if (rc) return rc;
+    for (int e = 1; e < 2 * c.k; ++e) {           // one launch: events 0 and 1 bracket the whole step, the rest follow it
+        rc = record_event(c.events, e, c.st);
+        if (rc) return rc;
+    }
+    return EGNN_OK;
+}
+
+// First use of a large graph at F = 1 (no SELL plan yet): plan-free column-blocked kernel (blocked.cuh)
+static int wavelet_blocked(const ChebArgs& c, const ChebWs& ws, const float* x0, float* out, float* t_all,
+                           int32_t normalize_l1) {
+    const int64_t n = c.rows;
+    const int C = ws.C, CB = ws.CB;
+    int rc = check_cuda(cudaMemsetAsync(ws.blk_counters, 0, sizeof(unsigned) * (size_t)c.k * (size_t)C, c.st),
+                        "memset batch counters");
+    if (rc) return rc;
+    blocked_bounds_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, c.st>>>(c.rowptr, c.colidx, (int)n, C, CB, ws.seg);
+    EGNN_LAUNCH_CHECK("blocked_bounds_kernel launch");
+    const size_t smem = sizeof(float) * (size_t)CB;
+    const void* fn = c.vals ? (const void*)blocked_spmv_kernel<true> : (const void*)blocked_spmv_kernel<false>;
+    rc = check_cuda(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
+                    "cudaFuncSetAttribute(blocked_spmv_kernel)");
+    if (rc) return rc;
+    BlockedParams bp{};
+    bp.colidx = c.colidx; bp.vals = c.vals; bp.seg = ws.seg; bp.part = ws.part;
+    bp.n = (int32_t)n; bp.C = C; bp.CB = CB; bp.n_cta = device_sm_count();
+    if (bp.n_cta < C) bp.n_cta = C;
+    BlockedEpilogueParams ep{};
+    ep.delta = c.delta;
+    ep.part = ws.part; ep.dinv = c.dinv; ep.iso = c.iso; ep.out = out; ep.n = (int32_t)n; ep.C = C; ep.S = c.S;
+    ep.a = c.a; ep.b = c.b;
+    const float* t_prev = x0;
+    const float* t_prev2 = nullptr;
+    for (int order = 1; order <= c.k; ++order) {
+        const bool last = order == c.k;
+        float* t_out = t_slot(c, ws, t_all, order, t_prev2);
+        rc = record_event(c.events, 2 * (order - 1), c.st);
+        if (rc) return rc;
+        bp.y = ws.y[(order - 1) & 1];
+        bp.counter = ws.blk_counters + (size_t)(order - 1) * C;
+        if (c.vals) blocked_spmv_kernel<true><<<bp.n_cta, kBlockedThreads, smem, c.st>>>(bp);
+        else blocked_spmv_kernel<false><<<bp.n_cta, kBlockedThreads, smem, c.st>>>(bp);
+        EGNN_LAUNCH_CHECK("blocked_spmv_kernel launch");
+        ep.y_prev = bp.y; ep.tprev = t_prev; ep.tprev2 = t_prev2; ep.tk = t_out;
+        ep.y_out = last ? nullptr : ws.y[order & 1];
+        ep.first = order == 1; ep.normalize = last && normalize_l1;
+        order_coefs(ep.c_prev, c.coeffs, c.k, c.S, order - 1);
+        order_coefs(ep.c_k, c.coeffs, c.k, c.S, order);
+        blocked_epilogue_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, c.st>>>(ep);
+        EGNN_LAUNCH_CHECK("blocked_epilogue_kernel launch");
+        rc = record_event(c.events, 2 * (order - 1) + 1, c.st);
+        if (rc) return rc;
+        t_prev2 = t_prev;
+        t_prev = t_out;
+    }
+    return EGNN_OK;
+}
+
+static int wavelet_wide(const ChebArgs& c, const ChebWs& ws, const float* x0, float* out, float* t_all,
+                        int32_t normalize_l1) {
+    const int64_t n = c.rows;
+    const int ldy = wide_ldy(c.f);
+    const RingConfig rcfg = ring_config(ldy);
+    WideParams wp = wide_params(c);
+    wp.out = out;
+    // ws.y[] hold dinv (.) T_k, rows padded to 16 bytes
+    prescale_pad_kernel<<<grid_for(n * ldy, 256), 256, 0, c.st>>>(x0, c.dinv, ws.y[0], n, c.f, ldy, 0);
+    EGNN_LAUNCH_CHECK("prescale_pad_kernel launch");
+    int rc = check_cuda(cudaMemsetAsync(ws.row_counters, 0, sizeof(unsigned) * (size_t)c.k * (size_t)rcfg.grid_y, c.st),
+                        "memset row counters");
+    if (rc) return rc;
+    const bool fuse_norm = normalize_l1 && rcfg.grid_y == 1;
+    // dynamic rows pay off where rows are short and one feature tile covers the signal (arxiv
+    // shape F = 128: 0.283 -> 0.23 ms per order); measured slower on long rows (Reddit shape
+    // F = 64: 2.13 -> 2.48) and on many feature tiles (Physics F = 8415: 2.77 -> 3.3)
+    const bool dynamic_rows = rcfg.grid_y == 1 && c.nnz < (int64_t)kWideDynamicMaxDegree * n;
+    const int sms = device_sm_count();
+    for (int order = 1; order <= c.k; ++order) {
+        const bool last = order == c.k;
+        wp.first = order == 1;
+        wp.normalize = last && fuse_norm;
+        wp.row_counter = dynamic_rows ? ws.row_counters + (size_t)(order - 1) * (size_t)rcfg.grid_y : nullptr;
+        wp.ysrc = ws.y[(order - 1) & 1];
+        wp.x0_own = order == 1 ? x0 : nullptr;
+        wp.y2_own = order == 1 ? nullptr : ws.y[order & 1];
+        wp.y_out = last ? nullptr : ws.y[order & 1];      // in place over dinv (.) T_{k-2} (own row only)
+        wp.tk_out = slab_of(t_all, (size_t)n * (size_t)c.f, order);
+        order_coefs(wp.c_prev, c.coeffs, c.k, c.S, order - 1);
+        order_coefs(wp.c_k, c.coeffs, c.k, c.S, order);
+        rc = record_event(c.events, 2 * (order - 1), c.st);
+        if (rc) return rc;
+        rc = launch_wide(wp, rcfg, sms, c.st);
+        if (rc) return rc;
+        rc = record_event(c.events, 2 * (order - 1) + 1, c.st);
+        if (rc) return rc;
+    }
+    return normalize_l1 && !fuse_norm ? launch_l1_normalize(out, n, c.S, c.f, c.st) : EGNN_OK;
+}
+
+static int wavelet_generic(const ChebArgs& c, const ChebWs& ws, const OrderConfig& cfg, const float* x0, float* out,
+                           float* t_all, int32_t normalize_l1) {
+    OrderParams p = order_params(c, cfg);
+    p.out = out;
+    const bool fuse_norm = normalize_l1 && cfg.grid_y == 1;
+    const float* t_prev = x0;         // T_{k-1}
+    const float* t_prev2 = nullptr;   // T_{k-2}
+    for (int order = 1; order <= c.k; ++order) {
+        const bool last = order == c.k;
+        float* t_out = t_slot(c, ws, t_all, order, t_prev2);
+        p.first = order == 1;
+        p.normalize = last && fuse_norm;
+        p.tprev_own = t_prev;
+        p.tprev2_own = t_prev2;
+        p.tk_own = t_out;
+        p.gsrc = cfg.prescaled ? ws.y[(order - 1) & 1] : t_prev;
+        p.y_own = (cfg.prescaled && !last) ? ws.y[order & 1] : nullptr;
+        order_coefs(p.c_prev, c.coeffs, c.k, c.S, order - 1);
+        order_coefs(p.c_k, c.coeffs, c.k, c.S, order);
+        int rc = record_event(c.events, 2 * (order - 1), c.st);
+        if (rc) return rc;
+        rc = launch_order(p, cfg, c.st);
+        if (rc) return rc;
+        rc = record_event(c.events, 2 * (order - 1) + 1, c.st);
+        if (rc) return rc;
+        t_prev2 = t_prev;
+        t_prev = t_out;
+    }
+    return normalize_l1 && !fuse_norm ? launch_l1_normalize(out, c.rows, c.S, c.f, c.st) : EGNN_OK;
+}
+
+extern "C" {
 
 size_t egnn_cheb_workspace_bytes(int64_t n, int32_t f) {
-    // two T ping-pong slabs + two pre-scaled gather slabs (narrow F only)
-    // f <= 4: two T slabs + two pre-scaled slabs; 4 < f < 8: two T slabs; f >= 8: two pre-scaled slabs
-    const size_t width = f >= kWideMinF ? (size_t)((f + 3) / 4 * 4) : (size_t)f;     // wide slabs have 16-byte rows
-    const size_t slab = align_up(sizeof(float) * (size_t)n * width, 256);
-    // wide path: + one row counter per (order, feature tile) for the dynamic row schedule
-    const size_t counters = f >= kWideMinF ? align_up(sizeof(unsigned) * (size_t)EGNN_MAX_ORDER * (size_t)((width + 127) / 128), 256) : 0;
-    // f == 1: + segment table, partial sums and counters of the plan-free blocked kernel
-    return slab * (f <= 4 ? 4 : 2) + counters + (f == 1 ? blocked_ws_bytes(n) : 0) + 256;
+    return cheb_ws_layout(nullptr, n, f).total_bytes;
 }
 
 int egnn_cheb_wavelet(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
@@ -584,251 +879,115 @@ int egnn_cheb_wavelet(const int32_t* rowptr, const int32_t* colidx, const float*
     EGNN_REQUIRE(vec_aligned(x0, f) && vec_aligned(out, f) && vec_aligned(t_all_or_null, f),
                  "x0, out and t_all must be 16-byte aligned when f % 4 == 0");
     if (n == 0) return EGNN_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-
-    OrderParams p{};
-    int rc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    ChebArgs c{};
+    c.rowptr = rowptr; c.colidx = colidx; c.vals = vals_or_null; c.row_order = row_order_or_null;
+    c.dinv = dinv; c.iso = iso; c.rows = n; c.nnz = nnz; c.f = f; c.k = k; c.S = n_scales;
+    c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.events = order_events_host; c.st = (cudaStream_t)stream;
+    int rc = fill_delta(c.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(p.delta.row[i] >= 0 && p.delta.row[i] < n && p.delta.col[i] >= 0 && p.delta.col[i] < n,
-                     "delta index out of range");
-
-    const size_t slab_elems = (size_t)n * (size_t)f;
-    if (k == 0) {
-        for (int s = 0; s < n_scales; ++s) p.c_prev[s] = coeffs_host[s];
-        order0_kernel<<<grid_for((int64_t)slab_elems * n_scales, 256), 256, 0, st>>>(x0, out, n, f, n_scales, p);
-        EGNN_LAUNCH_CHECK("order0_kernel launch");
-        if (t_all_or_null) {
-            rc = check_cuda(cudaMemcpyAsync(t_all_or_null, x0, sizeof(float) * slab_elems, cudaMemcpyDeviceToDevice, st), "copy T0");
-            if (rc) return rc;
-        }
-        if (normalize_l1) {
-            l1_normalize_kernel<<<grid_for(n * n_scales * 32, 256), 256, 0, st>>>(out, n * n_scales, f);
-            EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
-        }
-        return EGNN_OK;
-    }
+    if (k == 0) return wavelet_order0(c, x0, out, t_all_or_null, normalize_l1);
 
     const OrderConfig cfg = choose_config(n, nnz, f);
-    const size_t need = egnn_cheb_workspace_bytes(n, f);
-    if (workspace == nullptr || workspace_bytes < need) {
-        set_error("workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
-    const size_t slab = align_up(sizeof(float) * slab_elems, 256);
-    char* ws = (char*)align_up((size_t)workspace, 256);
-    float* tbuf[2] = {(float*)ws, (float*)(ws + slab)};
-    float* ybuf[2] = {(float*)(ws + 2 * slab), (float*)(ws + 3 * slab)};
-
+    rc = require_workspace(workspace, workspace_bytes, egnn_cheb_workspace_bytes(n, f), "workspace");
+    if (rc) return rc;
+    const ChebWs ws = cheb_ws_layout(workspace, n, f);
+    const size_t slab_elems = (size_t)n * (size_t)f;
     if (t_all_or_null) {
-        rc = check_cuda(cudaMemcpyAsync(t_all_or_null, x0, sizeof(float) * slab_elems, cudaMemcpyDeviceToDevice, st), "copy T0");
+        rc = check_cuda(cudaMemcpyAsync(t_all_or_null, x0, sizeof(float) * slab_elems, cudaMemcpyDeviceToDevice, c.st), "copy T0");
         if (rc) return rc;
     }
     if (cfg.prescaled && !sell_plan) {
-        prescale_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(x0, dinv, ybuf[0], n, f, 0);
+        prescale_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, c.st>>>(x0, dinv, ws.y[0], n, f, 0);
         EGNN_LAUNCH_CHECK("prescale_kernel launch");
     }
-
-    if (sell_plan) {
-        EGNN_REQUIRE(f == 1 && vals_or_null == nullptr, "the SELL plan serves F = 1 on a binary adjacency");
-        EGNN_REQUIRE(sell_plan->n == n && sell_plan->n_cols == n && sell_plan->row0 == 0 && sell_plan->vpart && sell_plan->slice_off && sell_plan->blk_slice_ptr &&
-                     sell_plan->rv_ptr && sell_plan->vslot && sell_plan->cta_info && sell_plan->hub && sell_plan->sched, "SELL plan does not match the graph or is not filled");
-        // all K orders in one persistent launch (sell_step.cuh); the first operand dinv (.) T_0 is
-        // computed inside it
-        SellStepParams sp{};
-        step_fill_plan(sp, sell_plan);
-        sp.delta = p.delta;
-        sp.w_base = w_base_or_null; sp.rowsum_base = rowsum_base_or_null; sp.patch_x0 = default_signal ? 1 : 0;
-        sp.dinv = dinv; sp.iso = iso; sp.x0 = x0;
-        sp.operand_first = y0_or_null;       // dinv (.) T_0 kept by the caller (fixed per graph for the default signal)
-        sp.operand[0] = ybuf[0]; sp.operand[1] = ybuf[1];
-        sp.ydst[0][0] = ybuf[0]; sp.ydst[1][0] = ybuf[1]; sp.n_dst = 1;
-        sp.tbuf[0] = tbuf[0]; sp.tbuf[1] = tbuf[1]; sp.t_all = t_all_or_null; sp.out = out;
-        sp.normalize = normalize_l1; sp.a = op_scale; sp.b = op_shift;
-        sp.world = 1; sp.rank = 0; sp.rows_per = n;
-        if (order_events_host) {
-            rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[0], st), "event record");
-            if (rc) return rc;
-        }
-        rc = run_sell_step(sp, k, n_scales, coeffs_host, false, st);
-        if (rc) return rc;
-        if (order_events_host) {                      // one launch: events 0 and 1 bracket the whole step, the rest follow it
-            for (int e = 1; e < 2 * k; ++e) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[e], st), "event record");
-                if (rc) return rc;
-            }
-        }
-        return EGNN_OK;
-    }
-
-    if (f == 1 && rows_sorted && (nnz >= kBlockedMinNnz || rows_sorted == 2) && nnz > 0) {
-        // first use of a large graph (no SELL plan yet): plan-free column-blocked kernel (blocked.cuh)
-        int C = 1, CB = 32;
-        narrow_geometry(n, &C, &CB);
-        char* extra = ws + 4 * slab;
-        int32_t* seg = (int32_t*)extra;
-        float* part = (float*)(extra + align_up(4 * (size_t)(C + 1) * (size_t)n, 256));
-        unsigned* counters = (unsigned*)((char*)part + align_up(4 * (size_t)C * (size_t)n, 256));
-        rc = check_cuda(cudaMemsetAsync(counters, 0, sizeof(unsigned) * (size_t)k * (size_t)C, st), "memset batch counters");
-        if (rc) return rc;
-        blocked_bounds_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, st>>>(rowptr, colidx, (int)n, C, CB, seg);
-        EGNN_LAUNCH_CHECK("blocked_bounds_kernel launch");
-        const size_t smem = sizeof(float) * (size_t)CB;
-        const void* fn = vals_or_null ? (const void*)blocked_spmv_kernel<true> : (const void*)blocked_spmv_kernel<false>;
-        rc = check_cuda(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
-                        "cudaFuncSetAttribute(blocked_spmv_kernel)");
-        if (rc) return rc;
-        BlockedParams bp{};
-        bp.colidx = colidx; bp.vals = vals_or_null; bp.seg = seg; bp.part = part;
-        bp.n = (int32_t)n; bp.C = C; bp.CB = CB; bp.n_cta = device_sm_count();
-        if (bp.n_cta < C) bp.n_cta = C;
-        BlockedEpilogueParams ep{};
-        ep.delta = p.delta;
-        ep.part = part; ep.dinv = dinv; ep.iso = iso; ep.out = out; ep.n = (int32_t)n; ep.C = C; ep.S = n_scales;
-        ep.a = op_scale; ep.b = op_shift;
-        const float* t_prev = x0;
-        const float* t_prev2 = nullptr;
-        for (int order = 1; order <= k; ++order) {
-            const bool last = order == k;
-            float* t_out;
-            if (t_all_or_null) t_out = t_all_or_null + (size_t)order * slab_elems;
-            else if (last) t_out = nullptr;
-            else if (order == 1) t_out = tbuf[0];
-            else if (order == 2) t_out = tbuf[1];
-            else t_out = const_cast<float*>(t_prev2);
-            if (order_events_host) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[2 * (order - 1)], st), "event record");
-                if (rc) return rc;
-            }
-            bp.y = ybuf[(order - 1) & 1];
-            bp.counter = counters + (size_t)(order - 1) * C;
-            if (vals_or_null) blocked_spmv_kernel<true><<<bp.n_cta, kBlockedThreads, smem, st>>>(bp);
-            else blocked_spmv_kernel<false><<<bp.n_cta, kBlockedThreads, smem, st>>>(bp);
-            EGNN_LAUNCH_CHECK("blocked_spmv_kernel launch");
-            ep.y_prev = bp.y; ep.tprev = t_prev; ep.tprev2 = t_prev2; ep.tk = t_out;
-            ep.y_out = last ? nullptr : ybuf[order & 1];
-            ep.first = order == 1; ep.normalize = last && normalize_l1;
-            for (int s = 0; s < n_scales; ++s) {
-                ep.c_prev[s] = coeffs_host[s * (k + 1) + order - 1];
-                ep.c_k[s] = coeffs_host[s * (k + 1) + order];
-            }
-            blocked_epilogue_kernel<<<(unsigned)ceil_div64(n, 256), 256, 0, st>>>(ep);
-            EGNN_LAUNCH_CHECK("blocked_epilogue_kernel launch");
-            if (order_events_host) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[2 * (order - 1) + 1], st), "event record");
-                if (rc) return rc;
-            }
-            t_prev2 = t_prev;
-            t_prev = t_out;
-        }
-        return EGNN_OK;
-    }
-
-    if (f >= kWideMinF) {
-        const int ldy = (f + 3) / 4 * 4;
-        const RingConfig rcfg = ring_config(ldy);
-        const size_t yslab = align_up(sizeof(float) * (size_t)n * (size_t)ldy, 256);
-        float* yb[2] = {(float*)ws, (float*)(ws + yslab)};       // the two slabs hold dinv (.) T_k, rows padded to 16 bytes
-        WideParams wp{};
-        wp.delta = p.delta;
-        wp.rowptr = rowptr; wp.colidx = colidx; wp.vals = vals_or_null;
-        wp.perm = row_order_or_null; wp.n_hub = row_order_or_null ? row_order_or_null + n : nullptr;
-        wp.dinv = dinv; wp.iso = iso; wp.out = out; wp.n_rows = n; wp.row0 = 0; wp.F = f; wp.ldy = ldy; wp.S = n_scales;
-        wp.a = op_scale; wp.b = op_shift;
-        prescale_pad_kernel<<<grid_for((int64_t)n * ldy, 256), 256, 0, st>>>(x0, dinv, yb[0], n, f, ldy, 0);
-        EGNN_LAUNCH_CHECK("prescale_pad_kernel launch");
-        unsigned* counters = (unsigned*)(ws + 2 * yslab);          // [k][grid_y], zeroed once per call
-        rc = check_cuda(cudaMemsetAsync(counters, 0, sizeof(unsigned) * (size_t)k * (size_t)rcfg.grid_y, st), "memset row counters");
-        if (rc) return rc;
-        const bool fuse_norm_w = normalize_l1 && rcfg.grid_y == 1;
-        const int sms = device_sm_count();
-        for (int order = 1; order <= k; ++order) {
-            const bool last = order == k;
-            wp.first = order == 1;
-            wp.normalize = last && fuse_norm_w;
-            // dynamic rows pay off where rows are short and one feature tile covers the signal (arxiv
-            // shape F = 128: 0.283 -> 0.23 ms per order); measured slower on long rows (Reddit shape
-            // F = 64: 2.13 -> 2.48) and on many feature tiles (Physics F = 8415: 2.77 -> 3.3)
-            const bool dynamic_rows = rcfg.grid_y == 1 && nnz < (int64_t)kWideDynamicMaxDegree * n;
-            wp.row_counter = dynamic_rows ? counters + (size_t)(order - 1) * (size_t)rcfg.grid_y : nullptr;
-            wp.ysrc = yb[(order - 1) & 1];
-            wp.x0_own = order == 1 ? x0 : nullptr;
-            wp.y2_own = order == 1 ? nullptr : yb[order & 1];
-            wp.y_out = last ? nullptr : yb[order & 1];      // in place over dinv (.) T_{k-2} (own row only)
-            wp.tk_out = t_all_or_null ? t_all_or_null + (size_t)order * slab_elems : nullptr;
-            for (int s = 0; s < n_scales; ++s) {
-                wp.c_prev[s] = coeffs_host[s * (k + 1) + order - 1];
-                wp.c_k[s] = coeffs_host[s * (k + 1) + order];
-            }
-            if (order_events_host) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[2 * (order - 1)], st), "event record");
-                if (rc) return rc;
-            }
-            rc = launch_wide(wp, rcfg, sms, st);
-            if (rc) return rc;
-            if (order_events_host) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[2 * (order - 1) + 1], st), "event record");
-                if (rc) return rc;
-            }
-        }
-        if (normalize_l1 && !fuse_norm_w) {
-            l1_normalize_kernel<<<grid_for(n * n_scales * 32, 256), 256, 0, st>>>(out, n * n_scales, f);
-            EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
-        }
-        return EGNN_OK;
-    }
-
-    p.rowptr = rowptr; p.colidx = colidx; p.vals = vals_or_null; p.dinv = dinv; p.iso = iso;
-    p.out = out; p.acc_ws = nullptr; p.n_rows = n; p.row0 = 0; p.F = f; p.S = n_scales;
-    p.a = op_scale; p.b = op_shift; p.mode = 0; p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
-
-    const bool fuse_norm = normalize_l1 && cfg.grid_y == 1;
-    const float* t_prev = x0;         // T_{k-1}
-    const float* t_prev2 = nullptr;   // T_{k-2}
-    for (int order = 1; order <= k; ++order) {
-        const bool last = order == k;
-        float* t_out;
-        if (t_all_or_null) t_out = t_all_or_null + (size_t)order * slab_elems;
-        else if (last) t_out = nullptr;                       // T_K itself is never read again
-        else if (order == 1) t_out = tbuf[0];
-        else if (order == 2) t_out = tbuf[1];
-        else t_out = const_cast<float*>(t_prev2);             // overwrite T_{k-2} in place
-        p.first = order == 1;
-        p.normalize = last && fuse_norm;
-        p.tprev_own = t_prev;
-        p.tprev2_own = t_prev2;
-        p.tk_own = t_out;
-        p.gsrc = cfg.prescaled ? ybuf[(order - 1) & 1] : t_prev;
-        p.y_own = (cfg.prescaled && !last) ? ybuf[order & 1] : nullptr;
-        for (int s = 0; s < n_scales; ++s) {
-            p.c_prev[s] = coeffs_host[s * (k + 1) + order - 1];
-            p.c_k[s] = coeffs_host[s * (k + 1) + order];
-        }
-        if (order_events_host) {
-            rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[2 * (order - 1)], st), "event record");
-            if (rc) return rc;
-        }
-        rc = launch_order(p, cfg, st);
-        if (rc) return rc;
-        if (order_events_host) {
-            rc = check_cuda(cudaEventRecord((cudaEvent_t)order_events_host[2 * (order - 1) + 1], st), "event record");
-            if (rc) return rc;
-        }
-        t_prev2 = t_prev;
-        t_prev = t_out;
-    }
-    if (normalize_l1 && !fuse_norm) {
-        l1_normalize_kernel<<<grid_for(n * n_scales * 32, 256), 256, 0, st>>>(out, n * n_scales, f);
-        EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
-    }
-    return EGNN_OK;
+    if (sell_plan)
+        return wavelet_sell(c, ws, sell_plan, x0, y0_or_null, out, t_all_or_null, normalize_l1, w_base_or_null,
+                            rowsum_base_or_null, default_signal);
+    if (f == 1 && rows_sorted && (nnz >= kBlockedMinNnz || rows_sorted == 2) && nnz > 0)
+        return wavelet_blocked(c, ws, x0, out, t_all_or_null, normalize_l1);
+    if (f >= kWideMinF) return wavelet_wide(c, ws, x0, out, t_all_or_null, normalize_l1);
+    return wavelet_generic(c, ws, cfg, x0, out, t_all_or_null, normalize_l1);
 }
 
 }  // extern "C"
 
 // ---- backward of the wavelet pass (csrc/adjoint.cuh) ------------------------------------------------
-// b_all_or_null: [K+1, n, f] receives Xbar (slab 0) and every Clenshaw vector b_m (slab m); the
-// generic path then keeps its b vectors there instead of the workspace ping-pong slabs.
+// Application j = 1..K produces b_m, m = K - j (b_0 = the signal's gradient).  b_all: [K+1, n, f]
+// receives Xbar (slab 0) and every Clenshaw vector b_m (slab m); the generic path then keeps its
+// b vectors there instead of the workspace ping-pong slabs.
+static int adjoint_wide(const ChebArgs& c, const ChebWs& ws, const float* cbar, const float* tbar, float* xbar,
+                        float* b_all) {
+    const int64_t n = c.rows;
+    const int k = c.k;
+    const size_t slab_elems = (size_t)n * (size_t)c.f;
+    const int ldy = wide_ldy(c.f);
+    const RingConfig rcfg = ring_config(ldy);
+    int rc = check_cuda(cudaMemsetAsync(ws.row_counters, 0, sizeof(unsigned) * (size_t)k * (size_t)rcfg.grid_y, c.st),
+                        "memset row counters");
+    if (rc) return rc;
+    // ws.y[] hold dinv (.) b, rows padded to 16 bytes
+    adjoint_prologue_kernel<<<grid_for(n * ldy, 256), 256, 0, c.st>>>(
+        cbar, slab_of(tbar, slab_elems, k), c.dinv, slab_of(b_all, slab_elems, k), ws.y[0], n, c.f, c.S, ldy,
+        coef_row(c.coeffs, k, c.S, k));
+    EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+    WideParams wp = wide_params(c);
+    wp.cbar = cbar;
+    const bool dynamic_rows = rcfg.grid_y == 1 && c.nnz < (int64_t)kWideDynamicMaxDegree * n;   // as the forward
+    const int sms = device_sm_count();
+    for (int j = 1; j <= k; ++j) {
+        const int m = k - j;
+        wp.row_counter = dynamic_rows ? ws.row_counters + (size_t)(j - 1) * (size_t)rcfg.grid_y : nullptr;
+        wp.ysrc = ws.y[(j - 1) & 1];
+        wp.y2_own = j == 1 ? nullptr : ws.y[j & 1];
+        wp.y_out = m == 0 ? nullptr : ws.y[j & 1];           // in place over dinv (.) b_{m+2} (own row only)
+        wp.tk_out = m == 0 ? xbar : slab_of(b_all, slab_elems, m);
+        wp.tbar = slab_of(tbar, slab_elems, m);
+        wp.c_adj = m == 0 ? 1.f : 2.f;
+        order_coefs(wp.c_k, c.coeffs, k, c.S, m);
+        rc = record_event(c.events, 2 * (j - 1), c.st);
+        if (rc) return rc;
+        rc = launch_wide<true>(wp, rcfg, sms, c.st);
+        if (rc) return rc;
+        rc = record_event(c.events, 2 * (j - 1) + 1, c.st);
+        if (rc) return rc;
+    }
+    return EGNN_OK;
+}
+
+static int adjoint_generic(const ChebArgs& c, const ChebWs& ws, const float* cbar, const float* tbar, float* xbar,
+                           float* b_all) {
+    const int64_t n = c.rows;
+    const int k = c.k;
+    const size_t slab_elems = (size_t)n * (size_t)c.f;
+    const OrderConfig cfg = choose_config(n, c.nnz, c.f);
+    // b_m of application j: ws.t[j & 1] (in place over b_{m+2}), or slab m of b_all
+    auto b_vec = [&](int j) { return b_all ? slab_of(b_all, slab_elems, k - j) : ws.t[j & 1]; };
+    adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, c.st>>>(
+        cbar, slab_of(tbar, slab_elems, k), c.dinv, b_vec(0), cfg.prescaled ? ws.y[0] : nullptr, n, c.f, c.S, c.f,
+        coef_row(c.coeffs, k, c.S, k));
+    EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+    OrderParams p = order_params(c, cfg);
+    p.cbar = cbar;
+    for (int j = 1; j <= k; ++j) {
+        const int m = k - j;
+        p.tprev_own = b_vec(j - 1);
+        p.tprev2_own = j == 1 ? nullptr : b_vec(j - 2);
+        p.tk_own = m == 0 ? xbar : b_vec(j);
+        p.gsrc = cfg.prescaled ? ws.y[(j - 1) & 1] : b_vec(j - 1);
+        p.y_own = (cfg.prescaled && m > 0) ? ws.y[j & 1] : nullptr;
+        p.tbar = slab_of(tbar, slab_elems, m);
+        p.c_adj = m == 0 ? 1.f : 2.f;
+        order_coefs(p.c_k, c.coeffs, k, c.S, m);
+        int rc = record_event(c.events, 2 * (j - 1), c.st);
+        if (rc) return rc;
+        rc = launch_order<true>(p, cfg, c.st);
+        if (rc) return rc;
+        rc = record_event(c.events, 2 * (j - 1) + 1, c.st);
+        if (rc) return rc;
+    }
+    return EGNN_OK;
+}
+
 static int cheb_adjoint_impl(const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
                              const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f, int32_t k,
                              int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
@@ -846,117 +1005,72 @@ static int cheb_adjoint_impl(const int32_t* rowptr_t, const int32_t* colidx_t, c
     EGNN_REQUIRE(vec_aligned(cbar, f) && vec_aligned(tbar_or_null, f) && vec_aligned(xbar, f) &&
                  vec_aligned(b_all_or_null, f), "cbar, tbar, xbar and b_all must be 16-byte aligned when f % 4 == 0");
     if (n == 0) return EGNN_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    OrderParams p{};
-    int rc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    ChebArgs c{};
+    c.rowptr = rowptr_t; c.colidx = colidx_t; c.vals = vals_t_or_null; c.row_order = row_order_or_null;
+    c.dinv = dinv; c.iso = iso; c.rows = n; c.nnz = nnz; c.f = f; c.k = k; c.S = n_scales;
+    c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.events = app_events_host; c.st = (cudaStream_t)stream;
+    int rc = fill_delta(c.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(p.delta.row[i] >= 0 && p.delta.row[i] < n && p.delta.col[i] >= 0 && p.delta.col[i] < n,
-                     "delta index out of range");
     const size_t slab_elems = (size_t)n * (size_t)f;
-    auto coef_row = [&](int m) {
-        CoefRow c{};
-        for (int s = 0; s < n_scales; ++s) c.c[s] = coeffs_host[s * (k + 1) + m];
-        return c;
-    };
-    auto tbar_at = [&](int m) { return tbar_or_null ? tbar_or_null + (size_t)m * slab_elems : nullptr; };
-    auto b_at = [&](int m) { return b_all_or_null ? b_all_or_null + (size_t)m * slab_elems : nullptr; };
-    auto copy_xbar = [&]() {
-        return b_all_or_null ? check_cuda(cudaMemcpyAsync(b_all_or_null, xbar, sizeof(float) * slab_elems,
-                                                          cudaMemcpyDeviceToDevice, st), "copy Xbar")
-                             : EGNN_OK;
-    };
     if (k == 0) {
-        adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
-            cbar, tbar_at(0), dinv, xbar, nullptr, n, f, n_scales, f, coef_row(0));
+        adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, c.st>>>(
+            cbar, tbar_or_null, dinv, xbar, nullptr, n, f, n_scales, f, coef_row(coeffs_host, 0, n_scales, 0));
         EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
-        return copy_xbar();
-    }
-    const size_t need = egnn_cheb_workspace_bytes(n, f);
-    if (workspace == nullptr || workspace_bytes < need) {
-        set_error("workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
-    char* ws = (char*)align_up((size_t)workspace, 256);
-    // application j = 1..K produces b_m, m = K - j (b_0 = the signal's gradient)
-    if (f >= kWideMinF) {
-        const int ldy = (f + 3) / 4 * 4;
-        const RingConfig rcfg = ring_config(ldy);
-        const size_t yslab = align_up(sizeof(float) * (size_t)n * (size_t)ldy, 256);
-        float* yb[2] = {(float*)ws, (float*)(ws + yslab)};        // dinv (.) b, rows padded to 16 bytes
-        unsigned* counters = (unsigned*)(ws + 2 * yslab);
-        rc = check_cuda(cudaMemsetAsync(counters, 0, sizeof(unsigned) * (size_t)k * (size_t)rcfg.grid_y, st), "memset row counters");
+    } else {
+        rc = require_workspace(workspace, workspace_bytes, egnn_cheb_workspace_bytes(n, f), "workspace");
         if (rc) return rc;
-        adjoint_prologue_kernel<<<grid_for((int64_t)n * ldy, 256), 256, 0, st>>>(
-            cbar, tbar_at(k), dinv, b_at(k), yb[0], n, f, n_scales, ldy, coef_row(k));
-        EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
-        WideParams wp{};
-        wp.delta = p.delta;
-        wp.rowptr = rowptr_t; wp.colidx = colidx_t; wp.vals = vals_t_or_null;
-        wp.perm = row_order_or_null; wp.n_hub = row_order_or_null ? row_order_or_null + n : nullptr;
-        wp.dinv = dinv; wp.iso = iso; wp.out = nullptr; wp.n_rows = n; wp.row0 = 0; wp.F = f; wp.ldy = ldy;
-        wp.S = n_scales; wp.a = op_scale; wp.b = op_shift; wp.first = 0; wp.normalize = 0;
-        wp.cbar = cbar; wp.x0_own = nullptr;
-        const bool dynamic_rows = rcfg.grid_y == 1 && nnz < (int64_t)kWideDynamicMaxDegree * n;   // as the forward
-        const int sms = device_sm_count();
-        for (int j = 1; j <= k; ++j) {
-            const int m = k - j;
-            wp.row_counter = dynamic_rows ? counters + (size_t)(j - 1) * (size_t)rcfg.grid_y : nullptr;
-            wp.ysrc = yb[(j - 1) & 1];
-            wp.y2_own = j == 1 ? nullptr : yb[j & 1];
-            wp.y_out = m == 0 ? nullptr : yb[j & 1];             // in place over dinv (.) b_{m+2} (own row only)
-            wp.tk_out = m == 0 ? xbar : b_at(m);
-            wp.tbar = tbar_at(m);
-            wp.c_adj = m == 0 ? 1.f : 2.f;
-            for (int s = 0; s < n_scales; ++s) wp.c_k[s] = coeffs_host[s * (k + 1) + m];
-            if (app_events_host) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1)], st), "event record");
-                if (rc) return rc;
-            }
-            rc = launch_wide<true>(wp, rcfg, sms, st);
-            if (rc) return rc;
-            if (app_events_host) {
-                rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1) + 1], st), "event record");
-                if (rc) return rc;
-            }
-        }
-        return copy_xbar();
-    }
-    const OrderConfig cfg = choose_config(n, nnz, f);
-    const size_t slab = align_up(sizeof(float) * slab_elems, 256);
-    float* tbuf[2] = {(float*)ws, (float*)(ws + slab)};
-    float* ybuf[2] = {(float*)(ws + 2 * slab), (float*)(ws + 3 * slab)};
-    // b_m of application j: tbuf[j & 1] (in place over b_{m+2}), or slab m of b_all
-    auto b_vec = [&](int j) { return b_all_or_null ? b_at(k - j) : tbuf[j & 1]; };
-    adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
-        cbar, tbar_at(k), dinv, b_vec(0), cfg.prescaled ? ybuf[0] : nullptr, n, f, n_scales, f, coef_row(k));
-    EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
-    p.rowptr = rowptr_t; p.colidx = colidx_t; p.vals = vals_t_or_null; p.dinv = dinv; p.iso = iso;
-    p.out = nullptr; p.acc_ws = nullptr; p.n_rows = n; p.row0 = 0; p.F = f; p.S = n_scales;
-    p.a = op_scale; p.b = op_shift; p.mode = 0; p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
-    p.first = 0; p.normalize = 0; p.cbar = cbar;
-    for (int j = 1; j <= k; ++j) {
-        const int m = k - j;
-        p.tprev_own = b_vec(j - 1);
-        p.tprev2_own = j == 1 ? nullptr : b_vec(j - 2);
-        p.tk_own = m == 0 ? xbar : b_vec(j);
-        p.gsrc = cfg.prescaled ? ybuf[(j - 1) & 1] : b_vec(j - 1);
-        p.y_own = (cfg.prescaled && m > 0) ? ybuf[j & 1] : nullptr;
-        p.tbar = tbar_at(m);
-        p.c_adj = m == 0 ? 1.f : 2.f;
-        for (int s = 0; s < n_scales; ++s) p.c_k[s] = coeffs_host[s * (k + 1) + m];
-        if (app_events_host) {
-            rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1)], st), "event record");
-            if (rc) return rc;
-        }
-        rc = launch_order<true>(p, cfg, st);
+        const ChebWs ws = cheb_ws_layout(workspace, n, f);
+        rc = f >= kWideMinF ? adjoint_wide(c, ws, cbar, tbar_or_null, xbar, b_all_or_null)
+                            : adjoint_generic(c, ws, cbar, tbar_or_null, xbar, b_all_or_null);
         if (rc) return rc;
-        if (app_events_host) {
-            rc = check_cuda(cudaEventRecord((cudaEvent_t)app_events_host[2 * (j - 1) + 1], st), "event record");
-            if (rc) return rc;
-        }
     }
-    return copy_xbar();
+    return b_all_or_null ? check_cuda(cudaMemcpyAsync(b_all_or_null, xbar, sizeof(float) * slab_elems,
+                                                      cudaMemcpyDeviceToDevice, c.st), "copy Xbar")
+                         : EGNN_OK;
+}
+
+// ---- one order (adjoint application) of a row shard ----------------------------------------------
+// Generic kernel, split over the rank's local and remote columns: phase 0 sums the local columns
+// into p.acc_ws, phase 1 adds the remote columns from the gathered operand and runs the epilogue,
+// phase 2 is one launch over the unsplit rows.  The edge flips ride with the launch that gathers
+// from the exchanged operand, so phase 0 does not look at them.  p comes filled for the local CSR.
+template <bool ADJ>
+static int order_sharded_phase(OrderParams& p, const OrderConfig& cfg, int32_t phase, const int32_t* rowptr_remote,
+                               const int32_t* colidx_remote, const float* gathered, const char* gathered_missing,
+                               const int32_t* delta_row_host, const int32_t* delta_col_host,
+                               const float* delta_val_host, int32_t n_delta, int64_t n, cudaStream_t st) {
+    if (phase == 0) {                 // local columns: gathers hit the rank's own slab
+        EGNN_REQUIRE(p.rowptr && p.acc_ws, "local half missing");
+        p.gsrc = p.tprev_own - p.row0 * (int64_t)p.F;      // indexed by global column, only own rows touched
+        p.mode = 1;
+        p.normalize = 0;
+        return launch_order<ADJ>(p, cfg, st);
+    }
+    int rc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
+    if (rc) return rc;
+    EGNN_REQUIRE(gathered != nullptr, gathered_missing);
+    p.gsrc = gathered;
+    if (phase == 1) {                 // remote columns + epilogue
+        EGNN_REQUIRE(rowptr_remote && p.acc_ws, "remote half missing");
+        p.rowptr = rowptr_remote; p.colidx = colidx_remote; p.mode = 2;
+    } else {                          // one launch over the unsplit rows
+        EGNN_REQUIRE(p.rowptr != nullptr, "csr missing");
+    }
+    return launch_order<ADJ>(p, cfg, st);
+}
+
+// Wide kernel with the exchange fused: order (application) `step` reads buffer (step - 1) & 1 of
+// the own window - the full operand, global rows - and, unless it is the last, stores the next
+// operand into buffer step & 1 of every rank's window (a plain store into the own rows at world 1).
+template <bool ADJ>
+static int wide_sharded_step(WideParams& wp, const RingConfig& rcfg, const egnn_peer_window* win, int step, bool last,
+                             cudaStream_t st) {
+    wp.ysrc = peer_operand(win, win->rank, (step - 1) & 1);
+    float* own_next = peer_operand(win, win->rank, step & 1) + wp.row0 * (int64_t)wp.ldy;
+    wp.y2_own = step == 1 ? nullptr : own_next;                  // dinv (.) T_{k-2} (b_{m+2}) of the own rows
+    wp.y_out = (!last && win->world == 1) ? own_next : nullptr;
+    fill_peer_push(wp.peer, win, step & 1, !last, false);
+    return launch_wide<ADJ>(wp, rcfg, device_sm_count(), st);
 }
 
 extern "C" {
@@ -1021,11 +1135,9 @@ int egnn_cheb_coeff_grad(const float* cbar, const float* t_all, int64_t n, int32
     EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && f >= 1, "bad shape");
     EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "k out of range");
     EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
-    const size_t need = egnn_cheb_coeff_grad_ws_bytes(k, n_scales);
-    if (workspace == nullptr || workspace_bytes < need) {
-        set_error("coefficient-gradient workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    int rc = require_workspace(workspace, workspace_bytes, egnn_cheb_coeff_grad_ws_bytes(k, n_scales),
+                               "coefficient-gradient workspace");
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     double* partial = (double*)align_up((size_t)workspace, 256);
     coeff_grad_partial_kernel<<<kCoefGradBlocks, kCoefGradThreads, 0, st>>>(cbar, t_all, n, f, k, n_scales, partial);
@@ -1057,11 +1169,8 @@ int egnn_csr_transpose(const int32_t* rowptr, const int32_t* colidx, const float
     EGNN_REQUIRE(nnz == 0 || (colidx && colidx_t), "null colidx");
     EGNN_REQUIRE((vals_or_null == nullptr) == (vals_t_or_null == nullptr), "vals and vals_t come together");
     EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
-    const size_t need = egnn_csr_transpose_ws_bytes(n, nnz);
-    if (workspace == nullptr || workspace_bytes < need) {
-        set_error("transpose workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    int rc = require_workspace(workspace, workspace_bytes, egnn_csr_transpose_ws_bytes(n, nnz), "transpose workspace");
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const size_t arr = align_up(4 * (size_t)(nnz > 0 ? nnz : 1), 256);
     char* ws = (char*)align_up((size_t)workspace, 256);
@@ -1071,7 +1180,7 @@ int egnn_csr_transpose(const int32_t* rowptr, const int32_t* colidx, const float
     int32_t* counts = (int32_t*)(ws + 3 * arr);
     void* cub_temp = ws + 3 * arr + align_up(4 * (size_t)(n + 1), 256);
     size_t cub_bytes = transpose_cub_bytes(n, nnz);
-    int rc = check_cuda(cudaMemsetAsync(counts, 0, sizeof(int32_t) * (size_t)(n + 1), st), "memset column counts");
+    rc = check_cuda(cudaMemsetAsync(counts, 0, sizeof(int32_t) * (size_t)(n + 1), st), "memset column counts");
     if (rc) return rc;
     if (nnz > 0) {
         transpose_count_kernel<<<grid_for(nnz, 256), 256, 0, st>>>(colidx, nnz, ids, counts);
@@ -1114,11 +1223,9 @@ int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const flo
     EGNN_REQUIRE((xbar_or_null == nullptr) || rowsum_or_null, "xbar needs rowsum");
     EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
     EGNN_REQUIRE(f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER, "bad f / k");
-    const size_t need = egnn_adj_grad_degree_ws_bytes(n);
-    if (workspace == nullptr || workspace_bytes < need) {
-        set_error("adjacency-gradient workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    int rc = require_workspace(workspace, workspace_bytes, egnn_adj_grad_degree_ws_bytes(n),
+                               "adjacency-gradient workspace");
+    if (rc) return rc;
     if (n == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
     double* r = (double*)align_up((size_t)workspace, 256);
@@ -1186,53 +1293,25 @@ int egnn_cheb_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_l
     const int64_t rows = row_end - row_begin;
     if (rows == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
-
-    OrderParams p{};
-    p.delta.n = 0;
-    if (phase != 0) {                 // edge flips ride with the launch that gathers from the exchanged operand
-        int drc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
-        if (drc) return drc;
-        for (int i = 0; i < n_delta; ++i)
-            EGNN_REQUIRE(p.delta.row[i] >= 0 && p.delta.row[i] < n && p.delta.col[i] >= 0 && p.delta.col[i] < n,
-                         "delta index out of range");
-    }
-    p.vals = nullptr; p.dinv = dinv_full; p.iso = iso_full;
-    p.tprev_own = t_prev_local; p.tprev2_own = t_prev2_local; p.tk_own = t_out_local; p.y_own = nullptr;
-    p.out = out_local; p.acc_ws = acc_ws; p.n_rows = rows; p.row0 = row_begin; p.F = f; p.S = n_scales;
-    p.a = op_scale; p.b = op_shift; p.first = order == 1;
-    for (int s = 0; s < n_scales; ++s) {
-        p.c_prev[s] = coeffs_host[s * (k_max + 1) + order - 1];
-        p.c_k[s] = coeffs_host[s * (k_max + 1) + order];
-    }
+    ChebArgs c{};
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.dinv = dinv_full; c.iso = iso_full;
+    c.rows = rows; c.row0 = row_begin; c.nnz = nnz_hint; c.f = f; c.k = k_max; c.S = n_scales;
+    c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
     OrderConfig cfg = choose_config(rows, nnz_hint, f);
     cfg.prescaled = false;            // sharded slabs carry plain T_k (what the exchange moves)
-    p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
+    OrderParams p = order_params(c, cfg);
+    p.tprev_own = t_prev_local; p.tprev2_own = t_prev2_local; p.tk_own = t_out_local;
+    p.out = out_local; p.acc_ws = acc_ws; p.first = order == 1;
+    order_coefs(p.c_prev, coeffs_host, k_max, n_scales, order - 1);
+    order_coefs(p.c_k, coeffs_host, k_max, n_scales, order);
     const bool last = order == k_max;
     const bool fuse_norm = normalize_l1 && cfg.grid_y == 1;
-    int rc;
-    if (phase == 0) {                 // local columns: gathers hit the rank's own slab
-        EGNN_REQUIRE(rowptr_local && acc_ws, "local half missing");
-        p.rowptr = rowptr_local; p.colidx = colidx_local;
-        p.gsrc = t_prev_local - row_begin * (int64_t)f;      // indexed by global column, only own rows touched
-        p.mode = 1; p.normalize = 0;
-        return launch_order(p, cfg, st);
-    }
-    EGNN_REQUIRE(t_prev_full != nullptr, "gathered T_{k-1} missing");
-    p.gsrc = t_prev_full;
     p.normalize = last && fuse_norm;
-    if (phase == 1) {                 // remote columns + epilogue
-        EGNN_REQUIRE(rowptr_remote && acc_ws, "remote half missing");
-        p.rowptr = rowptr_remote; p.colidx = colidx_remote; p.mode = 2;
-    } else {                          // one launch over the unsplit rows
-        EGNN_REQUIRE(rowptr_local != nullptr, "csr missing");
-        p.rowptr = rowptr_local; p.colidx = colidx_local; p.mode = 0;
-    }
-    rc = launch_order(p, cfg, st);
+    int rc = order_sharded_phase<false>(p, cfg, phase, rowptr_remote, colidx_remote, t_prev_full,
+                                        "gathered T_{k-1} missing", delta_row_host, delta_col_host, delta_val_host,
+                                        n_delta, n, st);
     if (rc) return rc;
-    if (last && normalize_l1 && !fuse_norm) {
-        l1_normalize_kernel<<<grid_for(rows * n_scales * 32, 256), 256, 0, st>>>(out_local, rows * n_scales, f);
-        EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
-    }
+    if (phase != 0 && last && normalize_l1 && !fuse_norm) return launch_l1_normalize(out_local, rows, n_scales, f, st);
     return EGNN_OK;
 }
 
@@ -1260,10 +1339,8 @@ int egnn_sell_prepare(const int32_t* rowptr, const int32_t* colidx, int64_t n, i
     EGNN_REQUIRE(rowptr && (colidx || nnz == 0), "null pointer");
     const int C = plan->n_blocks, CB = plan->col_block, lmax = plan->lmax;
     SellWs w = sell_ws_layout(workspace, n, nnz, C, lmax);
-    if (!workspace || workspace_bytes < w.total_bytes) {
-        set_error("sell workspace too small: need %zu bytes, got %zu", w.total_bytes, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    rc = require_workspace(workspace, workspace_bytes, w.total_bytes, "sell workspace");
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t cn = (int64_t)C * n;
     rc = check_cuda(cudaMemsetAsync(w.nv + cn, 0, 4, st), "memset"); if (rc) return rc;
@@ -1320,10 +1397,8 @@ int egnn_sell_fill(const int32_t* rowptr, const int32_t* colidx, int64_t n, int6
     EGNN_REQUIRE(plan->n_vrows == 0 || plan->vslot, "plan vslot not allocated");
     const int C = plan->n_blocks, CB = plan->col_block, lmax = plan->lmax;
     SellWs w = sell_ws_layout(workspace, n, nnz, C, lmax);
-    if (!workspace || workspace_bytes < w.total_bytes) {
-        set_error("sell workspace too small: need %zu bytes, got %zu", w.total_bytes, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    rc = require_workspace(workspace, workspace_bytes, w.total_bytes, "sell workspace");
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     rc = check_cuda(cudaMemcpyAsync(plan->slice_off, w.slice_off, 4 * (plan->n_slices + 1), cudaMemcpyDeviceToDevice, st), "copy slice_off"); if (rc) return rc;
     rc = check_cuda(cudaMemcpyAsync(plan->blk_slice_ptr, w.bsp, 4 * (C + 1), cudaMemcpyDeviceToDevice, st), "copy blk_slice_ptr"); if (rc) return rc;
@@ -1388,11 +1463,8 @@ int egnn_sell_step_sharded(const egnn_sell_plan* plan, const float* dinv_full, c
         EGNN_REQUIRE(order_end == k_max || (y_slab0 && y_slab1), "operand slabs missing");
     }
     SellStepParams sp{};
-    int rc = fill_delta(sp.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    int rc = fill_delta(sp.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, plan->n_cols);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(sp.delta.row[i] >= 0 && sp.delta.row[i] < plan->n_cols && sp.delta.col[i] >= 0 && sp.delta.col[i] < plan->n_cols,
-                     "delta index out of range");
     step_fill_plan(sp, plan);
     sp.w_base = w_base_or_null; sp.rowsum_base = rowsum_base_or_null; sp.patch_x0 = default_signal ? 1 : 0;
     sp.dinv = dinv_full; sp.iso = iso_full; sp.x0 = x0_local; sp.operand_first = y_first_full;
@@ -1431,11 +1503,9 @@ int egnn_calibration_metrics(const float* x, int32_t is_log, const int64_t* labe
                              size_t workspace_bytes, egnn_stream_t stream) {
     EGNN_REQUIRE(x && labels && out3, "null pointer");
     EGNN_REQUIRE(n >= 0 && n_classes >= 1 && n_bins >= 1 && n_bins <= kEceMaxBins, "bad shape");
-    const size_t need = egnn_calibration_metrics_ws_bytes(n_classes, n_bins);
-    if (!workspace || workspace_bytes < need) {
-        set_error("metrics workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
-        return EGNN_ERR_WORKSPACE;
-    }
+    int rc = require_workspace(workspace, workspace_bytes, egnn_calibration_metrics_ws_bytes(n_classes, n_bins),
+                               "metrics workspace");
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     char* base = (char*)align_up((size_t)workspace, 256);
     const size_t arr = align_up(8 * (size_t)n_classes * n_bins, 256);
@@ -1444,7 +1514,7 @@ int egnn_calibration_metrics(const float* x, int32_t is_log, const int64_t* labe
     ws.count = (unsigned long long*)(base + arr);
     ws.hits = (unsigned long long*)(base + 2 * arr);
     ws.scalars = (double*)(base + 3 * arr);
-    int rc = check_cuda(cudaMemsetAsync(base, 0, 3 * arr + 64, st), "memset metrics workspace");
+    rc = check_cuda(cudaMemsetAsync(base, 0, 3 * arr + 64, st), "memset metrics workspace");
     if (rc) return rc;
     if (n > 0) {
         ece_accumulate_kernel<<<grid_for(n * 32, 256), 256, 0, st>>>(x, is_log, labels, mask_or_null, n, n_classes, n_bins, ws);
@@ -1559,14 +1629,12 @@ int egnn_peer_prescale_push(const float* x_local, const float* dinv_full, int64_
     EGNN_REQUIRE(n_rows >= 0 && row0 >= 0 && f >= 1 && (n_rows == 0 || x_local), "bad shape");
     int rc = peer_check(win);
     if (rc) return rc;
-    EGNN_REQUIRE(win->f == (f >= kWideMinF ? (f + 3) / 4 * 4 : f) && row0 + n_rows <= (int64_t)win->world * win->rows_per,
+    EGNN_REQUIRE(win->f == (f >= kWideMinF ? wide_ldy(f) : f) && row0 + n_rows <= (int64_t)win->world * win->rows_per,
                  "window does not fit the signal");
     PeerPush pp{};
     fill_peer_push(pp, win, 0, true, true);
-    int64_t blocks = ceil_div64(n_rows > 0 ? n_rows * win->f : 1, 1024);      // at most one CTA per SM: one system fence each
-    const int sms = device_sm_count();
-    if (blocks > sms) blocks = sms;
-    peer_prescale_push_kernel<<<(unsigned)blocks, 1024, 0, (cudaStream_t)stream>>>(x_local, dinv_full, n_rows, row0, f, win->f, pp);
+    peer_prescale_push_kernel<<<push_grid(n_rows * win->f), 1024, 0, (cudaStream_t)stream>>>(x_local, dinv_full, n_rows,
+                                                                                            row0, f, win->f, pp);
     EGNN_LAUNCH_CHECK("peer_prescale_push_kernel launch");
     return EGNN_OK;
 }
@@ -1587,42 +1655,29 @@ int egnn_wide_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_l
     EGNN_REQUIRE(order > 1 || x0_local || row_end == row_begin, "T_0 rows missing");
     int rc = peer_check(win);
     if (rc) return rc;
-    const int ldy = (f + 3) / 4 * 4;
-    EGNN_REQUIRE(win->f == ldy && (int64_t)win->world * win->rows_per >= n_global, "window does not fit the signal");
+    EGNN_REQUIRE(win->f == wide_ldy(f) && (int64_t)win->world * win->rows_per >= n_global, "window does not fit the signal");
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t rows = row_end - row_begin;
-    const RingConfig rcfg = ring_config(ldy);
-    WideParams wp{};
-    rc = fill_delta(wp.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    ChebArgs c{};
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.vals = vals_or_null; c.row_order = row_order_or_null;
+    c.dinv = dinv_full; c.iso = iso_full; c.rows = rows; c.row0 = row_begin; c.f = f; c.k = k_max; c.S = n_scales;
+    c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
+    rc = fill_delta(c.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, n_global);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(wp.delta.row[i] >= 0 && wp.delta.row[i] < n_global && wp.delta.col[i] >= 0 && wp.delta.col[i] < n_global,
-                     "delta index out of range");
-    wp.rowptr = rowptr_local; wp.colidx = colidx_local; wp.vals = vals_or_null;
-    wp.perm = row_order_or_null; wp.n_hub = row_order_or_null ? row_order_or_null + rows : nullptr;
-    wp.dinv = dinv_full; wp.iso = iso_full; wp.out = out_local; wp.n_rows = rows; wp.row0 = row_begin;
-    wp.F = f; wp.ldy = ldy; wp.S = n_scales; wp.a = op_scale; wp.b = op_shift;
+    const RingConfig rcfg = ring_config(wide_ldy(f));
     const bool last = order == k_max;
     const bool fuse_norm = normalize_l1 && rcfg.grid_y == 1;
+    WideParams wp = wide_params(c);
+    wp.out = out_local;
     wp.first = order == 1;
     wp.normalize = last && fuse_norm;
-    wp.ysrc = peer_operand(win, win->rank, (order - 1) & 1);                  // full operand, global rows
     wp.x0_own = order == 1 ? x0_local : nullptr;
-    float* own_next = peer_operand(win, win->rank, order & 1) + row_begin * (int64_t)ldy;
-    wp.y2_own = order == 1 ? nullptr : own_next;                              // dinv (.) T_{k-2} of the own rows
-    wp.y_out = (!last && win->world == 1) ? own_next : nullptr;               // single rank: plain store
     wp.tk_out = t_out_local_or_null;
-    for (int s = 0; s < n_scales; ++s) {
-        wp.c_prev[s] = coeffs_host[s * (k_max + 1) + order - 1];
-        wp.c_k[s] = coeffs_host[s * (k_max + 1) + order];
-    }
-    fill_peer_push(wp.peer, win, order & 1, !last, false);
-    rc = launch_wide(wp, rcfg, device_sm_count(), st);
+    order_coefs(wp.c_prev, coeffs_host, k_max, n_scales, order - 1);
+    order_coefs(wp.c_k, coeffs_host, k_max, n_scales, order);
+    rc = wide_sharded_step<false>(wp, rcfg, win, order, last, st);
     if (rc) return rc;
-    if (last && normalize_l1 && !fuse_norm && rows > 0) {
-        l1_normalize_kernel<<<grid_for(rows * n_scales * 32, 256), 256, 0, st>>>(out_local, rows * n_scales, f);
-        EGNN_LAUNCH_CHECK("l1_normalize_kernel launch");
-    }
+    if (last && normalize_l1 && !fuse_norm && rows > 0) return launch_l1_normalize(out_local, rows, n_scales, f, st);
     return EGNN_OK;
 }
 
@@ -1662,50 +1717,26 @@ int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx
     cudaStream_t st = (cudaStream_t)stream;
     const size_t slab_elems = (size_t)rows * (size_t)f;
     const int m = k_max - app;
-    const float* tbar_m = tbar_local_or_null ? tbar_local_or_null + (size_t)m * slab_elems : nullptr;
+    const float* tbar_m = slab_of(tbar_local_or_null, slab_elems, m);
     if (app == 0) {
-        CoefRow c{};
-        for (int s = 0; s < n_scales; ++s) c.c[s] = coeffs_host[s * (k_max + 1) + k_max];
         adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
-            cbar_local, tbar_m, dinv_full + row_begin, b_out_local, nullptr, rows, f, n_scales, f, c);
+            cbar_local, tbar_m, dinv_full + row_begin, b_out_local, nullptr, rows, f, n_scales, f,
+            coef_row(coeffs_host, k_max, n_scales, k_max));
         EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
         return EGNN_OK;
     }
-    OrderParams p{};
-    p.delta.n = 0;
-    if (phase != 0) {                 // the flips (already transposed) ride with the launch that sees the exchange
-        rc = fill_delta(p.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
-        if (rc) return rc;
-        for (int i = 0; i < n_delta; ++i)
-            EGNN_REQUIRE(p.delta.row[i] >= 0 && p.delta.row[i] < n && p.delta.col[i] >= 0 && p.delta.col[i] < n,
-                         "delta index out of range");
-    }
-    p.vals = nullptr; p.dinv = dinv_full; p.iso = iso_full;
-    p.tprev_own = b_prev_local; p.tprev2_own = b_prev2_local_or_null; p.tk_own = b_out_local; p.y_own = nullptr;
-    p.out = nullptr; p.acc_ws = acc_ws; p.n_rows = rows; p.row0 = row_begin; p.F = f; p.S = n_scales;
-    p.a = op_scale; p.b = op_shift; p.first = 0; p.normalize = 0;
-    p.cbar = cbar_local; p.tbar = tbar_m; p.c_adj = m == 0 ? 1.f : 2.f;
-    for (int s = 0; s < n_scales; ++s) p.c_k[s] = coeffs_host[s * (k_max + 1) + m];
+    ChebArgs c{};
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.dinv = dinv_full; c.iso = iso_full;
+    c.rows = rows; c.row0 = row_begin; c.nnz = nnz_hint; c.f = f; c.k = k_max; c.S = n_scales;
+    c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
     OrderConfig cfg = choose_config(rows, nnz_hint, f);
     cfg.prescaled = false;            // sharded slabs carry plain b (what the exchange moves)
-    p.fl_log2 = cfg.fl_log2; p.nz_log2 = cfg.nz_log2;
-    if (phase == 0) {                 // local columns: gathers hit the rank's own slab
-        EGNN_REQUIRE(rowptr_local && acc_ws, "local half missing");
-        p.rowptr = rowptr_local; p.colidx = colidx_local;
-        p.gsrc = b_prev_local - row_begin * (int64_t)f;      // indexed by global column, only own rows touched
-        p.mode = 1;
-        return launch_order<true>(p, cfg, st);
-    }
-    EGNN_REQUIRE(b_prev_full != nullptr, "gathered b_{m+1} missing");
-    p.gsrc = b_prev_full;
-    if (phase == 1) {                 // remote columns + epilogue
-        EGNN_REQUIRE(rowptr_remote && acc_ws, "remote half missing");
-        p.rowptr = rowptr_remote; p.colidx = colidx_remote; p.mode = 2;
-    } else {                          // one launch over the unsplit rows
-        EGNN_REQUIRE(rowptr_local != nullptr, "csr missing");
-        p.rowptr = rowptr_local; p.colidx = colidx_local; p.mode = 0;
-    }
-    return launch_order<true>(p, cfg, st);
+    OrderParams p = order_params(c, cfg);
+    p.tprev_own = b_prev_local; p.tprev2_own = b_prev2_local_or_null; p.tk_own = b_out_local; p.acc_ws = acc_ws;
+    p.cbar = cbar_local; p.tbar = tbar_m; p.c_adj = m == 0 ? 1.f : 2.f;
+    order_coefs(p.c_k, coeffs_host, k_max, n_scales, m);
+    return order_sharded_phase<true>(p, cfg, phase, rowptr_remote, colidx_remote, b_prev_full, "gathered b_{m+1} missing",
+                                     delta_row_host, delta_col_host, delta_val_host, n_delta, n, st);
 }
 
 int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
@@ -1726,47 +1757,33 @@ int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx
                  "cbar, tbar and xbar must be 16-byte aligned when f % 4 == 0");
     rc = peer_check(win);
     if (rc) return rc;
-    const int ldy = (f + 3) / 4 * 4;
+    const int ldy = wide_ldy(f);
     EGNN_REQUIRE(win->f == ldy && (int64_t)win->world * win->rows_per >= n_global, "window does not fit the signal");
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t rows = row_end - row_begin;
     const size_t slab_elems = (size_t)rows * (size_t)f;
     const int m = k_max - app;
-    const float* tbar_m = tbar_local_or_null ? tbar_local_or_null + (size_t)m * slab_elems : nullptr;
+    const float* tbar_m = slab_of(tbar_local_or_null, slab_elems, m);
     if (app == 0) {                   // b_K = v_K, its operand into buffer 0 of every window
-        CoefRow c{};
-        for (int s = 0; s < n_scales; ++s) c.c[s] = coeffs_host[s * (k_max + 1) + k_max];
         PeerPush pp{};
         fill_peer_push(pp, win, 0, true, true);
-        int64_t blocks = ceil_div64(rows > 0 ? rows * ldy : 1, 1024);        // at most one CTA per SM, as the forward's push
-        const int sms = device_sm_count();
-        if (blocks > sms) blocks = sms;
-        adjoint_prologue_push_kernel<<<(unsigned)blocks, 1024, 0, st>>>(cbar_local, tbar_m, dinv_full, rows, row_begin,
-                                                                       f, n_scales, ldy, c, pp);
+        adjoint_prologue_push_kernel<<<push_grid(rows * ldy), 1024, 0, st>>>(
+            cbar_local, tbar_m, dinv_full, rows, row_begin, f, n_scales, ldy, coef_row(coeffs_host, k_max, n_scales, k_max),
+            pp);
         EGNN_LAUNCH_CHECK("adjoint_prologue_push_kernel launch");
         return EGNN_OK;
     }
-    const RingConfig rcfg = ring_config(ldy);
-    WideParams wp{};
-    rc = fill_delta(wp.delta, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    ChebArgs c{};
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.row_order = row_order_or_null;
+    c.dinv = dinv_full; c.iso = iso_full; c.rows = rows; c.row0 = row_begin; c.f = f; c.k = k_max; c.S = n_scales;
+    c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
+    rc = fill_delta(c.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, n_global);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(wp.delta.row[i] >= 0 && wp.delta.row[i] < n_global && wp.delta.col[i] >= 0 && wp.delta.col[i] < n_global,
-                     "delta index out of range");
-    wp.rowptr = rowptr_local; wp.colidx = colidx_local; wp.vals = nullptr;
-    wp.perm = row_order_or_null; wp.n_hub = row_order_or_null ? row_order_or_null + rows : nullptr;
-    wp.dinv = dinv_full; wp.iso = iso_full; wp.out = nullptr; wp.n_rows = rows; wp.row0 = row_begin;
-    wp.F = f; wp.ldy = ldy; wp.S = n_scales; wp.a = op_scale; wp.b = op_shift; wp.first = 0; wp.normalize = 0;
-    wp.ysrc = peer_operand(win, win->rank, (app - 1) & 1);                  // dinv (.) b_{m+1}, global rows
-    wp.x0_own = nullptr;
-    float* own_next = peer_operand(win, win->rank, app & 1) + row_begin * (int64_t)ldy;
-    wp.y2_own = app == 1 ? nullptr : own_next;                              // dinv (.) b_{m+2} of the own rows
-    wp.y_out = (m > 0 && win->world == 1) ? own_next : nullptr;             // single rank: plain store
+    WideParams wp = wide_params(c);
     wp.tk_out = m == 0 ? xbar_local : nullptr;
     wp.cbar = cbar_local; wp.tbar = tbar_m; wp.c_adj = m == 0 ? 1.f : 2.f;
-    for (int s = 0; s < n_scales; ++s) wp.c_k[s] = coeffs_host[s * (k_max + 1) + m];
-    fill_peer_push(wp.peer, win, app & 1, m > 0, false);
-    return launch_wide<true>(wp, rcfg, device_sm_count(), st);
+    order_coefs(wp.c_k, coeffs_host, k_max, n_scales, m);
+    return wide_sharded_step<true>(wp, ring_config(ldy), win, app, m == 0, st);
 }
 
 int egnn_graph_prep_sharded(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_or_null,
@@ -1786,15 +1803,8 @@ int egnn_graph_prep_sharded(const int32_t* rowptr_local, const int32_t* colidx_l
             rc = check_cuda(cudaMemsetAsync(unsorted_flag_or_null, 0, sizeof(int32_t), st), "memset flag"); if (rc) return rc;
         }
         if (n_rows == 0) return EGNN_OK;
-        const int g = grid_for(n_rows * 32, 256);
-        if (vals_or_null)
-            degree_kernel<true><<<g, 256, 0, st>>>(rowptr_local, colidx_local, vals_or_null, n_rows, rowsum_local,
-                                                   diag_full + row_begin, colsum_full, unsorted_flag_or_null, row_begin);
-        else
-            degree_kernel<false><<<g, 256, 0, st>>>(rowptr_local, colidx_local, nullptr, n_rows, rowsum_local,
-                                                    diag_full + row_begin, colsum_full, unsorted_flag_or_null, row_begin);
-        EGNN_LAUNCH_CHECK("degree_kernel launch");
-        return EGNN_OK;
+        return launch_degree(rowptr_local, colidx_local, vals_or_null, n_rows, rowsum_local, diag_full + row_begin,
+                             colsum_full, unsorted_flag_or_null, row_begin, st);
     }
     EGNN_REQUIRE(phase == 1 && dinv_full && iso_full, "bad phase or null outputs");
     if (n_global > 0) {    // after the all-reduce: normaliser of every node, x0 of the local rows
@@ -1827,10 +1837,8 @@ int egnn_gcn_propagate(const int32_t* rowptr, const int32_t* colidx, const float
     EGNN_REQUIRE(vec_aligned(m, h) && vec_aligned(bias_or_null, h) && vec_aligned(y, h),
                  "m, bias and y must be 16-byte aligned");
     DeltaList d;
-    rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(d.row[i] >= 0 && d.row[i] < n && d.col[i] >= 0 && d.col[i] < n, "delta index out of range");
     const unsigned grid = (unsigned)ceil_div64(n * 32, 256);
     if (vals_or_null)
         gcn_propagate_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(rowptr, colidx, vals_or_null, m, bias_or_null, y,
@@ -1852,10 +1860,8 @@ int egnn_gcn_target_logits(const int32_t* rowptr, const int32_t* colidx, const f
     EGNN_REQUIRE(vec_aligned(z1, h), "z1 must be 16-byte aligned");
     EGNN_REQUIRE(target >= 0 && target < n && n_classes >= 1, "bad target / classes");
     DeltaList d;
-    rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(d.row[i] >= 0 && d.row[i] < n && d.col[i] >= 0 && d.col[i] < n, "delta index out of range");
     if (vals_or_null)
         gcn_target_logits_kernel<true><<<1, 256, 0, (cudaStream_t)stream>>>(rowptr, colidx, vals_or_null, z1, w2, b2, target, h,
                                                                             n_classes, logits_out, ctx, d);
@@ -1878,10 +1884,8 @@ int egnn_gcn_structure_grad(const int32_t* rowptr, const int32_t* colidx, const 
     EGNN_REQUIRE(vec_aligned(z1, h) && vec_aligned(xw, h), "z1 and xw must be 16-byte aligned");
     EGNN_REQUIRE(target >= 0 && target < n && n_classes >= 1, "bad target / classes");
     DeltaList d;
-    rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta);
+    rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
     if (rc) return rc;
-    for (int i = 0; i < n_delta; ++i)
-        EGNN_REQUIRE(d.row[i] >= 0 && d.row[i] < n && d.col[i] >= 0 && d.col[i] < n, "delta index out of range");
     cudaStream_t st = (cudaStream_t)stream;
     rc = check_cuda(cudaMemsetAsync(grad_col, 0, sizeof(float) * n, st), "memset grad_col");
     if (rc) return rc;

@@ -315,7 +315,6 @@ class CsrGraph:
         """(dinv, iso, x0) of this graph with edge flips applied (UGCA
         recompute): flip e adds ``delta_vals[e]`` to ``A[rows[e], cols[e]]``."""
         n, dev = self.n, self.device
-        nd = len(delta_rows)
         lib = _cabi.load()
         with torch.cuda.device(dev):
             dinv = torch.empty_like(self.dinv)
@@ -323,10 +322,7 @@ class CsrGraph:
             x0 = torch.empty_like(self.x0)
             _cabi.check(lib.egnn_patch_degrees(
                 _cabi.ptr(self.w), _cabi.ptr(self.rowsum), _cabi.ptr(self.dinv), _cabi.ptr(self.iso),
-                _cabi.ptr(self.x0), n,
-                _cabi.host_array(C.c_int32, [int(v) for v in delta_rows]),
-                _cabi.host_array(C.c_int32, [int(v) for v in delta_cols]),
-                _cabi.host_array(C.c_float, [float(v) for v in delta_vals]), nd,
+                _cabi.ptr(self.x0), n, *_cabi.delta_args((delta_rows, delta_cols, delta_vals)),
                 _cabi.ptr(dinv), _cabi.ptr(iso), _cabi.ptr(x0), 0, n, _stream()), "egnn_patch_degrees")
         return dinv, iso, x0
 
@@ -337,15 +333,11 @@ class CsrGraph:
         pass that used them).  Returns ``(dinv, iso, x0, y0)``.  One pass at a time per graph."""
         if self._scratch is None:
             self._scratch = (self.dinv.clone(), self.iso.clone(), self.x0.clone(), self.y0().clone())
-        d_rows, d_cols, d_vals = deltas
         lib = _cabi.load()
         with torch.cuda.device(self.device):
             _cabi.check(lib.egnn_patch_nodes(
                 _cabi.ptr(self.w), _cabi.ptr(self.rowsum), _cabi.ptr(self.dinv), _cabi.ptr(self.iso), _cabi.ptr(self.x0),
-                _cabi.ptr(self.y0()), self.n,
-                _cabi.host_array(C.c_int32, [int(v) for v in d_rows]),
-                _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),
-                _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows),
+                _cabi.ptr(self.y0()), self.n, *_cabi.delta_args(deltas),
                 *[_cabi.ptr(t) for t in self._scratch], 1 if restore else 0, _stream()), "egnn_patch_nodes")
         return self._scratch
 

@@ -173,13 +173,6 @@ def _stream():
     return _cabi.current_stream()
 
 
-def _delta_args(deltas):
-    """(rows, cols, vals) -> the four delta arguments of the C ABI (host arrays + count)."""
-    d_rows, d_cols, d_vals = ([], [], []) if deltas is None else deltas
-    return (_cabi.host_array(C.c_int32, [int(v) for v in d_rows]), _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),
-            _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows))
-
-
 class CudaEngine:
     """Device side of the sharded path: thin calls into libegnn_b200."""
 
@@ -215,12 +208,11 @@ class CudaEngine:
 
     def patch_degrees(self, dinv, iso, x0_local, n_global, row_begin, n_rows, deltas):
         """(dinv, iso, x0_local) of the graph with edge flips applied (global ids)."""
-        d_rows, d_cols, d_vals = deltas
         dinv2, iso2 = torch.empty_like(dinv), torch.empty_like(iso)
         x02 = torch.empty(max(1, n_rows), dtype=torch.float32, device=self.device)
         _cabi.check(self.lib.egnn_patch_degrees(
             _cabi.ptr(self.w_full), _cabi.ptr(self.rowsum_local), _cabi.ptr(dinv), _cabi.ptr(iso), _cabi.ptr(x0_local),
-            n_global, *_delta_args(deltas), _cabi.ptr(dinv2), _cabi.ptr(iso2), _cabi.ptr(x02), row_begin, n_rows,
+            n_global, *_cabi.delta_args(deltas), _cabi.ptr(dinv2), _cabi.ptr(iso2), _cabi.ptr(x02), row_begin, n_rows,
             _stream()), "egnn_patch_degrees")
         return dinv2, iso2, x02[:n_rows]
 
@@ -235,7 +227,7 @@ class CudaEngine:
             _cabi.ptr(t_prev_full), _cabi.ptr(t_prev_local), _cabi.ptr(t_prev2_local), _cabi.ptr(t_out_local),
             _cabi.ptr(out_local), _cabi.ptr(acc_ws), n_global, nnz_hint, row_begin, row_end, f, order, k_max,
             n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), 1 if normalize else 0,
-            phase, *_delta_args(deltas), _stream()), "egnn_cheb_order_sharded")
+            phase, *_cabi.delta_args(deltas), _stream()), "egnn_cheb_order_sharded")
 
     # -- narrow path -----------------------------------------------------------
     def sell_plan(self, rowptr, colidx, n_rows, n_cols, row0, unsorted):
@@ -266,7 +258,7 @@ class CudaEngine:
             C.byref(plan), _cabi.ptr(dinv), _cabi.ptr(iso), _cabi.ptr(x0), _cabi.ptr(y_first_full),
             _cabi.ptr(ys[0]), _cabi.ptr(ys[1]), _cabi.ptr(tb[0]), _cabi.ptr(tb[1]), _cabi.ptr(t_all), _cabi.ptr(out),
             order_begin, order_end, k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale),
-            float(op_shift), 1 if normalize else 0, *_delta_args(deltas),
+            float(op_shift), 1 if normalize else 0, *_cabi.delta_args(deltas),
             _cabi.ptr(self.w_full) if base_rowsum is not None else None, _cabi.ptr(base_rowsum),
             1 if default_signal else 0,
             None if window is None else C.byref(window), _stream()), "egnn_sell_step_sharded")
@@ -290,7 +282,7 @@ class CudaEngine:
             _cabi.ptr(rowptr), _cabi.ptr(colidx), None, _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
             _cabi.ptr(x0_local), _cabi.ptr(t_out), _cabi.ptr(out), n_global, row_begin, row_end, f, order, k_max,
             n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), 1 if normalize else 0,
-            *_delta_args(deltas), C.byref(window), _stream()), "egnn_wide_order_sharded")
+            *_cabi.delta_args(deltas), C.byref(window), _stream()), "egnn_wide_order_sharded")
 
     # -- backward ------------------------------------------------------------------
     def adjoint(self, phase, local, remote, dinv, iso, b_prev_full, b_prev_local, b_prev2_local, b_out_local, cbar,
@@ -305,14 +297,14 @@ class CudaEngine:
             _cabi.ptr(b_prev_full), _cabi.ptr(b_prev_local), _cabi.ptr(b_prev2_local), _cabi.ptr(b_out_local),
             _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(acc_ws), n_global, nnz_hint, row_begin, row_end, f, app,
             k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), phase,
-            *_delta_args(deltas_t), _stream()), "egnn_cheb_adjoint_sharded")
+            *_cabi.delta_args(deltas_t), _stream()), "egnn_cheb_adjoint_sharded")
 
     def wide_adjoint(self, rowptr, colidx, row_order, dinv, iso, cbar, tbar, xbar, n_global, row_begin, row_end, f,
                      app, k_max, n_scales, coeffs, op_scale, op_shift, window, deltas_t=None):
         _cabi.check(self.lib.egnn_wide_adjoint_sharded(
             _cabi.ptr(rowptr), _cabi.ptr(colidx), _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
             _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar), n_global, row_begin, row_end, f, app, k_max, n_scales,
-            coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), *_delta_args(deltas_t),
+            coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), *_cabi.delta_args(deltas_t),
             C.byref(window), _stream()), "egnn_wide_adjoint_sharded")
 
     def coeff_grad(self, cbar, t_all):

@@ -22,8 +22,6 @@ features nor the weights change during an attack.
 """
 from __future__ import annotations
 
-import ctypes as C
-
 import torch
 
 from . import _cabi
@@ -36,12 +34,6 @@ CTX_FLOATS = 136
 
 def _stream():
     return _cabi.current_stream()
-
-
-def _delta_args(deltas):
-    d_rows, d_cols, d_vals = ([], [], []) if deltas is None else deltas
-    return (_cabi.host_array(C.c_int32, [int(v) for v in d_rows]), _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),
-            _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows))
 
 
 class StructureGradient:
@@ -116,7 +108,7 @@ class SparseGCNSurrogate:
             deg = torch.empty(g.n, dtype=torch.float32, device=dev)
             _cabi.check(self.lib.egnn_gcn_propagate(
                 _cabi.ptr(g.rowptr), _cabi.ptr(g.colidx), _cabi.ptr(g.vals), _cabi.ptr(self.xw), _cabi.ptr(self.b1),
-                _cabi.ptr(z1), _cabi.ptr(deg), g.n, self.h, *_delta_args(deltas), _stream()), "egnn_gcn_propagate")
+                _cabi.ptr(z1), _cabi.ptr(deg), g.n, self.h, *_cabi.delta_args(deltas), _stream()), "egnn_gcn_propagate")
         self._state = (key, z1, deg)
         return z1, deg
 
@@ -129,7 +121,7 @@ class SparseGCNSurrogate:
             _cabi.check(self.lib.egnn_gcn_target_logits(
                 _cabi.ptr(g.rowptr), _cabi.ptr(g.colidx), _cabi.ptr(g.vals), _cabi.ptr(z1), _cabi.ptr(self.w2),
                 _cabi.ptr(self.b2), int(target), g.n, self.h, self.n_classes, _cabi.ptr(logits), _cabi.ptr(gcn_ctx),
-                *_delta_args(deltas), _stream()), "egnn_gcn_target_logits")
+                *_cabi.delta_args(deltas), _stream()), "egnn_gcn_target_logits")
         return logits, gcn_ctx
 
     def _structure_grad(self, target, upstream, deltas, gcn_ctx):
@@ -142,7 +134,7 @@ class SparseGCNSurrogate:
                 _cabi.ptr(g.rowptr), _cabi.ptr(g.colidx), _cabi.ptr(g.vals), _cabi.ptr(upstream.to(torch.float32)),
                 _cabi.ptr(self.w2), _cabi.ptr(z1), _cabi.ptr(self.xw), _cabi.ptr(self.b1), _cabi.ptr(deg),
                 _cabi.ptr(gcn_ctx), int(target), g.n, self.h, self.n_classes, _cabi.ptr(row), _cabi.ptr(col),
-                *_delta_args(deltas), _stream()), "egnn_gcn_structure_grad")
+                *_cabi.delta_args(deltas), _stream()), "egnn_gcn_structure_grad")
         return StructureGradient(row, col)
 
     # -- what the attack calls ----------------------------------------------------
@@ -176,5 +168,5 @@ class SparseGCNSurrogate:
             h2 = torch.empty_like(h1)
             _cabi.check(self.lib.egnn_gcn_propagate(
                 _cabi.ptr(g.rowptr), _cabi.ptr(g.colidx), _cabi.ptr(g.vals), _cabi.ptr(h1), None, _cabi.ptr(h2), None,
-                g.n, self.h, *_delta_args(deltas), _stream()), "egnn_gcn_propagate")
+                g.n, self.h, *_cabi.delta_args(deltas), _stream()), "egnn_gcn_propagate")
         return h2 @ self.w2.t() + self.b2

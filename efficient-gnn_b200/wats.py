@@ -87,7 +87,6 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
     if coeffs.shape[1] != k + 1:
         raise ValueError("coeffs must be [S, K+1]")
     dinv, iso = (graph.dinv, graph.iso) if degree_vectors is None else degree_vectors
-    d_rows, d_cols, d_vals = ([], [], []) if deltas is None else deltas
     plan = None
     blocked = 0                   # plan-free column-blocked kernel (csrc/blocked.cuh): first use of a large graph
     if use_sell == "blocked":     # tests: force it whatever the size
@@ -112,10 +111,7 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
             _cabi.ptr(graph.rowptr), _cabi.ptr(graph.colidx), _cabi.ptr(graph.vals), _cabi.ptr(dinv),
             _cabi.ptr(iso), _cabi.ptr(x0), n, graph.nnz, f, k, n_scales,
             coeffs32.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift),
-            _cabi.ptr(out), _cabi.ptr(t_all), 1 if normalize else 0,
-            _cabi.host_array(C.c_int32, [int(v) for v in d_rows]),
-            _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),
-            _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows),
+            _cabi.ptr(out), _cabi.ptr(t_all), 1 if normalize else 0, *_cabi.delta_args(deltas),
             _cabi.ptr(ws), ws_bytes, _stream(), order_events,
             None if plan is None else C.byref(plan), _cabi.ptr(row_order),
             _cabi.ptr(y0 if y0 is not None else graph.y0()) if (plan is not None and (default_signal or y0 is not None)) else None,
@@ -135,7 +131,6 @@ def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, 
     lib = _cabi.load()
     n, f, dev = graph_t.n, int(cbar.shape[2]), graph_t.device
     dinv, iso = degree_vectors
-    d_rows, d_cols, d_vals = ([], [], []) if deltas is None else deltas
     row_order = graph_t.row_order() if (f >= WIDE_MIN_F and k >= 1) else None
     with torch.cuda.device(dev):
         xbar = torch.empty((n, f), dtype=torch.float32, device=dev)
@@ -145,10 +140,8 @@ def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, 
         args = (_cabi.ptr(graph_t.rowptr), _cabi.ptr(graph_t.colidx), _cabi.ptr(graph_t.vals), _cabi.ptr(dinv),
                 _cabi.ptr(iso), n, graph_t.nnz, f, k, int(coeffs.shape[0]), coeffs32.ctypes.data_as(C.c_void_p),
                 float(op_scale), float(op_shift), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar),
-                _cabi.host_array(C.c_int32, [int(v) for v in d_cols]),       # transposed flips: rows <-> cols
-                _cabi.host_array(C.c_int32, [int(v) for v in d_rows]),
-                _cabi.host_array(C.c_float, [float(v) for v in d_vals]), len(d_rows),
-                _cabi.ptr(ws), ws_bytes, _stream(), app_events, _cabi.ptr(row_order))
+                *_cabi.delta_args(deltas, transpose=True), _cabi.ptr(ws), ws_bytes, _stream(), app_events,
+                _cabi.ptr(row_order))
         if not keep_all:
             _cabi.check(lib.egnn_cheb_adjoint(*args), "egnn_cheb_adjoint")
             return xbar
