@@ -35,7 +35,7 @@ import torch.distributed as dist
 from torch.autograd.function import once_differentiable
 
 from . import _cabi
-from .wats import WIDE_MIN_F, _needs_grad, heat_coefficients
+from .wats import WIDE_MIN_F, _heat_scale_grad, _needs_grad, heat_coefficients
 
 __all__ = ["RowPartition", "BalancedOrder", "split_columns", "CudaEngine", "DistComm", "PeerExchange", "ShardedWavelet"]
 
@@ -448,16 +448,14 @@ class _ShardedPass(torch.autograd.Function):
         ctx.set_materialize_grads(False)
         s_grad = s is not None and ctx.needs_input_grad[1]
         want = spec.want_orders or s_grad
-        res = sw._pass(spec.k, spec.s, None if x0 is None else x0.detach(), spec.lambda_max, False, want, spec.deltas)
-        f = 1 if (x0 is None or x0.dim() == 1) else int(x0.shape[1])
+        comb, orders = sw._pass(spec.k, spec.s, None if x0 is None else x0.detach(), spec.lambda_max, False, want,
+                                spec.deltas)
+        f = comb.shape[2]
         if want:
-            _, orders, comb = res
             t_all = torch.stack([o.reshape(sw.rows, f) for o in orders])
         else:
-            comb = res
             t_all = comb.new_empty((0,))
             ctx.mark_non_differentiable(t_all)
-        comb = comb.reshape(sw.rows, -1, f)
         ctx.sw, ctx.spec, ctx.f = sw, spec, f
         ctx.x_shape = None if x0 is None else x0.shape
         ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
@@ -640,37 +638,36 @@ class ShardedWavelet:
         gradient, identical bits on every rank.  The backward is collective:
         every rank must call ``backward`` (once per call of ``features``, in
         the same order on every rank), with the same inputs requiring grad."""
+        k = int(k)
+        if deltas is not None and len(deltas[0]) == 0:
+            deltas = None
         x_in = None if X0_local is None else torch.as_tensor(X0_local)
         if _needs_grad(self.x0 if x_in is None else x_in, s):
-            return self._features_grad(int(k), s, x_in, lambda_max, normalize, return_parts, deltas)
-        return self._pass(k, s, X0_local, lambda_max, normalize, return_parts, deltas)
-
-    def _features_grad(self, k, s, x_in, lambda_max, normalize, return_parts, deltas):
-        """The differentiable pass: un-normalised combination (and the orders when wanted) through
-        :class:`_ShardedPass`, then the out-of-place normalisation (as ``graph_wavelet_features``)."""
-        s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
-        if deltas is None or len(deltas[0]) == 0:
-            deltas = None
-        x0 = x_in
-        if x0 is not None:
-            x0 = x0.to(device=self.device, dtype=torch.float32)
-        spec = _ShardedSpec(k, s_vals, float(lambda_max), return_parts, deltas)
-        s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
-        comb, t_all = _ShardedPass.apply(x0, s_in, self, spec)
-        feats = self.engine.l1_normalize(comb) if normalize else comb
+            # un-normalised combination (and the orders) through the autograd function, then the
+            # out-of-place normalisation (as graph_wavelet_features)
+            s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
+            x0 = None if x_in is None else x_in.to(device=self.device, dtype=torch.float32)
+            s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
+            comb, t_all = _ShardedPass.apply(x0, s_in, self, _ShardedSpec(k, s_vals, float(lambda_max), return_parts,
+                                                                          deltas))
+            feats = self.engine.l1_normalize(comb) if normalize else comb
+            orders = [t_all[i] for i in range(k + 1)] if return_parts else None
+        else:
+            comb, orders = self._pass(k, s, X0_local, lambda_max, normalize, return_parts, deltas)
+            feats = comb / (comb.abs().sum(dim=2, keepdim=True) + 1e-8) if (normalize and return_parts) else comb
         feats = feats.reshape(self.rows, -1)
-        if return_parts:
-            return feats, [t_all[i] for i in range(k + 1)], comb
-        return feats
+        return (feats, orders, comb) if return_parts else feats
 
     def _pass(self, k, s, X0_local, lambda_max, normalize, return_parts, deltas):
+        """The rank's rows of one pass: ``(out [rows, S, F], [T_0 .. T_K])``, the orders only when
+        ``return_parts`` (else just ``[T_0]``).  ``out`` is L1-normalised when ``normalize`` and not
+        ``return_parts``, else the un-normalised combination.  ``deltas``: a non-empty flip list or None."""
         eng, dev = self.engine, self.device
-        k = int(k)
         coeffs = np.ascontiguousarray(heat_coefficients(k, s), dtype=np.float32)
         n_scales = coeffs.shape[0]
         dinv, iso, x0_default = self.dinv, self.iso, self.x0
         base_rowsum = None
-        if deltas is not None and len(deltas[0]) > 0:
+        if deltas is not None:
             x_in = None if X0_local is None else torch.as_tensor(X0_local)
             f_in = 1 if (x_in is None or x_in.dim() == 1) else int(x_in.shape[1])
             if k >= 1 and f_in == 1 and self.plan is not None and self.peer is not None and self._rowsum_full is not None:
@@ -681,8 +678,6 @@ class ShardedWavelet:
             else:
                 dinv, iso, x0_default = eng.patch_degrees(self.dinv, self.iso, self.x0, self.n, self.row_begin,
                                                           self.rows, deltas)
-        else:
-            deltas = None
         x0 = x0_default.reshape(-1, 1) if X0_local is None else torch.as_tensor(X0_local)
         if x0.dim() == 1:
             x0 = x0.reshape(-1, 1)
@@ -698,22 +693,15 @@ class ShardedWavelet:
             # rows beyond self.rows (short last shard) are exchanged but never read: no fill needed
             return torch.empty((rp, f), dtype=torch.float32, device=dev)
 
-        def finish(out, orders):
-            out = out[:self.rows]
-            if k == 0 and fused_norm:
-                out = out / (out.abs().sum(dim=2, keepdim=True) + 1e-8)
-            if return_parts:
-                comb = out
-                feats = comb / (comb.abs().sum(dim=2, keepdim=True) + 1e-8) if normalize else comb
-                return feats.reshape(self.rows, -1), orders, comb
-            return out.reshape(self.rows, -1)
-
         # order 1 writes every (row, scale, column) of out, so it is not cleared either
         out = torch.empty((max(1, self.rows), n_scales, f), dtype=torch.float32, device=dev)
         orders = [x0]
         if k == 0:
             out[:self.rows] = torch.from_numpy(coeffs[:, 0]).to(dev).reshape(1, -1, 1) * x0.unsqueeze(1)
-            return finish(out, orders)
+            out = out[:self.rows]
+            if fused_norm:            # no kernel ran to fuse it into
+                out = out / (out.abs().sum(dim=2, keepdim=True) + 1e-8)
+            return out, orders
         use_plan = self.plan is not None and f == 1
         fused = use_plan and self.peer is not None
         fused_wide = self.fused_wide and f >= WIDE_MIN_F
@@ -732,7 +720,7 @@ class ShardedWavelet:
                 self.launches += 1
                 if return_parts:
                     orders.append(t_out)
-            return finish(out, orders)
+            return out[:self.rows], orders
         if use_plan:
             # narrow path: the persistent step kernel over the rank's SELL plan (csrc/sell_step.cuh)
             rows1 = max(1, self.rows)
@@ -772,7 +760,7 @@ class ShardedWavelet:
                 if base_rowsum is not None:       # T_0 of the flipped graph: the kernel wrote the touched rows
                     orders[0] = t_all[0, :self.rows].reshape(-1, 1)
                 orders += [t_all[i, :self.rows].reshape(-1, 1) for i in range(1, k + 1)]
-            return finish(out, orders)
+            return out[:self.rows], orders
         # generic CSR kernel, local / remote column halves around the exchange of T_{k-1}
         if self.rows == rp:
             t_prev = x0
@@ -809,7 +797,7 @@ class ShardedWavelet:
             if return_parts:
                 orders.append(t_out[:self.rows])
             t_prev2, t_prev = t_prev, t_out
-        return finish(out, orders)
+        return out[:self.rows], orders
 
     def gather_features(self, local_feats):
         """All ranks' feature rows, ``[N, S*F]`` on every rank.  A natural
@@ -952,9 +940,7 @@ class ShardedWavelet:
         total = parts[0]
         for r in range(1, self.world):
             total = total + parts[r]
-        alpha = torch.from_numpy(coeffs).to(self.device)
-        kk = torch.arange(k1, dtype=torch.float64, device=self.device)
-        return -(kk * alpha * total).sum(dim=1)
+        return _heat_scale_grad(coeffs, total)
 
 
 # --------------------------------------------------------------------------- #

@@ -26,6 +26,7 @@ from __future__ import annotations
 
 import ctypes as C
 import time
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -64,29 +65,19 @@ class WaveletResult:
         self.combined = combined      # [N, S, F] un-normalised S or None
 
 
-def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_scale: float,
-              op_shift: float, normalize: bool, want_orders: bool, deltas=None,
-              degree_vectors=None, order_events=None, use_sell=None, default_signal=False, y0=None,
-              patch_in_kernel=False):
-    """One call of egnn_cheb_wavelet.  Returns (out [N,S,F], t_all or None).
-    ``default_signal``: x0 is the graph's own log1p(degree) with its own degree
-    vectors, so the first operand dinv * x0 is the one cached on the graph; ``y0``: that
-    operand supplied by the caller (patched copy of the cached one, UGCA recompute).
-    ``patch_in_kernel``: ``deltas`` come with the BASE graph's vectors; on the SELL plan path the
-    step kernel re-derives the touched nodes itself (one launch per perturbed pass) - callers
-    check :func:`_patches_in_kernel` first."""
-    lib = _cabi.load()
-    n, dev = graph.n, graph.device
-    if x0.dim() == 1:
-        x0 = x0.unsqueeze(1)
-    if x0.shape[0] != n:
-        raise ValueError(f"X0 has {x0.shape[0]} rows, graph has {n} nodes")
-    x0 = _cabi.vec_ready(x0.detach().to(device=dev))
-    f = int(x0.shape[1])
-    n_scales = int(coeffs.shape[0])
-    if coeffs.shape[1] != k + 1:
-        raise ValueError("coeffs must be [S, K+1]")
-    dinv, iso = (graph.dinv, graph.iso) if degree_vectors is None else degree_vectors
+# How the forward of one pass runs (:func:`_resolve_route`; the default: the plan-free kernels).  ``plan``: the
+# SELL plan or None; ``blocked``: egnn_cheb_wavelet's ``rows_sorted`` code (0: no blocked kernel, 1: on a large
+# graph, 2: whatever the size); ``in_kernel``: the step kernel applies the flips' degree patches itself (the pass
+# gets the BASE graph's vectors); ``y0``: the step kernel takes the pre-scaled first operand dinv * x0.
+_Route = namedtuple("_Route", "plan blocked in_kernel y0", defaults=(None, 0, False, False))
+
+
+def _resolve_route(graph: CsrGraph, f: int, k: int, use_sell=None, differentiable=False, flips=False,
+                   default_signal=False) -> _Route:
+    """The route of one pass with an ``[N, f]`` signal and ``k`` orders, decided once; counts the pass in
+    ``graph.narrow_calls`` when it may take the plan.  ``use_sell``: None (automatic), True (plan whatever
+    the size), False (neither plan nor blocked kernel), ``"blocked"`` (blocked whatever the size, tests).
+    A differentiable pass with ``flips`` patches the degree vectors on the host: its backward needs them."""
     plan = None
     blocked = 0                   # plan-free column-blocked kernel (csrc/blocked.cuh): first use of a large graph
     if use_sell == "blocked":     # tests: force it whatever the size
@@ -100,6 +91,49 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
             plan = graph.sell_plan(force=bool(use_sell))
         if plan is None and graph.rows_sorted():
             blocked = 1
+    on_plan = plan is not None
+    return _Route(plan, blocked, on_plan and flips and not differentiable, on_plan and default_signal)
+
+
+def _width(x: torch.Tensor) -> int:
+    """F of an ``[N]`` or ``[N, F]`` signal."""
+    return 1 if x.dim() == 1 else int(x.shape[1])
+
+
+class _PassSpec:
+    """Everything of one pass but its differentiable inputs (the signal, the scales, the adjacency and
+    ``lambda_max``).  ``degree_vectors`` / ``y0``: patched for ``deltas`` (None: the graph's own);
+    ``default_signal``: the signal is the graph's log1p(degree) with the graph's vectors.  ``pattern``:
+    ``(rows, cols)`` int32 device tensors when the adjacency input is the value vector of a sparse COO
+    pattern (None: a dense ``[N, N]`` adjacency)."""
+
+    def __init__(self, graph, adjoint, k, coeffs, op_scale, op_shift, want_orders, route=_Route(), deltas=None,
+                 degree_vectors=None, default_signal=False, y0=None, lambda_max=None, pattern=None):
+        self.graph, self.adjoint, self.k, self.coeffs = graph, adjoint, k, coeffs
+        self.op_scale, self.op_shift, self.want_orders, self.route = op_scale, op_shift, want_orders, route
+        self.deltas, self.degree_vectors = deltas, degree_vectors
+        self.default_signal, self.y0 = default_signal, y0
+        self.lambda_max, self.pattern = lambda_max, pattern
+
+    def vectors(self):          # the (dinv, iso) the pass runs with
+        return (self.graph.dinv, self.graph.iso) if self.degree_vectors is None else self.degree_vectors
+
+
+def _run_cheb(spec: _PassSpec, x0: torch.Tensor, normalize: bool, want_orders: bool, order_events=None):
+    """One call of egnn_cheb_wavelet on ``spec.route``.  Returns (out [N,S,F], t_all or None)."""
+    lib = _cabi.load()
+    graph, route, k, coeffs = spec.graph, spec.route, spec.k, spec.coeffs
+    n, dev = graph.n, graph.device
+    if x0.dim() == 1:
+        x0 = x0.unsqueeze(1)
+    if x0.shape[0] != n:
+        raise ValueError(f"X0 has {x0.shape[0]} rows, graph has {n} nodes")
+    x0 = _cabi.vec_ready(x0.detach().to(device=dev))
+    f = int(x0.shape[1])
+    n_scales = int(coeffs.shape[0])
+    if coeffs.shape[1] != k + 1:
+        raise ValueError("coeffs must be [S, K+1]")
+    dinv, iso = spec.vectors()
     row_order = graph.row_order() if (f >= WIDE_MIN_F and k >= 1) else None
     with torch.cuda.device(dev):
         out = torch.empty((n, n_scales, f), dtype=torch.float32, device=dev)
@@ -110,27 +144,27 @@ def _run_cheb(graph: CsrGraph, x0: torch.Tensor, k: int, coeffs: np.ndarray, op_
         _cabi.check(lib.egnn_cheb_wavelet(
             _cabi.ptr(graph.rowptr), _cabi.ptr(graph.colidx), _cabi.ptr(graph.vals), _cabi.ptr(dinv),
             _cabi.ptr(iso), _cabi.ptr(x0), n, graph.nnz, f, k, n_scales,
-            coeffs32.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift),
-            _cabi.ptr(out), _cabi.ptr(t_all), 1 if normalize else 0, *_cabi.delta_args(deltas),
+            coeffs32.ctypes.data_as(C.c_void_p), float(spec.op_scale), float(spec.op_shift),
+            _cabi.ptr(out), _cabi.ptr(t_all), 1 if normalize else 0, *_cabi.delta_args(spec.deltas),
             _cabi.ptr(ws), ws_bytes, _stream(), order_events,
-            None if plan is None else C.byref(plan), _cabi.ptr(row_order),
-            _cabi.ptr(y0 if y0 is not None else graph.y0()) if (plan is not None and (default_signal or y0 is not None)) else None,
-            blocked,
-            _cabi.ptr(graph.w) if patch_in_kernel else None, _cabi.ptr(graph.rowsum) if patch_in_kernel else None,
-            1 if default_signal else 0), "egnn_cheb_wavelet")
+            None if route.plan is None else C.byref(route.plan), _cabi.ptr(row_order),
+            _cabi.ptr(spec.y0 if spec.y0 is not None else graph.y0()) if route.y0 else None,
+            route.blocked,
+            _cabi.ptr(graph.w) if route.in_kernel else None, _cabi.ptr(graph.rowsum) if route.in_kernel else None,
+            1 if spec.default_signal else 0), "egnn_cheb_wavelet")
     return out, t_all
 
 
-def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, op_scale: float, op_shift: float,
-                 cbar: torch.Tensor, tbar=None, deltas=None, app_events=None, keep_all: bool = False):
-    """One call of egnn_cheb_adjoint: the signal's gradient ``[N, F]`` from ``cbar`` ``[N, S, F]`` (and
-    ``tbar`` ``[K+1, N, F]``).  ``graph_t``: the transposed graph (:meth:`CsrGraph.adjoint`),
-    ``degree_vectors``: the forward's ``(dinv, iso)``, ``deltas``: the forward's flips, not yet
-    transposed.  ``keep_all``: egnn_cheb_adjoint_all instead, returns ``(xbar, b_all)`` with every
-    Clenshaw vector ``b_all`` ``[K+1, N, F]`` (slab 0: ``xbar``)."""
+def _run_adjoint(spec: _PassSpec, cbar: torch.Tensor, tbar=None, keep_all: bool = False, app_events=None):
+    """One call of egnn_cheb_adjoint over ``spec.adjoint()`` (the transposed graph,
+    :meth:`CsrGraph.adjoint`) with the forward's degree vectors and flips: the signal's gradient
+    ``[N, F]`` from ``cbar`` ``[N, S, F]`` (and ``tbar`` ``[K+1, N, F]``).  ``keep_all``:
+    egnn_cheb_adjoint_all instead, returns ``(xbar, b_all)`` with every Clenshaw vector ``b_all``
+    ``[K+1, N, F]`` (slab 0: ``xbar``)."""
     lib = _cabi.load()
+    graph_t, k, coeffs = spec.adjoint(), spec.k, spec.coeffs
     n, f, dev = graph_t.n, int(cbar.shape[2]), graph_t.device
-    dinv, iso = degree_vectors
+    dinv, iso = spec.vectors()
     row_order = graph_t.row_order() if (f >= WIDE_MIN_F and k >= 1) else None
     with torch.cuda.device(dev):
         xbar = torch.empty((n, f), dtype=torch.float32, device=dev)
@@ -139,8 +173,8 @@ def _run_adjoint(graph_t: CsrGraph, degree_vectors, k: int, coeffs: np.ndarray, 
         coeffs32 = np.ascontiguousarray(coeffs, dtype=np.float32)
         args = (_cabi.ptr(graph_t.rowptr), _cabi.ptr(graph_t.colidx), _cabi.ptr(graph_t.vals), _cabi.ptr(dinv),
                 _cabi.ptr(iso), n, graph_t.nnz, f, k, int(coeffs.shape[0]), coeffs32.ctypes.data_as(C.c_void_p),
-                float(op_scale), float(op_shift), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar),
-                *_cabi.delta_args(deltas, transpose=True), _cabi.ptr(ws), ws_bytes, _stream(), app_events,
+                float(spec.op_scale), float(spec.op_shift), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar),
+                *_cabi.delta_args(spec.deltas, transpose=True), _cabi.ptr(ws), ws_bytes, _stream(), app_events,
                 _cabi.ptr(row_order))
         if not keep_all:
             _cabi.check(lib.egnn_cheb_adjoint(*args), "egnn_cheb_adjoint")
@@ -164,18 +198,12 @@ def _coeff_grad(cbar: torch.Tensor, t_all: torch.Tensor) -> torch.Tensor:
     return g
 
 
-class _PassSpec:
-    """Everything of one pass but its differentiable inputs (the signal, the scales, the adjacency and
-    ``lambda_max``).  ``pattern``: ``(rows, cols)`` int32 device tensors when the adjacency input is
-    the value vector of a sparse COO pattern (None: a dense ``[N, N]`` adjacency)."""
-
-    def __init__(self, graph, adjoint, k, coeffs, op_scale, op_shift, want_orders, deltas=None, degree_vectors=None,
-                 use_sell=None, default_signal=False, y0=None, lambda_max=None, pattern=None):
-        self.graph, self.adjoint, self.k, self.coeffs = graph, adjoint, k, coeffs
-        self.op_scale, self.op_shift, self.want_orders = op_scale, op_shift, want_orders
-        self.deltas, self.degree_vectors, self.use_sell = deltas, degree_vectors, use_sell
-        self.default_signal, self.y0 = default_signal, y0
-        self.lambda_max, self.pattern = lambda_max, pattern
+def _heat_scale_grad(coeffs: np.ndarray, G: torch.Tensor) -> torch.Tensor:
+    """``ds_j = -sum_k k alpha[j,k] G[j,k]`` (float64) from the heat coefficients ``alpha``
+    (:func:`heat_coefficients`) and ``G[j, k] = <Cbar_j, T_k>``."""
+    alpha = torch.from_numpy(np.ascontiguousarray(coeffs, dtype=np.float64)).to(G.device)
+    kk = torch.arange(alpha.shape[1], dtype=torch.float64, device=G.device)
+    return -(kk * alpha * G).sum(dim=1)
 
 
 class _WaveletPass(torch.autograd.Function):
@@ -192,9 +220,7 @@ class _WaveletPass(torch.autograd.Function):
         ctx.set_materialize_grads(False)        # an output nobody differentiates arrives as None
         s_grad = s is not None and ctx.needs_input_grad[1]
         structure = (adj is not None and ctx.needs_input_grad[2]) or (lam is not None and ctx.needs_input_grad[3])
-        comb, t_all = _run_cheb(spec.graph, x0, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, False,
-                                spec.want_orders or s_grad or structure, spec.deltas, spec.degree_vectors,
-                                use_sell=spec.use_sell, default_signal=spec.default_signal, y0=spec.y0)
+        comb, t_all = _run_cheb(spec, x0, False, spec.want_orders or s_grad or structure)
         if t_all is None:
             t_all = comb.new_empty((0,))
             ctx.mark_non_differentiable(t_all)
@@ -218,19 +244,14 @@ class _WaveletPass(torch.autograd.Function):
         x_grad = s_grad = adj_grad = lam_grad = None
         structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
         if ctx.needs_input_grad[0] or structure:
-            dv = spec.degree_vectors if spec.degree_vectors is not None else (g.dinv, g.iso)
-            xbar = _run_adjoint(spec.adjoint(), dv, spec.k, spec.coeffs, spec.op_scale, spec.op_shift, cbar, tbar,
-                                spec.deltas, keep_all=structure)
+            xbar = _run_adjoint(spec, cbar, tbar, keep_all=structure)
             if structure:
                 xbar, b_all = xbar
             if ctx.needs_input_grad[0]:
                 x_grad = xbar.reshape(ctx.x_shape)
         if ctx.needs_input_grad[1]:
-            G = _coeff_grad(cbar, t_all)
-            alpha = torch.from_numpy(np.ascontiguousarray(spec.coeffs, dtype=np.float64)).to(G.device)
-            kk = torch.arange(spec.k + 1, dtype=torch.float64, device=G.device)
             shape, dev, dtype = ctx.s_meta
-            s_grad = (-(kk * alpha * G).sum(dim=1)).to(device=dev, dtype=dtype).reshape(shape)
+            s_grad = _heat_scale_grad(spec.coeffs, _coeff_grad(cbar, t_all)).to(device=dev, dtype=dtype).reshape(shape)
         if ctx.needs_input_grad[2]:
             adj_grad = _adjacency_grad(spec, b_all, t_all)
         if ctx.needs_input_grad[3]:
@@ -313,18 +334,37 @@ class _L1Normalize(torch.autograd.Function):
         return cbar
 
 
-def _needs_grad(x0, s=None) -> bool:
-    """The autograd path engages only in grad mode with an input that requires grad."""
-    return torch.is_grad_enabled() and (x0.requires_grad or (isinstance(s, torch.Tensor) and s.requires_grad))
+def _needs_grad(x0, s=None, adj=None, lam=None) -> bool:
+    """The autograd path engages only in grad mode with an input that requires grad (``adj`` / ``lam``:
+    the structure inputs of :func:`_structure_input`, None unless they do)."""
+    return adj is not None or lam is not None or \
+        (torch.is_grad_enabled() and (x0.requires_grad or (isinstance(s, torch.Tensor) and s.requires_grad)))
 
 
-def _differentiable_pass(spec: _PassSpec, x0: torch.Tensor, s=None, adj=None, lam=None):
-    """``(C, T)`` through :class:`_WaveletPass`; the device / dtype conversion of ``x0`` (and of ``adj``)
-    stays outside the function, so autograd routes the gradient back to a CPU or float64 leaf."""
-    x0 = x0.to(device=spec.graph.device, dtype=torch.float32)
-    if adj is not None:
-        adj = adj.to(device=spec.graph.device, dtype=torch.float32)
-    return _WaveletPass.apply(x0, s if (isinstance(s, torch.Tensor) and s.requires_grad) else None, adj, lam, spec)
+def _cheb_pass(spec: _PassSpec, x0: torch.Tensor, s=None, adj=None, lam=None, normalize=False,
+               order_events=None) -> WaveletResult:
+    """One pass of any public caller: through :class:`_WaveletPass` when an input needs a gradient
+    (:func:`_needs_grad`), else straight through :func:`_run_cheb`.  ``features`` is ``[N, S*F]``;
+    ``orders`` and ``combined`` are filled when ``spec.want_orders``.  Normalisation: out of place by
+    :class:`_L1Normalize` when differentiable, by a torch expression when the orders are kept, else
+    fused into the last order's kernel."""
+    if _needs_grad(x0, s, adj, lam):
+        # the device / dtype conversions stay outside the function, so autograd routes the gradient
+        # back to a CPU or float64 leaf
+        x0 = x0.to(device=spec.graph.device, dtype=torch.float32)
+        if adj is not None:
+            adj = adj.to(device=spec.graph.device, dtype=torch.float32)
+        s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
+        comb, t_all = _WaveletPass.apply(x0, s_in, adj, lam, spec)
+        feats = _L1Normalize.apply(comb) if normalize else comb
+    elif spec.want_orders:
+        comb, t_all = _run_cheb(spec, x0, False, True)
+        feats = comb / (comb.abs().sum(dim=2, keepdim=True) + 1e-8) if normalize else comb
+    else:
+        out, _ = _run_cheb(spec, x0, normalize, False, order_events)
+        return WaveletResult(out.flatten(1))
+    orders = [t_all[i] for i in range(spec.k + 1)] if spec.want_orders else None
+    return WaveletResult(feats.flatten(1), orders, comb)
 
 
 def _structure_input(adj_matrix, lambda_max, deltas):
@@ -340,16 +380,6 @@ def _structure_input(adj_matrix, lambda_max, deltas):
     lam = lambda_max if isinstance(lambda_max, torch.Tensor) and lambda_max.requires_grad and lambda_max.dim() == 0 \
         else None
     return adj, lam
-
-
-def _patches_in_kernel(graph: CsrGraph, f: int, k: int, use_sell) -> bool:
-    """Will a perturbed pass of this shape run on the SELL plan (whose kernel applies the degree
-    patches of the flips itself)?  Mirrors the plan choice of :func:`_run_cheb`."""
-    if f != 1 or k < 1 or use_sell is False or use_sell == "blocked":
-        return False
-    if use_sell or graph.narrow_calls >= 1 or graph.has_sell_plan():
-        return graph.sell_plan(force=bool(use_sell)) is not None
-    return False
 
 
 class LaplacianOperator:
@@ -400,15 +430,10 @@ class LaplacianOperator:
         """One operator application through the fused kernel (order-1 pass); differentiable
         w.r.t. ``x`` (backward: one application of the transposed operator)."""
         xt = torch.as_tensor(x)
-        vec = xt.dim() == 1
-        coeffs = np.array([[0.0, 1.0]])
-        if _needs_grad(xt):
-            out, _ = _differentiable_pass(_PassSpec(self.graph, self.graph.adjoint, 1, coeffs, self.scale, self.shift,
-                                                    False), xt)
-        else:
-            out, _ = _run_cheb(self.graph, xt, 1, coeffs, self.scale, self.shift, False, False)
-        y = out[:, 0, :]
-        return y[:, 0] if vec else y
+        spec = _PassSpec(self.graph, self.graph.adjoint, 1, np.array([[0.0, 1.0]]), self.scale, self.shift, False,
+                         _resolve_route(self.graph, _width(xt), 1))
+        y = _cheb_pass(spec, xt).features
+        return y[:, 0] if xt.dim() == 1 else y
 
     def rescaled(self, lambda_max: float = 2.0) -> "LaplacianOperator":
         """``(2/lambda_max) * L - I`` (calibration/WATS.py:55)."""
@@ -470,14 +495,9 @@ class ExplicitOperator:
         vec = xt.dim() == 1
         xt = (xt.unsqueeze(1) if vec else xt).to(device=self.diag.device, dtype=torch.float32)
         # kernel: theta * x - a * dinv_i * sum_{j != i} v_ij dinv_j x_j with a = -1, dinv = 1, theta = 0
-        coeffs = np.array([[0.0, 1.0]])
-        if _needs_grad(xt):
-            out, _ = _differentiable_pass(_PassSpec(self.graph, self._transpose, 1, coeffs, -1.0, 0.0, False,
-                                                    degree_vectors=self.unit, use_sell=False), xt)
-        else:
-            out, _ = _run_cheb(self.graph, xt, 1, coeffs, -1.0, 0.0, False, False,
-                               degree_vectors=self.unit, use_sell=False)
-        y = out[:, 0, :] + self.diag.unsqueeze(1) * xt
+        spec = _PassSpec(self.graph, self._transpose, 1, np.array([[0.0, 1.0]]), -1.0, 0.0, False,
+                         _resolve_route(self.graph, _width(xt), 1, use_sell=False), degree_vectors=self.unit)
+        y = _cheb_pass(spec, xt).features + self.diag.unsqueeze(1) * xt
         return y[:, 0] if vec else y
 
 
@@ -506,13 +526,10 @@ def chebyshev_polynomials(L, k, X0):
         for _ in range(2, k + 1):
             t_k.append(2 * (op @ t_k[-1]) - t_k[-2])
         return t_k
-    coeffs = np.zeros((1, k + 1))
     x0 = torch.as_tensor(X0)
-    if _needs_grad(x0):
-        _, t_all = _differentiable_pass(_PassSpec(L.graph, L.graph.adjoint, k, coeffs, L.scale, L.shift, True), x0)
-    else:
-        _, t_all = _run_cheb(L.graph, x0, k, coeffs, L.scale, L.shift, False, True)
-    return [t_all[i] for i in range(k + 1)]
+    spec = _PassSpec(L.graph, L.graph.adjoint, k, np.zeros((1, k + 1)), L.scale, L.shift, True,
+                     _resolve_route(L.graph, _width(x0), k))
+    return _cheb_pass(spec, x0).orders
 
 
 def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float = 2.0,
@@ -571,55 +588,32 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
     k = int(k)
     s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
     coeffs = heat_coefficients(k, s_vals)
-    degree_vectors = None
     x0 = graph.x0 if X0 is None else torch.as_tensor(X0)
-    grad = _needs_grad(x0, s) or adj_in is not None or lam_in is not None
-    y0 = None
-    in_kernel = False
-    if deltas is not None and len(deltas[0]) > 0:
-        # the backward needs the patched degree vectors, so a differentiable pass patches them itself
-        in_kernel = not grad and _patches_in_kernel(graph, 1 if x0.dim() == 1 else int(x0.shape[1]), k, _use_sell)
-        if not in_kernel:
-            # degree vectors of the flipped graph: only the touched entries of persistent scratch copies are
-            # written, and put back once the pass is queued (no copies of the N-vectors per perturbation)
-            dinv, iso, x0_patched, y0_patched = graph.patch_nodes(deltas)
-            degree_vectors = (dinv, iso)
-            if X0 is None:
-                x0, y0 = x0_patched, y0_patched
-        # else (SELL plan): the step kernel re-derives the touched nodes from the base vectors - one launch
-    else:
+    if deltas is not None and len(deltas[0]) == 0:
         deltas = None
-    op_scale = 2.0 / float(lambda_max)
-    default_signal = X0 is None and (deltas is None or in_kernel)
+    grad = _needs_grad(x0, s, adj_in, lam_in)
+    route = _resolve_route(graph, _width(x0), k, _use_sell, grad, deltas is not None, X0 is None)
+    # on the SELL plan the step kernel re-derives the nodes the flips touch from the base vectors (one launch);
+    # every other route gets the degree vectors of the flipped graph: only the touched entries of persistent
+    # scratch copies are written, and put back once the pass is queued (no copies of the N-vectors per perturbation)
+    patched = deltas is not None and not route.in_kernel
+    degree_vectors = y0 = None
+    if patched:
+        dinv, iso, x0_patched, y0_patched = graph.patch_nodes(deltas)
+        degree_vectors = (dinv, iso)
+        if X0 is None:
+            x0, y0 = x0_patched, y0_patched
+    lam_max = float(lambda_max)
     try:
-        if grad:
-            if degree_vectors is not None:       # the scratch vectors are restored below, the backward runs later
-                degree_vectors = tuple(v.clone() for v in degree_vectors)
-            spec = _PassSpec(graph, graph.adjoint, k, coeffs, op_scale, -1.0, return_parts, deltas, degree_vectors,
-                             _use_sell, default_signal, y0, float(lambda_max), pattern)
-            comb, t_all = _differentiable_pass(spec, x0, s, adj_in, lam_in)
-            feats = _L1Normalize.apply(comb) if normalize else comb
-            feats = feats.reshape(graph.n, -1)
-            return WaveletResult(feats, [t_all[i] for i in range(k + 1)], comb) if return_parts else feats
-        return _wavelet_pass(graph, x0, k, coeffs, op_scale, normalize, return_parts, deltas, degree_vectors,
-                             _order_events, _use_sell, default_signal, y0, in_kernel)
+        if grad and patched:       # the scratch vectors are restored below, the backward runs later
+            degree_vectors = tuple(v.clone() for v in degree_vectors)
+        spec = _PassSpec(graph, graph.adjoint, k, coeffs, 2.0 / lam_max, -1.0, return_parts, route, deltas,
+                         degree_vectors, X0 is None and not patched, y0, lam_max, pattern)
+        res = _cheb_pass(spec, x0, s, adj_in, lam_in, normalize, _order_events)
+        return res if return_parts else res.features
     finally:
-        if deltas is not None and not in_kernel:
+        if patched:
             graph.patch_nodes(deltas, restore=True)
-
-
-def _wavelet_pass(graph, x0, k, coeffs, op_scale, normalize, return_parts, deltas, degree_vectors, _order_events,
-                  _use_sell, default_signal, y0, patch_in_kernel=False):
-    if return_parts:
-        comb, t_all = _run_cheb(graph, x0, k, coeffs, op_scale, -1.0, False, True, deltas, degree_vectors,
-                                use_sell=_use_sell, default_signal=default_signal, y0=y0,
-                                patch_in_kernel=patch_in_kernel)
-        feats = comb / (comb.abs().sum(dim=2, keepdim=True) + 1e-8) if normalize else comb
-        feats = feats.reshape(graph.n, -1)
-        return WaveletResult(feats, [t_all[i] for i in range(k + 1)], comb)
-    out, _ = _run_cheb(graph, x0, k, coeffs, op_scale, -1.0, normalize, False, deltas, degree_vectors,
-                       _order_events, _use_sell, default_signal, y0, patch_in_kernel)
-    return out.reshape(graph.n, -1)
 
 
 def accuracy(outputs, labels):

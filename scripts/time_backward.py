@@ -21,7 +21,7 @@ sys.path.insert(0, ROOT)
 
 import efficient_gnn_b200 as egnn  # noqa: E402
 from efficient_gnn_b200 import synth  # noqa: E402
-from efficient_gnn_b200.wats import _run_adjoint  # noqa: E402
+from efficient_gnn_b200.wats import _PassSpec, _run_adjoint  # noqa: E402
 
 K = 3
 WORKLOADS = [("reddit", 1, [0.8]), ("reddit", 64, [0.8]), ("arxiv", 128, [0.8]),
@@ -104,18 +104,16 @@ def main():
                 egnn.graph_wavelet_features(g, k=K, s=scales, X0=x, _order_events=ev)
         # with the SELL plan events 0 and 1 bracket the whole step
         t_order = per_launch(fwd_orders, K, args.repeats, used=1) / K if sell else per_launch(fwd_orders, K, args.repeats)
-        gt = g.adjoint()
-        coeffs = egnn.heat_coefficients(K, scales)
+        spec = _PassSpec(g, g.adjoint, K, egnn.heat_coefficients(K, scales), 2.0, -1.0, False)
         cbar = torch.randn(n, len(scales), f, device="cuda", generator=gen)
-        t_app = per_launch(lambda ev: _run_adjoint(gt, (g.dinv, g.iso), K, coeffs, 2.0, -1.0, cbar, app_events=ev),
-                           K, args.repeats)
+        t_app = per_launch(lambda ev: _run_adjoint(spec, cbar, app_events=ev), K, args.repeats)
         row = dict(shape=shape, n=n, nnz=g.nnz, f=f, S=len(scales), k=K, forward_ms=t_fwd, forward_backward_ms=t_fb,
                    backward_over_forward=(t_fb - t_fwd) / t_fwd, forward_order_ms=t_order,
                    forward_order_kernel="sell_step (per order)" if sell else ("wide" if f >= 8 else "generic"),
                    adjoint_application_ms=t_app, application_over_order=t_app / t_order)
         rows.append(row)
         print(json.dumps(row))
-        del g, gt, x, xg, up, cbar
+        del g, spec, x, xg, up, cbar
         torch.cuda.empty_cache()
     if args.out:
         os.makedirs(args.out, exist_ok=True)

@@ -22,8 +22,8 @@ sys.path.insert(0, ROOT)
 
 import efficient_gnn_b200 as egnn  # noqa: E402
 from efficient_gnn_b200 import synth  # noqa: E402
-from efficient_gnn_b200.wats import (_PassSpec, _adjacency_grad, _lambda_max_grad, _run_adjoint,  # noqa: E402
-                                     _run_cheb)
+from efficient_gnn_b200.wats import (_PassSpec, _adjacency_grad, _lambda_max_grad, _resolve_route,  # noqa: E402
+                                     _run_adjoint, _run_cheb)
 
 K = 3
 # shape, F (None: default signal), adjacency layout
@@ -113,21 +113,22 @@ def main():
         state = {}
 
         def forward_kernels():
-            state["t"] = _run_cheb(g, x0, K, coeffs, op_scale, -1.0, False, True)[1]
+            route = _resolve_route(g, fw, K)       # per call, as every pass: the plan comes on the second
+            state["t"] = _run_cheb(_PassSpec(g, g.adjoint, K, coeffs, op_scale, -1.0, True, route), x0, False, True)[1]
 
         cbar = up.reshape(n, 1, fw).contiguous()
-
-        def adjoint_all():
-            state["b"] = _run_adjoint(g.adjoint(), (g.dinv, g.iso), K, coeffs, op_scale, -1.0, cbar, keep_all=True)[1]
-
-        row["forward_kernels_ms"] = timed(forward_kernels, args.repeats)
-        row["adjoint_all_ms"] = timed(adjoint_all, args.repeats)
         pattern = None
         if layout == "coo":
             c = a.coalesce().indices().to(torch.int32)
             pattern = (c[0].contiguous(), c[1].contiguous())
         spec = _PassSpec(g, g.adjoint, K, coeffs, op_scale, -1.0, True, default_signal=f is None, lambda_max=2.0,
                          pattern=pattern)
+
+        def adjoint_all():
+            state["b"] = _run_adjoint(spec, cbar, keep_all=True)[1]
+
+        row["forward_kernels_ms"] = timed(forward_kernels, args.repeats)
+        row["adjoint_all_ms"] = timed(adjoint_all, args.repeats)
         lib = egnn._cabi.load()
         gw = torch.empty(n, device="cuda")
         grho = torch.empty(n, device="cuda")
