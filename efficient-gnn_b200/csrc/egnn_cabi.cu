@@ -13,6 +13,7 @@
 #include "prep.cuh"
 #include "sell.cuh"
 #include "sell_step.cuh"
+#include "shard_grad.cuh"
 #include "structure_grad.cuh"
 #include "surrogate.cuh"
 #include "blocked.cuh"
@@ -501,7 +502,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 10; }
+int egnn_abi_version(void) { return 11; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -1034,11 +1035,13 @@ static int cheb_adjoint_impl(const int32_t* rowptr_t, const int32_t* colidx_t, c
 // into p.acc_ws, phase 1 adds the remote columns from the gathered operand and runs the epilogue,
 // phase 2 is one launch over the unsplit rows.  The edge flips ride with the launch that gathers
 // from the exchanged operand, so phase 0 does not look at them.  p comes filled for the local CSR.
+// Weighted shards: p.vals holds the local half's (or the unsplit rows') values, vals_remote the remote half's.
 template <bool ADJ>
 static int order_sharded_phase(OrderParams& p, const OrderConfig& cfg, int32_t phase, const int32_t* rowptr_remote,
-                               const int32_t* colidx_remote, const float* gathered, const char* gathered_missing,
-                               const int32_t* delta_row_host, const int32_t* delta_col_host,
-                               const float* delta_val_host, int32_t n_delta, int64_t n, cudaStream_t st) {
+                               const int32_t* colidx_remote, const float* vals_remote, const float* gathered,
+                               const char* gathered_missing, const int32_t* delta_row_host,
+                               const int32_t* delta_col_host, const float* delta_val_host, int32_t n_delta, int64_t n,
+                               cudaStream_t st) {
     if (phase == 0) {                 // local columns: gathers hit the rank's own slab
         EGNN_REQUIRE(p.rowptr && p.acc_ws, "local half missing");
         p.gsrc = p.tprev_own - p.row0 * (int64_t)p.F;      // indexed by global column, only own rows touched
@@ -1052,7 +1055,7 @@ static int order_sharded_phase(OrderParams& p, const OrderConfig& cfg, int32_t p
     p.gsrc = gathered;
     if (phase == 1) {                 // remote columns + epilogue
         EGNN_REQUIRE(rowptr_remote && p.acc_ws, "remote half missing");
-        p.rowptr = rowptr_remote; p.colidx = colidx_remote; p.mode = 2;
+        p.rowptr = rowptr_remote; p.colidx = colidx_remote; p.vals = vals_remote; p.mode = 2;
     } else {                          // one launch over the unsplit rows
         EGNN_REQUIRE(p.rowptr != nullptr, "csr missing");
     }
@@ -1274,27 +1277,31 @@ int egnn_adj_grad_dense(const float* dinv, const float* lam, const float* t, con
     return EGNN_OK;
 }
 
-int egnn_cheb_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
-                            const int32_t* rowptr_remote, const int32_t* colidx_remote,
-                            const float* dinv_full, const uint8_t* iso_full, const float* t_prev_full,
-                            const float* t_prev_local, const float* t_prev2_local, float* t_out_local,
-                            float* out_local, float* acc_ws, int64_t n, int64_t nnz_hint,
-                            int64_t row_begin, int64_t row_end, int32_t f, int32_t order, int32_t k_max,
-                            int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
-                            int32_t normalize_l1, int32_t phase,
-                            const int32_t* delta_row_host, const int32_t* delta_col_host,
-                            const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+}  // extern "C"
+
+// One order of a row shard, binary (vals_local == vals_remote == NULL) or weighted (both given).
+static int cheb_order_sharded_impl(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_local,
+                                   const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                                   const float* vals_remote, const float* dinv_full, const uint8_t* iso_full,
+                                   const float* t_prev_full, const float* t_prev_local, const float* t_prev2_local,
+                                   float* t_out_local, float* out_local, float* acc_ws, int64_t n, int64_t nnz_hint,
+                                   int64_t row_begin, int64_t row_end, int32_t f, int32_t order, int32_t k_max,
+                                   int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                                   int32_t normalize_l1, int32_t phase, const int32_t* delta_row_host,
+                                   const int32_t* delta_col_host, const float* delta_val_host, int32_t n_delta,
+                                   egnn_stream_t stream) {
     EGNN_REQUIRE(dinv_full && iso_full && out_local && coeffs_host && t_prev_local, "null pointer");
     EGNN_REQUIRE(row_begin >= 0 && row_end >= row_begin && row_end <= n, "bad row range");
     EGNN_REQUIRE(order >= 1 && order <= k_max && k_max <= EGNN_MAX_ORDER, "bad order");
     EGNN_REQUIRE(n_scales >= 1 && n_scales <= EGNN_MAX_SCALES, "n_scales out of range");
     EGNN_REQUIRE(phase >= 0 && phase <= 2, "bad phase");
     EGNN_REQUIRE(order == 1 || t_prev2_local, "T_{k-2} missing");
+    EGNN_REQUIRE((vals_local == nullptr) == (vals_remote == nullptr), "values of the local and remote halves come together");
     const int64_t rows = row_end - row_begin;
     if (rows == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
     ChebArgs c{};
-    c.rowptr = rowptr_local; c.colidx = colidx_local; c.dinv = dinv_full; c.iso = iso_full;
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.vals = vals_local; c.dinv = dinv_full; c.iso = iso_full;
     c.rows = rows; c.row0 = row_begin; c.nnz = nnz_hint; c.f = f; c.k = k_max; c.S = n_scales;
     c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
     OrderConfig cfg = choose_config(rows, nnz_hint, f);
@@ -1307,12 +1314,48 @@ int egnn_cheb_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_l
     const bool last = order == k_max;
     const bool fuse_norm = normalize_l1 && cfg.grid_y == 1;
     p.normalize = last && fuse_norm;
-    int rc = order_sharded_phase<false>(p, cfg, phase, rowptr_remote, colidx_remote, t_prev_full,
+    int rc = order_sharded_phase<false>(p, cfg, phase, rowptr_remote, colidx_remote, vals_remote, t_prev_full,
                                         "gathered T_{k-1} missing", delta_row_host, delta_col_host, delta_val_host,
                                         n_delta, n, st);
     if (rc) return rc;
     if (phase != 0 && last && normalize_l1 && !fuse_norm) return launch_l1_normalize(out_local, rows, n_scales, f, st);
     return EGNN_OK;
+}
+
+extern "C" {
+
+int egnn_cheb_order_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                            const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                            const float* dinv_full, const uint8_t* iso_full, const float* t_prev_full,
+                            const float* t_prev_local, const float* t_prev2_local, float* t_out_local,
+                            float* out_local, float* acc_ws, int64_t n, int64_t nnz_hint,
+                            int64_t row_begin, int64_t row_end, int32_t f, int32_t order, int32_t k_max,
+                            int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                            int32_t normalize_l1, int32_t phase,
+                            const int32_t* delta_row_host, const int32_t* delta_col_host,
+                            const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+    return cheb_order_sharded_impl(rowptr_local, colidx_local, nullptr, rowptr_remote, colidx_remote, nullptr,
+                                   dinv_full, iso_full, t_prev_full, t_prev_local, t_prev2_local, t_out_local,
+                                   out_local, acc_ws, n, nnz_hint, row_begin, row_end, f, order, k_max, n_scales,
+                                   coeffs_host, op_scale, op_shift, normalize_l1, phase, delta_row_host,
+                                   delta_col_host, delta_val_host, n_delta, stream);
+}
+
+int egnn_cheb_order_sharded_vals(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_local,
+                                 const int32_t* rowptr_remote, const int32_t* colidx_remote, const float* vals_remote,
+                                 const float* dinv_full, const uint8_t* iso_full, const float* t_prev_full,
+                                 const float* t_prev_local, const float* t_prev2_local, float* t_out_local,
+                                 float* out_local, float* acc_ws, int64_t n, int64_t nnz_hint,
+                                 int64_t row_begin, int64_t row_end, int32_t f, int32_t order, int32_t k_max,
+                                 int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                                 int32_t normalize_l1, int32_t phase,
+                                 const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                 const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+    return cheb_order_sharded_impl(rowptr_local, colidx_local, vals_local, rowptr_remote, colidx_remote, vals_remote,
+                                   dinv_full, iso_full, t_prev_full, t_prev_local, t_prev2_local, t_out_local,
+                                   out_local, acc_ws, n, nnz_hint, row_begin, row_end, f, order, k_max, n_scales,
+                                   coeffs_host, op_scale, op_shift, normalize_l1, phase, delta_row_host,
+                                   delta_col_host, delta_val_host, n_delta, stream);
 }
 
 int egnn_sell_geometry(int64_t n, int64_t nnz, int32_t* n_blocks, int32_t* col_block, int32_t* lmax) {
@@ -1694,21 +1737,23 @@ static int adjoint_sharded_check(int64_t n, int64_t row_begin, int64_t row_end, 
     return EGNN_OK;
 }
 
-int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
-                              const int32_t* rowptr_remote, const int32_t* colidx_remote,
-                              const float* dinv_full, const uint8_t* iso_full, const float* b_prev_full,
-                              const float* b_prev_local, const float* b_prev2_local_or_null, float* b_out_local,
-                              const float* cbar_local, const float* tbar_local_or_null, float* acc_ws,
-                              int64_t n, int64_t nnz_hint, int64_t row_begin, int64_t row_end, int32_t f,
-                              int32_t app, int32_t k_max, int32_t n_scales, const float* coeffs_host,
-                              float op_scale, float op_shift, int32_t phase,
-                              const int32_t* delta_row_host, const int32_t* delta_col_host,
-                              const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+// Binary (vals_local == vals_remote == NULL) or weighted (both given) shard of the transposed adjacency.
+static int cheb_adjoint_sharded_impl(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_local,
+                                     const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                                     const float* vals_remote, const float* dinv_full, const uint8_t* iso_full,
+                                     const float* b_prev_full, const float* b_prev_local,
+                                     const float* b_prev2_local_or_null, float* b_out_local, const float* cbar_local,
+                                     const float* tbar_local_or_null, float* acc_ws, int64_t n, int64_t nnz_hint,
+                                     int64_t row_begin, int64_t row_end, int32_t f, int32_t app, int32_t k_max,
+                                     int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                                     int32_t phase, const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                     const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
     EGNN_REQUIRE(dinv_full && iso_full && b_out_local && cbar_local && coeffs_host, "null pointer");
     int rc = adjoint_sharded_check(n, row_begin, row_end, f, app, k_max, n_scales);
     if (rc) return rc;
     EGNN_REQUIRE(phase >= 0 && phase <= 2, "bad phase");
     EGNN_REQUIRE(app == 0 || b_prev_local, "b_{m+1} rows missing");
+    EGNN_REQUIRE((vals_local == nullptr) == (vals_remote == nullptr), "values of the local and remote halves come together");
     EGNN_REQUIRE(vec_aligned(b_prev_full, f) && vec_aligned(b_prev_local, f) && vec_aligned(b_prev2_local_or_null, f) &&
                  vec_aligned(b_out_local, f) && vec_aligned(cbar_local, f) && vec_aligned(tbar_local_or_null, f) &&
                  vec_aligned(acc_ws, f), "b, cbar, tbar and acc_ws must be 16-byte aligned when f % 4 == 0");
@@ -1726,7 +1771,7 @@ int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx
         return EGNN_OK;
     }
     ChebArgs c{};
-    c.rowptr = rowptr_local; c.colidx = colidx_local; c.dinv = dinv_full; c.iso = iso_full;
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.vals = vals_local; c.dinv = dinv_full; c.iso = iso_full;
     c.rows = rows; c.row0 = row_begin; c.nnz = nnz_hint; c.f = f; c.k = k_max; c.S = n_scales;
     c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
     OrderConfig cfg = choose_config(rows, nnz_hint, f);
@@ -1735,26 +1780,65 @@ int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx
     p.tprev_own = b_prev_local; p.tprev2_own = b_prev2_local_or_null; p.tk_own = b_out_local; p.acc_ws = acc_ws;
     p.cbar = cbar_local; p.tbar = tbar_m; p.c_adj = m == 0 ? 1.f : 2.f;
     order_coefs(p.c_k, coeffs_host, k_max, n_scales, m);
-    return order_sharded_phase<true>(p, cfg, phase, rowptr_remote, colidx_remote, b_prev_full, "gathered b_{m+1} missing",
-                                     delta_row_host, delta_col_host, delta_val_host, n_delta, n, st);
+    return order_sharded_phase<true>(p, cfg, phase, rowptr_remote, colidx_remote, vals_remote, b_prev_full,
+                                     "gathered b_{m+1} missing", delta_row_host, delta_col_host, delta_val_host,
+                                     n_delta, n, st);
 }
 
-int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
-                              const int32_t* row_order_or_null, const float* dinv_full, const uint8_t* iso_full,
-                              const float* cbar_local, const float* tbar_local_or_null, float* xbar_local,
-                              int64_t n_global, int64_t row_begin, int64_t row_end, int32_t f, int32_t app,
-                              int32_t k_max, int32_t n_scales, const float* coeffs_host, float op_scale,
-                              float op_shift, const int32_t* delta_row_host, const int32_t* delta_col_host,
-                              const float* delta_val_host, int32_t n_delta, const egnn_peer_window* win,
-                              egnn_stream_t stream) {
+int egnn_cheb_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                              const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                              const float* dinv_full, const uint8_t* iso_full, const float* b_prev_full,
+                              const float* b_prev_local, const float* b_prev2_local_or_null, float* b_out_local,
+                              const float* cbar_local, const float* tbar_local_or_null, float* acc_ws,
+                              int64_t n, int64_t nnz_hint, int64_t row_begin, int64_t row_end, int32_t f,
+                              int32_t app, int32_t k_max, int32_t n_scales, const float* coeffs_host,
+                              float op_scale, float op_shift, int32_t phase,
+                              const int32_t* delta_row_host, const int32_t* delta_col_host,
+                              const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+    return cheb_adjoint_sharded_impl(rowptr_local, colidx_local, nullptr, rowptr_remote, colidx_remote, nullptr,
+                                     dinv_full, iso_full, b_prev_full, b_prev_local, b_prev2_local_or_null,
+                                     b_out_local, cbar_local, tbar_local_or_null, acc_ws, n, nnz_hint, row_begin,
+                                     row_end, f, app, k_max, n_scales, coeffs_host, op_scale, op_shift, phase,
+                                     delta_row_host, delta_col_host, delta_val_host, n_delta, stream);
+}
+
+int egnn_cheb_adjoint_sharded_vals(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_local,
+                                   const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                                   const float* vals_remote, const float* dinv_full, const uint8_t* iso_full,
+                                   const float* b_prev_full, const float* b_prev_local,
+                                   const float* b_prev2_local_or_null, float* b_out_local, const float* cbar_local,
+                                   const float* tbar_local_or_null, float* acc_ws, int64_t n, int64_t nnz_hint,
+                                   int64_t row_begin, int64_t row_end, int32_t f, int32_t app, int32_t k_max,
+                                   int32_t n_scales, const float* coeffs_host, float op_scale, float op_shift,
+                                   int32_t phase, const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                   const float* delta_val_host, int32_t n_delta, egnn_stream_t stream) {
+    return cheb_adjoint_sharded_impl(rowptr_local, colidx_local, vals_local, rowptr_remote, colidx_remote,
+                                     vals_remote, dinv_full, iso_full, b_prev_full, b_prev_local,
+                                     b_prev2_local_or_null, b_out_local, cbar_local, tbar_local_or_null, acc_ws, n,
+                                     nnz_hint, row_begin, row_end, f, app, k_max, n_scales, coeffs_host, op_scale,
+                                     op_shift, phase, delta_row_host, delta_col_host, delta_val_host, n_delta, stream);
+}
+
+// Fused wide adjoint of a binary or weighted shard; b_out_local_or_null [rows, f] receives b_m of every
+// application m >= 1 (app 0: b_K), as egnn_cheb_adjoint_all keeps them on one GPU.
+static int wide_adjoint_sharded_impl(const int32_t* rowptr_local, const int32_t* colidx_local,
+                                     const float* vals_or_null, const int32_t* row_order_or_null,
+                                     const float* dinv_full, const uint8_t* iso_full, const float* cbar_local,
+                                     const float* tbar_local_or_null, float* xbar_local, float* b_out_local_or_null,
+                                     int64_t n_global, int64_t row_begin, int64_t row_end, int32_t f, int32_t app,
+                                     int32_t k_max, int32_t n_scales, const float* coeffs_host, float op_scale,
+                                     float op_shift, const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                     const float* delta_val_host, int32_t n_delta, const egnn_peer_window* win,
+                                     egnn_stream_t stream) {
     EGNN_REQUIRE(rowptr_local && dinv_full && iso_full && cbar_local && coeffs_host && win, "null pointer");
     int rc = adjoint_sharded_check(n_global, row_begin, row_end, f, app, k_max, n_scales);
     if (rc) return rc;
     EGNN_REQUIRE(f >= kWideMinF, "the wide sharded adjoint serves f >= 8");
     EGNN_REQUIRE(k_max >= 1, "k_max = 0 has no application to exchange");
     EGNN_REQUIRE(app < k_max || xbar_local || row_end == row_begin, "xbar rows missing");
-    EGNN_REQUIRE(vec_aligned(cbar_local, f) && vec_aligned(tbar_local_or_null, f) && vec_aligned(xbar_local, f),
-                 "cbar, tbar and xbar must be 16-byte aligned when f % 4 == 0");
+    EGNN_REQUIRE(vec_aligned(cbar_local, f) && vec_aligned(tbar_local_or_null, f) && vec_aligned(xbar_local, f) &&
+                 vec_aligned(b_out_local_or_null, f),
+                 "cbar, tbar, xbar and b_out must be 16-byte aligned when f % 4 == 0");
     rc = peer_check(win);
     if (rc) return rc;
     const int ldy = wide_ldy(f);
@@ -1771,19 +1855,158 @@ int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx
             cbar_local, tbar_m, dinv_full, rows, row_begin, f, n_scales, ldy, coef_row(coeffs_host, k_max, n_scales, k_max),
             pp);
         EGNN_LAUNCH_CHECK("adjoint_prologue_push_kernel launch");
+        if (b_out_local_or_null && rows > 0) {        // and b_K itself into the caller's rows
+            adjoint_prologue_kernel<<<grid_for((int64_t)slab_elems, 256), 256, 0, st>>>(
+                cbar_local, tbar_m, dinv_full + row_begin, b_out_local_or_null, nullptr, rows, f, n_scales, f,
+                coef_row(coeffs_host, k_max, n_scales, k_max));
+            EGNN_LAUNCH_CHECK("adjoint_prologue_kernel launch");
+        }
         return EGNN_OK;
     }
     ChebArgs c{};
-    c.rowptr = rowptr_local; c.colidx = colidx_local; c.row_order = row_order_or_null;
+    c.rowptr = rowptr_local; c.colidx = colidx_local; c.vals = vals_or_null; c.row_order = row_order_or_null;
     c.dinv = dinv_full; c.iso = iso_full; c.rows = rows; c.row0 = row_begin; c.f = f; c.k = k_max; c.S = n_scales;
     c.coeffs = coeffs_host; c.a = op_scale; c.b = op_shift; c.st = st;
     rc = fill_delta(c.delta, delta_row_host, delta_col_host, delta_val_host, n_delta, n_global);
     if (rc) return rc;
     WideParams wp = wide_params(c);
-    wp.tk_out = m == 0 ? xbar_local : nullptr;
+    wp.tk_out = m == 0 ? xbar_local : b_out_local_or_null;
     wp.cbar = cbar_local; wp.tbar = tbar_m; wp.c_adj = m == 0 ? 1.f : 2.f;
     order_coefs(wp.c_k, coeffs_host, k_max, n_scales, m);
     return wide_sharded_step<true>(wp, ring_config(ldy), win, app, m == 0, st);
+}
+
+int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx_local,
+                              const int32_t* row_order_or_null, const float* dinv_full, const uint8_t* iso_full,
+                              const float* cbar_local, const float* tbar_local_or_null, float* xbar_local,
+                              int64_t n_global, int64_t row_begin, int64_t row_end, int32_t f, int32_t app,
+                              int32_t k_max, int32_t n_scales, const float* coeffs_host, float op_scale,
+                              float op_shift, const int32_t* delta_row_host, const int32_t* delta_col_host,
+                              const float* delta_val_host, int32_t n_delta, const egnn_peer_window* win,
+                              egnn_stream_t stream) {
+    return wide_adjoint_sharded_impl(rowptr_local, colidx_local, nullptr, row_order_or_null, dinv_full, iso_full,
+                                     cbar_local, tbar_local_or_null, xbar_local, nullptr, n_global, row_begin, row_end,
+                                     f, app, k_max, n_scales, coeffs_host, op_scale, op_shift, delta_row_host,
+                                     delta_col_host, delta_val_host, n_delta, win, stream);
+}
+
+int egnn_wide_adjoint_sharded_all(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_or_null,
+                                  const int32_t* row_order_or_null, const float* dinv_full, const uint8_t* iso_full,
+                                  const float* cbar_local, const float* tbar_local_or_null, float* xbar_local,
+                                  float* b_out_local_or_null, int64_t n_global, int64_t row_begin, int64_t row_end,
+                                  int32_t f, int32_t app, int32_t k_max, int32_t n_scales, const float* coeffs_host,
+                                  float op_scale, float op_shift, const int32_t* delta_row_host,
+                                  const int32_t* delta_col_host, const float* delta_val_host, int32_t n_delta,
+                                  const egnn_peer_window* win, egnn_stream_t stream) {
+    return wide_adjoint_sharded_impl(rowptr_local, colidx_local, vals_or_null, row_order_or_null, dinv_full, iso_full,
+                                     cbar_local, tbar_local_or_null, xbar_local, b_out_local_or_null, n_global,
+                                     row_begin, row_end, f, app, k_max, n_scales, coeffs_host, op_scale, op_shift,
+                                     delta_row_host, delta_col_host, delta_val_host, n_delta, win, stream);
+}
+
+// ---- gradient w.r.t. the edge weights of a row shard (csrc/shard_grad.cuh) ---------------------------
+// Lanes across the K*F / vec vectors of one entry: the next power of two, at most a warp.
+static int shard_fl_log2(int64_t kf, int vec) {
+    const int64_t nv = kf / vec;
+    const int l = pow2_ceil_log2(nv > 1 ? nv : 1);
+    return l > 5 ? 5 : l;
+}
+
+int egnn_adj_grad_stacks_sharded(const float* lam_all, int64_t lam_slab_rows, const float* t_all, int64_t t_slab_rows,
+                                 const float* dinv_full, int64_t n_global, int64_t row_begin, int64_t row_end,
+                                 int32_t f, int32_t k, float* pl_local, float* pt_local, egnn_stream_t stream) {
+    EGNN_REQUIRE(n_global >= 0 && n_global < (int64_t(1) << 31) && row_begin >= 0 && row_end >= row_begin &&
+                 row_end <= n_global, "bad row range");
+    EGNN_REQUIRE(f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER, "bad f / k");
+    const int64_t rows = row_end - row_begin;
+    EGNN_REQUIRE(lam_slab_rows >= rows && t_slab_rows >= rows, "slabs shorter than the rank's rows");
+    if (rows == 0 || k == 0) return EGNN_OK;
+    EGNN_REQUIRE(lam_all && t_all && dinv_full && pl_local && pt_local, "null pointer");
+    shard_grad_stacks_kernel<<<grid_for(rows * k * f, 256), 256, 0, (cudaStream_t)stream>>>(
+        lam_all, lam_slab_rows * f, t_all, t_slab_rows * f, dinv_full + row_begin, rows, f, k, pl_local, pt_local);
+    EGNN_LAUNCH_CHECK("shard_grad_stacks_kernel launch");
+    return EGNN_OK;
+}
+
+size_t egnn_adj_grad_degree_sharded_ws_bytes(int64_t rows) {
+    return 2 * align_up(sizeof(double) * (size_t)(rows > 0 ? rows : 1), 256) + 256;
+}
+
+static int launch_shard_dot(const int32_t* rowptr, const int32_t* colidx, const float* vals, const int32_t* perm,
+                            const float* own, const float* gath, int64_t rows, int64_t row0, int32_t kf,
+                            double* out, float* g_out, cudaStream_t st) {
+    const int vec = kf % 4 == 0 ? 4 : 1;
+    const int fl = shard_fl_log2(kf, vec);
+    const int blocks = grid_for(rows * 32, 256);
+    if (vec == 4)
+        shard_grad_dot_kernel<4><<<blocks, 256, 0, st>>>(rowptr, colidx, vals, perm, own, gath, rows, row0, kf, fl,
+                                                          out, g_out);
+    else
+        shard_grad_dot_kernel<1><<<blocks, 256, 0, st>>>(rowptr, colidx, vals, perm, own, gath, rows, row0, kf, fl,
+                                                          out, g_out);
+    EGNN_LAUNCH_CHECK("shard_grad_dot_kernel launch");
+    return EGNN_OK;
+}
+
+int egnn_adj_grad_degree_sharded(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                                 const int32_t* row_order_or_null, const int32_t* rowptr_t, const int32_t* colidx_t,
+                                 const float* vals_t_or_null, const int32_t* row_order_t_or_null,
+                                 const float* dinv_full, const uint8_t* iso_full, int64_t n_global, int64_t row_begin,
+                                 int64_t row_end, int32_t f, int32_t k, float op_scale, const float* pl_full,
+                                 const float* pt_full, const float* xbar_local_or_null,
+                                 const float* rowsum_local_or_null, float* g_out, float* gw_local, float* grho_local,
+                                 void* workspace, size_t workspace_bytes, egnn_stream_t stream) {
+    EGNN_REQUIRE(rowptr && rowptr_t && dinv_full && iso_full && g_out && gw_local && grho_local, "null pointer");
+    EGNN_REQUIRE(n_global >= 0 && n_global < (int64_t(1) << 31) && row_begin >= 0 && row_end >= row_begin &&
+                 row_end <= n_global, "bad row range");
+    EGNN_REQUIRE(f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER, "bad f / k");
+    EGNN_REQUIRE((vals_or_null == nullptr) == (vals_t_or_null == nullptr), "vals and vals_t come together");
+    EGNN_REQUIRE(k == 0 || (pl_full && pt_full), "null lambda / T stacks");
+    EGNN_REQUIRE((xbar_local_or_null == nullptr) || rowsum_local_or_null, "xbar needs rowsum");
+    const int64_t kf = (int64_t)k * f;
+    EGNN_REQUIRE(kf < (int64_t(1) << 31), "k * f out of int32 range");
+    EGNN_REQUIRE(vec_aligned(pl_full, (int32_t)(kf % 4 == 0 ? 4 : 1)) && vec_aligned(pt_full, (int32_t)(kf % 4 == 0 ? 4 : 1)),
+                 "the lambda / T stacks must be 16-byte aligned when k * f % 4 == 0");
+    const int64_t rows = row_end - row_begin;
+    int rc = require_workspace(workspace, workspace_bytes, egnn_adj_grad_degree_sharded_ws_bytes(rows),
+                               "adjacency-gradient workspace");
+    if (rc) return rc;
+    if (rows == 0) return EGNN_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    double* r = (double*)align_up((size_t)workspace, 256);
+    double* q = (double*)((char*)r + align_up(sizeof(double) * (size_t)rows, 256));
+    if (k == 0) {                     // no operator in the pass: g = 0, R = Q = 0, only grho
+        rc = check_cuda(cudaMemsetAsync(r, 0, 2 * align_up(sizeof(double) * (size_t)rows, 256), st), "memset R, Q");
+        if (rc) return rc;
+    } else {
+        rc = launch_shard_dot(rowptr, colidx, vals_or_null, row_order_or_null, pl_full, pt_full, rows, row_begin,
+                              (int32_t)kf, r, g_out, st);
+        if (rc) return rc;
+        rc = launch_shard_dot(rowptr_t, colidx_t, vals_t_or_null, row_order_t_or_null, pt_full, pl_full, rows,
+                              row_begin, (int32_t)kf, q, nullptr, st);
+        if (rc) return rc;
+    }
+    adj_grad_finish_kernel<<<grid_for(rows, 256), 256, 0, st>>>(r, q, dinv_full + row_begin, iso_full + row_begin,
+                                                                xbar_local_or_null, rowsum_local_or_null, rows,
+                                                                op_scale, gw_local, grho_local);
+    EGNN_LAUNCH_CHECK("adj_grad_finish_kernel launch");
+    return EGNN_OK;
+}
+
+int egnn_adj_grad_entries_sharded(const int32_t* rowptr, const int32_t* colidx, int64_t n_global, int64_t row_begin,
+                                  int64_t row_end, int32_t k, const float* g, const float* gw_full,
+                                  const float* grho_local, float op_scale, float* out, egnn_stream_t stream) {
+    EGNN_REQUIRE(n_global >= 0 && n_global < (int64_t(1) << 31) && row_begin >= 0 && row_end >= row_begin &&
+                 row_end <= n_global, "bad row range");
+    EGNN_REQUIRE(k >= 0 && k <= EGNN_MAX_ORDER, "bad k");
+    const int64_t rows = row_end - row_begin;
+    if (rows == 0) return EGNN_OK;   // a rank without rows: nothing to write (its buffers may be empty)
+    EGNN_REQUIRE(rowptr && gw_full && grho_local && out, "null pointer");
+    EGNN_REQUIRE(k == 0 || g, "null g");
+    shard_grad_entries_kernel<<<grid_for(rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+        rowptr, colidx, k == 0 ? nullptr : g, gw_full, grho_local, rows, row_begin, op_scale, out);
+    EGNN_LAUNCH_CHECK("shard_grad_entries_kernel launch");
+    return EGNN_OK;
 }
 
 int egnn_graph_prep_sharded(const int32_t* rowptr_local, const int32_t* colidx_local, const float* vals_or_null,

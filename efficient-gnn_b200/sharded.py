@@ -37,6 +37,8 @@ from torch.autograd.function import once_differentiable
 from . import _cabi
 from .wats import WIDE_MIN_F, _heat_scale_grad, _needs_grad, heat_coefficients
 
+_COEFF_GRAD_MAX_ROWS = 8            # EGNN_MAX_SCALES: rows of cbar one egnn_cheb_coeff_grad takes
+
 __all__ = ["RowPartition", "BalancedOrder", "split_columns", "CudaEngine", "DistComm", "PeerExchange", "ShardedWavelet"]
 
 
@@ -154,9 +156,11 @@ class BalancedOrder:
         return feats[self.inv.to(feats.device)]
 
 
-def split_columns(rowptr: torch.Tensor, colidx: torch.Tensor, col_begin: int, col_end: int):
+def split_columns(rowptr: torch.Tensor, colidx: torch.Tensor, col_begin: int, col_end: int, vals=None):
     """Split a row shard into (local-column CSR, remote-column CSR); entry
-    order inside each row is preserved.  Index plumbing only (torch ops)."""
+    order inside each row is preserved.  Each half is ``(rowptr, colidx)``, or
+    ``(rowptr, colidx, vals)`` when the shard's values are given.  Index
+    plumbing only (torch ops)."""
     n_rows = rowptr.numel() - 1
     counts = (rowptr[1:] - rowptr[:-1]).long()
     rows = torch.repeat_interleave(torch.arange(n_rows, device=rowptr.device), counts)
@@ -165,7 +169,8 @@ def split_columns(rowptr: torch.Tensor, colidx: torch.Tensor, col_begin: int, co
     for mask in (is_local, ~is_local):
         ptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=rowptr.device)
         ptr[1:] = torch.cumsum(torch.bincount(rows[mask], minlength=n_rows), 0)
-        out.append((ptr.to(torch.int32), colidx[mask].contiguous()))
+        half = (ptr.to(torch.int32), colidx[mask].contiguous())
+        out.append(half if vals is None else half + (vals[mask].contiguous(),))
     return out[0], out[1]
 
 
@@ -183,9 +188,16 @@ class CudaEngine:
         self.device = torch.device(device)
         self.lib = _cabi.load()
         self.comm_stream = torch.cuda.Stream(device=self.device)
+        self._one = torch.zeros(1, dtype=torch.float32, device=self.device)
+
+    def _vals(self, v):
+        """Values argument: None (binary), else a valid pointer even for an empty half."""
+        return None if v is None else _cabi.ptr(v if v.numel() else self._one)
 
     # -- degree vectors -----------------------------------------------------
-    def prep(self, rowptr, colidx, n_global, row_begin, n_rows, allreduce):
+    def prep(self, rowptr, colidx, n_global, row_begin, n_rows, allreduce, vals=None):
+        """``(dinv, iso, x0_local, unsorted)`` of the sharded graph (collective); ``vals``: the shard's
+        weights.  Keeps ``w_full`` / ``rowsum_local`` for the degree patches of edge flips."""
         dev, lib = self.device, self.lib
         colsum = torch.empty(n_global, dtype=torch.float64, device=dev)
         diag = torch.empty(n_global, dtype=torch.float32, device=dev)
@@ -195,7 +207,7 @@ class CudaEngine:
         x0 = torch.empty(max(1, n_rows), dtype=torch.float32, device=dev)
         flag = torch.zeros(1, dtype=torch.int32, device=dev)
         w = torch.empty(n_global, dtype=torch.float32, device=dev)
-        args = (_cabi.ptr(rowptr), _cabi.ptr(colidx), None, n_global, row_begin, n_rows)
+        args = (_cabi.ptr(rowptr), _cabi.ptr(colidx), self._vals(vals), n_global, row_begin, n_rows)
         _cabi.check(lib.egnn_graph_prep_sharded(*args, 0, _cabi.ptr(colsum), _cabi.ptr(diag), _cabi.ptr(rowsum),
                                                 None, None, None, _cabi.ptr(flag), None, _stream()), "prep phase 0")
         allreduce(colsum)
@@ -220,14 +232,28 @@ class CudaEngine:
     def order(self, phase, local, remote, dinv, iso, t_prev_full, t_prev_local, t_prev2_local, t_out_local,
               out_local, acc_ws, n_global, nnz_hint, row_begin, row_end, f, order, k_max, n_scales, coeffs,
               op_scale, op_shift, normalize, deltas=None):
-        lp, lc = (None, None) if local is None else local
-        rp, rc = (None, None) if remote is None else remote
-        _cabi.check(self.lib.egnn_cheb_order_sharded(
-            _cabi.ptr(lp), _cabi.ptr(lc), _cabi.ptr(rp), _cabi.ptr(rc), _cabi.ptr(dinv), _cabi.ptr(iso),
-            _cabi.ptr(t_prev_full), _cabi.ptr(t_prev_local), _cabi.ptr(t_prev2_local), _cabi.ptr(t_out_local),
-            _cabi.ptr(out_local), _cabi.ptr(acc_ws), n_global, nnz_hint, row_begin, row_end, f, order, k_max,
-            n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), 1 if normalize else 0,
-            phase, *_cabi.delta_args(deltas), _stream()), "egnn_cheb_order_sharded")
+        """One order on the rank's rows.  ``local`` / ``remote``: the halves of :func:`split_columns`
+        (3-tuples with the values on a weighted shard: egnn_cheb_order_sharded_vals)."""
+        halves, weighted = self._halves(local, remote)
+        tail = (_cabi.ptr(dinv), _cabi.ptr(iso), _cabi.ptr(t_prev_full), _cabi.ptr(t_prev_local),
+                _cabi.ptr(t_prev2_local), _cabi.ptr(t_out_local), _cabi.ptr(out_local), _cabi.ptr(acc_ws), n_global,
+                nnz_hint, row_begin, row_end, f, order, k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p),
+                float(op_scale), float(op_shift), 1 if normalize else 0, phase, *_cabi.delta_args(deltas), _stream())
+        if weighted:
+            _cabi.check(self.lib.egnn_cheb_order_sharded_vals(*halves, *tail), "egnn_cheb_order_sharded_vals")
+        else:
+            _cabi.check(self.lib.egnn_cheb_order_sharded(*halves, *tail), "egnn_cheb_order_sharded")
+
+    def _halves(self, local, remote):
+        """C arguments of the two halves: ``(rowptr, colidx)`` each, or ``(rowptr, colidx, vals)`` each
+        when either carries values; and whether they do."""
+        weighted = any(h is not None and len(h) == 3 for h in (local, remote))
+        out = []
+        for h in (local, remote):
+            rp_, ci_, v_ = (None, None, None) if h is None else (tuple(h) + (None,))[:3]
+            out += [_cabi.ptr(rp_), _cabi.ptr(ci_)] + ([self._vals(v_) if h is not None else _cabi.ptr(self._one)]
+                                                        if weighted else [])
+        return out, weighted
 
     # -- narrow path -----------------------------------------------------------
     def sell_plan(self, rowptr, colidx, n_rows, n_cols, row0, unsorted):
@@ -277,9 +303,9 @@ class CudaEngine:
         return order
 
     def wide_order(self, rowptr, colidx, row_order, dinv, iso, x0_local, t_out, out, n_global, row_begin, row_end, f,
-                   order, k_max, n_scales, coeffs, op_scale, op_shift, normalize, window, deltas=None):
+                   order, k_max, n_scales, coeffs, op_scale, op_shift, normalize, window, deltas=None, vals=None):
         _cabi.check(self.lib.egnn_wide_order_sharded(
-            _cabi.ptr(rowptr), _cabi.ptr(colidx), None, _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
+            _cabi.ptr(rowptr), _cabi.ptr(colidx), self._vals(vals), _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
             _cabi.ptr(x0_local), _cabi.ptr(t_out), _cabi.ptr(out), n_global, row_begin, row_end, f, order, k_max,
             n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), 1 if normalize else 0,
             *_cabi.delta_args(deltas), C.byref(window), _stream()), "egnn_wide_order_sharded")
@@ -289,23 +315,74 @@ class CudaEngine:
                 tbar, acc_ws, n_global, nnz_hint, row_begin, row_end, f, app, k_max, n_scales, coeffs, op_scale,
                 op_shift, deltas_t=None):
         """Application ``app`` of the adjoint on the rank's rows (include/egnn_b200.h
-        ``egnn_cheb_adjoint_sharded``); ``deltas_t``: the forward's flips, rows and columns swapped."""
-        lp, lc = (None, None) if local is None else local
-        rp, rc = (None, None) if remote is None else remote
-        _cabi.check(self.lib.egnn_cheb_adjoint_sharded(
-            _cabi.ptr(lp), _cabi.ptr(lc), _cabi.ptr(rp), _cabi.ptr(rc), _cabi.ptr(dinv), _cabi.ptr(iso),
-            _cabi.ptr(b_prev_full), _cabi.ptr(b_prev_local), _cabi.ptr(b_prev2_local), _cabi.ptr(b_out_local),
-            _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(acc_ws), n_global, nnz_hint, row_begin, row_end, f, app,
-            k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), phase,
-            *_cabi.delta_args(deltas_t), _stream()), "egnn_cheb_adjoint_sharded")
+        ``egnn_cheb_adjoint_sharded``, ``_vals`` when the halves carry values); ``deltas_t``: the
+        forward's flips, rows and columns swapped."""
+        halves, weighted = self._halves(local, remote)
+        tail = (_cabi.ptr(dinv), _cabi.ptr(iso), _cabi.ptr(b_prev_full), _cabi.ptr(b_prev_local),
+                _cabi.ptr(b_prev2_local), _cabi.ptr(b_out_local), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(acc_ws),
+                n_global, nnz_hint, row_begin, row_end, f, app, k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p),
+                float(op_scale), float(op_shift), phase, *_cabi.delta_args(deltas_t), _stream())
+        if weighted:
+            _cabi.check(self.lib.egnn_cheb_adjoint_sharded_vals(*halves, *tail), "egnn_cheb_adjoint_sharded_vals")
+        else:
+            _cabi.check(self.lib.egnn_cheb_adjoint_sharded(*halves, *tail), "egnn_cheb_adjoint_sharded")
 
     def wide_adjoint(self, rowptr, colidx, row_order, dinv, iso, cbar, tbar, xbar, n_global, row_begin, row_end, f,
-                     app, k_max, n_scales, coeffs, op_scale, op_shift, window, deltas_t=None):
-        _cabi.check(self.lib.egnn_wide_adjoint_sharded(
-            _cabi.ptr(rowptr), _cabi.ptr(colidx), _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
-            _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar), n_global, row_begin, row_end, f, app, k_max, n_scales,
-            coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift), *_cabi.delta_args(deltas_t),
-            C.byref(window), _stream()), "egnn_wide_adjoint_sharded")
+                     app, k_max, n_scales, coeffs, op_scale, op_shift, window, deltas_t=None, vals=None, b_out=None):
+        """``vals``: the transposed shard's values; ``b_out``: [rows, f] rows receiving b_m (app 0: b_K),
+        both through egnn_wide_adjoint_sharded_all."""
+        if vals is None and b_out is None:
+            _cabi.check(self.lib.egnn_wide_adjoint_sharded(
+                _cabi.ptr(rowptr), _cabi.ptr(colidx), _cabi.ptr(row_order), _cabi.ptr(dinv), _cabi.ptr(iso),
+                _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar), n_global, row_begin, row_end, f, app, k_max,
+                n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift),
+                *_cabi.delta_args(deltas_t), C.byref(window), _stream()), "egnn_wide_adjoint_sharded")
+            return
+        _cabi.check(self.lib.egnn_wide_adjoint_sharded_all(
+            _cabi.ptr(rowptr), _cabi.ptr(colidx), self._vals(vals), _cabi.ptr(row_order), _cabi.ptr(dinv),
+            _cabi.ptr(iso), _cabi.ptr(cbar), _cabi.ptr(tbar), _cabi.ptr(xbar), _cabi.ptr(b_out), n_global, row_begin,
+            row_end, f, app, k_max, n_scales, coeffs.ctypes.data_as(C.c_void_p), float(op_scale), float(op_shift),
+            *_cabi.delta_args(deltas_t), C.byref(window), _stream()), "egnn_wide_adjoint_sharded_all")
+
+    # -- edge-weight gradient (DESIGN.md section 13) ---------------------------------
+    def adj_grad_stacks(self, b_all, t_all, dinv, n_global, row_begin, row_end, rows_per, f, k):
+        """Pre-scaled node-major stacks ``(pl, pt)`` ``[rows_per, K*F]`` of the own rows: ``pl[i] = (m_k d_i
+        b_k[i])_k``, ``pt[i] = (d_i T_{k-1}[i])_k`` (egnn_adj_grad_stacks_sharded); rows past the rank's
+        are not written (exchanged, never read)."""
+        pl = torch.empty((rows_per, k * f), dtype=torch.float32, device=self.device)
+        pt = torch.empty_like(pl)
+        _cabi.check(self.lib.egnn_adj_grad_stacks_sharded(
+            _cabi.ptr(b_all), int(b_all.shape[1]), _cabi.ptr(t_all), int(t_all.shape[1]), _cabi.ptr(dinv), n_global,
+            row_begin, row_end, f, k, _cabi.ptr(pl), _cabi.ptr(pt), _stream()), "egnn_adj_grad_stacks_sharded")
+        return pl, pt
+
+    def adj_grad_degree(self, shard, shard_t, row_orders, dinv, iso, n_global, row_begin, row_end, f, k, op_scale,
+                        pl_full, pt_full, xbar, rowsum):
+        """``(g [nnz_local], gw [rows], grho [rows])``: ``g_ij`` at the shard's stored entries and the degree
+        terms of the own rows (egnn_adj_grad_degree_sharded).  ``shard`` / ``shard_t``: ``(rowptr, colidx,
+        vals or None)`` of the rank's rows of A and of A^T."""
+        rows = row_end - row_begin
+        (rp_, ci_, v_), (rpt, cit, vt) = shard, shard_t
+        g = torch.empty(max(1, int(ci_.numel())), dtype=torch.float32, device=self.device)
+        gw = torch.empty(max(1, rows), dtype=torch.float32, device=self.device)
+        grho = torch.empty_like(gw)
+        ws_bytes = int(self.lib.egnn_adj_grad_degree_sharded_ws_bytes(rows))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
+        _cabi.check(self.lib.egnn_adj_grad_degree_sharded(
+            _cabi.ptr(rp_), _cabi.ptr(ci_), self._vals(v_), _cabi.ptr(row_orders[0]), _cabi.ptr(rpt), _cabi.ptr(cit),
+            self._vals(vt), _cabi.ptr(row_orders[1]), _cabi.ptr(dinv), _cabi.ptr(iso), n_global, row_begin, row_end,
+            f, k, float(op_scale), _cabi.ptr(pl_full), _cabi.ptr(pt_full), _cabi.ptr(xbar), _cabi.ptr(rowsum),
+            _cabi.ptr(g), _cabi.ptr(gw), _cabi.ptr(grho), _cabi.ptr(ws), ws_bytes, _stream()),
+            "egnn_adj_grad_degree_sharded")
+        return g[:ci_.numel()], gw[:rows], grho[:rows]
+
+    def adj_grad_entries(self, rowptr, colidx, n_global, row_begin, row_end, k, g, gw_full, grho, op_scale):
+        """dLoss/dA at the shard's stored entries ``[nnz_local]`` (egnn_adj_grad_entries_sharded)."""
+        out = torch.empty(max(1, int(colidx.numel())), dtype=torch.float32, device=self.device)
+        _cabi.check(self.lib.egnn_adj_grad_entries_sharded(
+            _cabi.ptr(rowptr), _cabi.ptr(colidx), n_global, row_begin, row_end, k, _cabi.ptr(g), _cabi.ptr(gw_full),
+            _cabi.ptr(grho), float(op_scale), _cabi.ptr(out), _stream()), "egnn_adj_grad_entries_sharded")
+        return out[:colidx.numel()]
 
     def coeff_grad(self, cbar, t_all):
         """``G[s, k] = <cbar[:, s, :], T_k>`` of the local rows, float64 (egnn_cheb_coeff_grad)."""
@@ -429,27 +506,44 @@ class PeerExchange:
         self._opened, self._own = [], None
 
 
-class _ShardedSpec:
-    """Everything of one sharded pass but its differentiable inputs: ``s`` holds the scales' values."""
+class _ShardGraph:
+    """The shard one pass runs on: its values (None: binary), column halves, degree vectors, default
+    signal, and the in-degree weights / row sums the degree patches of edge flips start from."""
 
-    def __init__(self, k, s, lambda_max, want_orders, deltas):
+    def __init__(self, vals, halves, dinv, iso, x0, w_full, rowsum_local):
+        self.vals, (self.local_half, self.remote_half) = vals, halves
+        self.dinv, self.iso, self.x0 = dinv, iso, x0
+        self.w_full, self.rowsum_local = w_full, rowsum_local
+        self.adjoint_vals = None       # the values moved to the transpose, built once per graph (_adjoint_vals)
+
+
+class _ShardedSpec:
+    """Everything of one sharded pass but its differentiable inputs: ``s`` holds the scales' values,
+    ``graph`` the :class:`_ShardGraph` of the call, ``default_signal`` whether ``x0`` is its log1p(degree)."""
+
+    def __init__(self, k, s, lambda_max, want_orders, deltas, graph=None, default_signal=False):
         self.k, self.s, self.lambda_max, self.want_orders, self.deltas = k, s, lambda_max, want_orders, deltas
+        self.graph, self.default_signal = graph, default_signal
 
 
 class _ShardedPass(torch.autograd.Function):
     """``(C [rows, S, F], T [K+1, rows, F])`` of the rank's rows of one un-normalised pass as a function
-    of the local signal ``x0`` (None: the default signal) and the scales ``s`` (None when they need no
-    gradient).  ``T`` is empty unless the orders are wanted or ``s`` needs a gradient.  Backward: the
-    adjoint pass over the transposed shard (:meth:`ShardedWavelet._adjoint`) and the scale gradient from
-    every rank's float64 partials (:meth:`ShardedWavelet._scale_grad`); both are collective."""
+    of the local signal ``x0`` (None: the default signal), the scales ``s``, this rank's edge weights
+    ``ew`` and a 0-d ``lam`` = ``lambda_max`` (each None when it needs no gradient).  ``T`` is empty
+    unless the orders are wanted or ``s``, ``ew`` or ``lam`` needs a gradient.  Backward: the adjoint
+    pass over the transposed shard (:meth:`ShardedWavelet._adjoint`, keeping every Clenshaw vector for
+    ``ew`` / ``lam``), the scale gradient from every rank's float64 partials
+    (:meth:`ShardedWavelet._scale_grad`) and the edge-weight and ``lambda_max`` terms
+    (:meth:`ShardedWavelet._structure_grad`); all are collective."""
 
     @staticmethod
-    def forward(ctx, x0, s, sw, spec):
+    def forward(ctx, x0, s, ew, lam, sw, spec):
         ctx.set_materialize_grads(False)
         s_grad = s is not None and ctx.needs_input_grad[1]
-        want = spec.want_orders or s_grad
+        structure = (ew is not None and ctx.needs_input_grad[2]) or (lam is not None and ctx.needs_input_grad[3])
+        want = spec.want_orders or s_grad or structure
         comb, orders = sw._pass(spec.k, spec.s, None if x0 is None else x0.detach(), spec.lambda_max, False, want,
-                                spec.deltas)
+                                spec.deltas, spec.graph)
         f = comb.shape[2]
         if want:
             t_all = torch.stack([o.reshape(sw.rows, f) for o in orders])
@@ -459,7 +553,8 @@ class _ShardedPass(torch.autograd.Function):
         ctx.sw, ctx.spec, ctx.f = sw, spec, f
         ctx.x_shape = None if x0 is None else x0.shape
         ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
-        ctx.save_for_backward(t_all if s_grad else None)
+        ctx.lam_meta = None if lam is None else (lam.shape, lam.device, lam.dtype)
+        ctx.save_for_backward(t_all if (s_grad or structure) else None)
         return comb, t_all
 
     @staticmethod
@@ -471,13 +566,24 @@ class _ShardedPass(torch.autograd.Function):
         cbar = (_cabi.vec_ready(g_comb) if g_comb is not None else
                 torch.zeros((sw.rows, n_scales, f), dtype=torch.float32, device=sw.device))
         tbar = _cabi.vec_ready(g_orders) if (g_orders is not None and g_orders.numel()) else None
-        x_grad = s_grad = None
-        if ctx.needs_input_grad[0]:
-            x_grad = sw._adjoint(spec, cbar, tbar, f).reshape(ctx.x_shape)
+        x_grad = s_grad = ew_grad = lam_grad = None
+        structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
+        if ctx.needs_input_grad[0] or structure:
+            xbar = sw._adjoint(spec, cbar, tbar, f, keep_all=structure)
+            if structure:
+                xbar, b_all = xbar
+            if ctx.needs_input_grad[0]:
+                x_grad = xbar.reshape(ctx.x_shape)
         if ctx.needs_input_grad[1]:
             shape, dev, dtype = ctx.s_meta
             s_grad = sw._scale_grad(spec, cbar, t_all).to(device=dev, dtype=dtype).reshape(shape)
-        return x_grad, s_grad, None, None
+        if structure:
+            ew_grad, lam_grad = sw._structure_grad(spec, b_all, t_all, f, ctx.needs_input_grad[2],
+                                                   ctx.needs_input_grad[3])
+            if lam_grad is not None:
+                shape, dev, dtype = ctx.lam_meta
+                lam_grad = lam_grad.to(device=dev, dtype=dtype).reshape(shape)
+        return x_grad, s_grad, ew_grad, lam_grad, None, None
 
 
 class ShardedWavelet:
@@ -487,15 +593,23 @@ class ShardedWavelet:
     rows assigned by :class:`RowPartition`.  ``engine`` defaults to the CUDA
     engine; tests inject a CPU engine to drive this logic over gloo.
 
-    :meth:`features` is differentiable w.r.t. ``X0_local`` and a tensor ``s``
-    (DESIGN.md section 12).  The backward is collective, like DDP's: every rank
-    calls ``backward`` on a loss of its own rows, and the gradients are those of
-    the sum of the ranks' losses.  The adjacency and ``lambda_max`` get no
-    gradient here (single-GPU ``graph_wavelet_features`` gives those).
+    ``vals_local``: float32 weights of the rank's stored entries, in
+    ``colidx_local`` order (None: a binary shard).  Every call uses them: the
+    forward, edge flips (their degree patches start from the weighted in-degree
+    and row sums) and the backward.  The SELL plan is binary only, so when any
+    rank is weighted no rank takes it (the generic loop runs, or the fused wide
+    path at F >= 8 with peers), and a rank that passed no weights takes unit
+    weights, so that every rank runs the same kernels and collectives.
+
+    :meth:`features` is differentiable w.r.t. ``X0_local``, a tensor ``s``, the
+    rank's edge weights (``edge_weight=``) and a 0-d tensor ``lambda_max``
+    (DESIGN.md sections 12 and 13).  The backward is collective, like DDP's:
+    every rank calls ``backward`` on a loss of its own rows, and the gradients
+    are those of the sum of the ranks' losses.
     """
 
-    def __init__(self, rowptr_local, colidx_local, n_global: int, *, group=None, engine=None, device=None,
-                 use_sell: Optional[bool] = None, comm=None, peer_exchange: Optional[bool] = None):
+    def __init__(self, rowptr_local, colidx_local, n_global: int, *, vals_local=None, group=None, engine=None,
+                 device=None, use_sell: Optional[bool] = None, comm=None, peer_exchange: Optional[bool] = None):
         self.comm = comm if comm is not None else DistComm(group)
         self.rank, self.world = self.comm.rank, self.comm.world
         self.n = int(n_global)
@@ -509,20 +623,35 @@ class ShardedWavelet:
         self.rowptr = rowptr_local.to(torch.int32).contiguous()
         self.colidx = colidx_local.to(torch.int32).contiguous()
         self.nnz_local = int(self.colidx.numel())
-        self.dinv, self.iso, self.x0, unsorted = self.engine.prep(self.rowptr, self.colidx, self.n, self.row_begin,
-                                                                  self.rows, self._allreduce)
-        self.local_half, self.remote_half = split_columns(self.rowptr, self.colidx, self.row_begin, self.row_end)
+        self.vals = None if vals_local is None else self._check_weights(vals_local)
+        self.dinv, self.iso, self.x0, unsorted = self._prep(self.vals)
+        self.local_half, self.remote_half = split_columns(self.rowptr, self.colidx, self.row_begin, self.row_end,
+                                                          vals=self.vals)
+        self._base = _ShardGraph(self.vals, (self.local_half, self.remote_half), self.dinv, self.iso, self.x0,
+                                 getattr(self.engine, "w_full", None), getattr(self.engine, "rowsum_local", None))
         self.plan = None
-        if use_sell is not False:
+        if use_sell is not False and self.vals is None:      # the SELL plan is binary only
             self.plan = self.engine.sell_plan(self.rowptr, self.colidx, self.rows, self.n, self.row_begin, unsorted)
         # The narrow path exchanges the PRE-SCALED operand dinv * T, the generic path plain T:
         # every rank must run the same one.  A rank whose shard does not qualify for the plan
-        # (unsorted rows, too sparse, no rows) takes the plan away from all of them.
+        # (unsorted rows, too sparse, no rows) takes the plan away from all of them.  Weights are
+        # agreed on in the same all-reduce: when any rank is weighted, a binary rank takes unit
+        # weights, so that every rank runs the weighted kernels and the same collectives (the
+        # transpose of a weighted shard moves values) - its degree vectors do not change.
         if self.world > 1:
-            have = torch.tensor([1.0 if self.plan is not None else 0.0], dtype=torch.float64, device=self.device)
+            have = torch.tensor([1.0 if self.plan is not None else 0.0, 0.0 if self.vals is None else 1.0],
+                                dtype=torch.float64, device=self.device)
             self._allreduce(have)
-            if int(round(float(have.item()))) != self.world:
+            plan_ranks, weighted_ranks = (int(round(float(v))) for v in have.tolist())
+            if plan_ranks != self.world:
                 self.plan = None
+            if weighted_ranks and self.vals is None:
+                self.plan = None
+                self.vals = torch.ones(self.nnz_local, dtype=torch.float32, device=self.device)
+                self.local_half, self.remote_half = split_columns(self.rowptr, self.colidx, self.row_begin,
+                                                                  self.row_end, vals=self.vals)
+                self._base = _ShardGraph(self.vals, (self.local_half, self.remote_half), self.dinv, self.iso,
+                                         self.x0, self._base.w_full, self._base.rowsum_local)
         # Fused exchange over peer memory for the narrow path: needs real peers
         # (one process per GPU, NCCL group) and the plan on every rank.
         self.peer = None
@@ -574,7 +703,58 @@ class ShardedWavelet:
                 self._rowsum_full = full[:self.n].clone()
         self._adjoint_shard = None     # what the backward gathers over (built on first use, see _adjoint_csr)
         self._adjoint_order = None
+        self._t_route = None           # how the entries travel to the transpose (values of weighted calls)
+        self._half_index = {}          # positions of each half's entries, per CSR (_with_vals)
         self.launches = 0
+
+    def _check_weights(self, v):
+        v = torch.as_tensor(v).detach().to(device=self.device, dtype=torch.float32).reshape(-1).contiguous()
+        if v.numel() != self.nnz_local:
+            raise ValueError(f"rank {self.rank} stores {self.nnz_local} entries but got {v.numel()} weights")
+        return v
+
+    def _prep(self, vals):
+        """The sharded degree pass (collective); the weights travel only on a weighted shard, so an
+        injected engine sees the binary call it always saw."""
+        args = (self.rowptr, self.colidx, self.n, self.row_begin, self.rows, self._allreduce)
+        return self.engine.prep(*args) if vals is None else self.engine.prep(*args, vals=vals)
+
+    def _graph(self, edge_weight):
+        """:class:`_ShardGraph` of one call: the shard's own, or with ``edge_weight`` (detached) in place
+        of the stored weights and the degree vectors re-derived for them (collective)."""
+        if edge_weight is None:
+            return self._base
+        vals = self._check_weights(edge_weight)
+        eng = self.engine
+        kept = (getattr(eng, "w_full", None), getattr(eng, "rowsum_local", None))
+        dinv, iso, x0, _ = self._prep(vals)
+        halves = self._with_vals("fwd", self.colidx, (self.local_half, self.remote_half), vals)
+        g = _ShardGraph(vals, halves, dinv, iso, x0, getattr(eng, "w_full", None), getattr(eng, "rowsum_local", None))
+        eng.w_full, eng.rowsum_local = kept      # the shard's own vectors stay the engine's base
+        return g
+
+    def _with_vals(self, key, colidx, halves, vals):
+        """``halves`` (of :func:`split_columns` over ``colidx``) with ``vals`` split alongside: the entries'
+        positions in each half are found once per CSR, so a call's weights cost two gathers."""
+        if key not in self._half_index:
+            local = (colidx >= self.row_begin) & (colidx < self.row_end)
+            self._half_index[key] = (local.nonzero().squeeze(1), (~local).nonzero().squeeze(1))
+        il, ir = self._half_index[key]
+        (lp, lc), (rp_, rc) = (h[:2] for h in halves)
+        return (lp, lc, vals.index_select(0, il)), (rp_, rc, vals.index_select(0, ir))
+
+    def _patch(self, g, deltas):
+        """``(dinv, iso, x0_local)`` of ``g`` with the flips applied (the engine patches from ``g``'s
+        in-degree weights and row sums)."""
+        eng = self.engine
+        if g is self._base:
+            return eng.patch_degrees(g.dinv, g.iso, g.x0, self.n, self.row_begin, self.rows, deltas)
+        kept = (eng.w_full, eng.rowsum_local)
+        eng.w_full, eng.rowsum_local = g.w_full, g.rowsum_local
+        try:
+            return eng.patch_degrees(g.dinv, g.iso, g.x0, self.n, self.row_begin, self.rows, deltas)
+        finally:
+            eng.w_full, eng.rowsum_local = kept
 
     def _wide_window(self, ldy: int):
         """Exchange window for ``ldy``-wide operand rows (collective on first use)."""
@@ -618,8 +798,8 @@ class ShardedWavelet:
         self.comm.allgather(full, slab)
 
     # -- the path ------------------------------------------------------------------
-    def features(self, k=3, s=0.8, *, X0_local=None, lambda_max: float = 2.0, normalize: bool = True,
-                 return_parts: bool = False, deltas=None):
+    def features(self, k=3, s=0.8, *, X0_local=None, lambda_max=2.0, normalize: bool = True,
+                 return_parts: bool = False, deltas=None, edge_weight=None):
         """Features of the local rows ``[rows, S*F]`` (reference defaults
         k=3, s=0.8, X0 = log1p(degree)); with ``return_parts`` also the local
         slabs of every order and the un-normalised combination.
@@ -631,53 +811,79 @@ class ShardedWavelet:
         patches its replicated dinv/iso and the x0 of its own rows, and the
         order kernels add the flipped entries of the rows they own.
 
-        Differentiable w.r.t. ``X0_local`` and a 0-d / 1-d tensor ``s`` when
-        grad mode is on and one of them requires grad: every output then
-        carries a ``grad_fn`` (``deltas=`` is supported).  ``X0_local.grad``
-        receives this rank's rows of the gradient and ``s.grad`` the full scale
-        gradient, identical bits on every rank.  The backward is collective:
-        every rank must call ``backward`` (once per call of ``features``, in
-        the same order on every rank), with the same inputs requiring grad."""
+        ``edge_weight``: a ``[nnz_local]`` tensor that replaces this rank's
+        stored weights for this call (the degree vectors are re-derived:
+        collective, so every rank passes one or none does).
+
+        Differentiable w.r.t. ``X0_local``, a 0-d / 1-d tensor ``s``,
+        ``edge_weight`` and a 0-d tensor ``lambda_max`` when grad mode is on
+        and one of them requires grad: every output then carries a
+        ``grad_fn``.  ``X0_local.grad`` receives this rank's rows of the
+        gradient, ``edge_weight.grad`` dLoss/dA at this rank's stored entries,
+        ``s.grad`` and ``lambda_max.grad`` the full gradients, identical bits
+        on every rank (DESIGN.md sections 12 and 13).  ``deltas=`` works with
+        the first two; an ``edge_weight`` or ``lambda_max`` that requires grad
+        together with ``deltas`` raises ``ValueError``.  The backward is
+        collective: every rank must call ``backward`` (once per call of
+        ``features``, in the same order on every rank), with the same inputs
+        requiring grad."""
         k = int(k)
         if deltas is not None and len(deltas[0]) == 0:
             deltas = None
+        grad_on = torch.is_grad_enabled()
+        ew_in = edge_weight if (grad_on and isinstance(edge_weight, torch.Tensor) and edge_weight.requires_grad) \
+            else None
+        lam_in = lambda_max if (grad_on and isinstance(lambda_max, torch.Tensor) and lambda_max.requires_grad) \
+            else None
+        if lam_in is not None and lam_in.dim() != 0:
+            raise ValueError("a lambda_max that requires grad must be a 0-d tensor")
+        if deltas is not None and (ew_in is not None or lam_in is not None):
+            raise ValueError("edge flips (deltas=) are adjacency-forward-only: edge_weight and lambda_max cannot "
+                             "require grad with them")
+        lam_val = float(lambda_max.detach() if isinstance(lambda_max, torch.Tensor) else lambda_max)
+        graph = self._graph(edge_weight)
         x_in = None if X0_local is None else torch.as_tensor(X0_local)
-        if _needs_grad(self.x0 if x_in is None else x_in, s):
+        if _needs_grad(graph.x0 if x_in is None else x_in, s, ew_in, lam_in):
             # un-normalised combination (and the orders) through the autograd function, then the
-            # out-of-place normalisation (as graph_wavelet_features)
+            # out-of-place normalisation (as graph_wavelet_features); the device / dtype conversions stay
+            # outside the function, so autograd routes the gradients back to the callers' tensors
             s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
             x0 = None if x_in is None else x_in.to(device=self.device, dtype=torch.float32)
             s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
-            comb, t_all = _ShardedPass.apply(x0, s_in, self, _ShardedSpec(k, s_vals, float(lambda_max), return_parts,
-                                                                          deltas))
-            feats = self.engine.l1_normalize(comb) if normalize else comb
+            ew = None if ew_in is None else ew_in.to(device=self.device, dtype=torch.float32).reshape(-1)
+            spec = _ShardedSpec(k, s_vals, lam_val, return_parts, deltas, graph, default_signal=x_in is None)
+            comb, t_all = _ShardedPass.apply(x0, s_in, ew, lam_in, self, spec)
+            feats = self.engine.l1_normalize(comb) if (normalize and self.rows) else comb
             orders = [t_all[i] for i in range(k + 1)] if return_parts else None
         else:
-            comb, orders = self._pass(k, s, X0_local, lambda_max, normalize, return_parts, deltas)
+            comb, orders = self._pass(k, s, X0_local, lam_val, normalize, return_parts, deltas, graph)
             feats = comb / (comb.abs().sum(dim=2, keepdim=True) + 1e-8) if (normalize and return_parts) else comb
-        feats = feats.reshape(self.rows, -1)
+        feats = feats.flatten(1)          # [rows, S*F], also for a rank without rows
         return (feats, orders, comb) if return_parts else feats
 
-    def _pass(self, k, s, X0_local, lambda_max, normalize, return_parts, deltas):
+    def _pass(self, k, s, X0_local, lambda_max, normalize, return_parts, deltas, graph=None):
         """The rank's rows of one pass: ``(out [rows, S, F], [T_0 .. T_K])``, the orders only when
         ``return_parts`` (else just ``[T_0]``).  ``out`` is L1-normalised when ``normalize`` and not
-        ``return_parts``, else the un-normalised combination.  ``deltas``: a non-empty flip list or None."""
+        ``return_parts``, else the un-normalised combination.  ``deltas``: a non-empty flip list or None.
+        ``graph``: the call's :class:`_ShardGraph` (None: the shard's own)."""
         eng, dev = self.engine, self.device
+        g = self._base if graph is None else graph
+        plan = self.plan if g.vals is None else None          # the SELL plan is binary only
+        vals_kw = {} if g.vals is None else {"vals": g.vals}
         coeffs = np.ascontiguousarray(heat_coefficients(k, s), dtype=np.float32)
         n_scales = coeffs.shape[0]
-        dinv, iso, x0_default = self.dinv, self.iso, self.x0
+        dinv, iso, x0_default = g.dinv, g.iso, g.x0
         base_rowsum = None
         if deltas is not None:
             x_in = None if X0_local is None else torch.as_tensor(X0_local)
             f_in = 1 if (x_in is None or x_in.dim() == 1) else int(x_in.shape[1])
-            if k >= 1 and f_in == 1 and self.plan is not None and self.peer is not None and self._rowsum_full is not None:
+            if k >= 1 and f_in == 1 and plan is not None and self.peer is not None and self._rowsum_full is not None:
                 # fused narrow path: the step kernel gets the base graph's vectors plus the row sums of every
                 # node and re-derives the nodes the flips touch itself (same arithmetic on every rank) - a
                 # perturbed pass is one launch, and the first operand dinv * x0 stays known everywhere
                 base_rowsum = self._rowsum_full
             else:
-                dinv, iso, x0_default = eng.patch_degrees(self.dinv, self.iso, self.x0, self.n, self.row_begin,
-                                                          self.rows, deltas)
+                dinv, iso, x0_default = self._patch(g, deltas)
         x0 = x0_default.reshape(-1, 1) if X0_local is None else torch.as_tensor(X0_local)
         if x0.dim() == 1:
             x0 = x0.reshape(-1, 1)
@@ -702,7 +908,7 @@ class ShardedWavelet:
             if fused_norm:            # no kernel ran to fuse it into
                 out = out / (out.abs().sum(dim=2, keepdim=True) + 1e-8)
             return out, orders
-        use_plan = self.plan is not None and f == 1
+        use_plan = plan is not None and f == 1
         fused = use_plan and self.peer is not None
         fused_wide = self.fused_wide and f >= WIDE_MIN_F
         if fused_wide:
@@ -716,7 +922,7 @@ class ShardedWavelet:
                 t_out = torch.empty((self.rows, f), dtype=torch.float32, device=dev) if return_parts else None
                 eng.wide_order(self.rowptr, self.colidx, self._row_order, dinv, iso,
                                x0 if order == 1 else None, t_out, out, self.n, self.row_begin, self.row_end, f, order,
-                               k, n_scales, coeffs, op_scale, op_shift, fused_norm, win, deltas)
+                               k, n_scales, coeffs, op_scale, op_shift, fused_norm, win, deltas, **vals_kw)
                 self.launches += 1
                 if return_parts:
                     orders.append(t_out)
@@ -788,10 +994,10 @@ class ShardedWavelet:
             tail = (self.n, max(1, self.nnz_local), self.row_begin, self.row_end, f, order, k, n_scales, coeffs,
                     op_scale, op_shift, fused_norm)
             if self.rows:
-                eng.order(0, self.local_half, None, *common, None, t_prev, t_prev2, t_out, out, acc_ws, *tail)
+                eng.order(0, g.local_half, None, *common, None, t_prev, t_prev2, t_out, out, acc_ws, *tail)
             eng.join()
             if self.rows:
-                eng.order(1, None, self.remote_half, *common, full, t_prev, t_prev2, t_out, out, acc_ws, *tail,
+                eng.order(1, None, g.remote_half, *common, full, t_prev, t_prev2, t_out, out, acc_ws, *tail,
                           deltas=deltas)
                 self.launches += 2
             if return_parts:
@@ -833,7 +1039,9 @@ class ShardedWavelet:
             self.comm.alltoall(recv_counts, send_counts, [1] * world, [1] * world)
             recv = torch.empty((int(recv_counts.sum()), 2), dtype=torch.int64, device=dev)
             self.comm.alltoall(recv, send, recv_counts.tolist(), send_counts.tolist())
-            key = ((recv[:, 0] - self.row_begin) * n + recv[:, 1]).sort().values
+            key, order = ((recv[:, 0] - self.row_begin) * n + recv[:, 1]).sort(stable=True)
+            # the route of the entries, for the values of weighted calls (_adjoint_vals)
+            self._t_route = (by_owner, send_counts.tolist(), recv_counts.tolist(), order)
             rowptr_t = torch.zeros(self.rows + 1, dtype=torch.int64, device=dev)
             rowptr_t[1:] = torch.cumsum(torch.bincount(torch.div(key, n, rounding_mode="floor"), minlength=self.rows), 0)
             rowptr_t, colidx_t = rowptr_t.to(torch.int32), (key % n).to(torch.int32)
@@ -849,6 +1057,24 @@ class ShardedWavelet:
             return self.rowptr, self.colidx, self.local_half, self.remote_half
         return self._adjoint_shard
 
+    def _adjoint_vals(self, g):
+        """``(vals_t, local half, remote half)`` of :meth:`_adjoint_csr` with the values of the
+        :class:`_ShardGraph` ``g`` moved to their places in the transpose: one collective ``all_to_all``
+        along the route the entries took, once per graph (the shard's own, or one call's edge weights,
+        whose adjoint and gradient terms share it)."""
+        if g.adjoint_vals is not None:
+            return g.adjoint_vals
+        vals = g.vals
+        rowptr_t, colidx_t, local, remote = self._adjoint_csr()
+        by_owner, send_counts, recv_counts, order = self._t_route
+        recv = torch.empty(sum(recv_counts), dtype=torch.float32, device=self.device)
+        self.comm.alltoall(recv, vals.index_select(0, by_owner), recv_counts, send_counts)
+        vals_t = recv.index_select(0, order)
+        out = (vals_t,) + self._with_vals("fwd" if self._adjoint_shard is False else "adj", colidx_t, (local, remote),
+                                          vals_t)
+        g.adjoint_vals = out
+        return out
+
     def _adjoint_row_order(self):
         """egnn_row_order of :meth:`_adjoint_csr` (the fused wide adjoint's processing order)."""
         rowptr = self._adjoint_csr()[0]
@@ -860,48 +1086,61 @@ class ShardedWavelet:
             self._adjoint_order = self.engine.row_order(rowptr, self.rows)
         return self._adjoint_order
 
-    def _adjoint(self, spec, cbar, tbar, f):
+    def _adjoint(self, spec, cbar, tbar, f, keep_all=False):
         """This rank's rows of the signal's gradient ``[rows, F]`` from its rows of ``cbar`` ``[rows, S, F]``
         and ``tbar`` ``[K+1, rows, F]`` (collective: the operand of every application is exchanged).  The
-        forward's flips are applied transposed, with the forward's patched ``dinv`` / ``iso``."""
+        forward's flips are applied transposed, with the forward's patched ``dinv`` / ``iso``.
+        ``keep_all``: returns ``(xbar, b_all)`` with every Clenshaw vector ``b_all [K+1, rows_per, F]``
+        (slab 0: ``xbar``; the sharded analogue of egnn_cheb_adjoint_all)."""
         eng, dev, k = self.engine, self.device, spec.k
+        g = self._base if spec.graph is None else spec.graph
         coeffs = np.ascontiguousarray(heat_coefficients(k, spec.s), dtype=np.float32)
         n_scales = coeffs.shape[0]
         op_scale, op_shift = 2.0 / spec.lambda_max, -1.0
-        dinv, iso, deltas_t = self.dinv, self.iso, None
+        dinv, iso, deltas_t = g.dinv, g.iso, None
         if spec.deltas is not None:
-            dinv, iso, _ = eng.patch_degrees(self.dinv, self.iso, self.x0, self.n, self.row_begin, self.rows,
-                                             spec.deltas)
+            dinv, iso, _ = self._patch(g, spec.deltas)
             d_rows, d_cols, d_vals = spec.deltas
             deltas_t = (d_cols, d_rows, d_vals)
+        rp = self.part.rows_per
         if self.rows == 0:            # the fused kernels still take part in the exchange: valid pointers
             cbar = torch.zeros((1, n_scales, f), dtype=torch.float32, device=dev)
-        xbar = torch.empty((max(1, self.rows), f), dtype=torch.float32, device=dev)
+        b_all = torch.empty((k + 1, rp, f), dtype=torch.float32, device=dev) if keep_all else None
+        xbar = b_all[0] if keep_all else torch.empty((max(1, self.rows), f), dtype=torch.float32, device=dev)
+
+        def done():
+            return (xbar[:self.rows], b_all) if keep_all else xbar[:self.rows]
+
         coef = (k, n_scales, coeffs, op_scale, op_shift)
         if k == 0:                    # xbar = v_0: no operator application, nothing exchanged
             if self.rows:
                 eng.adjoint(2, None, None, dinv, iso, None, None, None, xbar, cbar, tbar, None, self.n, 1,
                             self.row_begin, self.row_end, f, 0, *coef)
                 self.launches += 1
-            return xbar[:self.rows]
+            return done()
         rowptr_t, colidx_t, local, remote = self._adjoint_csr()
+        vals_t = None
+        if g.vals is not None:
+            vals_t, local, remote = self._adjoint_vals(g)
         if self.fused_wide and f >= WIDE_MIN_F:
             # exchange fused: the operand dinv (.) b travels through the forward's window and flags
             win = self._wide_window((f + 3) // 4 * 4).window
             order = self._adjoint_row_order()
             for app in range(k + 1):
+                extra = {} if vals_t is None else {"vals": vals_t}
+                if keep_all and app < k:
+                    extra["b_out"] = b_all[k - app]
                 eng.wide_adjoint(rowptr_t, colidx_t, order, dinv, iso, cbar, tbar, xbar, self.n, self.row_begin,
-                                 self.row_end, f, app, *coef, win, deltas_t)
-                self.launches += 1
-            return xbar[:self.rows]
+                                 self.row_end, f, app, *coef, win, deltas_t, **extra)
+                self.launches += 2 if (keep_all and app == 0 and self.rows) else 1
+            return done()
         # generic CSR kernel, local / remote column halves around the exchange of b_{m+1} (as the forward)
-        rp = self.part.rows_per
 
         def slab():
             return torch.empty((rp, f), dtype=torch.float32, device=dev)
 
         tail = (self.n, max(1, int(colidx_t.numel())), self.row_begin, self.row_end, f)
-        b_prev = slab()
+        b_prev = b_all[k] if keep_all else slab()
         if self.rows:
             eng.adjoint(2, None, None, dinv, iso, None, None, None, b_prev, cbar, tbar, None, *tail, 0, *coef)
             self.launches += 1
@@ -910,7 +1149,10 @@ class ShardedWavelet:
         acc_ws = slab()
         for app in range(1, k + 1):
             m = k - app
-            b_out = xbar if m == 0 else (slab() if app <= 2 else b_prev2)    # in place over b_{m+2}
+            if keep_all:
+                b_out = b_all[m]                                                 # every b_m kept
+            else:
+                b_out = xbar if m == 0 else (slab() if app <= 2 else b_prev2)    # in place over b_{m+2}
             eng.fork()
             with eng.side_stream():
                 self._allgather(full, b_prev)
@@ -923,7 +1165,7 @@ class ShardedWavelet:
                             *coef, deltas_t=deltas_t)
                 self.launches += 2
             b_prev2, b_prev = b_prev, b_out
-        return xbar[:self.rows]
+        return done()
 
     def _scale_grad(self, spec, cbar, t_all):
         """``ds_j = -sum_k k alpha[j,k] G[j,k]`` with ``G = sum_r <cbar_r, T_r>`` over the ranks' rows: every
@@ -941,6 +1183,78 @@ class ShardedWavelet:
         for r in range(1, self.world):
             total = total + parts[r]
         return _heat_scale_grad(coeffs, total)
+
+    def _structure_grad(self, spec, b_all, t_all, f, want_weights, want_lam):
+        """``(dLoss/dA at this rank's stored entries [nnz_local], dLoss/dlambda_max)`` (each None unless
+        wanted) from the Clenshaw vectors ``b_all [K+1, rows_per, F]`` and the orders ``t_all [K+1, rows, F]``
+        (DESIGN.md section 13, collective).  Edge weights: the pre-scaled stacks ``m_k d (.) b_k`` and
+        ``d (.) T_{k-1}`` of every rank are all-gathered, each rank forms ``g``, ``R`` over its shard, ``Q``
+        over its rows of the transpose and ``gw`` / ``grho`` of its rows, ``gw`` is all-gathered and the
+        values at the stored entries follow.  ``lambda_max``: every rank's float64 partials ``<b_k, T_j>``
+        are all-gathered and added in rank order, so every rank holds the same bits."""
+        eng, dev, k = self.engine, self.device, spec.k
+        g = self._base if spec.graph is None else spec.graph
+        rp, rb, re_ = self.part.rows_per, self.row_begin, self.row_end
+        a = 2.0 / spec.lambda_max
+        ew_grad = lam_grad = None
+        if want_weights:
+            plf = ptf = None
+            if k >= 1:
+                pl, pt = eng.adj_grad_stacks(b_all, t_all, g.dinv, self.n, rb, re_, rp, f, k)
+                self.launches += 1 if self.rows else 0
+                plf = torch.empty((self.world * rp, k * f), dtype=pl.dtype, device=dev)
+                ptf = torch.empty_like(plf)
+                self._allgather(plf, pl)
+                self._allgather(ptf, pt)
+                rowptr_t, colidx_t = self._adjoint_csr()[:2]
+                vals_t = None if g.vals is None else self._adjoint_vals(g)[0]
+                orders = (self._forward_row_order(), self._adjoint_row_order())
+            else:                     # g = 0 and no transposed rows needed: only grho
+                rowptr_t, colidx_t, vals_t, orders = self.rowptr, self.colidx, g.vals, (None, None)
+            default = spec.default_signal and f == 1
+            xbar = b_all[0, :self.rows, 0].contiguous() if default else None
+            rowsum = g.rowsum_local if default else None
+            ge, gw, grho = eng.adj_grad_degree((self.rowptr, self.colidx, g.vals), (rowptr_t, colidx_t, vals_t),
+                                               orders, g.dinv, g.iso, self.n, rb, re_, f, k, a, plf, ptf, xbar,
+                                               rowsum)
+            pad = torch.zeros(rp, dtype=gw.dtype, device=dev)
+            pad[:self.rows] = gw
+            gw_full = torch.empty(self.world * rp, dtype=gw.dtype, device=dev)
+            self._allgather(gw_full, pad)
+            ew_grad = eng.adj_grad_entries(self.rowptr, self.colidx, self.n, rb, re_, k, ge if k >= 1 else None,
+                                           gw_full, grho, a)
+            self.launches += (3 if k >= 1 else 1) + 1 if self.rows else 0
+        if want_lam:
+            if k == 0:                # lambda_max does not enter the pass
+                lam_grad = torch.zeros((), dtype=torch.float64, device=dev)
+            else:
+                part = torch.zeros((k, k + 1), dtype=torch.float64, device=dev)
+                if self.rows:
+                    # <b_i, T_j> for every i in one egnn_cheb_coeff_grad per 8 orders: b_1..b_K take the
+                    # place of the scales (row i - 1 of the partials holds b_i against T_0..T_K)
+                    for c0 in range(1, k + 1, _COEFF_GRAD_MAX_ROWS):
+                        c1 = min(k + 1, c0 + _COEFF_GRAD_MAX_ROWS)
+                        part[c0 - 1:c1 - 1] = eng.coeff_grad(b_all[c0:c1, :self.rows].permute(1, 0, 2).contiguous(),
+                                                             t_all)
+                        self.launches += 2
+                full = torch.empty((self.world * k, k + 1), dtype=torch.float64, device=dev)
+                self._allgather(full, part)
+                parts = full.reshape(self.world, k, k + 1)
+                G = parts[0]
+                for r in range(1, self.world):
+                    G = G + parts[r]
+                total = torch.zeros((), dtype=torch.float64, device=dev)
+                for i in range(1, k + 1):
+                    total = total + G[i - 1, i] + (1.0 if i == 1 else 2.0) * G[i - 1, i - 1] + \
+                        (G[i - 1, i - 2] if i >= 2 else 0.0)
+                lam_grad = -total / float(spec.lambda_max)
+        return ew_grad, lam_grad
+
+    def _forward_row_order(self):
+        """egnn_row_order of the rank's own shard (longest rows first), built once."""
+        if self._row_order is None:
+            self._row_order = self.engine.row_order(self.rowptr, self.rows)
+        return self._row_order
 
 
 # --------------------------------------------------------------------------- #

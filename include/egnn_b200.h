@@ -602,6 +602,95 @@ int egnn_wide_adjoint_sharded(const int32_t* rowptr_local, const int32_t* colidx
                               const float* delta_val_host, int32_t n_delta,
                               const egnn_peer_window* win, egnn_stream_t stream);
 
+/* ---- weighted shards and the edge-weight gradient of a shard (new in ABI 11) --
+ * egnn_cheb_order_sharded_vals / egnn_cheb_adjoint_sharded_vals: the entries
+ * above with float32 values of the local and remote halves (in the halves'
+ * entry order; both NULL = binary, exactly the entries above).  The adjoint's
+ * values are those of the rank's rows of the TRANSPOSED adjacency.  The
+ * adjoint keeps every Clenshaw vector when the caller passes a distinct
+ * b_out_local per application instead of rotating over b_{m+2}.
+ * egnn_wide_adjoint_sharded_all: egnn_wide_adjoint_sharded with the values of
+ * the transposed shard and b_out_local_or_null [rows, f]: b_m of the own rows
+ * for every app with m >= 1 (app 0: b_K), the sharded analogue of
+ * egnn_cheb_adjoint_all.  b_out must be 16-byte aligned when f % 4 == 0.      */
+int egnn_cheb_order_sharded_vals(const int32_t* rowptr_local, const int32_t* colidx_local,
+                                 const float* vals_local_or_null,
+                                 const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                                 const float* vals_remote_or_null,
+                                 const float* dinv_full, const uint8_t* iso_full,
+                                 const float* t_prev_full, const float* t_prev_local,
+                                 const float* t_prev2_local, float* t_out_local,
+                                 float* out_local, float* acc_ws,
+                                 int64_t n, int64_t nnz_hint, int64_t row_begin, int64_t row_end,
+                                 int32_t f, int32_t order, int32_t k_max, int32_t n_scales,
+                                 const float* coeffs_host, float op_scale, float op_shift,
+                                 int32_t normalize_l1, int32_t phase,
+                                 const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                 const float* delta_val_host, int32_t n_delta,
+                                 egnn_stream_t stream);
+int egnn_cheb_adjoint_sharded_vals(const int32_t* rowptr_local, const int32_t* colidx_local,
+                                   const float* vals_local_or_null,
+                                   const int32_t* rowptr_remote, const int32_t* colidx_remote,
+                                   const float* vals_remote_or_null,
+                                   const float* dinv_full, const uint8_t* iso_full, const float* b_prev_full,
+                                   const float* b_prev_local, const float* b_prev2_local_or_null,
+                                   float* b_out_local, const float* cbar_local,
+                                   const float* tbar_local_or_null, float* acc_ws,
+                                   int64_t n, int64_t nnz_hint, int64_t row_begin, int64_t row_end,
+                                   int32_t f, int32_t app, int32_t k_max, int32_t n_scales,
+                                   const float* coeffs_host, float op_scale, float op_shift, int32_t phase,
+                                   const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                   const float* delta_val_host, int32_t n_delta, egnn_stream_t stream);
+int egnn_wide_adjoint_sharded_all(const int32_t* rowptr_local, const int32_t* colidx_local,
+                                  const float* vals_or_null, const int32_t* row_order_or_null,
+                                  const float* dinv_full, const uint8_t* iso_full, const float* cbar_local,
+                                  const float* tbar_local_or_null, float* xbar_local,
+                                  float* b_out_local_or_null,
+                                  int64_t n_global, int64_t row_begin, int64_t row_end,
+                                  int32_t f, int32_t app, int32_t k_max, int32_t n_scales,
+                                  const float* coeffs_host, float op_scale, float op_shift,
+                                  const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                  const float* delta_val_host, int32_t n_delta,
+                                  const egnn_peer_window* win, egnn_stream_t stream);
+
+/* Edge-weight gradient of a row shard (section 11's terms on the rows
+ * [row_begin, row_end); DESIGN.md section 13).  Pre-scaled, node-major
+ * stacks [rows, K*F] per rank, all-gathered by the caller into [N', K*F]
+ * (N' >= n_global, rank r's rows at row_begin_r):
+ *   pl[i] = (m_1 d_i lam_1[i], ..., m_K d_i lam_K[i]),  pt[i] = (d_i T_0[i], ..., d_i T_{K-1}[i])
+ * egnn_adj_grad_stacks_sharded: pl_local / pt_local [rows, K*F] from lam_all
+ *   [K+1, lam_slab_rows, f] (slab k = b_k; slab 0 unused) and t_all [K+1,
+ *   t_slab_rows, f] (the forward's orders of the own rows).
+ * egnn_adj_grad_degree_sharded: g_out[q] = g_ij at every stored entry q of
+ *   the shard (0 on the diagonal), R over the shard, Q over the rank's rows
+ *   of the transposed adjacency, then gw_local / grho_local [rows] (section
+ *   11; xbar/rowsum: default signal only).  row_order*_or_null: egnn_row_order
+ *   of the two CSRs (longest rows first).  pl_full / pt_full must be 16-byte
+ *   aligned when K*F % 4 == 0.  workspace: egnn_adj_grad_degree_sharded_ws_bytes.
+ * egnn_adj_grad_entries_sharded: out[q] = dLoss/dA at stored entry q = (i, j)
+ *   = [i != j] (-a g_q + gw_full[j]) + grho_local[i - row_begin], from the
+ *   all-gathered gw_full [N'] (g may be NULL when k == 0).
+ * Fixed summation order, no atomics: bitwise reproducible.                    */
+int egnn_adj_grad_stacks_sharded(const float* lam_all, int64_t lam_slab_rows, const float* t_all,
+                                 int64_t t_slab_rows, const float* dinv_full, int64_t n_global,
+                                 int64_t row_begin, int64_t row_end, int32_t f, int32_t k,
+                                 float* pl_local, float* pt_local, egnn_stream_t stream);
+size_t egnn_adj_grad_degree_sharded_ws_bytes(int64_t rows);
+int egnn_adj_grad_degree_sharded(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                                 const int32_t* row_order_or_null, const int32_t* rowptr_t,
+                                 const int32_t* colidx_t, const float* vals_t_or_null,
+                                 const int32_t* row_order_t_or_null, const float* dinv_full,
+                                 const uint8_t* iso_full, int64_t n_global, int64_t row_begin,
+                                 int64_t row_end, int32_t f, int32_t k, float op_scale,
+                                 const float* pl_full, const float* pt_full,
+                                 const float* xbar_local_or_null, const float* rowsum_local_or_null,
+                                 float* g_out, float* gw_local, float* grho_local,
+                                 void* workspace, size_t workspace_bytes, egnn_stream_t stream);
+int egnn_adj_grad_entries_sharded(const int32_t* rowptr, const int32_t* colidx, int64_t n_global,
+                                  int64_t row_begin, int64_t row_end, int32_t k, const float* g,
+                                  const float* gw_full, const float* grho_local, float op_scale,
+                                  float* out, egnn_stream_t stream);
+
 /* Degree pass of a row shard (scipy semantics as egnn_graph_prep).  phase 0:
  * row sums of the local rows, their diagonal entries into diag_full[row_begin..]
  * and the shard's contribution to the in-degree in colsum_full (both zeroed
