@@ -502,7 +502,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 11; }
+int egnn_abi_version(void) { return 12; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -1219,6 +1219,22 @@ int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const flo
                          float op_scale, const float* lam, const float* t, const float* xbar_or_null,
                          const float* rowsum_or_null, float* gw, float* grho, void* workspace,
                          size_t workspace_bytes, egnn_stream_t stream) {
+    return egnn_adj_grad_degree_flips(rowptr, colidx, vals_or_null, rowptr_t, colidx_t, vals_t_or_null, dinv, iso, n,
+                                      nnz, f, k, op_scale, lam, t, xbar_or_null, rowsum_or_null, nullptr, nullptr,
+                                      nullptr, 0, gw, grho, workspace, workspace_bytes, stream);
+}
+
+int egnn_adj_grad_degree_flips(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                               const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                               const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f,
+                               int32_t k, float op_scale, const float* lam, const float* t,
+                               const float* xbar_or_null, const float* rowsum_or_null,
+                               const int32_t* delta_row_host, const int32_t* delta_col_host,
+                               const float* delta_val_host, int32_t n_delta, float* gw, float* grho,
+                               void* workspace, size_t workspace_bytes, egnn_stream_t stream) {
+    DeltaList d;
+    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n);
+    if (rc) return rc;
     EGNN_REQUIRE(rowptr && rowptr_t && dinv && iso && gw && grho, "null pointer");
     EGNN_REQUIRE(nnz == 0 || (colidx && colidx_t), "null colidx");
     EGNN_REQUIRE((vals_or_null == nullptr) == (vals_t_or_null == nullptr), "vals and vals_t come together");
@@ -1226,8 +1242,8 @@ int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const flo
     EGNN_REQUIRE((xbar_or_null == nullptr) || rowsum_or_null, "xbar needs rowsum");
     EGNN_REQUIRE(n >= 0 && n < (int64_t(1) << 31) && nnz >= 0 && nnz < (int64_t(1) << 31), "n/nnz out of int32 range");
     EGNN_REQUIRE(f >= 1 && k >= 0 && k <= EGNN_MAX_ORDER, "bad f / k");
-    int rc = require_workspace(workspace, workspace_bytes, egnn_adj_grad_degree_ws_bytes(n),
-                               "adjacency-gradient workspace");
+    rc = require_workspace(workspace, workspace_bytes, egnn_adj_grad_degree_ws_bytes(n),
+                           "adjacency-gradient workspace");
     if (rc) return rc;
     if (n == 0) return EGNN_OK;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1239,6 +1255,10 @@ int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const flo
     EGNN_LAUNCH_CHECK("adj_grad_degree_kernel launch");
     adj_grad_degree_kernel<<<blocks, 256, 0, st>>>(rowptr_t, colidx_t, vals_t_or_null, dinv, t, lam, n, f, k, fl, q);
     EGNN_LAUNCH_CHECK("adj_grad_degree_kernel launch");
+    if (d.n > 0) {
+        adj_grad_flip_terms_kernel<<<1, 32 * kFlipWarps, 0, st>>>(d, dinv, lam, t, n, f, k, fl, r, q);
+        EGNN_LAUNCH_CHECK("adj_grad_flip_terms_kernel launch");
+    }
     adj_grad_finish_kernel<<<grid_for(n, 256), 256, 0, st>>>(r, q, dinv, iso, xbar_or_null, rowsum_or_null, n,
                                                              op_scale, gw, grho);
     EGNN_LAUNCH_CHECK("adj_grad_finish_kernel launch");

@@ -14,6 +14,7 @@
 #pragma once
 
 #include "common.cuh"
+#include "prep.cuh"
 
 namespace egnn {
 
@@ -77,6 +78,39 @@ adj_grad_degree_kernel(const int32_t* __restrict__ rowptr, const int32_t* __rest
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
         if (lane == 0) out[row] = (double)dinv[row] * s;
+    }
+}
+
+// Edge flips A' = A + sum_p v_p e_{r_p} e_{c_p}^T (DESIGN.md section 14): the flips' part of the degree
+// terms, R[r_p] += v_p g_{r_p c_p} and Q[c_p] += v_p g_{r_p c_p} for every off-diagonal flip, on top of
+// the two adj_grad_degree_kernel launches over the stored CSR.  One CTA of kFlipWarps warps, one warp
+// per flip (flips p and p + kFlipWarps share a warp): g_p by stack_dot with the lane layout and
+// summation of adj_grad_pairs_kernel, then one thread folds the products into R and Q in flip-list
+// order (no atomics: several flips on one node are bitwise reproducible).
+constexpr int kFlipWarps = 32;
+
+__global__ void __launch_bounds__(32 * kFlipWarps)
+adj_grad_flip_terms_kernel(DeltaList d, const float* __restrict__ dinv, const float* __restrict__ lam,
+                           const float* __restrict__ t, int64_t n, int32_t F, int32_t K, int32_t fl_log2,
+                           double* __restrict__ r_out, double* __restrict__ q_out) {
+    __shared__ double g[EGNN_MAX_DELTA];
+    const int lane = threadIdx.x & 31;
+    const int FL = 1 << fl_log2;
+    for (int p = threadIdx.x >> 5; p < d.n; p += kFlipWarps) {
+        const int r = d.row[p], c = d.col[p];
+        double s = 0.0;
+        if (lane < FL) s = stack_dot(lam, t, (int64_t)r * F, (int64_t)c * F, n * (int64_t)F, F, K, lane, FL);
+        for (int o = FL >> 1; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (lane == 0) g[p] = (double)dinv[r] * (double)dinv[c] * s;
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    for (int q = 0; q < d.n; ++q) {
+        const int r = d.row[q], c = d.col[q];
+        if (r == c) continue;                                // a diagonal flip enters only rho
+        const double vg = (double)d.val[q] * g[q];
+        r_out[r] += vg;
+        q_out[c] += vg;
     }
 }
 

@@ -17,10 +17,12 @@ device every entry point raises ``EgnnError``.
 ``s``): when grad mode is on and an input requires grad, the pass runs inside
 an autograd function whose backward is the adjoint (Clenshaw) pass of
 ``egnn_cheb_adjoint``.  ``graph_wavelet_features`` is also differentiable w.r.t. a
-dense or sparse COO adjacency tensor and a 0-d tensor ``lambda_max`` (DESIGN.md
-section 11).  Otherwise nothing changes: same kernels, nothing saved.
-``WATS`` and ``WaveletSession`` stay forward-only; the sharded path's gradients w.r.t. the
-signal and ``s`` are ``ShardedWavelet``'s (DESIGN.md section 12).
+dense or sparse COO adjacency tensor, a 0-d tensor ``lambda_max`` (DESIGN.md
+section 11) and the values of edge flips ``deltas`` (section 14), with or
+without flips.  Otherwise nothing changes: same kernels, nothing saved.
+``WATS`` passes a wavelet gradient to the adjacency only with
+``adjacency_grad=True``; ``WaveletSession`` stays forward-only; the sharded
+path's gradients are ``ShardedWavelet``'s (DESIGN.md sections 12-13).
 """
 from __future__ import annotations
 
@@ -101,22 +103,28 @@ def _width(x: torch.Tensor) -> int:
 
 
 class _PassSpec:
-    """Everything of one pass but its differentiable inputs (the signal, the scales, the adjacency and
-    ``lambda_max``).  ``degree_vectors`` / ``y0``: patched for ``deltas`` (None: the graph's own);
-    ``default_signal``: the signal is the graph's log1p(degree) with the graph's vectors.  ``pattern``:
-    ``(rows, cols)`` int32 device tensors when the adjacency input is the value vector of a sparse COO
-    pattern (None: a dense ``[N, N]`` adjacency)."""
+    """Everything of one pass but its differentiable inputs (the signal, the scales, the adjacency,
+    ``lambda_max`` and the flips' values).  ``degree_vectors`` / ``y0``: patched for ``deltas`` (None: the
+    graph's own); ``default_signal``: the signal is the graph's log1p(degree) with the graph's vectors.
+    ``rowsum``: the flipped graph's row sums when the signal is its log1p(degree) (``deltas`` with the
+    default signal, differentiable passes only).  ``pattern``: ``(rows, cols)`` int32 device tensors when
+    the adjacency input is the value vector of a sparse COO pattern (None: a dense ``[N, N]`` adjacency)."""
 
     def __init__(self, graph, adjoint, k, coeffs, op_scale, op_shift, want_orders, route=_Route(), deltas=None,
-                 degree_vectors=None, default_signal=False, y0=None, lambda_max=None, pattern=None):
+                 degree_vectors=None, default_signal=False, y0=None, lambda_max=None, pattern=None, rowsum=None):
         self.graph, self.adjoint, self.k, self.coeffs = graph, adjoint, k, coeffs
         self.op_scale, self.op_shift, self.want_orders, self.route = op_scale, op_shift, want_orders, route
         self.deltas, self.degree_vectors = deltas, degree_vectors
         self.default_signal, self.y0 = default_signal, y0
-        self.lambda_max, self.pattern = lambda_max, pattern
+        self.lambda_max, self.pattern, self.rowsum = lambda_max, pattern, rowsum
 
     def vectors(self):          # the (dinv, iso) the pass runs with
         return (self.graph.dinv, self.graph.iso) if self.degree_vectors is None else self.degree_vectors
+
+    def signal_rowsum(self):    # the row sums whose log1p is the signal, None for a caller's signal
+        if self.rowsum is not None:
+            return self.rowsum
+        return self.graph.rowsum if self.default_signal else None
 
 
 def _run_cheb(spec: _PassSpec, x0: torch.Tensor, normalize: bool, want_orders: bool, order_events=None):
@@ -209,17 +217,19 @@ def _heat_scale_grad(coeffs: np.ndarray, G: torch.Tensor) -> torch.Tensor:
 class _WaveletPass(torch.autograd.Function):
     """``(C [N,S,F], T [K+1,N,F])`` of one un-normalised pass as a function of the signal ``x0``, the
     scales ``s``, the adjacency ``adj`` (dense float32 ``[N, N]`` on the graph's device, or the float32
-    values of ``spec.pattern``) and a 0-d ``lam`` = ``lambda_max`` (each None when it needs no
-    gradient).  ``T`` is empty unless the orders are wanted or ``s``, ``adj`` or ``lam`` needs a
-    gradient (their backward reads them).  Backward: the adjoint pass on the transposed graph,
-    ``ds_j = -sum_k k alpha[j,k] <Cbar_j, T_k>``, and for ``adj`` / ``lam`` the adjacency terms of
-    DESIGN.md section 11 from every Clenshaw vector (egnn_cheb_adjoint_all)."""
+    values of ``spec.pattern``), a 0-d ``lam`` = ``lambda_max`` and the values ``dv`` of the flips
+    ``spec.deltas`` (each None when it needs no gradient).  With flips, ``adj`` is the base ``A`` of
+    ``A' = A + delta`` and its gradient is ``dLoss/dA'``.  ``T`` is empty unless the orders are wanted or
+    ``s``, ``adj``, ``lam`` or ``dv`` needs a gradient (their backward reads them).  Backward: the adjoint
+    pass on the transposed graph, ``ds_j = -sum_k k alpha[j,k] <Cbar_j, T_k>``, and for ``adj`` / ``lam``
+    / ``dv`` the adjacency terms of DESIGN.md sections 11 and 14 from every Clenshaw vector
+    (egnn_cheb_adjoint_all)."""
 
     @staticmethod
-    def forward(ctx, x0, s, adj, lam, spec):
+    def forward(ctx, x0, s, adj, lam, dv, spec):
         ctx.set_materialize_grads(False)        # an output nobody differentiates arrives as None
         s_grad = s is not None and ctx.needs_input_grad[1]
-        structure = (adj is not None and ctx.needs_input_grad[2]) or (lam is not None and ctx.needs_input_grad[3])
+        structure = any(v is not None and ctx.needs_input_grad[i] for i, v in ((2, adj), (3, lam), (4, dv)))
         comb, t_all = _run_cheb(spec, x0, False, spec.want_orders or s_grad or structure)
         if t_all is None:
             t_all = comb.new_empty((0,))
@@ -227,6 +237,7 @@ class _WaveletPass(torch.autograd.Function):
         ctx.spec, ctx.x_shape = spec, x0.shape
         ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
         ctx.lam_meta = None if lam is None else (lam.shape, lam.device, lam.dtype)
+        ctx.dv_meta = None if dv is None else (dv.shape, dv.device, dv.dtype)
         ctx.save_for_backward(t_all if (s_grad or structure) else None)
         return comb, t_all
 
@@ -241,8 +252,8 @@ class _WaveletPass(torch.autograd.Function):
         cbar = (_cabi.vec_ready(g_comb) if g_comb is not None else
                 torch.zeros((g.n, n_scales, f), dtype=torch.float32, device=g.device))
         tbar = _cabi.vec_ready(g_orders) if (g_orders is not None and g_orders.numel()) else None
-        x_grad = s_grad = adj_grad = lam_grad = None
-        structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
+        x_grad = s_grad = adj_grad = lam_grad = dv_grad = None
+        structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3] or ctx.needs_input_grad[4]
         if ctx.needs_input_grad[0] or structure:
             xbar = _run_adjoint(spec, cbar, tbar, keep_all=structure)
             if structure:
@@ -252,47 +263,66 @@ class _WaveletPass(torch.autograd.Function):
         if ctx.needs_input_grad[1]:
             shape, dev, dtype = ctx.s_meta
             s_grad = _heat_scale_grad(spec.coeffs, _coeff_grad(cbar, t_all)).to(device=dev, dtype=dtype).reshape(shape)
-        if ctx.needs_input_grad[2]:
-            adj_grad = _adjacency_grad(spec, b_all, t_all)
+        if ctx.needs_input_grad[2] or ctx.needs_input_grad[4]:
+            adj_grad, dv_grad = _adjacency_grad(spec, b_all, t_all, adjacency=ctx.needs_input_grad[2],
+                                                flips=ctx.needs_input_grad[4])
         if ctx.needs_input_grad[3]:
             shape, dev, dtype = ctx.lam_meta
             lam_grad = _lambda_max_grad(b_all, t_all, spec.lambda_max).to(device=dev, dtype=dtype).reshape(shape)
-        return x_grad, s_grad, adj_grad, lam_grad, None
+        if dv_grad is not None:
+            shape, dev, dtype = ctx.dv_meta
+            dv_grad = dv_grad.to(device=dev, dtype=dtype).reshape(shape)
+        return x_grad, s_grad, adj_grad, lam_grad, dv_grad, None
 
 
-def _adjacency_grad(spec: _PassSpec, b_all: torch.Tensor, t_all: torch.Tensor) -> torch.Tensor:
-    """``dLoss/dA`` from the Clenshaw vectors ``b_all`` and the orders ``t_all``: the degree terms
-    (egnn_adj_grad_degree over the CSR and its transpose), then either the dense ``[N, N]`` gradient
-    (egnn_adj_grad_dense) or its values at ``spec.pattern`` (egnn_adj_grad_pairs)."""
+def _adjacency_grad(spec: _PassSpec, b_all: torch.Tensor, t_all: torch.Tensor, adjacency: bool = True,
+                    flips: bool = False):
+    """``(dLoss/dA', dLoss/dv)`` of ``A' = A + delta`` (``A`` alone without ``spec.deltas``) from the
+    Clenshaw vectors ``b_all`` and the orders ``t_all``: the degree terms (egnn_adj_grad_degree_flips over
+    the CSR, its transpose and the flips, with the degree vectors and row sums of ``A'``), then
+    (``adjacency``) either the dense ``[N, N]`` gradient (egnn_adj_grad_dense) or its values at
+    ``spec.pattern``, and (``flips``) its values at the flips (egnn_adj_grad_pairs); None where not
+    asked for."""
     lib = _cabi.load()
     g, k = spec.graph, spec.k
     gt = spec.adjoint()
     n, f = g.n, int(b_all.shape[2])
     lam, t = b_all[1:], t_all[:k]                    # b_1..b_K and T_0..T_{K-1}: [K, N, F] stacks
-    signal = spec.default_signal and f == 1
+    dinv, iso = spec.vectors()
+    rowsum = spec.signal_rowsum() if f == 1 else None
+    adj_out = flip_out = None
     with torch.cuda.device(g.device):
         gw = torch.empty(n, dtype=torch.float32, device=g.device)
         grho = torch.empty(n, dtype=torch.float32, device=g.device)
         ws_bytes = int(lib.egnn_adj_grad_degree_ws_bytes(n))
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=g.device)
-        _cabi.check(lib.egnn_adj_grad_degree(
+        _cabi.check(lib.egnn_adj_grad_degree_flips(
             _cabi.ptr(g.rowptr), _cabi.ptr(g.colidx), _cabi.ptr(g.vals), _cabi.ptr(gt.rowptr), _cabi.ptr(gt.colidx),
-            _cabi.ptr(gt.vals), _cabi.ptr(g.dinv), _cabi.ptr(g.iso), n, g.nnz, f, k, float(spec.op_scale),
-            _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(b_all[0]) if signal else None,
-            _cabi.ptr(g.rowsum) if signal else None, _cabi.ptr(gw), _cabi.ptr(grho), _cabi.ptr(ws), ws_bytes,
-            _stream()), "egnn_adj_grad_degree")
-        if spec.pattern is None:
-            out = torch.empty((n, n), dtype=torch.float32, device=g.device)
-            _cabi.check(lib.egnn_adj_grad_dense(_cabi.ptr(g.dinv), _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(gw),
-                                                _cabi.ptr(grho), n, f, k, float(spec.op_scale), _cabi.ptr(out), n,
-                                                _stream()), "egnn_adj_grad_dense")
+            _cabi.ptr(gt.vals), _cabi.ptr(dinv), _cabi.ptr(iso), n, g.nnz, f, k, float(spec.op_scale),
+            _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(b_all[0]) if rowsum is not None else None, _cabi.ptr(rowsum),
+            *_cabi.delta_args(spec.deltas), _cabi.ptr(gw), _cabi.ptr(grho), _cabi.ptr(ws), ws_bytes,
+            _stream()), "egnn_adj_grad_degree_flips")
+
+        def pairs(rows, cols):
+            out = torch.empty(rows.numel(), dtype=torch.float32, device=g.device)
+            _cabi.check(lib.egnn_adj_grad_pairs(_cabi.ptr(rows), _cabi.ptr(cols), rows.numel(), _cabi.ptr(dinv),
+                                                _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(gw), _cabi.ptr(grho), n, f,
+                                                k, float(spec.op_scale), _cabi.ptr(out), _stream()),
+                        "egnn_adj_grad_pairs")
             return out
-        rows, cols = spec.pattern
-        out = torch.empty(rows.numel(), dtype=torch.float32, device=g.device)
-        _cabi.check(lib.egnn_adj_grad_pairs(_cabi.ptr(rows), _cabi.ptr(cols), rows.numel(), _cabi.ptr(g.dinv),
-                                            _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(gw), _cabi.ptr(grho), n, f, k,
-                                            float(spec.op_scale), _cabi.ptr(out), _stream()), "egnn_adj_grad_pairs")
-    return out
+
+        if adjacency and spec.pattern is None:
+            adj_out = torch.empty((n, n), dtype=torch.float32, device=g.device)
+            _cabi.check(lib.egnn_adj_grad_dense(_cabi.ptr(dinv), _cabi.ptr(lam), _cabi.ptr(t), _cabi.ptr(gw),
+                                                _cabi.ptr(grho), n, f, k, float(spec.op_scale), _cabi.ptr(adj_out), n,
+                                                _stream()), "egnn_adj_grad_dense")
+        elif adjacency:
+            adj_out = pairs(*spec.pattern)
+        if flips:
+            d_rows, d_cols, _ = spec.deltas
+            flip_out = pairs(torch.tensor([int(r) for r in d_rows], dtype=torch.int32).to(g.device),
+                             torch.tensor([int(c) for c in d_cols], dtype=torch.int32).to(g.device))
+    return adj_out, flip_out
 
 
 def _lambda_max_grad(b_all: torch.Tensor, t_all: torch.Tensor, lambda_max: float) -> torch.Tensor:
@@ -334,28 +364,28 @@ class _L1Normalize(torch.autograd.Function):
         return cbar
 
 
-def _needs_grad(x0, s=None, adj=None, lam=None) -> bool:
-    """The autograd path engages only in grad mode with an input that requires grad (``adj`` / ``lam``:
-    the structure inputs of :func:`_structure_input`, None unless they do)."""
-    return adj is not None or lam is not None or \
+def _needs_grad(x0, s=None, adj=None, lam=None, dv=None) -> bool:
+    """The autograd path engages only in grad mode with an input that requires grad (``adj`` / ``lam`` /
+    ``dv``: the structure inputs of :func:`_structure_input`, None unless they do)."""
+    return adj is not None or lam is not None or dv is not None or \
         (torch.is_grad_enabled() and (x0.requires_grad or (isinstance(s, torch.Tensor) and s.requires_grad)))
 
 
 def _cheb_pass(spec: _PassSpec, x0: torch.Tensor, s=None, adj=None, lam=None, normalize=False,
-               order_events=None) -> WaveletResult:
+               order_events=None, dv=None) -> WaveletResult:
     """One pass of any public caller: through :class:`_WaveletPass` when an input needs a gradient
     (:func:`_needs_grad`), else straight through :func:`_run_cheb`.  ``features`` is ``[N, S*F]``;
     ``orders`` and ``combined`` are filled when ``spec.want_orders``.  Normalisation: out of place by
     :class:`_L1Normalize` when differentiable, by a torch expression when the orders are kept, else
     fused into the last order's kernel."""
-    if _needs_grad(x0, s, adj, lam):
+    if _needs_grad(x0, s, adj, lam, dv):
         # the device / dtype conversions stay outside the function, so autograd routes the gradient
         # back to a CPU or float64 leaf
         x0 = x0.to(device=spec.graph.device, dtype=torch.float32)
         if adj is not None:
             adj = adj.to(device=spec.graph.device, dtype=torch.float32)
         s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
-        comb, t_all = _WaveletPass.apply(x0, s_in, adj, lam, spec)
+        comb, t_all = _WaveletPass.apply(x0, s_in, adj, lam, dv, spec)
         feats = _L1Normalize.apply(comb) if normalize else comb
     elif spec.want_orders:
         comb, t_all = _run_cheb(spec, x0, False, True)
@@ -368,18 +398,37 @@ def _cheb_pass(spec: _PassSpec, x0: torch.Tensor, s=None, adj=None, lam=None, no
 
 
 def _structure_input(adj_matrix, lambda_max, deltas):
-    """The adjacency and ``lambda_max`` inputs that need a gradient: ``(adj, lam)``, each None when not.
-    Only a dense strided ``[N, N]`` tensor and a sparse COO tensor take part, only a 0-d tensor
-    ``lambda_max``, and never with ``deltas``."""
-    if not torch.is_grad_enabled() or deltas is not None:
-        return None, None
+    """The adjacency, ``lambda_max`` and flip-value inputs that need a gradient: ``(adj, lam, dv)``, each
+    None when not.  Only a dense strided ``[N, N]`` tensor and a sparse COO tensor take part, only a 0-d
+    tensor ``lambda_max``, and only a 1-d float tensor ``deltas[2]`` with one value per flip."""
+    if not torch.is_grad_enabled():
+        return None, None, None
     adj = None
     if isinstance(adj_matrix, torch.Tensor) and adj_matrix.requires_grad and adj_matrix.dim() == 2 and \
             adj_matrix.layout in (torch.strided, torch.sparse_coo):
         adj = adj_matrix
     lam = lambda_max if isinstance(lambda_max, torch.Tensor) and lambda_max.requires_grad and lambda_max.dim() == 0 \
         else None
-    return adj, lam
+    dv = None
+    if deltas is not None and isinstance(deltas[2], torch.Tensor) and deltas[2].requires_grad:
+        dv = deltas[2]
+        if dv.dim() != 1 or dv.numel() != len(deltas[0]) or len(deltas[1]) != len(deltas[0]):
+            raise ValueError(f"deltas: {len(deltas[0])} rows, {len(deltas[1])} cols and values of shape "
+                             f"{tuple(dv.shape)}; want one value per flip")
+    return adj, lam, dv
+
+
+def _flipped_rowsum(graph: CsrGraph, deltas) -> torch.Tensor:
+    """Row sums of the graph with ``deltas`` applied, rounded as egnn_patch_nodes forms them for the
+    signal ``log1p(rowsum)``: each touched row's base sum plus the float32 sum of its flips in list order."""
+    add = {}
+    for r, v in zip(deltas[0], deltas[2]):
+        add[int(r)] = np.float32(add.get(int(r), np.float32(0.0)) + np.float32(v))
+    rowsum = graph.rowsum.clone()
+    if add:
+        idx = torch.tensor(list(add), dtype=torch.long).to(graph.device)
+        rowsum[idx] = rowsum[idx] + torch.tensor(list(add.values()), dtype=torch.float32).to(graph.device)
+    return rowsum
 
 
 class LaplacianOperator:
@@ -553,27 +602,34 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
     then carries a ``grad_fn``; ``deltas=`` is supported.  The forward then keeps
     the un-normalised combination and normalises out of place.
 
-    Also differentiable w.r.t. the adjacency and ``lambda_max`` (DESIGN.md
-    section 11) in grad mode, without ``deltas``, when one of these requires grad:
+    Also differentiable w.r.t. the adjacency, ``lambda_max`` and the flips'
+    values (DESIGN.md sections 11 and 14) in grad mode, when one of these
+    requires grad.  With ``deltas`` the pass runs on ``A' = A + delta`` (flips
+    add to ``A``; an entry may repeat, cancel a stored entry or sit on the
+    diagonal) and every gradient below is taken at ``A'``:
 
     * ``adj_matrix`` a dense strided ``[N, N]`` tensor (CPU or GPU, any float
-      dtype): its gradient is the full dense ``dLoss/dA``, diagonal and
+      dtype): its gradient is the full dense ``dLoss/dA'``, diagonal and
       unstored entries included;
     * ``adj_matrix`` a sparse COO tensor (e.g. ``torch.sparse_coo_tensor(
       edge_index, w, (N, N))`` with a leaf ``w``): the gradient at the stored
       pattern, which reaches ``w`` through torch's constructor and
       ``coalesce()`` (duplicates share their entry's gradient; explicit zeros,
       dropped from the graph, still get the gradient at their position);
-    * ``lambda_max`` a 0-d tensor.
+    * ``lambda_max`` a 0-d tensor;
+    * ``deltas=(rows, cols, vals)`` with ``vals`` a 1-d float tensor:
+      ``vals.grad[p] = dLoss/dA'`` at ``(rows[p], cols[p])`` (repeated entries
+      each get the entry's value), on any adjacency format, a ``CsrGraph``
+      included.
 
     An isolated node (zero column sum off the diagonal) has its normaliser held
     at 1: ``w^-1/2`` has no derivative at ``w = 0``.  That holds for every entry
     of its column: the unstored entries of a dense gradient, and explicit zeros
-    of a COO pattern (a column of explicit zeros only is isolated).  Every other adjacency
-    format (sparse CSR tensors, scipy matrices, ``CsrGraph``, ``(edge_index,
-    N)``) and every call with ``deltas`` stays forward-only in the adjacency.
+    of a COO pattern (a column of explicit zeros only is isolated).  Every other
+    adjacency format (sparse CSR tensors, scipy matrices, ``CsrGraph``,
+    ``(edge_index, N)``) stays forward-only in the adjacency itself.
     """
-    adj_in, lam_in = _structure_input(adj_matrix, lambda_max, deltas)
+    adj_in, lam_in, dv_in = _structure_input(adj_matrix, lambda_max, deltas)
     graph = as_graph(adj_matrix if adj_in is None else adj_matrix.detach())
     pattern = None
     if adj_in is not None and adj_in.layout == torch.sparse_coo:
@@ -585,19 +641,32 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
         adj_in = adj_in.values()
     elif adj_in is not None and tuple(adj_in.shape) != (graph.n, graph.n):
         raise ValueError(f"adjacency must be [N, N], got {tuple(adj_in.shape)}")
+    return _graph_features(graph, k, s, X0, lambda_max, normalize, return_parts, deltas, adj_in, pattern, lam_in,
+                           dv_in, _order_events, _use_sell)
+
+
+def _graph_features(graph: CsrGraph, k, s, X0, lambda_max, normalize, return_parts, deltas, adj_in=None,
+                    pattern=None, lam_in=None, dv_in=None, order_events=None, use_sell=None):
+    """:func:`graph_wavelet_features` on a resolved ``graph`` (with ``deltas`` on top) and its structure
+    inputs ``adj_in`` (a dense ``[N, N]`` tensor, or the values of ``pattern``), ``lam_in`` and ``dv_in``
+    (the flips' values), each None when it needs no gradient.  ``adj_in``'s gradient is ``dLoss/dA'`` of
+    the flipped graph: ``WATS.features_for`` hands in a leaf that IS the flipped graph, with the resident
+    graph and the flips that lead to it."""
     k = int(k)
     s_vals = s.detach().cpu().numpy() if isinstance(s, torch.Tensor) else s
     coeffs = heat_coefficients(k, s_vals)
     x0 = graph.x0 if X0 is None else torch.as_tensor(X0)
     if deltas is not None and len(deltas[0]) == 0:
-        deltas = None
-    grad = _needs_grad(x0, s, adj_in, lam_in)
-    route = _resolve_route(graph, _width(x0), k, _use_sell, grad, deltas is not None, X0 is None)
+        deltas = dv_in = None
+    if dv_in is not None:        # host values for the C ABI and the degree patches, read once
+        deltas = (deltas[0], deltas[1], dv_in.detach().cpu().tolist())
+    grad = _needs_grad(x0, s, adj_in, lam_in, dv_in)
+    route = _resolve_route(graph, _width(x0), k, use_sell, grad, deltas is not None, X0 is None)
     # on the SELL plan the step kernel re-derives the nodes the flips touch from the base vectors (one launch);
     # every other route gets the degree vectors of the flipped graph: only the touched entries of persistent
     # scratch copies are written, and put back once the pass is queued (no copies of the N-vectors per perturbation)
     patched = deltas is not None and not route.in_kernel
-    degree_vectors = y0 = None
+    degree_vectors = y0 = rowsum = None
     if patched:
         dinv, iso, x0_patched, y0_patched = graph.patch_nodes(deltas)
         degree_vectors = (dinv, iso)
@@ -607,9 +676,11 @@ def graph_wavelet_features(adj_matrix, k=3, s=0.8, *, X0=None, lambda_max: float
     try:
         if grad and patched:       # the scratch vectors are restored below, the backward runs later
             degree_vectors = tuple(v.clone() for v in degree_vectors)
+            if X0 is None and (adj_in is not None or dv_in is not None):
+                rowsum = _flipped_rowsum(graph, deltas)
         spec = _PassSpec(graph, graph.adjoint, k, coeffs, 2.0 / lam_max, -1.0, return_parts, route, deltas,
-                         degree_vectors, X0 is None and not patched, y0, lam_max, pattern)
-        res = _cheb_pass(spec, x0, s, adj_in, lam_in, normalize, _order_events)
+                         degree_vectors, X0 is None and not patched, y0, lam_max, pattern, rowsum)
+        res = _cheb_pass(spec, x0, s, adj_in, lam_in, normalize, order_events, dv_in)
         return res if return_parts else res.features
     finally:
         if patched:
@@ -643,13 +714,22 @@ class WATS(nn.Module):
     keep the reference's torch ops).
     ``_features_override`` exists for parity tests only: it injects a feature
     matrix computed elsewhere so two instances differ in nothing else.
-    The wavelet features are an input here, computed without gradients
-    (forward-only, as in the reference).
+    By default the wavelet features are an input here, computed without
+    gradients (forward-only, as in the reference).  ``adjacency_grad=True``
+    (with ``recompute_on_forward``) makes them a function of the adjacency
+    passed to ``forward``: a dense tensor that requires grad (the attack's
+    ``modified_adj`` leaf) receives the wavelet term of ``dLoss/dA`` on top of
+    the base model's.  Up to 64 entries that differ from the calibrator's own
+    adjacency run as edge flips on the resident graph (DESIGN.md section 14);
+    more run on a graph rebuilt from the tensor.  Each scale's one-column
+    feature is normalised on its own to about ``sign(S)``, so that term is
+    negligible next to a base model's, with one scale or several.
     """
 
     def __init__(self, base_model, features, labels, adj, val_mask, *, k: int = 3, s=0.8,
                  lambda_max: float = 2.0, recompute_on_forward: bool = False, train: bool = True,
-                 verbose: bool = True, fused_head: bool = True, _features_override=None):
+                 verbose: bool = True, fused_head: bool = True, adjacency_grad: bool = False,
+                 _features_override=None):
         super().__init__()
         self.device = torch.device('cuda' if torch.cuda.is_available() else 'cpu')
         if _features_override is None:
@@ -661,6 +741,7 @@ class WATS(nn.Module):
         self.val_idx = val_mask.to(self.device)
         self.k, self.s, self.lambda_max = int(k), s, float(lambda_max)
         self.recompute_on_forward = bool(recompute_on_forward)
+        self.adjacency_grad = bool(adjacency_grad)
         self.verbose = bool(verbose)
         self.fused_head = bool(fused_head)
 
@@ -684,25 +765,31 @@ class WATS(nn.Module):
     def features_for(self, adj=None, *, deltas=None):
         """Wavelet features of a perturbed graph: either a full adjacency
         (re-converted on the device) or edge flips on top of the base graph
-        (``deltas=(rows, cols, vals)``; no CSR rebuild)."""
+        (``deltas=(rows, cols, vals)``; no CSR rebuild).  With ``adjacency_grad``
+        a dense ``adj`` that requires grad receives ``dLoss/dA``."""
         if deltas is not None:
             return graph_wavelet_features(self.graph, k=self.k, s=self.s, lambda_max=self.lambda_max,
                                           deltas=deltas)
         if adj is None:
             return self.wavelet_feats
+        leaf = isinstance(adj, torch.Tensor) and self.adjacency_grad and adj.requires_grad and torch.is_grad_enabled()
         # a dense adjacency that differs from the calibrator's own in a few entries (what the attack
         # passes: calib_fga.py:897-908): take the flips and keep the resident graph and its plan
         if isinstance(adj, torch.Tensor) and adj.layout == torch.strided and self.graph is not None \
                 and isinstance(self.adj, torch.Tensor) and adj.shape == self.adj.shape:
-            flips = deltas_from_dense(self.adj, adj.to(self.adj.device))
+            flips = deltas_from_dense(self.adj, adj.detach().to(self.adj.device))
+            if flips is not None and leaf:
+                # the leaf is the flipped graph itself: its gradient is dLoss/dA' of the flipped pass
+                return _graph_features(self.graph, self.k, self.s, None, self.lambda_max, True, False, flips,
+                                       adj_in=adj)
             if flips is not None:
                 if not flips[0]:
                     return self.wavelet_feats
                 return graph_wavelet_features(self.graph, k=self.k, s=self.s, lambda_max=self.lambda_max,
                                               deltas=flips)
-        # the calibrator's features are an input, not a function of the adjacency: a leaf that requires
-        # grad (the attack's modified_adj) gets no wavelet gradient here, whatever the number of flips
-        if isinstance(adj, torch.Tensor):
+        # by default the calibrator's features are an input, not a function of the adjacency: a leaf that
+        # requires grad (the attack's modified_adj) gets no wavelet gradient, whatever the number of flips
+        if isinstance(adj, torch.Tensor) and not leaf:
             adj = adj.detach()
         return graph_wavelet_features(adj, k=self.k, s=self.s, lambda_max=self.lambda_max)
 

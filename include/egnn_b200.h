@@ -321,6 +321,25 @@ int egnn_adj_grad_degree(const int32_t* rowptr, const int32_t* colidx, const flo
                          int32_t k, float op_scale, const float* lam, const float* t,
                          const float* xbar_or_null, const float* rowsum_or_null, float* gw, float* grho,
                          void* workspace, size_t workspace_bytes, egnn_stream_t stream);
+
+/* egnn_adj_grad_degree of a perturbed graph A' = A + sum_p v_p e_r e_c^T (new
+ * in ABI 12; egnn_adj_grad_degree is this call without flips).  The CSR (and
+ * its transpose) hold A; the flips (host arrays, n_delta <= EGNN_MAX_DELTA,
+ * indices in [0, n), repeats allowed) add their terms to R and Q:
+ *   R_r += v_p g_rc,  Q_c += v_p g_rc   for every flip p = (r, c, v) with r != c
+ * (a diagonal flip enters only the row sums), folded in flip-list order.  dinv,
+ * iso and rowsum_or_null must be those of A' (egnn_patch_nodes, plus the
+ * flips' row sums), as in the perturbed forward.  dLoss/dA'_rc of the flips
+ * themselves: egnn_adj_grad_pairs on the flip list with these gw and grho.
+ * A refused flip list launches nothing.                                      */
+int egnn_adj_grad_degree_flips(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                               const int32_t* rowptr_t, const int32_t* colidx_t, const float* vals_t_or_null,
+                               const float* dinv, const uint8_t* iso, int64_t n, int64_t nnz, int32_t f,
+                               int32_t k, float op_scale, const float* lam, const float* t,
+                               const float* xbar_or_null, const float* rowsum_or_null,
+                               const int32_t* delta_row_host, const int32_t* delta_col_host,
+                               const float* delta_val_host, int32_t n_delta, float* gw, float* grho,
+                               void* workspace, size_t workspace_bytes, egnn_stream_t stream);
 int egnn_adj_grad_pairs(const int32_t* rows, const int32_t* cols, int64_t n_pairs, const float* dinv,
                         const float* lam, const float* t, const float* gw, const float* grho,
                         int64_t n, int32_t f, int32_t k, float op_scale, float* out, egnn_stream_t stream);
