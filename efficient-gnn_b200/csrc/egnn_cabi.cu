@@ -502,7 +502,7 @@ using namespace egnn;
 
 extern "C" {
 
-int egnn_abi_version(void) { return 12; }
+int egnn_abi_version(void) { return 13; }
 
 const char* egnn_last_error(void) { return last_error_buf(); }
 
@@ -1976,6 +1976,29 @@ int egnn_adj_grad_degree_sharded(const int32_t* rowptr, const int32_t* colidx, c
                                  const float* pt_full, const float* xbar_local_or_null,
                                  const float* rowsum_local_or_null, float* g_out, float* gw_local, float* grho_local,
                                  void* workspace, size_t workspace_bytes, egnn_stream_t stream) {
+    return egnn_adj_grad_degree_sharded_flips(rowptr, colidx, vals_or_null, row_order_or_null, rowptr_t, colidx_t,
+                                              vals_t_or_null, row_order_t_or_null, dinv_full, iso_full, n_global,
+                                              row_begin, row_end, f, k, op_scale, pl_full, pt_full,
+                                              xbar_local_or_null, rowsum_local_or_null, nullptr, nullptr, nullptr, 0,
+                                              nullptr, g_out, gw_local, grho_local, workspace, workspace_bytes,
+                                              stream);
+}
+
+int egnn_adj_grad_degree_sharded_flips(const int32_t* rowptr, const int32_t* colidx, const float* vals_or_null,
+                                       const int32_t* row_order_or_null, const int32_t* rowptr_t,
+                                       const int32_t* colidx_t, const float* vals_t_or_null,
+                                       const int32_t* row_order_t_or_null, const float* dinv_full,
+                                       const uint8_t* iso_full, int64_t n_global, int64_t row_begin, int64_t row_end,
+                                       int32_t f, int32_t k, float op_scale, const float* pl_full,
+                                       const float* pt_full, const float* xbar_local_or_null,
+                                       const float* rowsum_local_or_null, const int32_t* delta_row_host,
+                                       const int32_t* delta_col_host, const float* delta_val_host, int32_t n_delta,
+                                       float* g_flips_out, float* g_out, float* gw_local, float* grho_local,
+                                       void* workspace, size_t workspace_bytes, egnn_stream_t stream) {
+    DeltaList d;
+    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n_global);
+    if (rc) return rc;
+    EGNN_REQUIRE(d.n == 0 || g_flips_out, "null g_flips_out");
     EGNN_REQUIRE(rowptr && rowptr_t && dinv_full && iso_full && g_out && gw_local && grho_local, "null pointer");
     EGNN_REQUIRE(n_global >= 0 && n_global < (int64_t(1) << 31) && row_begin >= 0 && row_end >= row_begin &&
                  row_end <= n_global, "bad row range");
@@ -1988,16 +2011,20 @@ int egnn_adj_grad_degree_sharded(const int32_t* rowptr, const int32_t* colidx, c
     EGNN_REQUIRE(vec_aligned(pl_full, (int32_t)(kf % 4 == 0 ? 4 : 1)) && vec_aligned(pt_full, (int32_t)(kf % 4 == 0 ? 4 : 1)),
                  "the lambda / T stacks must be 16-byte aligned when k * f % 4 == 0");
     const int64_t rows = row_end - row_begin;
-    int rc = require_workspace(workspace, workspace_bytes, egnn_adj_grad_degree_sharded_ws_bytes(rows),
-                               "adjacency-gradient workspace");
+    rc = require_workspace(workspace, workspace_bytes, egnn_adj_grad_degree_sharded_ws_bytes(rows),
+                           "adjacency-gradient workspace");
     if (rc) return rc;
-    if (rows == 0) return EGNN_OK;
+    if (rows == 0) return EGNN_OK;    // a rank without rows: no term of its own (its flip values are all 0)
     cudaStream_t st = (cudaStream_t)stream;
     double* r = (double*)align_up((size_t)workspace, 256);
     double* q = (double*)((char*)r + align_up(sizeof(double) * (size_t)rows, 256));
     if (k == 0) {                     // no operator in the pass: g = 0, R = Q = 0, only grho
         rc = check_cuda(cudaMemsetAsync(r, 0, 2 * align_up(sizeof(double) * (size_t)rows, 256), st), "memset R, Q");
         if (rc) return rc;
+        if (d.n > 0) {
+            rc = check_cuda(cudaMemsetAsync(g_flips_out, 0, sizeof(float) * (size_t)d.n, st), "memset g_flips");
+            if (rc) return rc;
+        }
     } else {
         rc = launch_shard_dot(rowptr, colidx, vals_or_null, row_order_or_null, pl_full, pt_full, rows, row_begin,
                               (int32_t)kf, r, g_out, st);
@@ -2005,6 +2032,19 @@ int egnn_adj_grad_degree_sharded(const int32_t* rowptr, const int32_t* colidx, c
         rc = launch_shard_dot(rowptr_t, colidx_t, vals_t_or_null, row_order_t_or_null, pt_full, pl_full, rows,
                               row_begin, (int32_t)kf, q, nullptr, st);
         if (rc) return rc;
+        if (d.n > 0) {
+            const int vec = kf % 4 == 0 ? 4 : 1;
+            const int fl = shard_fl_log2(kf, vec);
+            if (vec == 4)
+                shard_grad_flip_terms_kernel<4><<<1, 32 * kShardFlipWarps, 0, st>>>(d, pl_full, pt_full, rows,
+                                                                                     row_begin, (int32_t)kf, fl,
+                                                                                     g_flips_out, r, q);
+            else
+                shard_grad_flip_terms_kernel<1><<<1, 32 * kShardFlipWarps, 0, st>>>(d, pl_full, pt_full, rows,
+                                                                                     row_begin, (int32_t)kf, fl,
+                                                                                     g_flips_out, r, q);
+            EGNN_LAUNCH_CHECK("shard_grad_flip_terms_kernel launch");
+        }
     }
     adj_grad_finish_kernel<<<grid_for(rows, 256), 256, 0, st>>>(r, q, dinv_full + row_begin, iso_full + row_begin,
                                                                 xbar_local_or_null, rowsum_local_or_null, rows,
@@ -2026,6 +2066,23 @@ int egnn_adj_grad_entries_sharded(const int32_t* rowptr, const int32_t* colidx, 
     shard_grad_entries_kernel<<<grid_for(rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(
         rowptr, colidx, k == 0 ? nullptr : g, gw_full, grho_local, rows, row_begin, op_scale, out);
     EGNN_LAUNCH_CHECK("shard_grad_entries_kernel launch");
+    return EGNN_OK;
+}
+
+int egnn_adj_grad_flips_sharded(const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                const float* delta_val_host, int32_t n_delta, const float* g_flips,
+                                const float* gw_full, const float* grho_local, int64_t n_global, int64_t row_begin,
+                                int64_t row_end, float op_scale, float* out, egnn_stream_t stream) {
+    EGNN_REQUIRE(n_global >= 0 && n_global < (int64_t(1) << 31) && row_begin >= 0 && row_end >= row_begin &&
+                 row_end <= n_global, "bad row range");
+    DeltaList d;
+    int rc = fill_delta(d, delta_row_host, delta_col_host, delta_val_host, n_delta, n_global);
+    if (rc) return rc;
+    if (d.n == 0) return EGNN_OK;
+    EGNN_REQUIRE(g_flips && gw_full && grho_local && out, "null pointer");
+    shard_grad_flip_values_kernel<<<1, EGNN_MAX_DELTA, 0, (cudaStream_t)stream>>>(
+        d, g_flips, gw_full, grho_local, row_end - row_begin, row_begin, op_scale, out);
+    EGNN_LAUNCH_CHECK("shard_grad_flip_values_kernel launch");
     return EGNN_OK;
 }
 

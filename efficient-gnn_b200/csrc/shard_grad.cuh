@@ -8,10 +8,13 @@
 // of length K*F (no per-product index arithmetic), read with 16-byte loads when K*F % 4 == 0.
 //   R_i = sum_{j != i} A_ij <PL[i], PT[j]>      over the rank's rows of A (g_ij kept per entry)
 //   Q_i = sum_{j != i} A^T_ij <PT[i], PL[j]>    over the rank's rows of A^T
+// With edge flips (section 15) the stacks are built on the flipped graph's d, and the flips add their
+// part of R / Q and get their own gradient (shard_grad_flip_terms_kernel, shard_grad_flip_values_kernel).
 // Every sum runs in a fixed order (float32 chunks, float64 carry, no atomics): bitwise reproducible.
 #pragma once
 
 #include "common.cuh"
+#include "prep.cuh"
 
 namespace egnn {
 
@@ -146,6 +149,75 @@ shard_grad_entries_kernel(const int32_t* __restrict__ rowptr, const int32_t* __r
             __stcs(out + q, v);
         }
     }
+}
+
+// Edge flips A' = A + sum_p v_p e_{r_p} e_{c_p}^T on a row shard (DESIGN.md section 15).  g_p =
+// <PL[r_p], PT[c_p]> of every flip from the all-gathered stacks, with the lane layout and summation of
+// shard_grad_dot_kernel (so a flip on a stored entry gets that entry's g bit for bit, and every rank the
+// same g_p), written to g_out [n_delta]; then R[r_p] += v_p g_p on the rank that owns row r_p and
+// Q[c_p] += v_p g_p on the rank that owns row c_p, for every off-diagonal flip, on top of the two
+// shard_grad_dot_kernel launches.  One CTA of kShardFlipWarps warps, one warp per flip; one thread folds
+// the products in flip-list order (no atomics: several flips on one node are bitwise reproducible).
+constexpr int kShardFlipWarps = 32;
+
+template <int VEC>
+__global__ void __launch_bounds__(32 * kShardFlipWarps)
+shard_grad_flip_terms_kernel(DeltaList d, const float* __restrict__ pl, const float* __restrict__ pt, int64_t rows,
+                             int64_t row0, int32_t KF, int32_t fl_log2, float* __restrict__ g_out,
+                             double* __restrict__ r_out, double* __restrict__ q_out) {
+    using V = ShardVec<VEC>;
+    __shared__ double g[EGNN_MAX_DELTA];
+    const int lane = threadIdx.x & 31;
+    const int FL = 1 << fl_log2;
+    const int nvec = KF / VEC;
+    for (int p = threadIdx.x >> 5; p < d.n; p += kShardFlipWarps) {
+        const float* orow = pl + (int64_t)d.row[p] * KF;
+        const float* grow = pt + (int64_t)d.col[p] * KF;
+        double hi = 0.0;
+        if (lane < FL) {
+            float acc = 0.f;
+            int cnt = 0;
+            for (int c = lane; c < nvec; c += FL) {
+                acc = V::dot(V::load(orow + (int64_t)c * VEC), V::load(grow + (int64_t)c * VEC), acc);
+                cnt += VEC;
+                if (cnt >= kShardGradChunk) { hi += (double)acc; acc = 0.f; cnt = 0; }
+            }
+            hi += (double)acc;
+        }
+        for (int m = FL >> 1; m > 0; m >>= 1) hi += __shfl_xor_sync(0xffffffffu, hi, m);
+        if (lane == 0) {
+            g[p] = hi;
+            g_out[p] = (float)hi;
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    for (int p = 0; p < d.n; ++p) {
+        const int64_t r = d.row[p] - row0, c = d.col[p] - row0;
+        if (r == c) continue;                                // a diagonal flip enters only rho
+        const double vg = (double)d.val[p] * g[p];
+        if (r >= 0 && r < rows) r_out[r] += vg;
+        if (c >= 0 && c < rows) q_out[c] += vg;
+    }
+}
+
+// dLoss/dv_p of the flips whose row this rank owns, out[p] = grho_{r_p} + [r_p != c_p] ((float)(-a g_p) +
+// gw_full[c_p]) (the arithmetic of shard_grad_entries_kernel), and 0 for every other flip: the caller
+// adds the ranks' rows, so the owner's value reaches every rank unchanged.  One thread per flip.
+__global__ void __launch_bounds__(EGNN_MAX_DELTA)
+shard_grad_flip_values_kernel(DeltaList d, const float* __restrict__ g, const float* __restrict__ gw_full,
+                              const float* __restrict__ grho, int64_t rows, int64_t row0, float a,
+                              float* __restrict__ out) {
+    const int p = threadIdx.x;
+    if (p >= d.n) return;
+    const int64_t r = d.row[p] - row0;
+    const int c = d.col[p];
+    float v = 0.f;
+    if (r >= 0 && r < rows) {
+        v = grho[r];
+        if (r + row0 != c) v += (float)(-(double)a * (double)g[p]) + gw_full[c];
+    }
+    out[p] = v;
 }
 
 }  // namespace egnn

@@ -35,7 +35,7 @@ import torch.distributed as dist
 from torch.autograd.function import once_differentiable
 
 from . import _cabi
-from .wats import WIDE_MIN_F, _heat_scale_grad, _needs_grad, heat_coefficients
+from .wats import WIDE_MIN_F, _heat_scale_grad, _needs_grad, _structure_input, heat_coefficients
 
 _COEFF_GRAD_MAX_ROWS = 8            # EGNN_MAX_SCALES: rows of cbar one egnn_cheb_coeff_grad takes
 
@@ -376,6 +376,36 @@ class CudaEngine:
             "egnn_adj_grad_degree_sharded")
         return g[:ci_.numel()], gw[:rows], grho[:rows]
 
+    def adj_grad_degree_flips(self, shard, shard_t, row_orders, dinv, iso, n_global, row_begin, row_end, f, k,
+                              op_scale, pl_full, pt_full, xbar, rowsum, deltas):
+        """:meth:`adj_grad_degree` of the flipped graph ``A + delta`` (``dinv`` / ``iso`` / stacks / ``rowsum``
+        of ``A'``; egnn_adj_grad_degree_sharded_flips): ``(g, gw, grho, g_flips [n_delta])``, the flips'
+        ``g_p`` on every rank and their part of the own rows' degree terms."""
+        rows = row_end - row_begin
+        (rp_, ci_, v_), (rpt, cit, vt) = shard, shard_t
+        g = torch.empty(max(1, int(ci_.numel())), dtype=torch.float32, device=self.device)
+        gw = torch.empty(max(1, rows), dtype=torch.float32, device=self.device)
+        grho = torch.empty_like(gw)
+        g_flips = torch.empty(len(deltas[0]), dtype=torch.float32, device=self.device)
+        ws_bytes = int(self.lib.egnn_adj_grad_degree_sharded_ws_bytes(rows))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
+        _cabi.check(self.lib.egnn_adj_grad_degree_sharded_flips(
+            _cabi.ptr(rp_), _cabi.ptr(ci_), self._vals(v_), _cabi.ptr(row_orders[0]), _cabi.ptr(rpt), _cabi.ptr(cit),
+            self._vals(vt), _cabi.ptr(row_orders[1]), _cabi.ptr(dinv), _cabi.ptr(iso), n_global, row_begin, row_end,
+            f, k, float(op_scale), _cabi.ptr(pl_full), _cabi.ptr(pt_full), _cabi.ptr(xbar), _cabi.ptr(rowsum),
+            *_cabi.delta_args(deltas), _cabi.ptr(g_flips), _cabi.ptr(g), _cabi.ptr(gw), _cabi.ptr(grho), _cabi.ptr(ws),
+            ws_bytes, _stream()), "egnn_adj_grad_degree_sharded_flips")
+        return g[:ci_.numel()], gw[:rows], grho[:rows], g_flips
+
+    def adj_grad_flips(self, deltas, g_flips, gw_full, grho, n_global, row_begin, row_end, op_scale):
+        """``dLoss/dv_p`` of the flips whose row this rank owns, 0 for the others, ``[n_delta]``
+        (egnn_adj_grad_flips_sharded)."""
+        out = torch.empty(len(deltas[0]), dtype=torch.float32, device=self.device)
+        _cabi.check(self.lib.egnn_adj_grad_flips_sharded(
+            *_cabi.delta_args(deltas), _cabi.ptr(g_flips), _cabi.ptr(gw_full), _cabi.ptr(grho), n_global, row_begin,
+            row_end, float(op_scale), _cabi.ptr(out), _stream()), "egnn_adj_grad_flips_sharded")
+        return out
+
     def adj_grad_entries(self, rowptr, colidx, n_global, row_begin, row_end, k, g, gw_full, grho, op_scale):
         """dLoss/dA at the shard's stored entries ``[nnz_local]`` (egnn_adj_grad_entries_sharded)."""
         out = torch.empty(max(1, int(colidx.numel())), dtype=torch.float32, device=self.device)
@@ -529,18 +559,21 @@ class _ShardedSpec:
 class _ShardedPass(torch.autograd.Function):
     """``(C [rows, S, F], T [K+1, rows, F])`` of the rank's rows of one un-normalised pass as a function
     of the local signal ``x0`` (None: the default signal), the scales ``s``, this rank's edge weights
-    ``ew`` and a 0-d ``lam`` = ``lambda_max`` (each None when it needs no gradient).  ``T`` is empty
-    unless the orders are wanted or ``s``, ``ew`` or ``lam`` needs a gradient.  Backward: the adjoint
-    pass over the transposed shard (:meth:`ShardedWavelet._adjoint`, keeping every Clenshaw vector for
-    ``ew`` / ``lam``), the scale gradient from every rank's float64 partials
-    (:meth:`ShardedWavelet._scale_grad`) and the edge-weight and ``lambda_max`` terms
-    (:meth:`ShardedWavelet._structure_grad`); all are collective."""
+    ``ew``, a 0-d ``lam`` = ``lambda_max`` and the values ``dv`` ``[n_delta]`` of the flips
+    ``spec.deltas`` (each None when it needs no gradient; the pass applies the flips' values as
+    ``spec.deltas`` holds them, detached).  ``T`` is empty unless the orders are wanted or ``s``, ``ew``,
+    ``lam`` or ``dv`` needs a gradient.  Backward: the flipped graph's degree vectors are patched once
+    and shared by the adjoint pass over the transposed shard (:meth:`ShardedWavelet._adjoint`, keeping
+    every Clenshaw vector for ``ew`` / ``lam`` / ``dv``) and the adjacency terms; the scale gradient
+    comes from every rank's float64 partials (:meth:`ShardedWavelet._scale_grad`) and the edge-weight,
+    ``lambda_max`` and flip-value terms from :meth:`ShardedWavelet._structure_grad`; all are
+    collective."""
 
     @staticmethod
-    def forward(ctx, x0, s, ew, lam, sw, spec):
+    def forward(ctx, x0, s, ew, lam, dv, sw, spec):
         ctx.set_materialize_grads(False)
         s_grad = s is not None and ctx.needs_input_grad[1]
-        structure = (ew is not None and ctx.needs_input_grad[2]) or (lam is not None and ctx.needs_input_grad[3])
+        structure = any(v is not None and ctx.needs_input_grad[i] for i, v in ((2, ew), (3, lam), (4, dv)))
         want = spec.want_orders or s_grad or structure
         comb, orders = sw._pass(spec.k, spec.s, None if x0 is None else x0.detach(), spec.lambda_max, False, want,
                                 spec.deltas, spec.graph)
@@ -554,6 +587,7 @@ class _ShardedPass(torch.autograd.Function):
         ctx.x_shape = None if x0 is None else x0.shape
         ctx.s_meta = None if s is None else (s.shape, s.device, s.dtype)
         ctx.lam_meta = None if lam is None else (lam.shape, lam.device, lam.dtype)
+        ctx.dv_shape = None if dv is None else dv.shape
         ctx.save_for_backward(t_all if (s_grad or structure) else None)
         return comb, t_all
 
@@ -566,10 +600,14 @@ class _ShardedPass(torch.autograd.Function):
         cbar = (_cabi.vec_ready(g_comb) if g_comb is not None else
                 torch.zeros((sw.rows, n_scales, f), dtype=torch.float32, device=sw.device))
         tbar = _cabi.vec_ready(g_orders) if (g_orders is not None and g_orders.numel()) else None
-        x_grad = s_grad = ew_grad = lam_grad = None
-        structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
+        x_grad = s_grad = ew_grad = lam_grad = dv_grad = None
+        structure = ctx.needs_input_grad[2] or ctx.needs_input_grad[3] or ctx.needs_input_grad[4]
+        vectors = None
+        if spec.deltas is not None and (ctx.needs_input_grad[0] or structure):
+            # the flipped graph's dinv / iso, patched once for the adjoint and the adjacency terms
+            vectors = sw._patch(sw._base if spec.graph is None else spec.graph, spec.deltas)[:2]
         if ctx.needs_input_grad[0] or structure:
-            xbar = sw._adjoint(spec, cbar, tbar, f, keep_all=structure)
+            xbar = sw._adjoint(spec, cbar, tbar, f, keep_all=structure, vectors=vectors)
             if structure:
                 xbar, b_all = xbar
             if ctx.needs_input_grad[0]:
@@ -578,12 +616,15 @@ class _ShardedPass(torch.autograd.Function):
             shape, dev, dtype = ctx.s_meta
             s_grad = sw._scale_grad(spec, cbar, t_all).to(device=dev, dtype=dtype).reshape(shape)
         if structure:
-            ew_grad, lam_grad = sw._structure_grad(spec, b_all, t_all, f, ctx.needs_input_grad[2],
-                                                   ctx.needs_input_grad[3])
+            ew_grad, lam_grad, dv_grad = sw._structure_grad(spec, b_all, t_all, f, ctx.needs_input_grad[2],
+                                                            ctx.needs_input_grad[3], ctx.needs_input_grad[4],
+                                                            vectors=vectors)
             if lam_grad is not None:
                 shape, dev, dtype = ctx.lam_meta
                 lam_grad = lam_grad.to(device=dev, dtype=dtype).reshape(shape)
-        return x_grad, s_grad, ew_grad, lam_grad, None, None
+            if dv_grad is not None:
+                dv_grad = dv_grad.reshape(ctx.dv_shape)
+        return x_grad, s_grad, ew_grad, lam_grad, dv_grad, None, None
 
 
 class ShardedWavelet:
@@ -816,17 +857,23 @@ class ShardedWavelet:
         collective, so every rank passes one or none does).
 
         Differentiable w.r.t. ``X0_local``, a 0-d / 1-d tensor ``s``,
-        ``edge_weight`` and a 0-d tensor ``lambda_max`` when grad mode is on
-        and one of them requires grad: every output then carries a
-        ``grad_fn``.  ``X0_local.grad`` receives this rank's rows of the
-        gradient, ``edge_weight.grad`` dLoss/dA at this rank's stored entries,
-        ``s.grad`` and ``lambda_max.grad`` the full gradients, identical bits
-        on every rank (DESIGN.md sections 12 and 13).  ``deltas=`` works with
-        the first two; an ``edge_weight`` or ``lambda_max`` that requires grad
-        together with ``deltas`` raises ``ValueError``.  The backward is
-        collective: every rank must call ``backward`` (once per call of
-        ``features``, in the same order on every rank), with the same inputs
-        requiring grad."""
+        ``edge_weight``, a 0-d tensor ``lambda_max`` and a 1-d tensor of flip
+        values ``deltas[2]`` when grad mode is on and one of them requires
+        grad: every output then carries a ``grad_fn``.  ``X0_local.grad``
+        receives this rank's rows of the gradient, ``edge_weight.grad``
+        dLoss/dA at this rank's stored entries, ``s.grad`` and
+        ``lambda_max.grad`` the full gradients, identical bits on every rank
+        (DESIGN.md sections 12 and 13).  With ``deltas``, the pass runs on
+        ``A' = A + delta`` and the gradients are those of ``A'``: a flip-value
+        tensor (one value per flip) receives ``dLoss/dA'`` at each flip, the
+        full ``[n_delta]`` vector with the same bits on every rank (a repeated
+        entry gives each of its flips the entry's value; a zero-valued flip
+        scores a candidate edge without changing the graph), and
+        ``lambda_max`` that of the flipped pass (section 15).  An
+        ``edge_weight`` that requires grad together with ``deltas`` raises
+        ``ValueError``.  The backward is collective: every rank must call
+        ``backward`` (once per call of ``features``, in the same order on every
+        rank), with the same inputs requiring grad."""
         k = int(k)
         if deltas is not None and len(deltas[0]) == 0:
             deltas = None
@@ -837,13 +884,15 @@ class ShardedWavelet:
             else None
         if lam_in is not None and lam_in.dim() != 0:
             raise ValueError("a lambda_max that requires grad must be a 0-d tensor")
-        if deltas is not None and (ew_in is not None or lam_in is not None):
-            raise ValueError("edge flips (deltas=) are adjacency-forward-only: edge_weight and lambda_max cannot "
-                             "require grad with them")
+        if deltas is not None and ew_in is not None:
+            raise ValueError("edge flips (deltas=) cannot come with an edge_weight that requires grad")
+        dv_in = _structure_input(None, None, deltas)[2]
+        if dv_in is not None:        # host values for the C ABI and the degree patches, read once
+            deltas = (deltas[0], deltas[1], dv_in.detach().cpu().tolist())
         lam_val = float(lambda_max.detach() if isinstance(lambda_max, torch.Tensor) else lambda_max)
         graph = self._graph(edge_weight)
         x_in = None if X0_local is None else torch.as_tensor(X0_local)
-        if _needs_grad(graph.x0 if x_in is None else x_in, s, ew_in, lam_in):
+        if _needs_grad(graph.x0 if x_in is None else x_in, s, ew_in, lam_in, dv_in):
             # un-normalised combination (and the orders) through the autograd function, then the
             # out-of-place normalisation (as graph_wavelet_features); the device / dtype conversions stay
             # outside the function, so autograd routes the gradients back to the callers' tensors
@@ -851,8 +900,9 @@ class ShardedWavelet:
             x0 = None if x_in is None else x_in.to(device=self.device, dtype=torch.float32)
             s_in = s if (isinstance(s, torch.Tensor) and s.requires_grad) else None
             ew = None if ew_in is None else ew_in.to(device=self.device, dtype=torch.float32).reshape(-1)
+            dv = None if dv_in is None else dv_in.to(device=self.device, dtype=torch.float32)
             spec = _ShardedSpec(k, s_vals, lam_val, return_parts, deltas, graph, default_signal=x_in is None)
-            comb, t_all = _ShardedPass.apply(x0, s_in, ew, lam_in, self, spec)
+            comb, t_all = _ShardedPass.apply(x0, s_in, ew, lam_in, dv, self, spec)
             feats = self.engine.l1_normalize(comb) if (normalize and self.rows) else comb
             orders = [t_all[i] for i in range(k + 1)] if return_parts else None
         else:
@@ -1086,12 +1136,13 @@ class ShardedWavelet:
             self._adjoint_order = self.engine.row_order(rowptr, self.rows)
         return self._adjoint_order
 
-    def _adjoint(self, spec, cbar, tbar, f, keep_all=False):
+    def _adjoint(self, spec, cbar, tbar, f, keep_all=False, vectors=None):
         """This rank's rows of the signal's gradient ``[rows, F]`` from its rows of ``cbar`` ``[rows, S, F]``
         and ``tbar`` ``[K+1, rows, F]`` (collective: the operand of every application is exchanged).  The
-        forward's flips are applied transposed, with the forward's patched ``dinv`` / ``iso``.
-        ``keep_all``: returns ``(xbar, b_all)`` with every Clenshaw vector ``b_all [K+1, rows_per, F]``
-        (slab 0: ``xbar``; the sharded analogue of egnn_cheb_adjoint_all)."""
+        forward's flips are applied transposed, with the forward's patched ``dinv`` / ``iso`` (``vectors``
+        when the caller patched them already, else patched here).  ``keep_all``: returns ``(xbar, b_all)``
+        with every Clenshaw vector ``b_all [K+1, rows_per, F]`` (slab 0: ``xbar``; the sharded analogue of
+        egnn_cheb_adjoint_all)."""
         eng, dev, k = self.engine, self.device, spec.k
         g = self._base if spec.graph is None else spec.graph
         coeffs = np.ascontiguousarray(heat_coefficients(k, spec.s), dtype=np.float32)
@@ -1099,7 +1150,7 @@ class ShardedWavelet:
         op_scale, op_shift = 2.0 / spec.lambda_max, -1.0
         dinv, iso, deltas_t = g.dinv, g.iso, None
         if spec.deltas is not None:
-            dinv, iso, _ = self._patch(g, spec.deltas)
+            dinv, iso = self._patch(g, spec.deltas)[:2] if vectors is None else vectors
             d_rows, d_cols, d_vals = spec.deltas
             deltas_t = (d_cols, d_rows, d_vals)
         rp = self.part.rows_per
@@ -1184,23 +1235,31 @@ class ShardedWavelet:
             total = total + parts[r]
         return _heat_scale_grad(coeffs, total)
 
-    def _structure_grad(self, spec, b_all, t_all, f, want_weights, want_lam):
-        """``(dLoss/dA at this rank's stored entries [nnz_local], dLoss/dlambda_max)`` (each None unless
-        wanted) from the Clenshaw vectors ``b_all [K+1, rows_per, F]`` and the orders ``t_all [K+1, rows, F]``
-        (DESIGN.md section 13, collective).  Edge weights: the pre-scaled stacks ``m_k d (.) b_k`` and
-        ``d (.) T_{k-1}`` of every rank are all-gathered, each rank forms ``g``, ``R`` over its shard, ``Q``
-        over its rows of the transpose and ``gw`` / ``grho`` of its rows, ``gw`` is all-gathered and the
-        values at the stored entries follow.  ``lambda_max``: every rank's float64 partials ``<b_k, T_j>``
-        are all-gathered and added in rank order, so every rank holds the same bits."""
+    def _structure_grad(self, spec, b_all, t_all, f, want_weights, want_lam, want_flips=False, vectors=None):
+        """``(dLoss/dA at this rank's stored entries [nnz_local], dLoss/dlambda_max, dLoss/dv [n_delta])``
+        (each None unless wanted) from the Clenshaw vectors ``b_all [K+1, rows_per, F]`` and the orders
+        ``t_all [K+1, rows, F]`` (DESIGN.md sections 13 and 15, collective).  Edge weights and flip values:
+        the pre-scaled stacks ``m_k d (.) b_k`` and ``d (.) T_{k-1}`` of every rank are all-gathered, each
+        rank forms ``g``, ``R`` over its shard, ``Q`` over its rows of the transpose (plus the flips' part of
+        both) and ``gw`` / ``grho`` of its rows, ``gw`` is all-gathered and the values at the stored entries
+        follow; each flip's value comes from the rank that owns its row, and the ranks' ``[n_delta]`` rows
+        are all-gathered and added in rank order.  ``lambda_max``: every rank's float64 partials
+        ``<b_k, T_j>`` are all-gathered and added in rank order, so every rank holds the same bits.  With
+        flips, ``vectors`` holds the flipped graph's ``(dinv, iso)`` (patched here when None), and the
+        default signal's row sums are those of ``A + delta``."""
         eng, dev, k = self.engine, self.device, spec.k
         g = self._base if spec.graph is None else spec.graph
         rp, rb, re_ = self.part.rows_per, self.row_begin, self.row_end
         a = 2.0 / spec.lambda_max
-        ew_grad = lam_grad = None
-        if want_weights:
+        ew_grad = lam_grad = dv_grad = None
+        deltas = spec.deltas
+        dinv, iso = g.dinv, g.iso
+        if deltas is not None and (want_weights or want_flips):
+            dinv, iso = self._patch(g, deltas)[:2] if vectors is None else vectors
+        if want_weights or want_flips:
             plf = ptf = None
             if k >= 1:
-                pl, pt = eng.adj_grad_stacks(b_all, t_all, g.dinv, self.n, rb, re_, rp, f, k)
+                pl, pt = eng.adj_grad_stacks(b_all, t_all, dinv, self.n, rb, re_, rp, f, k)
                 self.launches += 1 if self.rows else 0
                 plf = torch.empty((self.world * rp, k * f), dtype=pl.dtype, device=dev)
                 ptf = torch.empty_like(plf)
@@ -1214,16 +1273,35 @@ class ShardedWavelet:
             default = spec.default_signal and f == 1
             xbar = b_all[0, :self.rows, 0].contiguous() if default else None
             rowsum = g.rowsum_local if default else None
-            ge, gw, grho = eng.adj_grad_degree((self.rowptr, self.colidx, g.vals), (rowptr_t, colidx_t, vals_t),
-                                               orders, g.dinv, g.iso, self.n, rb, re_, f, k, a, plf, ptf, xbar,
-                                               rowsum)
+            shards = ((self.rowptr, self.colidx, g.vals), (rowptr_t, colidx_t, vals_t), orders)
+            if deltas is None:
+                ge, gw, grho = eng.adj_grad_degree(*shards, dinv, iso, self.n, rb, re_, f, k, a, plf, ptf, xbar,
+                                                   rowsum)
+            else:
+                if default:
+                    rowsum = self._flipped_rowsum(rowsum, deltas)
+                ge, gw, grho, g_flips = eng.adj_grad_degree_flips(*shards, dinv, iso, self.n, rb, re_, f, k, a, plf,
+                                                                  ptf, xbar, rowsum, deltas)
+                self.launches += 1 if (self.rows and k >= 1) else 0
             pad = torch.zeros(rp, dtype=gw.dtype, device=dev)
             pad[:self.rows] = gw
             gw_full = torch.empty(self.world * rp, dtype=gw.dtype, device=dev)
             self._allgather(gw_full, pad)
-            ew_grad = eng.adj_grad_entries(self.rowptr, self.colidx, self.n, rb, re_, k, ge if k >= 1 else None,
-                                           gw_full, grho, a)
-            self.launches += (3 if k >= 1 else 1) + 1 if self.rows else 0
+            if want_weights:
+                ew_grad = eng.adj_grad_entries(self.rowptr, self.colidx, self.n, rb, re_, k, ge if k >= 1 else None,
+                                               gw_full, grho, a)
+                self.launches += 1 if self.rows else 0
+            self.launches += (3 if k >= 1 else 1) if self.rows else 0
+            if want_flips:
+                mine = eng.adj_grad_flips(deltas, g_flips, gw_full, grho, self.n, rb, re_, a)
+                self.launches += 1
+                n_delta = len(deltas[0])
+                full = torch.empty(self.world * n_delta, dtype=mine.dtype, device=dev)
+                self._allgather(full, mine.contiguous())
+                full = full.reshape(self.world, n_delta)
+                dv_grad = full[0]
+                for r in range(1, self.world):
+                    dv_grad = dv_grad + full[r]
         if want_lam:
             if k == 0:                # lambda_max does not enter the pass
                 lam_grad = torch.zeros((), dtype=torch.float64, device=dev)
@@ -1248,7 +1326,22 @@ class ShardedWavelet:
                     total = total + G[i - 1, i] + (1.0 if i == 1 else 2.0) * G[i - 1, i - 1] + \
                         (G[i - 1, i - 2] if i >= 2 else 0.0)
                 lam_grad = -total / float(spec.lambda_max)
-        return ew_grad, lam_grad
+        return ew_grad, lam_grad, dv_grad
+
+    def _flipped_rowsum(self, rowsum_local, deltas):
+        """Row sums of the own rows with ``deltas`` applied, rounded as egnn_patch_degrees forms them for
+        the signal ``log1p(rowsum)``: each touched row's base sum plus the float32 sum of its flips in list
+        order (the sharded analogue of ``wats._flipped_rowsum``)."""
+        add = {}
+        for r, v in zip(deltas[0], deltas[2]):
+            r = int(r)
+            if self.row_begin <= r < self.row_end:
+                add[r - self.row_begin] = np.float32(add.get(r - self.row_begin, np.float32(0.0)) + np.float32(v))
+        rowsum = torch.as_tensor(rowsum_local).clone()
+        if add:
+            idx = torch.tensor(list(add), dtype=torch.long, device=rowsum.device)
+            rowsum[idx] = rowsum[idx] + torch.tensor(list(add.values()), dtype=torch.float32).to(rowsum.device)
+        return rowsum
 
     def _forward_row_order(self):
         """egnn_row_order of the rank's own shard (longest rows first), built once."""

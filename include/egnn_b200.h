@@ -710,6 +710,39 @@ int egnn_adj_grad_entries_sharded(const int32_t* rowptr, const int32_t* colidx, 
                                   const float* gw_full, const float* grho_local, float op_scale,
                                   float* out, egnn_stream_t stream);
 
+/* ---- gradients through the edge flips of a row shard (new in ABI 13) --------
+ * The pass ran on A' = A + sum_p v_p e_{r_p} e_{c_p}^T (every rank passes the
+ * same global flip list: host arrays, n_delta <= EGNN_MAX_DELTA, indices below
+ * n_global, checked before anything launches); DESIGN.md section 15.
+ * egnn_adj_grad_degree_sharded_flips: egnn_adj_grad_degree_sharded (which is
+ *   this call without flips) with dinv_full / iso_full / pl_full / pt_full of
+ *   A', plus g_flips_out[p] = g_{r_p c_p} = <pl[r_p], pt[c_p]> of every flip
+ *   (device, [n_delta]; the same bits on every rank) and the flips' part of
+ *   the degree terms: R[r_p] += v_p g_p on the rank owning row r_p, Q[c_p] +=
+ *   v_p g_p on the rank owning row c_p, for every off-diagonal flip, folded in
+ *   flip-list order.  rowsum_local: the row sums of A' (default signal only).
+ * egnn_adj_grad_flips_sharded: out[p] = dLoss/dv_p = grho_local[r_p - row_begin]
+ *   + [r_p != c_p] (-a g_flips[p] + gw_full[c_p]) for the flips whose row this
+ *   rank owns, 0 for the others (device, [n_delta]); the caller adds the
+ *   ranks' rows in rank order, which hands every rank the owner's bits.       */
+int egnn_adj_grad_degree_sharded_flips(const int32_t* rowptr, const int32_t* colidx,
+                                       const float* vals_or_null, const int32_t* row_order_or_null,
+                                       const int32_t* rowptr_t, const int32_t* colidx_t,
+                                       const float* vals_t_or_null, const int32_t* row_order_t_or_null,
+                                       const float* dinv_full, const uint8_t* iso_full, int64_t n_global,
+                                       int64_t row_begin, int64_t row_end, int32_t f, int32_t k,
+                                       float op_scale, const float* pl_full, const float* pt_full,
+                                       const float* xbar_local_or_null, const float* rowsum_local_or_null,
+                                       const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                       const float* delta_val_host, int32_t n_delta, float* g_flips_out,
+                                       float* g_out, float* gw_local, float* grho_local,
+                                       void* workspace, size_t workspace_bytes, egnn_stream_t stream);
+int egnn_adj_grad_flips_sharded(const int32_t* delta_row_host, const int32_t* delta_col_host,
+                                const float* delta_val_host, int32_t n_delta, const float* g_flips,
+                                const float* gw_full, const float* grho_local, int64_t n_global,
+                                int64_t row_begin, int64_t row_end, float op_scale, float* out,
+                                egnn_stream_t stream);
+
 /* Degree pass of a row shard (scipy semantics as egnn_graph_prep).  phase 0:
  * row sums of the local rows, their diagonal entries into diag_full[row_begin..]
  * and the shard's contribution to the in-degree in colsum_full (both zeroed

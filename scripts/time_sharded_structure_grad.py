@@ -136,9 +136,9 @@ def main():
         saved = {}
         orig = sw._structure_grad
 
-        def grab(spec, b_all, t_all, f_, want_w, want_lam):
+        def grab(spec, b_all, t_all, f_, *wants, **kw):
             saved.update(spec=spec, b_all=b_all, t_all=t_all)
-            return orig(spec, b_all, t_all, f_, want_w, want_lam)
+            return orig(spec, b_all, t_all, f_, *wants, **kw)
 
         sw._structure_grad = grab
         fwd_bwd_w()
